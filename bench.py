@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py -- GVox/s of the map -> cubes -> stitched-volume hot path (BASELINE.json).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A step = one pass of the whole hot path over one synthetic map: B-spline resample to
 the 1 A grid, exact median/p99.9 normalisation, 24-channel AF3 rasterisation, 64^3 cube
@@ -23,6 +23,10 @@ Further blocks of the same JSON line (each a different BASELINE config, never th
   e2e / e2e_aa_prob_resident / e2e_dropin
                            host buffers in, host volumes out; the last one through the reference-named
                            classes (DataPreprocessor -> GridCreator -> CryoEMPredictor), MRC + PDB on tmpfs
+
+`--dump-outputs DIR` writes the four stitched volumes of the headline's last timed step (dump_outputs: a
+fixed, seeded sample of voxels, float32) so that two builds can be compared output for output.  With
+N > 1 it holds rank 0's slab only; the other ranks' slabs are not written.
 
 Prints ONE JSON line (rank 0).  `--impl reference` times the UNMODIFIED reference (staged by
 oracle/make_ref.py) as it is -- its .mrc / .npz files on tmpfs, its worker pools -- on a bounded
@@ -76,7 +80,16 @@ def parse_args():
                     help='also time K steps with this many maps in flight (one pipeline + stream each); 0 = skip')
     ap.add_argument('--cpu-kind', default='as_is', choices=['as_is', 'port'],
                     help='reference arm: the unmodified reference with its file I/O (default) or the in-memory port')
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write the four volumes of the last timed step as DIR/<name>.npy (rank 0; a fixed sample '
+                         'of voxels when the volumes exceed DUMP_VOXELS), to compare two builds output for output')
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error('--steps must be >= 1 and --warmup >= 0')
+    if args.dump_outputs and args.impl == 'reference':
+        # the reference arm times a smaller CPU sample of the workload, so its volumes are not comparable
+        ap.error('--dump-outputs writes the GPU path (--impl ours) only')
+    return args
 
 
 def peaks():
@@ -374,6 +387,27 @@ def make_measure(ctx):
 
 def stage_table(stages, steps):
     return {k: round(v[1] / steps, 4) for k, v in stages.items()}
+
+
+DUMP_VOXELS = 1 << 19      # 23 float32 channels + a float64 index a voxel: 50 MiB, under 64 MB
+
+
+def dump_outputs(out_dir, vols):
+    """The four volumes ``pipe.run`` returned as out_dir/<name>.npy, float32, channels first.  Volumes larger
+    than DUMP_VOXELS are sampled at the same voxels on every run (a seeded choice, independent of the build);
+    sample_voxel_index.npy holds their flat C-order indices into the volume, as float64."""
+    import torch
+    n = vols.backbone_probability.numel()
+    if n > DUMP_VOXELS:
+        idx = np.sort(np.random.default_rng(2022).choice(n, DUMP_VOXELS, replace=False))
+    else:
+        idx = np.arange(n)
+    os.makedirs(out_dir, exist_ok=True)
+    idx_dev = torch.from_numpy(idx).to(vols.device)
+    for k, v in vols.as_dict().items():
+        flat = v.reshape(-1, n) if v.dim() == 4 else v.reshape(n)
+        np.save(os.path.join(out_dir, f'{k}.npy'), flat[..., idx_dev].cpu().numpy())
+    np.save(os.path.join(out_dir, 'sample_voxel_index.npy'), idx.astype(np.float64))
 
 
 # ------------------------------------------------------------------ configs[3]: strong scaling of ONE 720^3 map
@@ -803,6 +837,8 @@ def run_ours(args):
     dom_stage = max((k for k in single_kernel_stages if k in stages_all), key=lambda k: stages_all[k][1])
     del vols
     ms_per_step, stages, launches, clk, vols, host_ms = measure(pipe, inputs, model_fn, True, only={dom_stage})
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, vols)
     n_vox_rank = int(np.prod(pipe.normalized.shape)) if world == 1 else pipe.owned_voxels
     n_vox = n_vox_rank * world
     value = n_vox / (ms_per_step * 1e-3) / 1e9

@@ -32,6 +32,12 @@ def _save(name, **kw):
     print(f'  wrote {name}: {os.path.getsize(path) / 1024:.0f} KiB')
 
 
+def byte_planes(a):
+    """float32 array -> (4,) + shape uint8, byte k of every value in plane k (deflates far better)."""
+    a = np.ascontiguousarray(a, dtype=np.float32)
+    return np.ascontiguousarray(np.moveaxis(a.view(np.uint8).reshape(a.shape + (4,)), -1, 0))
+
+
 def golden_preprocess():
     """R1-R4: map (26,30,22) at anisotropic voxel -> normalised map + AF3 voxels."""
     rng = np.random.default_rng(2022)
@@ -202,8 +208,11 @@ def golden_stitch():
     o = orc.postprocess_and_stitch(bb, ca, aa, meta, orig_shape)
     for name in vols:
         assert np.array_equal(o[name], vols[name]), name
+    # float volumes as byte planes and the argmax as uint8 (lossless; tests/_golden.py reads them back):
+    # plain float32 deflates to just over 1 MB
+    packed = {k + '_planes': byte_planes(v) for k, v in vols.items() if k != 'amino_acid_prediction'}
     _save('stitch.npz', meta=meta, orig_shape=np.array(orig_shape), logits_seed=np.int64(99),
-          **{k: v for k, v in vols.items()})
+          amino_acid_prediction=vols['amino_acid_prediction'].astype(np.uint8), **packed)
 
 
 CANDIDATE_CASES = [dict(shape=(56, 44, 40), n_residues=(60, 25), seed=1, wall_margin=3.0),

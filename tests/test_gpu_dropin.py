@@ -199,10 +199,10 @@ def test_zero_af3_cubes_are_batched_apart(cuda, tmp_path):
 
 def test_reference_batching_reproduces_the_mixed_batches(cuda, tmp_path):
     """D8, ``reference_batching=True``: cubes in the reference's glob order, mixed batches, MICA's branch taken
-    on the whole batch -- compared with the UNMODIFIED reference predictor run on the same files and model."""
+    on the whole batch -- compared with the oracle's statement of that batch (one model call on all three cubes,
+    then the reference's stitch, pinned by stitch.npz) and, where a copy of it is present, with the UNMODIFIED
+    reference predictor run on the same files and model."""
     from oracle import ref_harness
-    if not ref_harness.available():
-        pytest.skip('no reference staged')
     session.clear()
     grids = _d8_case(tmp_path, materialize=True)
     model = BranchingModel()
@@ -211,6 +211,17 @@ def test_reference_batching_reproduces_the_mixed_batches(cuda, tmp_path):
     pr.batch_threshold = 1
     ok, got = pr.run_prediction()
     assert ok and model.seen == [(3, False)]                    # one mixed batch: nobody takes the zero branch
+    norm = mrc.read_mrc(str(tmp_path / 'resampled_normalized_map.mrc')).data
+    af3 = [mrc.read_mrc(str(tmp_path / 'AF3_encodings' / f'{name}_encoding.mrc')).data for name in pdb.CHANNEL_NAMES]
+    o_cubes, o_meta, o_shape, _ = orc.extract_cubes(norm)
+    o_af = torch.from_numpy(np.stack([orc.extract_cubes(a)[0] for a in af3], axis=1))
+    o_model = BranchingModel()
+    with torch.no_grad():
+        logits = o_model(torch.from_numpy(o_cubes[:, None]), o_af)
+    assert o_model.seen == [(3, False)]
+    _check_mixed_batches(got, orc.postprocess_and_stitch(*logits, o_meta, o_shape))
+    if not ref_harness.available():
+        return
     ref_harness._setup_path()
     from utils.predict import CryoEMPredictor as RefPredictor
     with ref_harness._quiet():
@@ -224,6 +235,10 @@ def test_reference_batching_reproduces_the_mixed_batches(cuda, tmp_path):
         assert good and rp.run_inference(loader)
         good, want = rp.reconstruct_and_save_volumes()
     assert good and rp.model.seen == [(3, False)]
+    _check_mixed_batches(got, want)
+
+
+def _check_mixed_batches(got, want):
     for k in ('backbone_probability', 'carbon_alpha_probability', 'amino_acid_probability'):
         assert np.abs(got[k] - want[k]).max() <= 1e-5, k
     top2 = np.sort(want['amino_acid_probability'], axis=0)[-2:]

@@ -14,6 +14,8 @@ from mica_b200 import _lib, ops, synthetic
 from mica_b200.pipeline import MapHeader, MapPipeline
 from oracle import mica_oracle as orc
 
+from _golden import load_stitch
+
 pytestmark = pytest.mark.gpu
 
 TOL = 1e-5
@@ -580,7 +582,7 @@ def test_pipeline_overlap_window_option(cuda):
 
 
 def test_postproc_stitch_golden(cuda, golden_dir):
-    g = np.load(os.path.join(golden_dir, 'stitch.npz'))
+    g = load_stitch(golden_dir)
     cube_shape = tuple(int(v) for v in g['orig_shape'])
     want, got, _ = _stitch_case(cube_shape, 48, 8, cuda, seed=int(g['logits_seed']))
     ref = {k: g[k] for k in want}

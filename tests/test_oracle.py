@@ -10,6 +10,8 @@ from oracle import mica_oracle as orc
 from oracle import ref_harness as rh
 from mica_b200 import synthetic
 
+from _golden import load_stitch
+
 
 def test_normalize_and_encode_match_reference_golden(golden_dir):
     g = np.load(os.path.join(golden_dir, 'preprocess_small.npz'))
@@ -40,7 +42,7 @@ def test_cubes_match_reference_golden(golden_dir):
 
 
 def test_stitch_matches_reference_golden(golden_dir):
-    g = np.load(os.path.join(golden_dir, 'stitch.npz'))
+    g = load_stitch(golden_dir)
     bb, ca, aa = synthetic.synthetic_logits(len(g['meta']), 64, seed=int(g['logits_seed']))
     got = orc.postprocess_and_stitch(bb, ca, aa, g['meta'], tuple(g['orig_shape']))
     for k, v in got.items():
