@@ -44,6 +44,7 @@ SIGNATURES = {
     'mica_resample_force_generic': (_i, [_i]),
     'mica_resample_slab_source_planes': (_i, [_i, _i, _i, _i, _p, _p]),
     'mica_bspline_resample_f32': (_i, [_p, _i, _i, _i, _i, _i, _p, _i, _i, _i, _i, _i, _p, _sz, _i, _p]),
+    'mica_last_resample_path': (_i, [_i]),
     'mica_select_workspace_bytes': (_sz, []),
     'mica_select_workspace_bytes_for': (_sz, [_i64]),
     'mica_select_set_compact': (_i, [_p, _sz, _p]),

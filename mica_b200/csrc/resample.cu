@@ -1312,10 +1312,15 @@ static int prefilter_lines() {   // lines per shared-memory tile of the segment-
 
 static int g_force_generic = 0;   // tests: run the general kernels on shapes the fast ones would take
 
+// mica_last_resample_path: the MICA_RS_* kernel each pass of this thread's last resample launched (-1 = none)
+enum { kPassZ = 0, kPassY = 1, kPassX = 2, kPassInterp = 3 };
+static thread_local int g_resample_path[4] = {-1, -1, -1, -1};
+
 constexpr size_t kMaxTileBytes = 200 * 1024;
 
 template <typename TIn, typename TOut>
-static int launch_cols(const TIn* in, TOut* out, int n, int n_cols, int n_outer, ColStrides S, cudaStream_t st) {
+static int launch_cols(const TIn* in, TOut* out, int n, int n_cols, int n_outer, ColStrides S, cudaStream_t st,
+                       int pass) {
   if (n_cols <= 0 || n_outer <= 0 || n <= 0) return MICA_OK;
   size_t per_col = (size_t)n * sizeof(double);
   if (!g_force_generic && n >= kMinSegLine && per_col * 32 <= kMaxTileBytes) {
@@ -1323,19 +1328,23 @@ static int launch_cols(const TIn* in, TOut* out, int n, int n_cols, int n_outer,
       size_t smem = per_col * 16;
       MICA_CUDA(cudaFuncSetAttribute(prefilter_cols_seg<TIn, TOut, 16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
       prefilter_cols_seg<TIn, TOut, 16><<<dim3((n_cols + 15) / 16, n_outer), 256, smem, st>>>(in, out, n, n_cols, S);
+      g_resample_path[pass] = MICA_RS_COLS_SEG16;
     } else {
       size_t smem = per_col * 32;
       MICA_CUDA(cudaFuncSetAttribute(prefilter_cols_seg<TIn, TOut, 32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
       prefilter_cols_seg<TIn, TOut, 32><<<dim3((n_cols + 31) / 32, n_outer), 256, smem, st>>>(in, out, n, n_cols, S);
+      g_resample_path[pass] = MICA_RS_COLS_SEG32;
     }
   } else if (per_col * 32 <= kMaxTileBytes) {
     size_t smem = per_col * 32;
     MICA_CUDA(cudaFuncSetAttribute(prefilter_cols<TIn, TOut, 32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     prefilter_cols<TIn, TOut, 32><<<dim3((n_cols + 31) / 32, n_outer), 256, smem, st>>>(in, out, n, n_cols, S);
+    g_resample_path[pass] = MICA_RS_COLS32;
   } else if (per_col * 8 <= kMaxTileBytes) {
     size_t smem = per_col * 8;
     MICA_CUDA(cudaFuncSetAttribute(prefilter_cols<TIn, TOut, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     prefilter_cols<TIn, TOut, 8><<<dim3((n_cols + 7) / 8, n_outer), 256, smem, st>>>(in, out, n, n_cols, S);
+    g_resample_path[pass] = MICA_RS_COLS8;
   } else {
     return set_error(MICA_ERR_INVALID, "line of %d samples too long for the shared-memory prefilter", n);
   }
@@ -1346,16 +1355,20 @@ static int launch_cols(const TIn* in, TOut* out, int n, int n_cols, int n_outer,
 // the old all-float64 path keeps its global-memory sweep for lines that fit no tile
 template <typename TIn>
 static int launch_cols_f64(const TIn* in, double* out, int n, int64_t line_stride, int n_cols,
-                           int64_t outer_stride, int n_outer, cudaStream_t st) {
+                           int64_t outer_stride, int n_outer, cudaStream_t st, int pass) {
   if (n_cols <= 0 || n_outer <= 0 || n <= 0) return MICA_OK;
   if ((size_t)n * sizeof(double) * 8 <= kMaxTileBytes) {
     ColStrides S{line_stride, line_stride, outer_stride, outer_stride};
-    return launch_cols<TIn, double>(in, out, n, n_cols, n_outer, S, st);
+    return launch_cols<TIn, double>(in, out, n, n_cols, n_outer, S, st, pass);
   }
   prefilter_cols_global<TIn><<<dim3((n_cols + 127) / 128, n_outer), 128, 0, st>>>(in, out, n, line_stride, n_cols, outer_stride);
+  g_resample_path[pass] = MICA_RS_COLS_GLOBAL;
   MICA_LAUNCH_CHECK("prefilter_cols_global");
   return MICA_OK;
 }
+
+// a row that fits no 4-row shared-memory tile is swept in global memory, one row per CTA along grid y
+static bool row_fits_smem(int n) { return (size_t)(n | 1) * sizeof(double) * 4 <= kMaxTileBytes; }
 
 static int launch_rows(double* data, int n, int64_t n_rows, cudaStream_t st) {
   if (n <= 0 || n_rows <= 0) return MICA_OK;
@@ -1365,22 +1378,27 @@ static int launch_rows(double* data, int n, int64_t n_rows, cudaStream_t st) {
       size_t smem = per_row * 16;
       MICA_CUDA(cudaFuncSetAttribute(prefilter_rows_seg<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
       prefilter_rows_seg<16><<<(unsigned)ceil_div64(n_rows, 16), 256, smem, st>>>(data, n, n_rows);
+      g_resample_path[kPassX] = MICA_RS_ROWS_SEG16;
     } else {
       size_t smem = per_row * 32;
       MICA_CUDA(cudaFuncSetAttribute(prefilter_rows_seg<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
       prefilter_rows_seg<32><<<(unsigned)ceil_div64(n_rows, 32), 256, smem, st>>>(data, n, n_rows);
+      g_resample_path[kPassX] = MICA_RS_ROWS_SEG32;
     }
   } else if (per_row * 32 <= kMaxTileBytes) {
     size_t smem = per_row * 32;
     MICA_CUDA(cudaFuncSetAttribute(prefilter_rows<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     prefilter_rows<32><<<(unsigned)ceil_div64(n_rows, 32), 256, smem, st>>>(data, n, n_rows);
-  } else if (per_row * 4 <= kMaxTileBytes) {
+    g_resample_path[kPassX] = MICA_RS_ROWS32;
+  } else if (row_fits_smem(n)) {
     size_t smem = per_row * 4;
     MICA_CUDA(cudaFuncSetAttribute(prefilter_rows<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     prefilter_rows<4><<<(unsigned)ceil_div64(n_rows, 4), 256, smem, st>>>(data, n, n_rows);
+    g_resample_path[kPassX] = MICA_RS_ROWS4;
   } else {
     // a row is a column of a [n_rows x n] matrix with unit line stride
     prefilter_cols_global<double><<<dim3(1, (unsigned)n_rows), 1, 0, st>>>(data, data, n, 1, 1, n);
+    g_resample_path[kPassX] = MICA_RS_COLS_GLOBAL;
   }
   MICA_LAUNCH_CHECK("prefilter_rows");
   return MICA_OK;
@@ -1444,20 +1462,24 @@ extern "C" int mica_resample_slab_source_planes(int sz, int nz, int dst_z0, int 
   return MICA_OK;
 }
 
-static bool reg_cols_ok(int src_nz_local, int sy) {
-  return !getenv("MICA_RESAMPLE_NOREG") && src_nz_local <= 64 * kColLen && sy <= 64 * kColLen;
-}
-// sz = planes of the whole map, src_nz_local = planes of the block in memory.  The choice follows the WHOLE line
-// wherever it can, so that a thin block of a long line (the last rank of a z-slab partition) runs the same
-// arithmetic as the whole map: the register column pass takes a block of any length.
+// The register column pass (cols_reg_kernel) takes lines of any length: a CTA runs 8 segments of <= kColLen samples
+// and the grid has ceil(segments / 8) CTAs along y.
+static bool reg_cols_ok() { return !getenv("MICA_RESAMPLE_NOREG"); }
+// sz = planes of the whole map, src_nz_local = planes of the block in memory.  The choice follows the WHOLE line,
+// so that every block of a z-slab partition runs the same kernels as the whole map (the z pass numbers its segments
+// on the whole line: the same bits): no bound but the register pass's 8-plane minimum looks at the block.  Only the
+// MICA_RESAMPLE_NOREG pipe kernels hold a line in shared memory, and they cut the block into its own segments.
 static bool fast_path_ok(int sz, int src_nz_local, int sy, int sx, int ny, int nx) {
   if (g_force_generic || getenv("MICA_NO_TMA") || getenv("MICA_RESAMPLE_OLD")) return false;
-  if (src_nz_local > 1760 || sy > 1760 || sx > 1760) return false;   // 64 segments x kRegSeg samples, tile in smem
+  if (sy > 1760 || sx > 1760) return false;              // lines the shared-memory tiles of the pipe kernels hold
   if (sz < kMinSegLine || sy < kMinSegLine || sx < kMinSegLine) return false;             // segment-parallel sweeps
-  if (src_nz_local < (reg_cols_ok(src_nz_local, sy) ? 8 : kMinSegLine)) return false;
-  if (cols_pipe_smem(src_nz_local, 8) > kPipeSmemMax || cols_pipe_smem(sy, 8) > kPipeSmemMax ||
-      rows_pipe_smem(sx, 8) > kPipeSmemMax)
+  if (reg_cols_ok()) {
+    if (src_nz_local < 8) return false;
+  } else if (src_nz_local < kMinSegLine || cols_pipe_smem(src_nz_local, 8) > kPipeSmemMax ||
+             cols_pipe_smem(sy, 8) > kPipeSmemMax) {
     return false;
+  }
+  if (rows_pipe_smem(sx, 8) > kPipeSmemMax) return false;
   const double zoom_y = ny > 1 ? (double)(sy - 1) / (double)(ny - 1) : 1.0;
   if ((int)floor(7.0 * zoom_y) + 5 > 16) return false;                                    // y span of an 8-row tile
   return tensor_map_encode_fn() != nullptr;
@@ -1465,7 +1487,8 @@ static bool fast_path_ok(int sz, int src_nz_local, int sy, int sx, int ny, int n
 
 // persistent grid: as many CTAs as fit (shared memory bound), tiles dealt round-robin
 template <int L, int THREADS>
-static int launch_cols_pipe_t(const float* in, float* out, int n, int n_cols, int n_outer, ColStrides S, cudaStream_t st) {
+static int launch_cols_pipe_t(const float* in, float* out, int n, int n_cols, int n_outer, ColStrides S, cudaStream_t st,
+                              int pass) {
   const size_t smem = cols_pipe_smem(n, L);
   MICA_CUDA(cudaFuncSetAttribute(cols_pipe_kernel<L, THREADS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   int per_sm = (int)((size_t)225 * 1024 / (smem + 1024));
@@ -1474,14 +1497,17 @@ static int launch_cols_pipe_t(const float* in, float* out, int n, int n_cols, in
   long long grid = (long long)kNumSMs * per_sm;
   if (grid > tiles) grid = tiles;
   cols_pipe_kernel<L, THREADS><<<(unsigned)grid, THREADS, smem, st>>>(in, out, n, n_cols, n_outer, S);
+  g_resample_path[pass] =
+      L == 8 ? MICA_RS_COLS_PIPE_8_512 : THREADS == 256 ? MICA_RS_COLS_PIPE_16_256 : MICA_RS_COLS_PIPE_16_512;
   MICA_LAUNCH_CHECK("cols_pipe_kernel");
   return MICA_OK;
 }
-static int launch_cols_pipe(const float* in, float* out, int n, int n_cols, int n_outer, ColStrides S, cudaStream_t st) {
+static int launch_cols_pipe(const float* in, float* out, int n, int n_cols, int n_outer, ColStrides S, cudaStream_t st,
+                            int pass) {
   if (n_cols <= 0 || n_outer <= 0) return MICA_OK;
-  if (cols_pipe_smem(n, 16) <= 110 * 1024) return launch_cols_pipe_t<16, 256>(in, out, n, n_cols, n_outer, S, st);
-  if (cols_pipe_smem(n, 16) <= kPipeSmemMax) return launch_cols_pipe_t<16, 512>(in, out, n, n_cols, n_outer, S, st);
-  return launch_cols_pipe_t<8, 512>(in, out, n, n_cols, n_outer, S, st);
+  if (cols_pipe_smem(n, 16) <= 110 * 1024) return launch_cols_pipe_t<16, 256>(in, out, n, n_cols, n_outer, S, st, pass);
+  if (cols_pipe_smem(n, 16) <= kPipeSmemMax) return launch_cols_pipe_t<16, 512>(in, out, n, n_cols, n_outer, S, st, pass);
+  return launch_cols_pipe_t<8, 512>(in, out, n, n_cols, n_outer, S, st, pass);
 }
 // register-only column pass: 32 columns x 8 segments per CTA, segments of <= kColLen samples.  The line in memory
 // is samples [g0, g0 + n) of a line of ng; the segments of the GLOBAL line that hold samples [need_lo, need_hi]
@@ -1491,7 +1517,7 @@ static void cols_reg_geometry(int ng, int* n_seg, int* len) {
   *len = (ng + *n_seg - 1) / *n_seg;
 }
 static int launch_cols_reg(const float* in, float* out, int n, int n_cols, int n_outer, ColStrides S, cudaStream_t st,
-                           int g0, int ng, int need_lo, int need_hi) {
+                           int pass, int g0, int ng, int need_lo, int need_hi) {
   if (n_cols <= 0 || n_outer <= 0 || need_hi < need_lo) return MICA_OK;
   MICA_REQUIRE(n_outer <= 65535, "too many outer lines for the launch grid");
   int n_seg_g, len;
@@ -1499,11 +1525,13 @@ static int launch_cols_reg(const float* in, float* out, int n, int n_cols, int n
   const int seg0 = need_lo / len, n_seg = need_hi / len - seg0 + 1;
   cols_reg_kernel<<<dim3((n_cols + 31) / 32, (n_seg + 7) / 8, n_outer), 256, 0, st>>>(in, out, n, n_cols, S, len, n_seg,
                                                                                    g0, ng, seg0);
+  g_resample_path[pass] = MICA_RS_COLS_REG;
   MICA_LAUNCH_CHECK("cols_reg_kernel");
   return MICA_OK;
 }
-static int launch_cols_reg(const float* in, float* out, int n, int n_cols, int n_outer, ColStrides S, cudaStream_t st) {
-  return launch_cols_reg(in, out, n, n_cols, n_outer, S, st, 0, n, 0, n - 1);
+static int launch_cols_reg(const float* in, float* out, int n, int n_cols, int n_outer, ColStrides S, cudaStream_t st,
+                           int pass) {
+  return launch_cols_reg(in, out, n, n_cols, n_outer, S, st, pass, 0, n, 0, n - 1);
 }
 
 template <int L, int THREADS>
@@ -1517,6 +1545,8 @@ static int launch_rows_pipe_t(const float* in, int64_t in_pitch, double* out, in
   long long grid = (long long)kNumSMs * per_sm;
   if (grid > tiles) grid = tiles;
   rows_pipe_interp_kernel<L, THREADS><<<(unsigned)grid, THREADS, smem, st>>>(in, in_pitch, out, out_pitch, n, nx, n_rows, tx);
+  g_resample_path[kPassX] =
+      L == 8 ? MICA_RS_ROWS_PIPE_8_512 : THREADS == 256 ? MICA_RS_ROWS_PIPE_16_256 : MICA_RS_ROWS_PIPE_16_512;
   MICA_LAUNCH_CHECK("rows_pipe_interp_kernel");
   return MICA_OK;
 }
@@ -1533,6 +1563,7 @@ static int launch_rows_reg_t(const float* in, int64_t in_pitch, double* out, int
   int len = (n + SEGS - 1) / SEGS;
   if (len % 2 == 0 && len < kColLen) ++len;      // odd segment length: the lanes of a row hit distinct banks
   rows_reg_interp_kernel<SEGS><<<(unsigned)grid, 16 * SEGS, smem, st>>>(in, in_pitch, out, out_pitch, n, nx, n_rows, tx, len);
+  g_resample_path[kPassX] = SEGS == 16 ? MICA_RS_ROWS_REG16 : MICA_RS_ROWS_REG32;
   MICA_LAUNCH_CHECK("rows_reg_interp_kernel");
   return MICA_OK;
 }
@@ -1565,12 +1596,16 @@ extern "C" int mica_bspline_resample_f32(const float* src, int sz, int sy, int s
                                          float* dst, int nz, int ny, int nx, int dst_z0, int dst_nz_local,
                                          void* workspace, size_t workspace_bytes, int order, mica_stream_t stream) {
   cudaStream_t st = (cudaStream_t)stream;
+  for (int& k : g_resample_path) k = -1;
   MICA_REQUIRE(src && dst && workspace, "null pointer");
   MICA_REQUIRE(order == 3 || order == 1, "order must be 3 or 1 (got %d)", order);
   MICA_REQUIRE(sz > 0 && sy > 0 && sx > 0 && nz > 0 && ny > 0 && nx > 0, "empty shape");
   MICA_REQUIRE(src_z0 >= 0 && src_nz_local > 0 && src_z0 + src_nz_local <= sz, "bad source slab");
   MICA_REQUIRE(dst_z0 >= 0 && dst_nz_local >= 0 && dst_z0 + dst_nz_local <= nz, "bad output slab");
   MICA_REQUIRE(ny <= 65535 && dst_nz_local <= 65535, "output too large for the launch grid");
+  MICA_REQUIRE(order != 3 || row_fits_smem(sx) || (int64_t)src_nz_local * sy <= 65535,
+               "rows of %d samples are prefiltered one per CTA: at most 65535 of them fit the launch grid (got %lld)",
+               sx, (long long)src_nz_local * sy);
   if (workspace_bytes < mica_resample_workspace_bytes(src_nz_local, sy, sx, nz, ny, nx, order))
     return set_error(MICA_ERR_WORKSPACE, "resample workspace too small");
   if (dst_nz_local == 0) return MICA_OK;
@@ -1598,7 +1633,7 @@ extern "C" int mica_bspline_resample_f32(const float* src, int sz, int sy, int s
     double* xr = (double*)((char*)coeff + align_up((size_t)2 * src_nz_local * sy * p32 * sizeof(float), 256));
     // axis 0 (z): columns (y, x0..x0+15) of length src_nz_local; float32 in (row pitch sx), float32 out (pitch p32)
     const bool pipe = !getenv("MICA_RESAMPLE_NOPIPE");
-    const bool regcols = reg_cols_ok(src_nz_local, sy);
+    const bool regcols = reg_cols_ok();
     float* c32b = c32 + (size_t)src_nz_local * sy * p32;      // second float32 volume (the register pass is not in place)
     const ColStrides Sz{plane, sy * p32, sx, p32}, Sy{p32, p32, sy * p32, sy * p32};
     int rc;
@@ -1609,16 +1644,16 @@ extern "C" int mica_bspline_resample_f32(const float* src, int sz, int sy, int s
     needed_planes(sz, nz, dst_z0, dst_nz_local, src_z0, src_nz_local, &c_lo, &c_hi);
     const int l0 = c_lo - src_z0, cnt = c_hi - c_lo + 1;
     if (regcols) {
-      rc = launch_cols_reg(src, c32b, src_nz_local, sx, sy, Sz, st, src_z0, sz, c_lo, c_hi);
+      rc = launch_cols_reg(src, c32b, src_nz_local, sx, sy, Sz, st, kPassZ, src_z0, sz, c_lo, c_hi);
       if (rc) return rc;
-      rc = launch_cols_reg(c32b + (size_t)l0 * sy * p32, c32 + (size_t)l0 * sy * p32, sy, sx, cnt, Sy, st);
+      rc = launch_cols_reg(c32b + (size_t)l0 * sy * p32, c32 + (size_t)l0 * sy * p32, sy, sx, cnt, Sy, st, kPassY);
     } else {
-      rc = pipe ? launch_cols_pipe(src, c32, src_nz_local, sx, sy, Sz, st)
-                : launch_cols<float, float>(src, c32, src_nz_local, sx, sy, Sz, st);
+      rc = pipe ? launch_cols_pipe(src, c32, src_nz_local, sx, sy, Sz, st, kPassZ)
+                : launch_cols<float, float>(src, c32, src_nz_local, sx, sy, Sz, st, kPassZ);
       if (rc) return rc;
       // axis 1 (y): in place, per z plane, lines of length sy with stride p32
-      rc = pipe ? launch_cols_pipe(c32, c32, sy, sx, src_nz_local, Sy, st)
-                : launch_cols<float, float>(c32, c32, sy, sx, src_nz_local, Sy, st);
+      rc = pipe ? launch_cols_pipe(c32, c32, sy, sx, src_nz_local, Sy, st, kPassY)
+                : launch_cols<float, float>(c32, c32, sy, sx, src_nz_local, Sy, st, kPassY);
     }
     if (rc) return rc;
     // axis 2 (x): prefilter + interpolate the rows -> x-resampled float64 volume
@@ -1631,6 +1666,7 @@ extern "C" int mica_bspline_resample_f32(const float* src, int sz, int sy, int s
       const size_t smem = (size_t)(sx | 1) * sizeof(double) * 16;
       MICA_CUDA(cudaFuncSetAttribute(rows_prefilter_interp_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
       rows_prefilter_interp_kernel<16><<<(unsigned)ceil_div64(n_rows, 16), 256, smem, st>>>(c32, p32, xr, p64, sx, nx, n_rows, tx);
+      g_resample_path[kPassX] = MICA_RS_ROWS_PREFILTER_INTERP;
       MICA_LAUNCH_CHECK("rows_prefilter_interp_kernel");
     }
     zwin_kernel<<<(dst_nz_local + 127) / 128, 128, 0, st>>>(tz, zw, dst_nz_local, src_nz_local);
@@ -1657,19 +1693,21 @@ extern "C" int mica_bspline_resample_f32(const float* src, int sz, int sy, int s
     if (rows == 12) {
       MICA_CUDA(cudaFuncSetAttribute(march_yz_tma_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
       march_yz_tma_kernel<3><<<mgrid, 256, smem, st>>>(tmap, zw, ty, dst, ny, nx, dst_nz_local, zchunk);
+      g_resample_path[kPassInterp] = MICA_RS_MARCH_YZ_TMA3;
     } else {
       MICA_CUDA(cudaFuncSetAttribute(march_yz_tma_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
       march_yz_tma_kernel<4><<<mgrid, 256, smem, st>>>(tmap, zw, ty, dst, ny, nx, dst_nz_local, zchunk);
+      g_resample_path[kPassInterp] = MICA_RS_MARCH_YZ_TMA4;
     }
     MICA_LAUNCH_CHECK("march_yz_tma_kernel");
   } else if (order == 3) {
     const int64_t plane = (int64_t)sy * sx;
     MICA_REQUIRE(plane <= 0x7fffffffLL && src_nz_local <= 65535, "source plane too large");
     // axis 0 (z): lines of length src_nz_local, stride plane; reads float32, writes float64
-    int rc = launch_cols_f64<float>(src, coeff, src_nz_local, plane, (int)plane, 0, 1, st);
+    int rc = launch_cols_f64<float>(src, coeff, src_nz_local, plane, (int)plane, 0, 1, st, kPassZ);
     if (rc) return rc;
     // axis 1 (y): per z plane, lines of length sy, stride sx
-    rc = launch_cols_f64<double>(coeff, coeff, sy, sx, sx, plane, src_nz_local, st);
+    rc = launch_cols_f64<double>(coeff, coeff, sy, sx, sx, plane, src_nz_local, st, kPassY);
     if (rc) return rc;
     // axis 2 (x): contiguous rows
     rc = launch_rows(coeff, sx, (int64_t)src_nz_local * sy, st);
@@ -1711,25 +1749,34 @@ extern "C" int mica_bspline_resample_f32(const float* src, int sz, int sy, int s
         if (rows == 12) {
           MICA_CUDA(cudaFuncSetAttribute(march3_tma_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
           march3_tma_kernel<3><<<mgrid, 256, smem, st>>>(tmap, xb, zw, ty, tx, dst, ny, nx, dst_nz_local, zchunk);
+          g_resample_path[kPassInterp] = MICA_RS_MARCH3_TMA3;
         } else {
           MICA_CUDA(cudaFuncSetAttribute(march3_tma_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
           march3_tma_kernel<4><<<mgrid, 256, smem, st>>>(tmap, xb, zw, ty, tx, dst, ny, nx, dst_nz_local, zchunk);
+          g_resample_path[kPassInterp] = MICA_RS_MARCH3_TMA4;
         }
         MICA_LAUNCH_CHECK("march3_tma_kernel");
       } else {
-        if (span_y <= 12)
+        if (span_y <= 12) {
           march3_kernel<3><<<mgrid, 256, 0, st>>>(coeff, sy, sx, zw, ty, tx, dst, ny, nx, dst_nz_local, zchunk);
-        else
+          g_resample_path[kPassInterp] = MICA_RS_MARCH3_3;
+        } else {
           march3_kernel<4><<<mgrid, 256, 0, st>>>(coeff, sy, sx, zw, ty, tx, dst, ny, nx, dst_nz_local, zchunk);
+          g_resample_path[kPassInterp] = MICA_RS_MARCH3_4;
+        }
         MICA_LAUNCH_CHECK("march3_kernel");
       }
     } else {
       gather3_kernel<<<grid, 128, 0, st>>>(coeff, sy, sx, tz, ty, tx, dst, ny, nx);
+      g_resample_path[kPassInterp] = MICA_RS_GATHER3;
       MICA_LAUNCH_CHECK("gather3_kernel");
     }
   } else {
     gather1_kernel<<<grid, 128, 0, st>>>(src, sy, sx, tz, ty, tx, dst, ny, nx);
+    g_resample_path[kPassInterp] = MICA_RS_GATHER1;
     MICA_LAUNCH_CHECK("gather1_kernel");
   }
   return MICA_OK;
 }
+
+extern "C" int mica_last_resample_path(int pass) { return pass >= 0 && pass < 4 ? g_resample_path[pass] : -1; }
