@@ -185,6 +185,12 @@ int mica_peer_alloc(void** dev_ptr, void* ipc_handle_out /* 64 bytes, nullable *
 int mica_peer_open(const void* ipc_handle, void** dev_ptr);
 int mica_peer_close(void* dev_ptr);
 int mica_peer_free(void* dev_ptr);
+/* Inside ONE process: lets kernels running on `device` load from and store to memory allocated on
+ * `peer_device` (cudaDeviceEnablePeerAccess).  device == peer_device is a no-op; a pair already enabled (by
+ * this library or by PyTorch) counts as success; a pair without a peer path is MICA_ERR_INVALID.  The caller's
+ * current device is restored.  (CUDA IPC handles cannot be opened by the process that made them, so
+ * mica_peer_open does not serve several GPUs driven from one process.) */
+int mica_peer_enable(int device, int peer_device);
 int mica_select_peer_reduce(void* workspace, void* const* peer_bufs, int rank, int world, int parity, int epoch,
                             int step /* host step 0..MICA_SELECT_PASSES-1; a step that is not due on the device
                                         (the fallback after an accepted guided pass) skips the handshake */,

@@ -65,6 +65,7 @@ SIGNATURES = {
     'mica_peer_open': (_i, [_p, C.POINTER(_p)]),
     'mica_peer_close': (_i, [_p]),
     'mica_peer_free': (_i, [_p]),
+    'mica_peer_enable': (_i, [_i, _i]),
     'mica_select_peer_reduce': (_i, [_p, _p, _i, _i, _i, _i, _i, _p]),
     'mica_halo_buffer_bytes': (_sz, [_i64]),
     'mica_ipc_alloc': (_i, [_sz, C.POINTER(_p), _p]),

@@ -1113,6 +1113,27 @@ extern "C" int mica_peer_open(const void* ipc_handle, void** dev_ptr) {
   return MICA_OK;
 }
 
+extern "C" int mica_peer_enable(int device, int peer_device) {
+  MICA_REQUIRE(device >= 0 && peer_device >= 0, "bad device pair (%d, %d)", device, peer_device);
+  if (device == peer_device) return MICA_OK;
+  int can = 0;
+  MICA_CUDA(cudaDeviceCanAccessPeer(&can, device, peer_device));
+  MICA_REQUIRE(can, "device %d cannot access the memory of device %d (no peer path between them)", device,
+               peer_device);
+  int prev = 0;
+  MICA_CUDA(cudaGetDevice(&prev));
+  MICA_CUDA(cudaSetDevice(device));
+  cudaError_t e = cudaDeviceEnablePeerAccess(peer_device, 0);
+  if (e == cudaErrorPeerAccessAlreadyEnabled) {   // e.g. enabled by PyTorch for a copy: not an error, and
+    cudaGetLastError();                           // must not be reported by a later launch check
+    e = cudaSuccess;
+  }
+  const cudaError_t restore = cudaSetDevice(prev);
+  MICA_CUDA(e);
+  MICA_CUDA(restore);
+  return MICA_OK;
+}
+
 extern "C" int mica_peer_close(void* dev_ptr) {
   if (dev_ptr) MICA_CUDA(cudaIpcCloseMemHandle(dev_ptr));
   return MICA_OK;

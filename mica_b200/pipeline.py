@@ -12,6 +12,7 @@ preprocessing.py, create_grids.py, predict.py) are thin shells over this class.
 """
 from __future__ import annotations
 
+import bisect
 import functools
 import time
 from contextlib import contextmanager
@@ -155,6 +156,45 @@ def run_model_chunks(model_fn, x, af, flags_host, ijk, stitch, model_batch=None,
                 gx, gaf, gijk = x[idx], af[idx], ijk[idx].contiguous()
             bb, ca, aa = model_fn(gx, gaf)
             stitch(bb, ca, aa, gijk)
+
+
+def _chunk_starts(n_cubes, super_batch, model_batch):
+    """Where the model calls of a one-device run start: the visiting order is cut into super-batches of
+    ``super_batch`` cubes and each of them into chunks of ``model_batch`` (``run_model_chunks``)."""
+    sb, mb = max(1, int(super_batch)), max(1, int(model_batch))
+    return [c for s in range(0, n_cubes, sb) for c in range(s, min(n_cubes, s + sb), mb)]
+
+
+def deal_cubes(n_cubes, super_batch, model_batch, n_workers):
+    """Deal a map's cubes over ``n_workers`` devices without changing any model call.
+
+    Returns one contiguous range (lo, hi) of the visiting order per worker.  Every bound is where a
+    model call of the one-device run starts (or the end), so the calls the workers make -- with
+    ``worker_batches`` -- are exactly the one-device calls: with TF32 convolutions a cube's logits depend on
+    the batch it is convolved in, and MICA's zero-AF3 branch is taken per batch (D8).  Each bound is the
+    chunk start nearest to an even split, so every worker's count is within one chunk (``model_batch``
+    cubes) of ``n_cubes / n_workers``; with fewer chunks than workers some ranges are empty."""
+    n, w = int(n_cubes), int(n_workers)
+    if w < 1:
+        raise MicaError(f'n_workers must be >= 1, got {n_workers}')
+    cuts = _chunk_starts(n, super_batch, model_batch) + [n]
+    bounds = [0]
+    for r in range(1, w):
+        target = n * r / w
+        i = bisect.bisect_left(cuts, target)
+        if i == len(cuts) or (i > 0 and target - cuts[i - 1] <= cuts[i] - target):
+            i -= 1
+        bounds.append(max(bounds[-1], cuts[i]))
+    bounds.append(n)
+    return [(bounds[r], bounds[r + 1]) for r in range(w)]
+
+
+def worker_batches(lo, hi, super_batch):
+    """A worker's range cut at the one-device super-batch boundaries inside it, as (b0, b1) relative to ``lo``:
+    the super-batches ``MapPipeline.predict_and_stitch(batches=)`` then feeds to ``run_model_chunks``."""
+    sb = max(1, int(super_batch))
+    cuts = [lo] + list(range((lo // sb + 1) * sb, hi, sb)) + [hi]
+    return [(a - lo, b - lo) for a, b in zip(cuts[:-1], cuts[1:]) if b > a]
 
 
 class MapPipeline:
@@ -367,7 +407,8 @@ class MapPipeline:
     # ---------------------------------------------------------------- stage 5 (+model)
     @_on_device
     def predict_and_stitch(self, model_fn, vols: ops.StitchedVolumes | None = None, on_batch=None, *,
-                           model_batch=None, d8='none', order=None, stitch_fn=None, overlap_window=None):
+                           model_batch=None, d8='none', order=None, stitch_fn=None, overlap_window=None,
+                           batches=None):
         """run_inference + reconstruct_volume (utils/predict.py:307-587) without the
         per-cube files.  ``model_fn(exp_map, af_features) -> (bb, ca, aa)`` logits, enqueued
         on the current stream.  With ``prefetch`` the cubes of batch n+1 are cut on a side
@@ -383,7 +424,9 @@ class MapPipeline:
         softmax/argmax + stitch (multi-GPU: cores owned by another rank go to its volumes).
         ``overlap_window`` ('uniform' | 'triangle' | 'core' | W weights): the north_star's overlap-weighted
         stitching instead of the reference's centre-crop paste (``ops.OverlapStitcher``; NOT the reference's
-        arithmetic, see DESIGN.md D2) -- whole map on one GPU only."""
+        arithmetic, see DESIGN.md D2) -- whole map on one GPU only.  ``batches``: the super-batches as
+        (b0, b1) ranges of the (ordered) cube list, each at most ``batch_cubes`` long, instead of the even cut
+        (``worker_batches``: a worker's share of a map dealt over several devices)."""
         if self.normalized is None:
             raise MicaError('no normalised map')
         self.cube_index()
@@ -402,7 +445,12 @@ class MapPipeline:
             self._set_cube_origins(self.ijk_host[order], ('ordered', id(order), len(order)))
             self._ijk_key = None                          # the next map starts from the loop order again
         n = len(self.ijk_host)
-        batches = [(b0, min(n, b0 + self.batch_cubes)) for b0 in range(0, n, self.batch_cubes)]
+        if batches is None:
+            batches = [(b0, min(n, b0 + self.batch_cubes)) for b0 in range(0, n, self.batch_cubes)]
+        else:
+            batches = [(int(b0), int(b1)) for b0, b1 in batches]
+            if any(not 0 <= b0 < b1 <= n or b1 - b0 > self.batch_cubes for b0, b1 in batches):
+                raise MicaError(f'batches must be non-empty ranges of the {n} cubes, at most {self.batch_cubes} long')
         if not batches:
             return overlap.finalize() if overlap is not None else vols
         want_flags = d8 == 'split' and (model_batch is None or int(model_batch) > 1)
@@ -624,3 +672,20 @@ def shared_pipeline(device) -> MapPipeline:
     if pipe is None:
         pipe = _SHARED[dev.index] = MapPipeline(dev)
     return pipe
+
+
+_WORKERS: dict = {}
+
+
+def worker_pipeline(device, slot: int):
+    """(MapPipeline, stream) of one worker of a map dealt over several devices in one process
+    (``CryoEMPredictor(devices=)``), kept per (GPU, slot) across maps like ``shared_pipeline``: ``slot`` n is
+    the n-th worker on that GPU, each with its own cube buffers and stream."""
+    dev = torch.device(device)
+    if dev.type != 'cuda' or dev.index is None:
+        raise MicaError(f'worker_pipeline needs an indexed CUDA device, got {device!r}')
+    key = (dev.index, int(slot))
+    w = _WORKERS.get(key)
+    if w is None:
+        w = _WORKERS[key] = (MapPipeline(dev), torch.cuda.Stream(dev))
+    return w

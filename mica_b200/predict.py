@@ -10,24 +10,77 @@ buffers, the AF3 channels are rasterised straight from the docked atoms, the mod
 reference's batches (1, or <= 8 above 200 cubes), its logits are post-processed and their cores
 pasted into the four volumes, and finished layers of the volumes stream to pinned host memory
 while later cubes are still in the model.  When only the reference's ``.npz`` files exist on
-disk, the cubes are uploaded from them instead."""
+disk, the cubes are uploaded from them instead.
+
+With ``devices=`` (or ``MICA_DEVICES``) the cubes of one map are dealt over several GPUs of this process:
+one thread, ``MapPipeline``, stream and model replica per device, every model call the same as on one
+device, every core stored into one volume block on the predictor's ``device`` over NVLink."""
 from __future__ import annotations
 
+import copy
 import glob
 import logging
 import os
 import re
+import threading
 import time
+from collections.abc import Mapping
 
 import numpy as np
 import torch
 
 from . import ops, pdb, session
-from .pipeline import MapPipeline, _SlabDrain, run_model_chunks, shared_pipeline
+from ._lib import check, lib
+from .pipeline import (MapPipeline, _SlabDrain, deal_cubes, run_model_chunks, shared_pipeline, worker_batches,
+                       worker_pipeline)
 
 MAP_TYPES = ('backbone_probability', 'carbon_alpha_probability', 'amino_acid_prediction',
              'amino_acid_probability')
 SMALL_VOLUMES = MAP_TYPES[:3]
+
+
+def parse_devices(spec, n_visible: int, allow_repeats: bool = True):
+    """``devices=`` / ``MICA_DEVICES`` -> a list of CUDA device indices, or None for the one-device path.
+
+    None or '' -> None; 'all' -> every visible device; '0,2,3' or a list of ints, 'N' or 'cuda:N' strings or
+    ``torch.device`` -> those devices.  Repeats (several workers on one GPU) only with ``allow_repeats``.
+    Anything else raises ValueError."""
+    if spec is None:
+        return None
+    if isinstance(spec, str):
+        text = spec.strip()
+        if not text:
+            return None
+        if text.lower() == 'all':
+            if n_visible < 1:
+                raise ValueError('devices=all: no CUDA device is visible')
+            return list(range(n_visible))
+        items = text.split(',')
+    else:
+        items = list(spec)
+        if not items:
+            return None
+    out = []
+    for it in items:
+        try:
+            if isinstance(it, torch.device):
+                d = it
+            elif isinstance(it, (int, np.integer)) and not isinstance(it, bool):
+                d = torch.device('cuda', int(it))
+            elif isinstance(it, str) and it.strip().isdigit():
+                d = torch.device('cuda', int(it.strip()))
+            elif isinstance(it, str):
+                d = torch.device(it.strip())
+            else:
+                raise ValueError
+        except (ValueError, RuntimeError):
+            raise ValueError(f'devices: cannot read {it!r} as a CUDA device (in {spec!r})') from None
+        if d.type != 'cuda' or d.index is None or not 0 <= d.index < n_visible:
+            raise ValueError(f'devices: {it!r} is not one of the {n_visible} visible CUDA devices (in {spec!r})')
+        out.append(d.index)
+    if not allow_repeats and len(set(out)) != len(out):
+        raise ValueError(f'devices: {spec!r} lists a device twice')
+    return out
 
 
 class HostPool:
@@ -105,7 +158,7 @@ class DeviceVolume:
 class CryoEMPredictor:
     def __init__(self, model_path, grids_path, output_path, save_output=True, device='cuda', quiet=False,
                  model=None, keep_on_device=True, host_volumes=None, host_pool=None, reference_batching=False,
-                 super_batch=256, release_inputs=True):
+                 super_batch=256, release_inputs=True, devices=None):
         """Additions to the reference signature (all optional):
 
         ``model``               an already loaded model (callable ``(exp_map, af_features) -> (bb, ca, aa)``).
@@ -124,7 +177,19 @@ class CryoEMPredictor:
                                 the grid files exist, mixed batches of ``optimal_batch_size``.
         ``super_batch``         cubes cut / stitched per kernel launch.
         ``release_inputs``      drop the consumed session entries (normalised map, atoms, cube indices) when
-                                done, as Solver.nnPred deletes the files (utils/modeler.py:753-758)."""
+                                done, as Solver.nnPred deletes the files (utils/modeler.py:753-758).
+        ``devices``             deal the map's cubes over several GPUs of this process: 'all', '0,2,3', or a list
+                                of ints / 'cuda:N'; None reads ``MICA_DEVICES`` when ``run_prediction`` is called
+                                (unset or empty: one device).  ``device`` is always worker 0 and receives the
+                                volumes.  A device listed n times in ``devices`` runs n workers, each with its
+                                own stream.  Every model call sees the cubes, in the order, it sees on one device
+                                with the same options, so the volumes do not depend on the device count.  The
+                                model is loaded once per GPU; an ``nn.Module`` given as ``model`` is deep-copied
+                                to the other GPUs, or ``model`` may be a {device: callable} mapping."""
+        self.devices = devices
+        self.worker_cubes = None                        # cubes each worker ran (several devices only)
+        self._workers = None
+        self._models = None
         self.keep_on_device = bool(keep_on_device)
         self.host_volumes = SMALL_VOLUMES if host_volumes is None else tuple(host_volumes)
         self.host_pool = host_pool
@@ -206,28 +271,79 @@ class CryoEMPredictor:
         finally:
             self.timing_stats['strategy_selection'] = time.time() - t0
 
+    # ------------------------------------------------------------------ several devices
+    def _resolve_workers(self):
+        """The worker devices (worker 0 = ``device``), or None for the one-device path."""
+        from_env = self.devices is None
+        spec = os.environ.get('MICA_DEVICES') if from_env else self.devices
+        if spec is None or (isinstance(spec, str) and not spec.strip()):
+            return None
+        idx = parse_devices(spec, torch.cuda.device_count(), allow_repeats=not from_env)
+        if idx is None:
+            return None
+        primary = torch.device(self.device)
+        if primary.type != 'cuda':
+            raise ops._lib.MicaError(f'devices= needs a CUDA device, got device={self.device!r}')
+        if primary.index is None:
+            primary = torch.device('cuda', torch.cuda.current_device())
+        if primary.index in idx:
+            idx.remove(primary.index)                   # its first listing is worker 0
+        workers = [primary] + [torch.device('cuda', i) for i in idx]
+        return workers if len(workers) > 1 else None
+
+    def _replicate_model(self, devs):
+        """{device: callable} for every distinct worker device; False (logged) if the model cannot be placed."""
+        model = self.model
+        if isinstance(model, Mapping):
+            given = {}
+            for k, v in model.items():
+                d = torch.device('cuda', k) if isinstance(k, int) else torch.device(k)
+                given[torch.device('cuda', torch.cuda.current_device()) if d.index is None else d] = v
+            missing = [str(d) for d in devs if d not in given]
+            if missing:
+                self.logger.error(f'model mapping has no entry for {", ".join(missing)}')
+                return False
+            self._models = {d: given[d] for d in devs}
+            return True
+        if len(devs) > 1 and not isinstance(model, torch.nn.Module):
+            self.logger.error('a model that is not an nn.Module cannot be copied to several devices: '
+                              'pass model={device: callable}')
+            return False
+        self._models = {devs[0]: model}
+        for d in devs[1:]:
+            self._models[d] = copy.deepcopy(model).to(d)
+        return True
+
     # utils/predict.py:217-258
     def load_model(self):
         t0 = time.time()
         try:
+            devs = list(dict.fromkeys(self._workers)) if self._workers else None
             if self.model is not None:
-                return True
+                return True if devs is None else self._replicate_model(devs)
             if not os.path.exists(self.model_path):
                 self.logger.error(f'Model file not found: {self.model_path}')
                 return False
-            from models.model import MICA                       # the reference's model, unchanged
-            model = MICA().to(self.device)
-            checkpoint = torch.load(self.model_path, map_location=self.device)
-            state = {k.replace('module.', ''): v.to(self.device) for k, v in checkpoint['model_state_dict'].items()}
-            model.load_state_dict(state, strict=False)
-            model.eval()
-            self.model = model
+            if devs is None:
+                self.model = self._load_checkpoint(self.device)
+                return True
+            self._models = {d: self._load_checkpoint(d) for d in devs}
+            self.model = self._models[devs[0]]
             return True
         except Exception as e:
             self.logger.error(f'Model loading failed: {e}')
             return False
         finally:
             self.timing_stats['model_loading'] = time.time() - t0
+
+    def _load_checkpoint(self, device):
+        from models.model import MICA                           # the reference's model, unchanged
+        model = MICA().to(device)
+        checkpoint = torch.load(self.model_path, map_location=device)
+        state = {k.replace('module.', ''): v.to(device) for k, v in checkpoint['model_state_dict'].items()}
+        model.load_state_dict(state, strict=False)
+        model.eval()
+        return model
 
     # ------------------------------------------------------------------ inference + stitch
     def _model_batch(self):
@@ -300,6 +416,8 @@ class CryoEMPredictor:
     def run_inference_and_reconstruct(self):
         """run_inference + reconstruct_volume (utils/predict.py:307-512) fused.  Returns
         (device volumes, {name: pinned host tensor})."""
+        if self._workers:
+            return self._run_on_devices(self._workers)
         dev = torch.device(self.device)
         s = self._source
         gs, pad = s['grid_size'], s['padding']
@@ -341,6 +459,126 @@ class CryoEMPredictor:
             torch.cuda.synchronize(dev)
             return vols, out_host
 
+    def _run_on_devices(self, workers):
+        """The map's cubes dealt over ``workers`` (``deal_cubes``), one thread each.  Every worker stores its
+        cores into ONE 23-channel block on workers[0] (``postproc_stitch_peer`` with a one-entry owner table);
+        the host copies run once, after the last worker has finished.  Returns what
+        ``run_inference_and_reconstruct`` returns."""
+        s = self._source
+        gs, pad = s['grid_size'], s['padding']
+        primary, n, mb = workers[0], len(s['ijk']), self._model_batch()
+        d8 = 'reference' if self.reference_batching else 'split'
+        resident = s['kind'] == 'resident'
+        slots = [sum(1 for d in workers[:w] if d == workers[w]) for w in range(len(workers))]
+        streams = [worker_pipeline(d, slot)[1] for d, slot in zip(workers, slots)]
+        pipes = [None] * len(workers)
+        if resident:
+            # the normalised map (and the atoms, or a dense AF3 volume) once per device; workers on one device
+            # share them.  Worker 0 continues on the map's own pipeline when that lives on the primary device.
+            m, a = s['map'], s['af3']
+            inputs = {}
+            for w, (dev, slot) in enumerate(zip(workers, slots)):
+                if w == 0 and m['volume'].device == dev:
+                    pipes[0] = self._pipeline(dev)
+                    continue
+                if dev not in inputs:
+                    af3 = None
+                    if a is not None and a.get('atoms') is None:
+                        vol = a['volume']
+                        af3 = (vol.get() if hasattr(vol, 'get') else vol).to(dev)
+                    inputs[dev] = (m['volume'].to(dev),
+                                   tuple(t.to(dev) for t in a['atoms']) if a is not None and a.get('atoms') is not None
+                                   else None, af3)
+                norm, atoms, af3 = inputs[dev]
+                pipe = worker_pipeline(dev, slot)[0]
+                pipe.configure(grid_size=gs, padding=pad, batch_cubes=max(1, min(self.super_batch, n)))
+                pipe.set_normalized(norm, m['header'])
+                if atoms is not None:
+                    if not pipe.encode_af3(*atoms):
+                        raise IndexError('atom index outside the grid')
+                else:
+                    pipe.af3, pipe._atoms_binned = af3, False
+                pipes[w] = pipe
+            order = self._reference_order() if self.reference_batching else None
+            order = np.arange(n, dtype=np.int64) if order is None else np.asarray(order, dtype=np.int64)
+            pipes[0].cube_index()
+            cube_shape = pipes[0].cube_shape
+            super_batch = max(1, min(self.super_batch, n))
+            self._pipe = pipes[0]
+        else:
+            if primary.type != 'cuda':
+                raise ops._lib.MicaError('mica_b200 has no CPU path')
+            cube_shape = s['cube_shape']
+            super_batch = max(mb, 1) * 4
+            ijk_dev = {d: torch.from_numpy(np.ascontiguousarray(s['ijk'], dtype=np.int32)).to(d)
+                       for d in dict.fromkeys(workers)}
+        ranges = deal_cubes(n, super_batch, mb, len(workers))
+        self.worker_cubes = [hi - lo for lo, hi in ranges]
+        X, Y, Z = (int(v) for v in cube_shape)
+        for d in dict.fromkeys(workers):
+            check(lib.mica_peer_enable(d.index, primary.index), f'peer_enable({d} -> {primary})')
+        with torch.cuda.device(primary):
+            block = torch.zeros(23 * X * Y * Z, dtype=torch.float32, device=primary)
+            zeroed = torch.cuda.Event()
+            zeroed.record()
+        vols = ops.StitchedVolumes.from_block(block, cube_shape, (0, 0, 0), (X, Y, Z))
+        tables = {d: torch.tensor([block.data_ptr()], dtype=torch.int64, device=d) for d in dict.fromkeys(workers)}
+        for dev, st in zip(workers, streams):
+            st.wait_stream(torch.cuda.current_stream(dev))     # inputs copied / binned on the current streams
+            st.wait_event(zeroed)
+        for model in self._models.values():
+            if hasattr(model, 'eval'):
+                model.eval()
+
+        def body(w):
+            lo, hi = ranges[w]
+            if hi <= lo:
+                return
+            dev, table, model = workers[w], tables[workers[w]], self._models[workers[w]]
+
+            def stitch(bb, ca, aa, ijk, _vols=None):
+                ops.postproc_stitch_peer(bb.contiguous().float(), ca.contiguous().float(), aa.contiguous().float(),
+                                         ijk, cube_shape, table, (0, X), gs, pad)
+            with torch.cuda.device(dev), torch.cuda.stream(streams[w]), torch.no_grad():
+                if resident:
+                    pipes[w].predict_and_stitch(model, vols, model_batch=mb, d8=d8, order=order[lo:hi],
+                                                batches=worker_batches(lo, hi, super_batch), stitch_fn=stitch)
+                    return
+                for b0, b1 in worker_batches(lo, hi, super_batch):
+                    x, af, flags = self._fetch_files(lo + b0, lo + b1, dev)
+                    run_model_chunks(model, x, af, flags.cpu().numpy(), ijk_dev[dev][lo + b0:lo + b1], stitch, mb, d8)
+
+        errors = [None] * len(workers)
+
+        def run(w):
+            try:
+                body(w)
+            except BaseException as e:                   # re-raised below, after every worker has stopped
+                errors[w] = e
+
+        threads = [threading.Thread(target=run, args=(w,), name=f'mica-worker-{w}') for w in range(len(workers))]
+        try:
+            for t in threads:
+                t.start()
+        finally:
+            for t in threads:
+                if t.ident is not None:
+                    t.join()
+            for st in streams:
+                st.synchronize()                         # the primary reads the block only after every worker
+            for w, pipe in enumerate(pipes):
+                if pipe is not None and pipe is not pipes[0]:
+                    pipe.release_map()                   # the per-device copies of this map's inputs
+        for e in errors:
+            if e is not None:
+                raise e
+        out_host = self._host_buffers(vols)
+        with torch.cuda.device(primary):
+            for k, t in out_host.items():
+                t.copy_(getattr(vols, k), non_blocking=True)
+            torch.cuda.current_stream(primary).synchronize()
+        return vols, out_host
+
     def _release(self):
         s = self._source or {}
         if s.get('kind') != 'resident':
@@ -358,6 +596,7 @@ class CryoEMPredictor:
     def run_prediction(self):
         t_total = time.time()
         try:
+            self._workers = self._resolve_workers()
             if not self.select_processing_strategy():
                 return False, {}
             if not self.load_model():
