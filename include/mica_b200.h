@@ -93,27 +93,21 @@ int mica_bspline_resample_f32(const float* src, int sz, int sy, int sx, int src_
 /* diagnostic: the kernel the last mica_bspline_resample_f32 call on this thread launched for one pass
  * (pass 0 = z prefilter, 1 = y prefilter, 2 = x pass, 3 = interpolation), one of the MICA_RS_* ids below;
  * -1 when that pass did not run (order 1 has no prefilter; a call that failed its argument checks ran none).
- * The fast path's x pass prefilters and interpolates x in one kernel; its pass 3 then interpolates y and z. */
+ * The fast path's x pass prefilters and interpolates x in one kernel; its pass 3 then interpolates y and z.
+ * An id keeps its number for good: the gaps are kernels that no longer exist. */
 int mica_last_resample_path(int pass);
 #define MICA_RS_COLS_SEG16 1          /* prefilter_cols_seg<16>: 16 lines x 16 segments in shared memory */
-#define MICA_RS_COLS_SEG32 2          /* prefilter_cols_seg<32> */
 #define MICA_RS_COLS32 3              /* prefilter_cols<32>: one thread per line */
 #define MICA_RS_COLS8 4               /* prefilter_cols<8>: one thread per line, long lines */
 #define MICA_RS_COLS_GLOBAL 5         /* prefilter_cols_global: one thread per line, in global memory */
 #define MICA_RS_ROWS_SEG16 6          /* prefilter_rows_seg<16> */
-#define MICA_RS_ROWS_SEG32 7          /* prefilter_rows_seg<32> */
 #define MICA_RS_ROWS32 8              /* prefilter_rows<32>: one thread per row */
 #define MICA_RS_ROWS4 9               /* prefilter_rows<4>: one thread per row, long rows */
 #define MICA_RS_COLS_REG 10           /* cols_reg_kernel: register segments numbered on the whole line */
-#define MICA_RS_COLS_PIPE_16_256 11   /* cols_pipe_kernel<16, 256> */
-#define MICA_RS_COLS_PIPE_16_512 12   /* cols_pipe_kernel<16, 512> */
-#define MICA_RS_COLS_PIPE_8_512 13    /* cols_pipe_kernel<8, 512> */
 #define MICA_RS_ROWS_REG16 14         /* rows_reg_interp_kernel<16> */
 #define MICA_RS_ROWS_REG32 15         /* rows_reg_interp_kernel<32> */
-#define MICA_RS_ROWS_PIPE_16_256 16   /* rows_pipe_interp_kernel<16, 256> */
 #define MICA_RS_ROWS_PIPE_16_512 17   /* rows_pipe_interp_kernel<16, 512> */
 #define MICA_RS_ROWS_PIPE_8_512 18    /* rows_pipe_interp_kernel<8, 512> */
-#define MICA_RS_ROWS_PREFILTER_INTERP 19 /* rows_prefilter_interp_kernel<16> */
 #define MICA_RS_MARCH_YZ_TMA3 20      /* march_yz_tma_kernel<3>: 12 staged rows */
 #define MICA_RS_MARCH_YZ_TMA4 21      /* march_yz_tma_kernel<4>: 16 staged rows */
 #define MICA_RS_MARCH3_TMA3 22        /* march3_tma_kernel<3> */

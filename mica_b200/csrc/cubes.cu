@@ -155,8 +155,6 @@ __device__ __forceinline__ uint32_t smem_u32(const void* p) {
 }
 
 struct TmaExtractParams {
-  int l2_hint;       // 1: the box loads carry an L2 evict_last policy (the 8x overlapping windows re-read the
-                     // same source lines; the output is written with evict-first .cs stores)
   const int32_t* ijk;
   float* out;
   int64_t out_cube_stride;
@@ -188,19 +186,10 @@ extract_tma_kernel(const __grid_constant__ CUtensorMap tmap, TmaExtractParams P)
   if (threadIdx.x == 0) {
     const uint32_t bytes = (uint32_t)BT * W * 128u;
     asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar_a), "r"(bytes) : "memory");
-    if (P.l2_hint) {
-      uint64_t policy;
-      asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(policy));
-      asm volatile(
-          "cp.async.bulk.tensor.4d.shared::cluster.global.tile.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1, {%2, %3, %4, %5}], [%6], %7;"
-          ::"r"(tile_a), "l"(&tmap), "r"(i0 + a0), "r"(k0 - P.off_c), "r"(j0 + b0 - P.off_b), "r"(ch), "r"(bar_a), "l"(policy)
-          : "memory");
-    } else {
-      asm volatile(
-          "cp.async.bulk.tensor.4d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4, %5}], [%6];"
-          ::"r"(tile_a), "l"(&tmap), "r"(i0 + a0), "r"(k0 - P.off_c), "r"(j0 + b0 - P.off_b), "r"(ch), "r"(bar_a)
-          : "memory");
-    }
+    asm volatile(
+        "cp.async.bulk.tensor.4d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4, %5}], [%6];"
+        ::"r"(tile_a), "l"(&tmap), "r"(i0 + a0), "r"(k0 - P.off_c), "r"(j0 + b0 - P.off_b), "r"(ch), "r"(bar_a)
+        : "memory");
   }
   {  // wait for the box (phase 0)
     uint32_t done = 0;
@@ -315,14 +304,9 @@ extern "C" int mica_extract_cubes(const float* vol, int64_t chan_stride, int n_c
                             (cuuint64_t)(n_channels > 1 ? chan_stride : (int64_t)nz_local * ny * nx) * 4};
       cuuint32_t box[4] = {32, (cuuint32_t)W, (cuuint32_t)kTmaBT, 1};
       cuuint32_t estr[4] = {1, 1, 1, 1};
-      CUtensorMapL2promotion promo = CU_TENSOR_MAP_L2_PROMOTION_L2_64B;   // measured best of the four on B200
-      if (const char* e = getenv("MICA_TMA_L2PROMO")) {   // experiment knob: 0 none, 1 64B, 2 128B, 3 256B
-        const int v = atoi(e);
-        promo = v == 0 ? CU_TENSOR_MAP_L2_PROMOTION_NONE : v == 1 ? CU_TENSOR_MAP_L2_PROMOTION_L2_64B
-              : v == 2 ? CU_TENSOR_MAP_L2_PROMOTION_L2_128B : CU_TENSOR_MAP_L2_PROMOTION_L2_256B;
-      }
+      // L2 promotion: 64B measured best of none / 64B / 128B / 256B on B200
       CUresult r = enc(&tmap, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, (void*)vol, gdim, gstr, box, estr,
-                       CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, promo,
+                       CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_64B,
                        CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
       if (r == CUDA_SUCCESS) {
         use_tma = true;
@@ -345,7 +329,6 @@ extern "C" int mica_extract_cubes(const float* vol, int64_t chan_stride, int n_c
     dim3 grid(W, nb, n_channels), block(32, 8);
     if (use_tma) {
       TmaExtractParams T;
-      T.l2_hint = getenv("MICA_EXTRACT_L2HINT") ? atoi(getenv("MICA_EXTRACT_L2HINT")) : 0;
       T.ijk = P.ijk;
       T.out = P.out;
       T.out_cube_stride = out_cube_stride;

@@ -9,22 +9,34 @@
 // as outside the map (mode='constant') and yields 0.
 //
 // Kernels (all HBM-bound, see DESIGN.md for the byte counts):
-//   taps_kernel          per-axis tap index / weight tables (tiny)
-//   prefilter_cols_seg   IIR along a strided axis (z or y): a [n x 32] float64 tile of 32
-//   prefilter_rows_seg   neighbouring lines (rows: [32 x n], contiguous axis) is staged in
-//                        shared memory with coalesced loads; every line is cut into 8 segments
+//   taps_kernel, zwin_kernel  per-axis tap index / weight tables; the z taps folded into 4-plane windows (tiny)
+// Fast path (order 3, the conditions are in fast_path_ok):
+//   cols_reg_kernel      z and y prefilter, float32 in and out: a thread owns <= 26 samples of one column and
+//                        runs both recursions over them and 16 samples either side in registers (no shared
+//                        memory, no barrier); segments are numbered on the whole line, so a z-slab of a map
+//                        gets the whole map's bits
+//   rows_reg_interp_kernel   x pass, rows of <= 832 samples: cp.async-staged rows, swept by the same register
+//                        segments, interpolated along x into the x-resampled float64 volume
+//   rows_pipe_interp_kernel  x pass, rows of 833-1759 samples: the same, swept in a float64 shared-memory tile
+//   march_yz_tma_kernel  y and z interpolation: TMA boxes of the x-resampled volume in an mbarrier ring, a
+//                        4-plane register window marched along z
+// General path (float64 throughout; short or very long lines, strong down-sampling, MICA_NO_TMA):
+//   prefilter_cols_seg   IIR along a strided axis (z or y): a [n x 16] float64 tile of 16
+//   prefilter_rows_seg   neighbouring lines (rows: [16 x n], contiguous axis) is staged in
+//                        shared memory with coalesced loads; every line is cut into 16 segments
 //                        swept concurrently, each warmed up over the kHorizon samples before
 //                        (causal) / after (anticausal) it -- the pole's impulse response has
 //                        decayed below double rounding by then -- so all 256 threads recurse
-//   march3_kernel        separable 4x4x4 gather: a CTA owns an [8 y x 64 x] output column and
-//                        marches along z; each source plane is x-interpolated from global
-//                        memory into shared memory (software-pipelined one plane ahead),
-//                        y-interpolated into a 4-plane register window, and every output
-//                        plane is 4 FMAs from that window: ~4 global + ~4 shared loads per
-//                        output voxel instead of 64 global loads
-//   prefilter_cols / prefilter_rows / gather3 / gather1
-//                        general fall-backs (short or very long lines, strong down-sampling,
-//                        trilinear): one thread per line / one thread per output voxel
+//   prefilter_cols / prefilter_rows   one thread per line in shared memory (short or long lines)
+//   prefilter_cols_global             one thread per line in global memory (lines that fit no tile)
+//   march3_tma_kernel    separable 4x4x4 gather: a CTA owns an [8 y x 64 x] output column and
+//                        marches along z; each source plane arrives as a TMA box, is
+//                        x-interpolated into shared memory, y-interpolated into a 4-plane
+//                        register window, and every output plane is 4 FMAs from that window
+//   march3_kernel        the same march fed by register prefetch (odd sx, wide x spans, MICA_NO_TMA)
+//   gather3_kernel       one thread per output voxel (axes under 4 samples, strong down-sampling,
+//                        mica_resample_force_generic)
+// Order 1: gather1_kernel, trilinear, one thread per output voxel, no prefilter.
 #include <cuda.h>
 #include <stdlib.h>
 
@@ -100,9 +112,10 @@ __global__ void taps_kernel(Tap* __restrict__ taps, int n_local, int k0, int n_i
 constexpr double kPole = -0.26794919243112270647;  // sqrt(3) - 2
 constexpr int kInitHorizon = 56;                    // |pole|^56 ~ 1e-32: below double rounding
 
-// One thread filters one line held in shared memory; `stride` is the distance (in
-// doubles) between successive samples of the line inside the tile.
-__device__ __forceinline__ void iir_line(double* line, int n, int stride) {
+// One thread filters one line in place; `stride` is the distance (in doubles) between
+// successive samples of the line (int inside a shared-memory tile, int64_t in global memory).
+template <typename Stride>
+__device__ __forceinline__ void iir_line(double* line, int n, Stride stride) {
   if (n < 2) return;
   const double z = kPole;
   // causal initialisation, mirror boundary, SciPy's pairing of k and n-1-k
@@ -138,14 +151,14 @@ constexpr double kGain = (1.0 - kPole) * (1.0 - 1.0 / kPole);  // = 6
 // lines along a strided axis.  grid = (ceil(n_cols / CW), n_outer)
 // Strides of a column pass: sample k of column j of outer index o sits at
 //   in [o * outer_in  + k * line_in  + j]     out[o * outer_out + k * line_out + j]
-// (in and out differ when the output volume has a padded row pitch or another element type).
+// (in and out differ when the output volume has a padded row pitch).
 struct ColStrides {
   int64_t line_in, line_out, outer_in, outer_out;
 };
 
-template <typename TIn, typename TOut, int CW>
+template <typename TIn, int CW>
 __global__ void __launch_bounds__(256)
-prefilter_cols(const TIn* __restrict__ in, TOut* __restrict__ out, int n, int n_cols, ColStrides S) {
+prefilter_cols(const TIn* __restrict__ in, double* __restrict__ out, int n, int n_cols, ColStrides S) {
   extern __shared__ double tile[];  // [n][CW]
   const int col0 = blockIdx.x * CW;
   const int64_t base_in = (int64_t)blockIdx.y * S.outer_in + col0, base_out = (int64_t)blockIdx.y * S.outer_out + col0;
@@ -160,7 +173,7 @@ prefilter_cols(const TIn* __restrict__ in, TOut* __restrict__ out, int n, int n_
   __syncthreads();
   for (int e = threadIdx.x; e < n * CW; e += blockDim.x) {
     int k = e / CW, j = e % CW;
-    if (j < ncol) out[base_out + (int64_t)k * S.line_out + j] = (TOut)tile[e];
+    if (j < ncol) out[base_out + (int64_t)k * S.line_out + j] = tile[e];
   }
 }
 
@@ -247,7 +260,7 @@ __device__ __forceinline__ void iir_segment(double* line, int n, int stride, int
   }
 }
 
-// Register-blocked variant for the pipelined passes.  iir_segment walks shared memory inside the
+// Register-blocked variant for the pipelined row pass.  iir_segment walks shared memory inside the
 // dependent chain (load -> FMA -> store per sample: ncu shows the warps waiting on the shared-memory
 // scoreboard 5 cycles per issued instruction).  Here a thread first pulls its segment (<= LMAX samples) and
 // its warm-up samples into registers with independent loads, runs both recursions register to register and
@@ -317,9 +330,9 @@ __device__ __forceinline__ void iir_segment_reg(double* line, int n, int k0, int
 
 // lines along a strided axis.  grid = (ceil(n_cols / L), n_outer), block = 256, tile [n][L],
 // 256 / L segments per line
-template <typename TIn, typename TOut, int L>
+template <typename TIn, int L>
 __global__ void __launch_bounds__(256)
-prefilter_cols_seg(const TIn* __restrict__ in, TOut* __restrict__ out, int n, int n_cols, ColStrides S) {
+prefilter_cols_seg(const TIn* __restrict__ in, double* __restrict__ out, int n, int n_cols, ColStrides S) {
   extern __shared__ double tile[];
   constexpr int kSegs = 256 / L;
   const int col0 = blockIdx.x * L;
@@ -337,9 +350,9 @@ prefilter_cols_seg(const TIn* __restrict__ in, TOut* __restrict__ out, int n, in
   iir_segment(tile + j, n, L, k0, k1, j < ncol && k0 < k1);
   __syncthreads();
   if (j < ncol) {
-    TOut* q = out + base_out + j;
+    double* q = out + base_out + j;
 #pragma unroll 8
-    for (int k = seg; k < n; k += kSegs) q[(int64_t)k * S.line_out] = (TOut)tile[k * L + j];
+    for (int k = seg; k < n; k += kSegs) q[(int64_t)k * S.line_out] = tile[k * L + j];
   }
 }
 
@@ -375,32 +388,7 @@ __global__ void prefilter_cols_global(const TIn* __restrict__ in, double* __rest
   const int64_t base = (int64_t)blockIdx.y * outer_stride + col;
   const double gain = (n >= 2) ? kGain : 1.0;
   for (int k = 0; k < n; ++k) out[base + k * line_stride] = (double)in[base + k * line_stride] * gain;
-  // iir_line with a 64-bit stride
-  double* line = out + base;
-  const double z = kPole;
-  if (n < 2) return;
-  double z_n_1 = pow(z, (double)(n - 1));
-  double c0 = line[0] + z_n_1 * line[(n - 1) * line_stride];
-  double z_i = z;
-  int lim = min(n - 1, kInitHorizon);
-  for (int k = 1; k < lim; ++k) {
-    c0 += z_i * (line[k * line_stride] + z_n_1 * line[(n - 1 - k) * line_stride]);
-    z_i *= z;
-  }
-  c0 /= (1.0 - z_n_1 * z_n_1);
-  line[0] = c0;
-  double prev = c0;
-  for (int k = 1; k < n; ++k) {
-    prev = fma(z, prev, line[k * line_stride]);
-    line[k * line_stride] = prev;
-  }
-  double last = (z / (z * z - 1.0)) * (prev + z * line[(n - 2) * line_stride]);
-  line[(n - 1) * line_stride] = last;
-  prev = last;
-  for (int k = n - 2; k >= 0; --k) {
-    prev = z * (prev - line[k * line_stride]);
-    line[k * line_stride] = prev;
-  }
+  iir_line(out + base, n, line_stride);
 }
 
 // ------------------------------------------------------------------- gather
@@ -720,15 +708,9 @@ cols_reg_kernel(const float* __restrict__ in, float* __restrict__ out, int n, in
     cols_reg_segment<true>(p, q, S.line_in, S.line_out, n, g0, ng, k0, k1);
 }
 
-// ------------------------------------------------- cp.async-pipelined prefilter passes (fast path)
-// The passes above load a tile, sweep it, store it -- and reach ~30 % of the HBM bandwidth because the three
-// phases of a CTA do not overlap.  Here a persistent CTA walks over its tiles with the float32 input of the
-// NEXT tile(s) already in flight (cp.async into a small staging ring: no registers, any alignment), converts
-// the staged tile into one float64 work tile, sweeps it (iir_segment, exact float64 as before) and writes
-// the result straight from the work tile.
-__device__ __forceinline__ void cp_async4(uint32_t dst, const void* src) {
-  asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(dst), "l"(src) : "memory");
-}
+// ------------------------------------------------- x pass of the fast path: prefilter + interpolation
+// A persistent CTA walks over its tiles of rows with the float32 input of the NEXT tile already in flight
+// (cp.async into a small staging ring: no registers), sweeps the staged tile and interpolates it along x.
 __device__ __forceinline__ void cp_async16(uint32_t dst, const void* src) {
   asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst), "l"(src) : "memory");
 }
@@ -737,86 +719,8 @@ template <int N>
 __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
 
 constexpr int kPipeStages = 2;
-
-// lines along a strided axis (z or y): tile = [n samples] x [L columns]; tiles are numbered
-// outer * x_tiles + x_tile.  float32 in, float32 out.  block = THREADS, dynamic smem =
-// n * L * (4 * kPipeStages + 8) bytes.
-constexpr int kRegSeg = 32;    // longest segment a thread keeps in registers
+constexpr int kRegSeg = 32;    // longest segment a thread of rows_pipe_interp_kernel keeps in registers
 constexpr int kRegHorizon = 20;
-
-template <int L, int THREADS>
-__global__ void __launch_bounds__(THREADS, THREADS == 256 ? 2 : 1)
-cols_pipe_kernel(const float* __restrict__ in, float* __restrict__ out, int n, int n_cols, int n_outer, ColStrides S) {
-  extern __shared__ __align__(16) uint8_t pipe_smem[];
-  constexpr int kSegs = THREADS / L;
-  double* work = reinterpret_cast<double*>(pipe_smem);                       // [n][L]
-  float* stage0 = reinterpret_cast<float*>(pipe_smem + (size_t)n * L * 8);   // kPipeStages x [n][L]
-  const uint32_t stage_a = smem_addr(stage0);
-  const int x_tiles = (n_cols + L - 1) / L;
-  const long long n_tiles = (long long)x_tiles * n_outer;
-  const bool in16 = ((((uintptr_t)in) | ((uintptr_t)(S.line_in * 4)) | ((uintptr_t)(S.outer_in * 4))) & 15) == 0;
-  const bool out16 = ((((uintptr_t)out) | ((uintptr_t)(S.line_out * 4)) | ((uintptr_t)(S.outer_out * 4))) & 15) == 0;
-
-  auto prefetch = [&](long long tile, int sidx) {
-    if (tile < n_tiles) {
-      const int xt = (int)(tile % x_tiles);
-      const long long o = tile / x_tiles;
-      const int col0 = xt * L, ncol = min(L, n_cols - col0);
-      const float* g = in + o * S.outer_in + col0;
-      const uint32_t dst = stage_a + (uint32_t)sidx * (uint32_t)(n * L * 4);
-      if (in16 && ncol == L) {
-        for (int e = threadIdx.x; e < n * (L / 4); e += THREADS) {
-          const int k = e / (L / 4), c = e - k * (L / 4);
-          cp_async16(dst + (uint32_t)((k * L + 4 * c) * 4), g + (int64_t)k * S.line_in + 4 * c);
-        }
-      } else {
-        for (int e = threadIdx.x; e < n * L; e += THREADS) {
-          const int k = e / L, j = e - k * L;
-          if (j < ncol) cp_async4(dst + (uint32_t)(e * 4), g + (int64_t)k * S.line_in + j);
-        }
-      }
-    }
-    cp_async_commit();
-  };
-
-  long long tile = blockIdx.x;
-  for (int i = 0; i < kPipeStages - 1; ++i) prefetch(tile + (long long)i * gridDim.x, i);
-  int sidx = 0;
-  const int j = threadIdx.x & (L - 1), seg = threadIdx.x / L;
-  const int len = (n + kSegs - 1) / kSegs;
-  const int k0 = seg * len, k1 = min(n, k0 + len);
-  for (; tile < n_tiles; tile += gridDim.x) {
-    // keep the ring full: the load of tile + (stages-1) strides goes into the stage freed last iteration
-    prefetch(tile + (long long)(kPipeStages - 1) * gridDim.x, (sidx + kPipeStages - 1) % kPipeStages);
-    cp_async_wait<kPipeStages - 1>();
-    __syncthreads();                                   // this tile's staged samples are visible to everybody
-    const float* st = stage0 + (size_t)sidx * n * L;
-    for (int e = threadIdx.x; e < n * L; e += THREADS) work[e] = (double)st[e] * kGain;
-    __syncthreads();
-    const int xt = (int)(tile % x_tiles);
-    const long long o = tile / x_tiles;
-    const int col0 = xt * L, ncol = min(L, n_cols - col0);
-    iir_segment_reg<kRegSeg, kRegHorizon, L>(work + j, n, k0, k1, j < ncol && k0 < k1);
-    __syncthreads();
-    float* q = out + o * S.outer_out + col0;
-    if (out16 && ncol == L) {
-      for (int e = threadIdx.x; e < n * (L / 4); e += THREADS) {
-        const int k = e / (L / 4), c = e - k * (L / 4);
-        const double* w = work + k * L + 4 * c;
-        const float4 v = make_float4((float)w[0], (float)w[1], (float)w[2], (float)w[3]);
-        *reinterpret_cast<float4*>(q + (int64_t)k * S.line_out + 4 * c) = v;
-      }
-    } else {
-      for (int e = threadIdx.x; e < n * L; e += THREADS) {
-        const int k = e / L, jj = e - k * L;
-        if (jj < ncol) q[(int64_t)k * S.line_out + jj] = (float)work[e];
-      }
-    }
-    __syncthreads();                                   // work tile and stage sidx are free again
-    sidx = (sidx + 1) % kPipeStages;
-  }
-  cp_async_wait<0>();
-}
 
 // x axis, register form (rows of <= 32 x kColLen samples): as rows_pipe_interp_kernel below, but the sweep is the
 // register-only segment of the column pass -- a thread pulls the 58-sample window of its segment out of the
@@ -886,12 +790,12 @@ rows_reg_interp_kernel(const float* __restrict__ in, int64_t in_pitch, double* _
   cp_async_wait<0>();
 }
 
-// x axis: rows of the (z,y)-filtered float32 volume (row pitch in_pitch, a multiple of 4) are staged by
-// cp.async, prefiltered in a float64 work tile and interpolated to the nx output columns at once: what leaves
-// the SM is the x-RESAMPLED float64 volume [rows][out_pitch], so the march that follows only interpolates
-// along y and z.  dynamic smem = L * (n | 1) * 8 + kPipeStages * L * in_pitch * 4 bytes.
+// x axis, rows too long for the register form: rows of the (z,y)-filtered float32 volume (row pitch in_pitch, a
+// multiple of 4) are staged by cp.async, prefiltered in a float64 work tile and interpolated to the nx output
+// columns at once: what leaves the SM is the x-RESAMPLED float64 volume [rows][out_pitch], so the march that
+// follows only interpolates along y and z.  dynamic smem = L * (n | 1) * 8 + kPipeStages * L * in_pitch * 4 bytes.
 template <int L, int THREADS>
-__global__ void __launch_bounds__(THREADS, THREADS == 256 ? 2 : 1)
+__global__ void __launch_bounds__(THREADS, 1)
 rows_pipe_interp_kernel(const float* __restrict__ in, int64_t in_pitch, double* __restrict__ out, int64_t out_pitch,
                         int n, int nx, int64_t n_rows, const Tap* __restrict__ tx) {
   extern __shared__ __align__(16) uint8_t pipe_smem[];
@@ -1103,49 +1007,8 @@ march3_tma_kernel(const __grid_constant__ CUtensorMap tmap, int xb, const ZWin* 
   }
 }
 
-// ------------------------------------------------- x axis: prefilter + interpolation in one pass
-// The rows of the (z,y)-filtered float32 volume are prefiltered along x in a shared-memory tile
-// (segment-parallel, float64) and interpolated to the nx output columns at once: what leaves the SM
-// is the x-RESAMPLED volume [rows][nx] in float64, so the march that follows only interpolates along
-// y and z and reads its planes as ready-made TMA boxes.  grid = ceil(n_rows / L), block = 256.
-template <int L>
-__global__ void __launch_bounds__(256)
-rows_prefilter_interp_kernel(const float* __restrict__ in, int64_t in_pitch, double* __restrict__ out,
-                             int64_t out_pitch, int n, int nx, int64_t n_rows, const Tap* __restrict__ tx) {
-  extern __shared__ double tile[];
-  constexpr int kSegs = 256 / L;
-  const int pitch = n | 1;
-  const int64_t row0 = (int64_t)blockIdx.x * L;
-  const int nrow = (int)min((int64_t)L, n_rows - row0);
-  const float* g = in + row0 * in_pitch;
-  for (int r = threadIdx.x >> 5; r < nrow; r += 8) {
-    const float* gr = g + (int64_t)r * in_pitch;
-#pragma unroll 4
-    for (int k = threadIdx.x & 31; k < n; k += 32) tile[r * pitch + k] = (double)gr[k] * kGain;
-  }
-  __syncthreads();
-  {
-    const int r = threadIdx.x & (L - 1), seg = threadIdx.x / L;
-    const int len = (n + kSegs - 1) / kSegs;
-    const int k0 = seg * len, k1 = min(n, k0 + len);
-    iir_segment(tile + r * pitch, n, 1, k0, k1, r < nrow && k0 < k1);
-  }
-  __syncthreads();
-  // a thread owns output columns x, x + 256, ...: its taps stay in registers while it walks the rows
-  for (int x = threadIdx.x; x < nx; x += 256) {
-    const Tap T = tx[x];
-    double* o = out + row0 * out_pitch + x;
-#pragma unroll 4
-    for (int r = 0; r < nrow; ++r) {
-      const double* row = tile + r * pitch;
-      o[(int64_t)r * out_pitch] = T.w[0] * row[T.idx[0]] + T.w[1] * row[T.idx[1]] + T.w[2] * row[T.idx[2]] +
-                                  T.w[3] * row[T.idx[3]];
-    }
-  }
-}
-
 // ------------------------------------------------- marching y/z interpolation, TMA-fed
-// Input: the x-resampled float64 volume [sz_l][sy][nxp] (rows_prefilter_interp_kernel).  A CTA owns an
+// Input: the x-resampled float64 volume [sz_l][sy][nxp] of the x pass.  A CTA owns an
 // [8 y x 64 x] output column and marches along z: each source plane's rows arrive as ONE
 // cp.async.bulk.tensor box ([ROWS y] x [64 x]) in a kYzStages-deep mbarrier ring issued by one elected
 // thread; y-interpolation reads the box in place into a 4-plane register window and every output plane
@@ -1301,15 +1164,6 @@ gather1_kernel(const float* __restrict__ src, int sy, int sx, const Tap* __restr
 
 static size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
-static int prefilter_lines() {   // lines per shared-memory tile of the segment-parallel prefilter
-  static int v = 0;
-  if (!v) {
-    const char* e = getenv("MICA_PREFILTER_LINES");
-    v = (e && atoi(e) == 32) ? 32 : 16;
-  }
-  return v;
-}
-
 static int g_force_generic = 0;   // tests: run the general kernels on shapes the fast ones would take
 
 // mica_last_resample_path: the MICA_RS_* kernel each pass of this thread's last resample launched (-1 = none)
@@ -1318,52 +1172,35 @@ static thread_local int g_resample_path[4] = {-1, -1, -1, -1};
 
 constexpr size_t kMaxTileBytes = 200 * 1024;
 
-template <typename TIn, typename TOut>
-static int launch_cols(const TIn* in, TOut* out, int n, int n_cols, int n_outer, ColStrides S, cudaStream_t st,
-                       int pass) {
-  if (n_cols <= 0 || n_outer <= 0 || n <= 0) return MICA_OK;
-  size_t per_col = (size_t)n * sizeof(double);
-  if (!g_force_generic && n >= kMinSegLine && per_col * 32 <= kMaxTileBytes) {
-    if (prefilter_lines() == 16) {
-      size_t smem = per_col * 16;
-      MICA_CUDA(cudaFuncSetAttribute(prefilter_cols_seg<TIn, TOut, 16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      prefilter_cols_seg<TIn, TOut, 16><<<dim3((n_cols + 15) / 16, n_outer), 256, smem, st>>>(in, out, n, n_cols, S);
-      g_resample_path[pass] = MICA_RS_COLS_SEG16;
-    } else {
-      size_t smem = per_col * 32;
-      MICA_CUDA(cudaFuncSetAttribute(prefilter_cols_seg<TIn, TOut, 32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      prefilter_cols_seg<TIn, TOut, 32><<<dim3((n_cols + 31) / 32, n_outer), 256, smem, st>>>(in, out, n, n_cols, S);
-      g_resample_path[pass] = MICA_RS_COLS_SEG32;
-    }
-  } else if (per_col * 32 <= kMaxTileBytes) {
-    size_t smem = per_col * 32;
-    MICA_CUDA(cudaFuncSetAttribute(prefilter_cols<TIn, TOut, 32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    prefilter_cols<TIn, TOut, 32><<<dim3((n_cols + 31) / 32, n_outer), 256, smem, st>>>(in, out, n, n_cols, S);
-    g_resample_path[pass] = MICA_RS_COLS32;
-  } else if (per_col * 8 <= kMaxTileBytes) {
-    size_t smem = per_col * 8;
-    MICA_CUDA(cudaFuncSetAttribute(prefilter_cols<TIn, TOut, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    prefilter_cols<TIn, TOut, 8><<<dim3((n_cols + 7) / 8, n_outer), 256, smem, st>>>(in, out, n, n_cols, S);
-    g_resample_path[pass] = MICA_RS_COLS8;
-  } else {
-    return set_error(MICA_ERR_INVALID, "line of %d samples too long for the shared-memory prefilter", n);
-  }
-  MICA_LAUNCH_CHECK("prefilter_cols");
-  return MICA_OK;
-}
-
-// the old all-float64 path keeps its global-memory sweep for lines that fit no tile
+// general path, z and y axes: float32 (z) or float64 (y, in place) in, float64 out; lines that fit no tile are
+// swept in global memory
 template <typename TIn>
 static int launch_cols_f64(const TIn* in, double* out, int n, int64_t line_stride, int n_cols,
                            int64_t outer_stride, int n_outer, cudaStream_t st, int pass) {
   if (n_cols <= 0 || n_outer <= 0 || n <= 0) return MICA_OK;
-  if ((size_t)n * sizeof(double) * 8 <= kMaxTileBytes) {
-    ColStrides S{line_stride, line_stride, outer_stride, outer_stride};
-    return launch_cols<TIn, double>(in, out, n, n_cols, n_outer, S, st, pass);
+  const ColStrides S{line_stride, line_stride, outer_stride, outer_stride};
+  const size_t per_col = (size_t)n * sizeof(double);
+  if (!g_force_generic && n >= kMinSegLine && per_col * 32 <= kMaxTileBytes) {
+    const size_t smem = per_col * 16;
+    MICA_CUDA(cudaFuncSetAttribute(prefilter_cols_seg<TIn, 16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    prefilter_cols_seg<TIn, 16><<<dim3((n_cols + 15) / 16, n_outer), 256, smem, st>>>(in, out, n, n_cols, S);
+    g_resample_path[pass] = MICA_RS_COLS_SEG16;
+  } else if (per_col * 32 <= kMaxTileBytes) {
+    const size_t smem = per_col * 32;
+    MICA_CUDA(cudaFuncSetAttribute(prefilter_cols<TIn, 32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    prefilter_cols<TIn, 32><<<dim3((n_cols + 31) / 32, n_outer), 256, smem, st>>>(in, out, n, n_cols, S);
+    g_resample_path[pass] = MICA_RS_COLS32;
+  } else if (per_col * 8 <= kMaxTileBytes) {
+    const size_t smem = per_col * 8;
+    MICA_CUDA(cudaFuncSetAttribute(prefilter_cols<TIn, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    prefilter_cols<TIn, 8><<<dim3((n_cols + 7) / 8, n_outer), 256, smem, st>>>(in, out, n, n_cols, S);
+    g_resample_path[pass] = MICA_RS_COLS8;
+  } else {
+    prefilter_cols_global<TIn><<<dim3((n_cols + 127) / 128, n_outer), 128, 0, st>>>(in, out, n, line_stride, n_cols,
+                                                                                    outer_stride);
+    g_resample_path[pass] = MICA_RS_COLS_GLOBAL;
   }
-  prefilter_cols_global<TIn><<<dim3((n_cols + 127) / 128, n_outer), 128, 0, st>>>(in, out, n, line_stride, n_cols, outer_stride);
-  g_resample_path[pass] = MICA_RS_COLS_GLOBAL;
-  MICA_LAUNCH_CHECK("prefilter_cols_global");
+  MICA_LAUNCH_CHECK("prefilter_cols");
   return MICA_OK;
 }
 
@@ -1374,17 +1211,10 @@ static int launch_rows(double* data, int n, int64_t n_rows, cudaStream_t st) {
   if (n <= 0 || n_rows <= 0) return MICA_OK;
   size_t per_row = (size_t)(n | 1) * sizeof(double);
   if (!g_force_generic && n >= kMinSegLine && per_row * 32 <= kMaxTileBytes) {
-    if (prefilter_lines() == 16) {
-      size_t smem = per_row * 16;
-      MICA_CUDA(cudaFuncSetAttribute(prefilter_rows_seg<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      prefilter_rows_seg<16><<<(unsigned)ceil_div64(n_rows, 16), 256, smem, st>>>(data, n, n_rows);
-      g_resample_path[kPassX] = MICA_RS_ROWS_SEG16;
-    } else {
-      size_t smem = per_row * 32;
-      MICA_CUDA(cudaFuncSetAttribute(prefilter_rows_seg<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      prefilter_rows_seg<32><<<(unsigned)ceil_div64(n_rows, 32), 256, smem, st>>>(data, n, n_rows);
-      g_resample_path[kPassX] = MICA_RS_ROWS_SEG32;
-    }
+    size_t smem = per_row * 16;
+    MICA_CUDA(cudaFuncSetAttribute(prefilter_rows_seg<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    prefilter_rows_seg<16><<<(unsigned)ceil_div64(n_rows, 16), 256, smem, st>>>(data, n, n_rows);
+    g_resample_path[kPassX] = MICA_RS_ROWS_SEG16;
   } else if (per_row * 32 <= kMaxTileBytes) {
     size_t smem = per_row * 32;
     MICA_CUDA(cudaFuncSetAttribute(prefilter_rows<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -1428,7 +1258,6 @@ extern "C" int mica_resample_force_generic(int on) {
 constexpr size_t kPipeSmemMax = 220 * 1024;
 static int64_t pitch_f32(int sx) { return ((int64_t)sx + 3) / 4 * 4; }
 static int64_t pitch_f64(int nx) { return ((int64_t)nx + 1) / 2 * 2; }
-static size_t cols_pipe_smem(int n, int L) { return (size_t)n * L * (4 * kPipeStages + 8); }
 static size_t rows_pipe_smem(int n, int L) {
   return (((size_t)L * (n | 1) * 8 + 15) & ~(size_t)15) + (size_t)kPipeStages * L * pitch_f32(n) * 4;
 }
@@ -1462,53 +1291,22 @@ extern "C" int mica_resample_slab_source_planes(int sz, int nz, int dst_z0, int 
   return MICA_OK;
 }
 
-// The register column pass (cols_reg_kernel) takes lines of any length: a CTA runs 8 segments of <= kColLen samples
-// and the grid has ceil(segments / 8) CTAs along y.
-static bool reg_cols_ok() { return !getenv("MICA_RESAMPLE_NOREG"); }
 // sz = planes of the whole map, src_nz_local = planes of the block in memory.  The choice follows the WHOLE line,
 // so that every block of a z-slab partition runs the same kernels as the whole map (the z pass numbers its segments
-// on the whole line: the same bits): no bound but the register pass's 8-plane minimum looks at the block.  Only the
-// MICA_RESAMPLE_NOREG pipe kernels hold a line in shared memory, and they cut the block into its own segments.
+// on the whole line: the same bits): no bound but the register pass's 8-plane minimum looks at the block.
 static bool fast_path_ok(int sz, int src_nz_local, int sy, int sx, int ny, int nx) {
-  if (g_force_generic || getenv("MICA_NO_TMA") || getenv("MICA_RESAMPLE_OLD")) return false;
-  if (sy > 1760 || sx > 1760) return false;              // lines the shared-memory tiles of the pipe kernels hold
+  if (g_force_generic || getenv("MICA_NO_TMA")) return false;
+  // No kernel needs this bound (the y pass, cols_reg_kernel, takes lines of any length): it only keeps maps with y
+  // lines of more than 1760 samples on the general path they have always taken.
+  if (sy > 1760) return false;
   if (sz < kMinSegLine || sy < kMinSegLine || sx < kMinSegLine) return false;             // segment-parallel sweeps
-  if (reg_cols_ok()) {
-    if (src_nz_local < 8) return false;
-  } else if (src_nz_local < kMinSegLine || cols_pipe_smem(src_nz_local, 8) > kPipeSmemMax ||
-             cols_pipe_smem(sy, 8) > kPipeSmemMax) {
-    return false;
-  }
-  if (rows_pipe_smem(sx, 8) > kPipeSmemMax) return false;
+  if (src_nz_local < 8) return false;
+  if (rows_pipe_smem(sx, 8) > kPipeSmemMax) return false;            // 8 rows in the x pass's tile: sx <= 1759
   const double zoom_y = ny > 1 ? (double)(sy - 1) / (double)(ny - 1) : 1.0;
   if ((int)floor(7.0 * zoom_y) + 5 > 16) return false;                                    // y span of an 8-row tile
   return tensor_map_encode_fn() != nullptr;
 }
 
-// persistent grid: as many CTAs as fit (shared memory bound), tiles dealt round-robin
-template <int L, int THREADS>
-static int launch_cols_pipe_t(const float* in, float* out, int n, int n_cols, int n_outer, ColStrides S, cudaStream_t st,
-                              int pass) {
-  const size_t smem = cols_pipe_smem(n, L);
-  MICA_CUDA(cudaFuncSetAttribute(cols_pipe_kernel<L, THREADS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  int per_sm = (int)((size_t)225 * 1024 / (smem + 1024));
-  per_sm = per_sm < 1 ? 1 : (per_sm > 2048 / THREADS ? 2048 / THREADS : per_sm);
-  const long long tiles = (long long)((n_cols + L - 1) / L) * n_outer;
-  long long grid = (long long)kNumSMs * per_sm;
-  if (grid > tiles) grid = tiles;
-  cols_pipe_kernel<L, THREADS><<<(unsigned)grid, THREADS, smem, st>>>(in, out, n, n_cols, n_outer, S);
-  g_resample_path[pass] =
-      L == 8 ? MICA_RS_COLS_PIPE_8_512 : THREADS == 256 ? MICA_RS_COLS_PIPE_16_256 : MICA_RS_COLS_PIPE_16_512;
-  MICA_LAUNCH_CHECK("cols_pipe_kernel");
-  return MICA_OK;
-}
-static int launch_cols_pipe(const float* in, float* out, int n, int n_cols, int n_outer, ColStrides S, cudaStream_t st,
-                            int pass) {
-  if (n_cols <= 0 || n_outer <= 0) return MICA_OK;
-  if (cols_pipe_smem(n, 16) <= 110 * 1024) return launch_cols_pipe_t<16, 256>(in, out, n, n_cols, n_outer, S, st, pass);
-  if (cols_pipe_smem(n, 16) <= kPipeSmemMax) return launch_cols_pipe_t<16, 512>(in, out, n, n_cols, n_outer, S, st, pass);
-  return launch_cols_pipe_t<8, 512>(in, out, n, n_cols, n_outer, S, st, pass);
-}
 // register-only column pass: 32 columns x 8 segments per CTA, segments of <= kColLen samples.  The line in memory
 // is samples [g0, g0 + n) of a line of ng; the segments of the GLOBAL line that hold samples [need_lo, need_hi]
 // (global numbers) are computed.
@@ -1534,19 +1332,23 @@ static int launch_cols_reg(const float* in, float* out, int n, int n_cols, int n
   return launch_cols_reg(in, out, n, n_cols, n_outer, S, st, pass, 0, n, 0, n - 1);
 }
 
+// persistent grid of the x pass: as many CTAs as fit an SM's shared memory (at most max_per_sm), no more than there
+// are tiles of L rows; the tiles are dealt round-robin
+static unsigned rows_grid(size_t smem, int max_per_sm, int64_t n_rows, int L) {
+  int per_sm = (int)((size_t)225 * 1024 / (smem + 1024));
+  per_sm = per_sm < 1 ? 1 : (per_sm > max_per_sm ? max_per_sm : per_sm);
+  const long long tiles = (n_rows + L - 1) / L;
+  const long long grid = (long long)kNumSMs * per_sm;
+  return (unsigned)(grid < tiles ? grid : tiles);
+}
 template <int L, int THREADS>
 static int launch_rows_pipe_t(const float* in, int64_t in_pitch, double* out, int64_t out_pitch, int n, int nx,
                               int64_t n_rows, const Tap* tx, cudaStream_t st) {
   const size_t smem = rows_pipe_smem(n, L);
   MICA_CUDA(cudaFuncSetAttribute(rows_pipe_interp_kernel<L, THREADS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  int per_sm = (int)((size_t)225 * 1024 / (smem + 1024));
-  per_sm = per_sm < 1 ? 1 : (per_sm > 2048 / THREADS ? 2048 / THREADS : per_sm);
-  const long long tiles = (n_rows + L - 1) / L;
-  long long grid = (long long)kNumSMs * per_sm;
-  if (grid > tiles) grid = tiles;
-  rows_pipe_interp_kernel<L, THREADS><<<(unsigned)grid, THREADS, smem, st>>>(in, in_pitch, out, out_pitch, n, nx, n_rows, tx);
-  g_resample_path[kPassX] =
-      L == 8 ? MICA_RS_ROWS_PIPE_8_512 : THREADS == 256 ? MICA_RS_ROWS_PIPE_16_256 : MICA_RS_ROWS_PIPE_16_512;
+  rows_pipe_interp_kernel<L, THREADS><<<rows_grid(smem, 2048 / THREADS, n_rows, L), THREADS, smem, st>>>(
+      in, in_pitch, out, out_pitch, n, nx, n_rows, tx);
+  g_resample_path[kPassX] = L == 8 ? MICA_RS_ROWS_PIPE_8_512 : MICA_RS_ROWS_PIPE_16_512;
   MICA_LAUNCH_CHECK("rows_pipe_interp_kernel");
   return MICA_OK;
 }
@@ -1555,27 +1357,22 @@ static int launch_rows_reg_t(const float* in, int64_t in_pitch, double* out, int
                              int64_t n_rows, const Tap* tx, cudaStream_t st) {
   const size_t smem = rows_pipe_smem(n, 16);
   MICA_CUDA(cudaFuncSetAttribute(rows_reg_interp_kernel<SEGS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  int per_sm = (int)((size_t)225 * 1024 / (smem + 1024));
-  per_sm = per_sm < 1 ? 1 : (per_sm > 512 / (16 * SEGS) ? 512 / (16 * SEGS) : per_sm);
-  const long long tiles = (n_rows + 15) / 16;
-  long long grid = (long long)kNumSMs * per_sm;
-  if (grid > tiles) grid = tiles;
   int len = (n + SEGS - 1) / SEGS;
   if (len % 2 == 0 && len < kColLen) ++len;      // odd segment length: the lanes of a row hit distinct banks
-  rows_reg_interp_kernel<SEGS><<<(unsigned)grid, 16 * SEGS, smem, st>>>(in, in_pitch, out, out_pitch, n, nx, n_rows, tx, len);
+  rows_reg_interp_kernel<SEGS><<<rows_grid(smem, 512 / (16 * SEGS), n_rows, 16), 16 * SEGS, smem, st>>>(
+      in, in_pitch, out, out_pitch, n, nx, n_rows, tx, len);
   g_resample_path[kPassX] = SEGS == 16 ? MICA_RS_ROWS_REG16 : MICA_RS_ROWS_REG32;
   MICA_LAUNCH_CHECK("rows_reg_interp_kernel");
   return MICA_OK;
 }
 
+// x pass: the register form for rows of <= 32 segments of kColLen (832 samples), the shared-memory sweep of 16 rows
+// per tile while they fit kPipeSmemMax (879 samples), of 8 rows beyond
 static int launch_rows_pipe(const float* in, int64_t in_pitch, double* out, int64_t out_pitch, int n, int nx,
                             int64_t n_rows, const Tap* tx, cudaStream_t st) {
   if (n_rows <= 0) return MICA_OK;
-  if (!getenv("MICA_RESAMPLE_NOREG") && rows_pipe_smem(n, 16) <= kPipeSmemMax) {
-    if (n <= 16 * kColLen) return launch_rows_reg_t<16>(in, in_pitch, out, out_pitch, n, nx, n_rows, tx, st);
-    if (n <= 32 * kColLen) return launch_rows_reg_t<32>(in, in_pitch, out, out_pitch, n, nx, n_rows, tx, st);
-  }
-  if (rows_pipe_smem(n, 16) <= 110 * 1024) return launch_rows_pipe_t<16, 256>(in, in_pitch, out, out_pitch, n, nx, n_rows, tx, st);
+  if (n <= 16 * kColLen) return launch_rows_reg_t<16>(in, in_pitch, out, out_pitch, n, nx, n_rows, tx, st);
+  if (n <= 32 * kColLen) return launch_rows_reg_t<32>(in, in_pitch, out, out_pitch, n, nx, n_rows, tx, st);
   if (rows_pipe_smem(n, 16) <= kPipeSmemMax) return launch_rows_pipe_t<16, 512>(in, in_pitch, out, out_pitch, n, nx, n_rows, tx, st);
   return launch_rows_pipe_t<8, 512>(in, in_pitch, out, out_pitch, n, nx, n_rows, tx, st);
 }
@@ -1631,44 +1428,23 @@ extern "C" int mica_bspline_resample_f32(const float* src, int sz, int sy, int s
     const int64_t p32 = pitch_f32(sx), p64 = pitch_f64(nx);
     float* c32 = (float*)coeff;
     double* xr = (double*)((char*)coeff + align_up((size_t)2 * src_nz_local * sy * p32 * sizeof(float), 256));
-    // axis 0 (z): columns (y, x0..x0+15) of length src_nz_local; float32 in (row pitch sx), float32 out (pitch p32)
-    const bool pipe = !getenv("MICA_RESAMPLE_NOPIPE");
-    const bool regcols = reg_cols_ok();
     float* c32b = c32 + (size_t)src_nz_local * sy * p32;      // second float32 volume (the register pass is not in place)
     const ColStrides Sz{plane, sy * p32, sx, p32}, Sy{p32, p32, sy * p32, sy * p32};
-    int rc;
     // source planes whose coefficients the z taps of this output slab can touch (global numbers, one plane of
     // margin): the whole line for a whole map; for a z-slab the planes beyond them are prefilter horizon only
     // and take no part in the y and x passes
     int c_lo, c_hi;
     needed_planes(sz, nz, dst_z0, dst_nz_local, src_z0, src_nz_local, &c_lo, &c_hi);
     const int l0 = c_lo - src_z0, cnt = c_hi - c_lo + 1;
-    if (regcols) {
-      rc = launch_cols_reg(src, c32b, src_nz_local, sx, sy, Sz, st, kPassZ, src_z0, sz, c_lo, c_hi);
-      if (rc) return rc;
-      rc = launch_cols_reg(c32b + (size_t)l0 * sy * p32, c32 + (size_t)l0 * sy * p32, sy, sx, cnt, Sy, st, kPassY);
-    } else {
-      rc = pipe ? launch_cols_pipe(src, c32, src_nz_local, sx, sy, Sz, st, kPassZ)
-                : launch_cols<float, float>(src, c32, src_nz_local, sx, sy, Sz, st, kPassZ);
-      if (rc) return rc;
-      // axis 1 (y): in place, per z plane, lines of length sy with stride p32
-      rc = pipe ? launch_cols_pipe(c32, c32, sy, sx, src_nz_local, Sy, st, kPassY)
-                : launch_cols<float, float>(c32, c32, sy, sx, src_nz_local, Sy, st, kPassY);
-    }
+    // axis 0 (z): float32 in (row pitch sx) -> c32b (row pitch p32); axis 1 (y): c32b -> c32
+    int rc = launch_cols_reg(src, c32b, src_nz_local, sx, sy, Sz, st, kPassZ, src_z0, sz, c_lo, c_hi);
+    if (rc) return rc;
+    rc = launch_cols_reg(c32b + (size_t)l0 * sy * p32, c32 + (size_t)l0 * sy * p32, sy, sx, cnt, Sy, st, kPassY);
     if (rc) return rc;
     // axis 2 (x): prefilter + interpolate the rows -> x-resampled float64 volume
-    if (pipe) {
-      rc = launch_rows_pipe(c32 + (size_t)l0 * sy * p32, p32, xr + (size_t)l0 * sy * p64, p64, sx, nx, (int64_t)cnt * sy,
-                            tx, st);
-      if (rc) return rc;
-    } else {
-      const int64_t n_rows = (int64_t)src_nz_local * sy;
-      const size_t smem = (size_t)(sx | 1) * sizeof(double) * 16;
-      MICA_CUDA(cudaFuncSetAttribute(rows_prefilter_interp_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      rows_prefilter_interp_kernel<16><<<(unsigned)ceil_div64(n_rows, 16), 256, smem, st>>>(c32, p32, xr, p64, sx, nx, n_rows, tx);
-      g_resample_path[kPassX] = MICA_RS_ROWS_PREFILTER_INTERP;
-      MICA_LAUNCH_CHECK("rows_prefilter_interp_kernel");
-    }
+    rc = launch_rows_pipe(c32 + (size_t)l0 * sy * p32, p32, xr + (size_t)l0 * sy * p64, p64, sx, nx, (int64_t)cnt * sy,
+                          tx, st);
+    if (rc) return rc;
     zwin_kernel<<<(dst_nz_local + 127) / 128, 128, 0, st>>>(tz, zw, dst_nz_local, src_nz_local);
     MICA_LAUNCH_CHECK("zwin_kernel");
     const int xt = (nx + 63) / 64, yt = (ny + 7) / 8;

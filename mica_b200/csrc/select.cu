@@ -287,12 +287,12 @@ select_sample_kernel(const float* __restrict__ x, long long n, SelectState* __re
 }
 
 __global__ void __launch_bounds__(512)
-select_hist0_guided_kernel(const float* __restrict__ x, long long n, SelectState* __restrict__ s, int allow_compacting) {
+select_hist0_guided_kernel(const float* __restrict__ x, long long n, SelectState* __restrict__ s) {
   __shared__ unsigned h[kBins];
   __shared__ unsigned long long lump[2];
   __shared__ float stage_all[16][kCompStage];
   if (s->phase0 != 1 || s->status != MICA_NORM_PENDING) return;
-  if (allow_compacting && s->comp_cap > 0) return;   // select_guided_compact_kernel serves this workspace
+  if (s->comp_cap > 0) return;   // select_guided_compact_kernel serves this workspace
   for (int i = threadIdx.x; i < kBins; i += blockDim.x) h[i] = 0;
   if (threadIdx.x < 2) lump[threadIdx.x] = 0ull;
   __syncthreads();
@@ -1034,14 +1034,13 @@ extern "C" int mica_select_hist(const float* x, int64_t n_local, void* workspace
   } else if (step == 1) {
     // which form runs is decided on the device (whether the workspace has a compact buffer): the other
     // kernels return at once.  Small inputs never have one, so they only get the histogramming form.
-    const int compacting = !getenv("MICA_SELECT_OLD_GUIDED");
-    if (compacting && n_local >= (1 << 22)) {
+    if (n_local >= (1 << 22)) {
       select_guided_compact_kernel<<<grid, 512, 0, st>>>(x, n_local, s);
       MICA_LAUNCH_CHECK("select_guided_compact_kernel");
       select_hist0_compact_kernel<<<kNumSMs * 2, 512, 0, st>>>(s);
       MICA_LAUNCH_CHECK("select_hist0_compact_kernel");
     }
-    select_hist0_guided_kernel<<<grid, 512, 0, st>>>(x, n_local, s, compacting);
+    select_hist0_guided_kernel<<<grid, 512, 0, st>>>(x, n_local, s);
     MICA_LAUNCH_CHECK("select_hist0_guided_kernel");
   } else if (step == 2) {
     // full digit-0 histogram: at most kHist0MaxPerWarp elements per warp (16-bit counters), >= two CTAs per SM

@@ -55,10 +55,20 @@ def _starts(n, n_seg):
     return list(range(0, n, length))
 
 
+def _reg_row_starts(n, n_seg):
+    """rows_reg_interp_kernel: ceil(n / n_seg) samples per segment, made odd (distinct banks) while below 26."""
+    length = -(-n // n_seg)
+    if length % 2 == 0 and length < 26:
+        length += 1
+    return list(range(0, n, length))
+
+
 # segment starts of the kernel a case targets along its long axis
 SEGS = {
     'rows_pipe_16_512': lambda n: _starts(n, 512 // 16),
     'rows_pipe_8_512': lambda n: _starts(n, 512 // 8),
+    'rows_reg32': lambda n: _reg_row_starts(n, 32),
+    'seg16': lambda n: _starts(n, 256 // 16),               # prefilter_cols_seg<16> / prefilter_rows_seg<16>
     'cols_reg': lambda n: _starts(n, -(-n // 26)),          # segments of <= kColLen = 26 samples
     'whole_line': lambda n: [],                             # one thread sweeps the whole line: edges only
 }
@@ -119,8 +129,8 @@ CASES = {
     # d: y columns longer than 64 register segments (1664 samples)
     'd_y1700_cols_reg': ((96, 1700, 96), 1.06, ('COLS_REG', 'COLS_REG', 'ROWS_REG16', 'MARCH_YZ_TMA3'),
                          ('COLS32', 'COLS8', 'ROWS32', 'GATHER3'), {1: 'cols_reg'}, {}),
-    # z lines longer than 64 register segments (1664) and than the pipe kernels' 1760-sample tile: the z pass follows
-    # the whole line, so these maps and their z-slabs run the same kernels (test_long_z_slab_ranks_reproduce_one_gpu)
+    # z lines longer than 64 register segments (1664) and than 1760 samples: the z pass follows the whole line, so
+    # these maps and their z-slabs run the same kernels (test_long_z_slab_ranks_reproduce_one_gpu)
     'z1700_cols_reg': ((1700, 96, 96), 1.06, ('COLS_REG', 'COLS_REG', 'ROWS_REG16', 'MARCH_YZ_TMA3'),
                        ('COLS8', 'COLS32', 'ROWS32', 'GATHER3'), {0: 'cols_reg'}, {}),
     'z1800_cols_reg': ((1800, 96, 96), 1.06, ('COLS_REG', 'COLS_REG', 'ROWS_REG16', 'MARCH_YZ_TMA3'),
@@ -143,7 +153,27 @@ CASES = {
                        None, {0: 'whole_line'}, {}),
     'i_x7000_global': ((8, 8, 7000), 1.2, ('COLS32', 'COLS32', 'COLS_GLOBAL', 'MARCH3_TMA3'),
                        None, {2: 'whole_line'}, {}),
+    # k: x rows of 417-832 samples: the register row pass with 32 segments per row
+    'k_rows_reg32_x700': ((96, 96, 700), 1.2, ('COLS_REG', 'COLS_REG', 'ROWS_REG32', 'MARCH_YZ_TMA3'),
+                          ('COLS32', 'COLS32', 'ROWS32', 'GATHER3'), {2: 'rows_reg32'}, {}),
+    # l: MICA_NO_TMA=1 on a y span of <= 12 rows: the register-prefetch march staging 12 rows per plane
+    'l_no_tma_march3_3': ((96, 96, 96), 1.2, ('COLS_SEG16', 'COLS_SEG16', 'ROWS_SEG16', 'MARCH3_3'),
+                          ('COLS32', 'COLS32', 'ROWS32', 'GATHER3'), {0: 'seg16', 1: 'seg16', 2: 'seg16'},
+                          {'MICA_NO_TMA': '1'}),
 }
+TRILINEAR_ROUTE = (None, None, None, 'GATHER1')   # order 1: no prefilter (test_resample_trilinear_long_rows)
+
+
+def test_every_route_id_is_pinned():
+    """Every MICA_RS_* id the header defines is the route of some test here, and every name a test expects is an id
+    there: a kernel the resample can report has a case, and an id whose kernel is gone does not linger."""
+    named = set(TRILINEAR_ROUTE)
+    for _, _, want_route, generic_route, _, _ in CASES.values():
+        named.update(want_route)
+        named.update(generic_route or ())
+    named.discard(None)
+    assert sorted(set(RS) - named) == []
+    assert sorted(named - set(RS)) == []
 
 
 @pytest.mark.parametrize('kind', ['noise', 'impulses'])
@@ -182,7 +212,7 @@ def test_resample_trilinear_long_rows(cuda, kind):
     shape, voxel, axes = (96, 96, 958), 1.2, {2: 'whole_line'}
     src, want = _reference(shape, voxel, kind, tuple(sorted(axes.items())), order=1)
     got, r = _resample(cuda, src, want.shape, order=1)
-    assert r == (None, None, None, 'GATHER1')
+    assert r == TRILINEAR_ROUTE
     assert _rel_err(got, want) <= BAR
 
 
@@ -224,7 +254,7 @@ def test_resample_slab_on_long_lines(cuda, monkeypatch, case, slabs, want_route,
 def test_long_z_slab_ranks_reproduce_one_gpu(cuda, sz):
     """The ranks of a z-slab partition (SlabPlan blocks, emulated one after the other) resample their planes to
     the same bits as one GPU resampling the whole map, also where the z line is longer than 64 register segments
-    (1664) or the pipe kernels' 1760-sample tile: the column kernel is chosen from the whole line."""
+    (1664) or 1760 samples: the column kernel is chosen from the whole line."""
     shape, voxel = (sz, 96, 96), (np.float32(1.06),) * 3
     src = torch.from_numpy(np.random.default_rng(sz).normal(size=shape).astype(np.float32)).to(cuda)
     out_shape = ops.zoom_output_shape(shape, voxel)
