@@ -90,6 +90,21 @@ int mica_bspline_resample_f32(const float* src, int sz, int sy, int sx, int src_
                               float* dst, int nz, int ny, int nx, int dst_z0, int dst_nz_local,
                               void* workspace, size_t workspace_bytes, int order, mica_stream_t stream);
 
+/* Sample types of a map, numbered as the MRC2014 modes that carry them. */
+#define MICA_DTYPE_I8 0  /* int8, MRC mode 0 */
+#define MICA_DTYPE_I16 1 /* int16, MRC mode 1 */
+#define MICA_DTYPE_F32 2 /* float32, MRC mode 2 */
+#define MICA_DTYPE_U16 6 /* uint16, MRC mode 6 */
+
+/* mica_bspline_resample_f32 for any of these types: src and dst hold samples of src_dtype / dst_dtype.  The pairs
+ * accepted are float32 -> float32 (the same call as mica_bspline_resample_f32) and an integer type -> the same
+ * integer type: scipy.ndimage.zoom on an integer array, which interpolates in float64 and stores into the input's
+ * type rounding half away from zero and saturating at the type's range (DESIGN.md D12).  Integer maps always run
+ * the float64 general path; zoom == (1,1,1) is again the caller's copy.  Any other pair is MICA_ERR_INVALID. */
+int mica_resample(const void* src, int src_dtype, int sz, int sy, int sx, int src_z0, int src_nz_local,
+                  void* dst, int dst_dtype, int nz, int ny, int nx, int dst_z0, int dst_nz_local,
+                  void* workspace, size_t workspace_bytes, int order, mica_stream_t stream);
+
 /* diagnostic: the kernel the last mica_bspline_resample_f32 call on this thread launched for one pass
  * (pass 0 = z prefilter, 1 = y prefilter, 2 = x pass, 3 = interpolation), one of the MICA_RS_* ids below;
  * -1 when that pass did not run (order 1 has no prefilter; a call that failed its argument checks ran none).
@@ -160,6 +175,28 @@ int mica_select_result_async(const void* workspace, void* host_record, mica_stre
  * Reads median / percentile from the workspace on the device; leaves y untouched
  * when the status is not MICA_NORM_OK. */
 int mica_normalize_apply_f32(const float* x, float* y, int64_t n, const void* workspace, mica_stream_t stream);
+
+/* ------------------------------------------------- R2/R3 normalisation of integer maps (DESIGN.md D12)
+ * The reference normalises an int8 / int16 / uint16 map as the integer array zoom returned: np.median is
+ * float64 (the middle element, or the mean of the two middle ones), the positives (x > med) * (x - med) are
+ * float64, np.percentile(pos, 99.9) interpolates in float64 and the normalised map is the float64 expression
+ * cast to float32.  Values have at most 16 bits, so one exact histogram of 2^8 / 2^16 bins gives every rank:
+ * mica_int_order_stats is one pass over x plus one single-CTA pick that finds the median, count(x <= med),
+ * n_pos, the percentile and the status word (MICA_NORM_*) on the device.  Single GPU only. */
+size_t mica_int_stats_workspace_bytes(void);
+/* x: device samples of `dtype` (MICA_DTYPE_I8 / I16 / U16), n of them; workspace of the size above */
+int mica_int_order_stats(const void* x, int dtype, int64_t n, void* workspace, mica_stream_t stream);
+/* synchronises the stream; any out pointer may be NULL */
+int mica_int_stats_result(const void* workspace, double* median, double* p999, int64_t* n_pos, int* norm_status,
+                          mica_stream_t stream);
+/* the same without the synchronisation: the 32-byte record {double median, double p999, int64 n_pos,
+ * int32 status, int32 0} is copied into host_record (pinned memory) in stream order */
+#define MICA_INT_STATS_RESULT_BYTES 32
+int mica_int_stats_result_async(const void* workspace, void* host_record, mica_stream_t stream);
+/* y (float32) = float32(min(m, p) / p), m = (x > med) * (x - med), evaluated in float64 exactly as NumPy does
+ * on the integer array: +0.0 at or below the median.  Leaves y untouched when the status is not MICA_NORM_OK. */
+int mica_normalize_apply_int(const void* x, int dtype, float* y, int64_t n, const void* workspace,
+                             mica_stream_t stream);
 
 /* ------------------------------------------- multi-GPU: histogram exchange over peer memory
  * No reference counterpart (the reference is single-process); replaces the NCCL all-reduce

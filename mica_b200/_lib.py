@@ -14,6 +14,8 @@ LIB_PATH = os.path.join(_HERE, 'libmica_b200.so')
 MICA_OK = 0
 ERR_NAMES = {-1: 'MICA_ERR_INVALID', -2: 'MICA_ERR_CUDA', -3: 'MICA_ERR_WORKSPACE', -4: 'MICA_ERR_NO_DEVICE'}
 NORM_OK, NORM_NO_POSITIVE, NORM_ZERO_PCTL, NORM_PENDING, NORM_PEER_TIMEOUT = 0, 1, 2, 3, 4
+DTYPE_I8, DTYPE_I16, DTYPE_F32, DTYPE_U16 = 0, 1, 2, 6      # MICA_DTYPE_*: the MRC modes of these sample types
+INT_STATS_RESULT_BYTES = 32
 SELECT_HIST_WORDS = 4096
 SELECT_PASSES = 7
 
@@ -44,6 +46,7 @@ SIGNATURES = {
     'mica_resample_force_generic': (_i, [_i]),
     'mica_resample_slab_source_planes': (_i, [_i, _i, _i, _i, _p, _p]),
     'mica_bspline_resample_f32': (_i, [_p, _i, _i, _i, _i, _i, _p, _i, _i, _i, _i, _i, _p, _sz, _i, _p]),
+    'mica_resample': (_i, [_p, _i, _i, _i, _i, _i, _i, _p, _i, _i, _i, _i, _i, _i, _p, _sz, _i, _p]),
     'mica_last_resample_path': (_i, [_i]),
     'mica_select_workspace_bytes': (_sz, []),
     'mica_select_workspace_bytes_for': (_sz, [_i64]),
@@ -58,6 +61,12 @@ SIGNATURES = {
     'mica_select_result': (_i, [_p, C.POINTER(_f), C.POINTER(_f), C.POINTER(_i64), C.POINTER(_i), _p]),
     'mica_select_result_async': (_i, [_p, _p, _p]),
     'mica_normalize_apply_f32': (_i, [_p, _p, _i64, _p, _p]),
+    'mica_int_stats_workspace_bytes': (_sz, []),
+    'mica_int_order_stats': (_i, [_p, _i, _i64, _p, _p]),
+    'mica_int_stats_result': (_i, [_p, C.POINTER(C.c_double), C.POINTER(C.c_double), C.POINTER(_i64), C.POINTER(_i),
+                                   _p]),
+    'mica_int_stats_result_async': (_i, [_p, _p, _p]),
+    'mica_normalize_apply_int': (_i, [_p, _i, _p, _i64, _p, _p]),
     'mica_normalize_force_reference_arith': (_i, [_i]),
     'mica_select_set_thresholds': (_i, [_p, _f, _f, _p]),
     'mica_peer_buffer_bytes': (_sz, []),

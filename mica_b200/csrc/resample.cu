@@ -37,6 +37,10 @@
 //   gather3_kernel       one thread per output voxel (axes under 4 samples, strong down-sampling,
 //                        mica_resample_force_generic)
 // Order 1: gather1_kernel, trilinear, one thread per output voxel, no prefilter.
+//
+// Integer maps (int8 / int16 / uint16, DESIGN.md D12) always take the general path: its z prefilter reads the
+// map's own type, and its interpolation kernels store with SciPy's integer rule (store_out).  The fast path's
+// float32 coefficients are not exact enough to round to the reference's integers.
 #include <cuda.h>
 #include <stdlib.h>
 
@@ -50,6 +54,35 @@ struct Tap {
   int idx[4];
   double w[4];
 };
+
+template <typename T>
+struct IntRange;
+template <>
+struct IntRange<int8_t> {
+  static constexpr double lo = -128.0, hi = 127.0;
+};
+template <>
+struct IntRange<int16_t> {
+  static constexpr double lo = -32768.0, hi = 32767.0;
+};
+template <>
+struct IntRange<uint16_t> {
+  static constexpr double lo = 0.0, hi = 65535.0;
+};
+
+// SciPy's store of an interpolated float64 value into the output array: float32 rounds to nearest; an integer
+// type rounds half away from zero (t > 0 ? t + 0.5 : t - 0.5, truncated toward zero) and saturates at the
+// type's range -- the cubic spline overshoots the input range on noisy maps
+template <typename T>
+__device__ __forceinline__ void store_out(T* p, double v) {
+  if constexpr (std::is_same<T, float>::value) {
+    st_stream(p, (float)v);
+  } else {
+    double t = v > 0.0 ? v + 0.5 : v - 0.5;
+    t = t < IntRange<T>::lo ? IntRange<T>::lo : (t > IntRange<T>::hi ? IntRange<T>::hi : t);
+    *p = (T)(int)t;
+  }
+}
 
 __device__ __forceinline__ int mirror_index(long idx, int len) {
   // SciPy ni_interpolation.c edge handling for NI_EXTEND_MIRROR-like taps
@@ -393,9 +426,10 @@ __global__ void prefilter_cols_global(const TIn* __restrict__ in, double* __rest
 
 // ------------------------------------------------------------------- gather
 // grid = (ceil(nx/128), ny, nz_local); one output voxel per thread
+template <typename TOut>
 __global__ void __launch_bounds__(128)
 gather3_kernel(const double* __restrict__ c, int sy, int sx, const Tap* __restrict__ tz,
-               const Tap* __restrict__ ty, const Tap* __restrict__ tx, float* __restrict__ dst, int ny,
+               const Tap* __restrict__ ty, const Tap* __restrict__ tx, TOut* __restrict__ dst, int ny,
                int nx) {
   int x = blockIdx.x * blockDim.x + threadIdx.x;
   if (x >= nx) return;
@@ -418,7 +452,7 @@ gather3_kernel(const double* __restrict__ c, int sy, int sx, const Tap* __restri
     }
     acc += Tz.w[l] * accy;
   }
-  st_stream(dst + ((int64_t)z * ny + y) * nx + x, (float)acc);
+  store_out(dst + ((int64_t)z * ny + y) * nx + x, acc);
 }
 
 
@@ -455,10 +489,10 @@ __global__ void zwin_kernel(const Tap* __restrict__ tz, ZWin* __restrict__ zw, i
 }
 
 // grid = (ceil(nx / 64), ceil(ny / 8), z chunks), block = 256.  NI * 4 = source rows staged per plane.
-template <int NI>
+template <int NI, typename TOut>
 __global__ void __launch_bounds__(256)
 march3_kernel(const double* __restrict__ c, int sy, int sx, const ZWin* __restrict__ zw,
-              const Tap* __restrict__ ty, const Tap* __restrict__ tx, float* __restrict__ dst, int ny, int nx,
+              const Tap* __restrict__ ty, const Tap* __restrict__ tx, TOut* __restrict__ dst, int ny, int nx,
               int nz_local, int zchunk) {
   constexpr int TX = 64, TY = 8, ROWS = NI * 4;
   __shared__ double A[2][ROWS][TX];
@@ -542,7 +576,7 @@ march3_kernel(const double* __restrict__ c, int sy, int sx, const ZWin* __restri
       for (int o = 0; o < 2; ++o) {
         const int y = y0 + lr + 4 * o;
         const double acc = Wz.w[0] * v[o][0] + Wz.w[1] * v[o][1] + Wz.w[2] * v[o][2] + Wz.w[3] * v[o][3];
-        if (x < nx && y < ny) st_stream(dst + ((int64_t)zc * ny + y) * nx + x, (float)acc);
+        if (x < nx && y < ny) store_out(dst + ((int64_t)zc * ny + y) * nx + x, acc);
       }
       ++zc;
       if (zc < z_end) next_emit = zw[zc].base + 3;
@@ -856,10 +890,11 @@ rows_pipe_interp_kernel(const float* __restrict__ in, int64_t in_pitch, double* 
 }
 
 // grid = (ceil(nx / 64), ceil(ny / 8), z chunks), block = 256; dynamic smem = ring + 1 KB alignment slack
-template <int NI>
-__global__ void __launch_bounds__(256, 3)
+// Integer outputs: 2 CTAs per SM, so that the saturating store fits the register budget without spilling.
+template <int NI, typename TOut>
+__global__ void __launch_bounds__(256, std::is_same<TOut, float>::value ? 3 : 2)
 march3_tma_kernel(const __grid_constant__ CUtensorMap tmap, int xb, const ZWin* __restrict__ zw,
-                  const Tap* __restrict__ ty, const Tap* __restrict__ tx, float* __restrict__ dst, int ny, int nx,
+                  const Tap* __restrict__ ty, const Tap* __restrict__ tx, TOut* __restrict__ dst, int ny, int nx,
                   int nz_local, int zchunk) {
   constexpr int TX = 64, TY = 8, ROWS = NI * 4;
   extern __shared__ uint8_t march_smem[];
@@ -954,7 +989,7 @@ march3_tma_kernel(const __grid_constant__ CUtensorMap tmap, int xb, const ZWin* 
   };
   // running output pointers (advance one plane per emitted z)
   const int64_t out_plane = (int64_t)ny * nx;
-  float* outp[2];
+  TOut* outp[2];
   bool outok[2];
 #pragma unroll
   for (int o = 0; o < 2; ++o) {
@@ -993,7 +1028,7 @@ march3_tma_kernel(const __grid_constant__ CUtensorMap tmap, int xb, const ZWin* 
 #pragma unroll
       for (int o = 0; o < 2; ++o) {
         const double acc = Wz.w[0] * v[o][0] + Wz.w[1] * v[o][1] + Wz.w[2] * v[o][2] + Wz.w[3] * v[o][3];
-        if (outok[o]) st_stream(outp[o], (float)acc);
+        if (outok[o]) store_out(outp[o], acc);
         outp[o] += out_plane;
       }
       ++zc;
@@ -1135,9 +1170,10 @@ march_yz_tma_kernel(const __grid_constant__ CUtensorMap tmap, const ZWin* __rest
   if (p + 2 <= p_last) step(I2(), p + 2);
 }
 
+template <typename TIn, typename TOut>
 __global__ void __launch_bounds__(128)
-gather1_kernel(const float* __restrict__ src, int sy, int sx, const Tap* __restrict__ tz,
-               const Tap* __restrict__ ty, const Tap* __restrict__ tx, float* __restrict__ dst, int ny,
+gather1_kernel(const TIn* __restrict__ src, int sy, int sx, const Tap* __restrict__ tz,
+               const Tap* __restrict__ ty, const Tap* __restrict__ tx, TOut* __restrict__ dst, int ny,
                int nx) {
   int x = blockIdx.x * blockDim.x + threadIdx.x;
   if (x >= nx) return;
@@ -1149,17 +1185,17 @@ gather1_kernel(const float* __restrict__ src, int sy, int sx, const Tap* __restr
   double acc = 0.0;
 #pragma unroll
   for (int l = 0; l < 2; ++l) {
-    const float* pz = src + (int64_t)Tz.idx[l] * plane;
+    const TIn* pz = src + (int64_t)Tz.idx[l] * plane;
     double accy = 0.0;
 #pragma unroll
     for (int m = 0; m < 2; ++m) {
-      const float* row = pz + (int64_t)Ty.idx[m] * sx;
+      const TIn* row = pz + (int64_t)Ty.idx[m] * sx;
       double r = Tx.w[0] * (double)row[Tx.idx[0]] + Tx.w[1] * (double)row[Tx.idx[1]];
       accy += Ty.w[m] * r;
     }
     acc += Tz.w[l] * accy;
   }
-  st_stream(dst + ((int64_t)z * ny + y) * nx + x, (float)acc);
+  store_out(dst + ((int64_t)z * ny + y) * nx + x, acc);
 }
 
 static size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
@@ -1389,11 +1425,13 @@ extern "C" size_t mica_resample_workspace_bytes(int src_nz_local, int sy, int sx
   return taps + coeff + 512;
 }
 
-extern "C" int mica_bspline_resample_f32(const float* src, int sz, int sy, int sx, int src_z0, int src_nz_local,
-                                         float* dst, int nz, int ny, int nx, int dst_z0, int dst_nz_local,
-                                         void* workspace, size_t workspace_bytes, int order, mica_stream_t stream) {
+// T = the map's sample type, in and out.  Integer maps never take the fast path (see the file header).
+template <typename T>
+static int resample_impl(const T* src, int sz, int sy, int sx, int src_z0, int src_nz_local, T* dst, int nz, int ny,
+                         int nx, int dst_z0, int dst_nz_local, void* workspace, size_t workspace_bytes, int order,
+                         mica_stream_t stream) {
+  constexpr bool kF32 = std::is_same<T, float>::value;
   cudaStream_t st = (cudaStream_t)stream;
-  for (int& k : g_resample_path) k = -1;
   MICA_REQUIRE(src && dst && workspace, "null pointer");
   MICA_REQUIRE(order == 3 || order == 1, "order must be 3 or 1 (got %d)", order);
   MICA_REQUIRE(sz > 0 && sy > 0 && sx > 0 && nz > 0 && ny > 0 && nx > 0, "empty shape");
@@ -1422,7 +1460,9 @@ extern "C" int mica_bspline_resample_f32(const float* src, int sz, int sy, int s
   MICA_LAUNCH_CHECK("taps_kernel(x)");
 
   dim3 grid((nx + 127) / 128, ny, dst_nz_local);
-  if (order == 3 && fast_path_ok(sz, src_nz_local, sy, sx, ny, nx)) {
+  if (kF32 && order == 3 && fast_path_ok(sz, src_nz_local, sy, sx, ny, nx)) {
+    const float* srcf = (const float*)src;
+    float* dstf = (float*)dst;
     const int64_t plane = (int64_t)sy * sx;
     MICA_REQUIRE(plane <= 0x7fffffffLL && src_nz_local <= 65535 && sy <= 65535, "source plane too large");
     const int64_t p32 = pitch_f32(sx), p64 = pitch_f64(nx);
@@ -1437,7 +1477,7 @@ extern "C" int mica_bspline_resample_f32(const float* src, int sz, int sy, int s
     needed_planes(sz, nz, dst_z0, dst_nz_local, src_z0, src_nz_local, &c_lo, &c_hi);
     const int l0 = c_lo - src_z0, cnt = c_hi - c_lo + 1;
     // axis 0 (z): float32 in (row pitch sx) -> c32b (row pitch p32); axis 1 (y): c32b -> c32
-    int rc = launch_cols_reg(src, c32b, src_nz_local, sx, sy, Sz, st, kPassZ, src_z0, sz, c_lo, c_hi);
+    int rc = launch_cols_reg(srcf, c32b, src_nz_local, sx, sy, Sz, st, kPassZ, src_z0, sz, c_lo, c_hi);
     if (rc) return rc;
     rc = launch_cols_reg(c32b + (size_t)l0 * sy * p32, c32 + (size_t)l0 * sy * p32, sy, sx, cnt, Sy, st, kPassY);
     if (rc) return rc;
@@ -1468,19 +1508,19 @@ extern "C" int mica_bspline_resample_f32(const float* src, int sz, int sy, int s
     const size_t smem = (size_t)kYzStages * rows * 64 * 8 + 128;
     if (rows == 12) {
       MICA_CUDA(cudaFuncSetAttribute(march_yz_tma_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      march_yz_tma_kernel<3><<<mgrid, 256, smem, st>>>(tmap, zw, ty, dst, ny, nx, dst_nz_local, zchunk);
+      march_yz_tma_kernel<3><<<mgrid, 256, smem, st>>>(tmap, zw, ty, dstf, ny, nx, dst_nz_local, zchunk);
       g_resample_path[kPassInterp] = MICA_RS_MARCH_YZ_TMA3;
     } else {
       MICA_CUDA(cudaFuncSetAttribute(march_yz_tma_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      march_yz_tma_kernel<4><<<mgrid, 256, smem, st>>>(tmap, zw, ty, dst, ny, nx, dst_nz_local, zchunk);
+      march_yz_tma_kernel<4><<<mgrid, 256, smem, st>>>(tmap, zw, ty, dstf, ny, nx, dst_nz_local, zchunk);
       g_resample_path[kPassInterp] = MICA_RS_MARCH_YZ_TMA4;
     }
     MICA_LAUNCH_CHECK("march_yz_tma_kernel");
   } else if (order == 3) {
     const int64_t plane = (int64_t)sy * sx;
     MICA_REQUIRE(plane <= 0x7fffffffLL && src_nz_local <= 65535, "source plane too large");
-    // axis 0 (z): lines of length src_nz_local, stride plane; reads float32, writes float64
-    int rc = launch_cols_f64<float>(src, coeff, src_nz_local, plane, (int)plane, 0, 1, st, kPassZ);
+    // axis 0 (z): lines of length src_nz_local, stride plane; reads the map's type, writes float64
+    int rc = launch_cols_f64<T>(src, coeff, src_nz_local, plane, (int)plane, 0, 1, st, kPassZ);
     if (rc) return rc;
     // axis 1 (y): per z plane, lines of length sy, stride sx
     rc = launch_cols_f64<double>(coeff, coeff, sy, sx, sx, plane, src_nz_local, st, kPassY);
@@ -1523,36 +1563,62 @@ extern "C" int mica_bspline_resample_f32(const float* src, int sz, int sy, int s
       if (tma_ok) {
         const size_t smem = (size_t)kMarchStages * (((size_t)rows * xb + 15) / 16 * 16) * 8 + 128;
         if (rows == 12) {
-          MICA_CUDA(cudaFuncSetAttribute(march3_tma_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-          march3_tma_kernel<3><<<mgrid, 256, smem, st>>>(tmap, xb, zw, ty, tx, dst, ny, nx, dst_nz_local, zchunk);
+          MICA_CUDA(cudaFuncSetAttribute(march3_tma_kernel<3, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+          march3_tma_kernel<3, T><<<mgrid, 256, smem, st>>>(tmap, xb, zw, ty, tx, dst, ny, nx, dst_nz_local, zchunk);
           g_resample_path[kPassInterp] = MICA_RS_MARCH3_TMA3;
         } else {
-          MICA_CUDA(cudaFuncSetAttribute(march3_tma_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-          march3_tma_kernel<4><<<mgrid, 256, smem, st>>>(tmap, xb, zw, ty, tx, dst, ny, nx, dst_nz_local, zchunk);
+          MICA_CUDA(cudaFuncSetAttribute(march3_tma_kernel<4, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+          march3_tma_kernel<4, T><<<mgrid, 256, smem, st>>>(tmap, xb, zw, ty, tx, dst, ny, nx, dst_nz_local, zchunk);
           g_resample_path[kPassInterp] = MICA_RS_MARCH3_TMA4;
         }
         MICA_LAUNCH_CHECK("march3_tma_kernel");
       } else {
         if (span_y <= 12) {
-          march3_kernel<3><<<mgrid, 256, 0, st>>>(coeff, sy, sx, zw, ty, tx, dst, ny, nx, dst_nz_local, zchunk);
+          march3_kernel<3, T><<<mgrid, 256, 0, st>>>(coeff, sy, sx, zw, ty, tx, dst, ny, nx, dst_nz_local, zchunk);
           g_resample_path[kPassInterp] = MICA_RS_MARCH3_3;
         } else {
-          march3_kernel<4><<<mgrid, 256, 0, st>>>(coeff, sy, sx, zw, ty, tx, dst, ny, nx, dst_nz_local, zchunk);
+          march3_kernel<4, T><<<mgrid, 256, 0, st>>>(coeff, sy, sx, zw, ty, tx, dst, ny, nx, dst_nz_local, zchunk);
           g_resample_path[kPassInterp] = MICA_RS_MARCH3_4;
         }
         MICA_LAUNCH_CHECK("march3_kernel");
       }
     } else {
-      gather3_kernel<<<grid, 128, 0, st>>>(coeff, sy, sx, tz, ty, tx, dst, ny, nx);
+      gather3_kernel<T><<<grid, 128, 0, st>>>(coeff, sy, sx, tz, ty, tx, dst, ny, nx);
       g_resample_path[kPassInterp] = MICA_RS_GATHER3;
       MICA_LAUNCH_CHECK("gather3_kernel");
     }
   } else {
-    gather1_kernel<<<grid, 128, 0, st>>>(src, sy, sx, tz, ty, tx, dst, ny, nx);
+    gather1_kernel<T, T><<<grid, 128, 0, st>>>(src, sy, sx, tz, ty, tx, dst, ny, nx);
     g_resample_path[kPassInterp] = MICA_RS_GATHER1;
     MICA_LAUNCH_CHECK("gather1_kernel");
   }
   return MICA_OK;
+}
+
+extern "C" int mica_resample(const void* src, int src_dtype, int sz, int sy, int sx, int src_z0, int src_nz_local,
+                             void* dst, int dst_dtype, int nz, int ny, int nx, int dst_z0, int dst_nz_local,
+                             void* workspace, size_t workspace_bytes, int order, mica_stream_t stream) {
+  for (int& k : g_resample_path) k = -1;
+  MICA_REQUIRE(src_dtype == dst_dtype, "resample writes the source's own type (src dtype %d, dst dtype %d)", src_dtype,
+               dst_dtype);
+#define MICA_RESAMPLE_AS(T)                                                                                          \
+  resample_impl<T>((const T*)src, sz, sy, sx, src_z0, src_nz_local, (T*)dst, nz, ny, nx, dst_z0, dst_nz_local,     \
+                   workspace, workspace_bytes, order, stream)
+  switch (src_dtype) {
+    case MICA_DTYPE_F32: return MICA_RESAMPLE_AS(float);
+    case MICA_DTYPE_I8: return MICA_RESAMPLE_AS(int8_t);
+    case MICA_DTYPE_I16: return MICA_RESAMPLE_AS(int16_t);
+    case MICA_DTYPE_U16: return MICA_RESAMPLE_AS(uint16_t);
+    default: return set_error(MICA_ERR_INVALID, "unknown dtype code %d", src_dtype);
+  }
+#undef MICA_RESAMPLE_AS
+}
+
+extern "C" int mica_bspline_resample_f32(const float* src, int sz, int sy, int sx, int src_z0, int src_nz_local,
+                                         float* dst, int nz, int ny, int nx, int dst_z0, int dst_nz_local,
+                                         void* workspace, size_t workspace_bytes, int order, mica_stream_t stream) {
+  return mica_resample(src, MICA_DTYPE_F32, sz, sy, sx, src_z0, src_nz_local, dst, MICA_DTYPE_F32, nz, ny, nx, dst_z0,
+                       dst_nz_local, workspace, workspace_bytes, order, stream);
 }
 
 extern "C" int mica_last_resample_path(int pass) { return pass >= 0 && pass < 4 ? g_resample_path[pass] : -1; }

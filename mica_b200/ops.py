@@ -94,27 +94,38 @@ def resample_slab_source_planes(sz: int, nz: int, dst_z0: int, dst_nz_local: int
     return int(lo.value), int(hi.value)
 
 
+#: sample types of the maps resample / normalize take -> MICA_DTYPE_* code
+MAP_DTYPES = {torch.float32: _lib.DTYPE_F32, torch.int8: _lib.DTYPE_I8, torch.int16: _lib.DTYPE_I16,
+              torch.uint16: _lib.DTYPE_U16}
+#: integer maps (MRC modes 0, 1, 6): rounded resample, float64 statistics (DESIGN.md D12)
+INT_DTYPES = (torch.int8, torch.int16, torch.uint16)
+
+
 @device_guard
 def resample(src: torch.Tensor, out_shape, order: int = 3, *, src_z0: int = 0, src_shape=None,
              dst_z0: int = 0, dst_nz_local=None, out: torch.Tensor | None = None) -> torch.Tensor:
     """Cubic B-spline (order=3) / trilinear (order=1) resample of ``src`` (sz,sy,sx) to
     the global shape ``out_shape``.  Slab form: ``src`` holds global planes
     [src_z0, src_z0+len) of a (src_shape) volume; planes [dst_z0, dst_z0+dst_nz_local)
-    of the output are produced."""
-    p_src = _dev(src, torch.float32, 'src')
+    of the output are produced.  ``src`` is float32, int8, int16 or uint16 and the output has its
+    type: an integer map is resampled in float64 and rounded as scipy.ndimage.zoom stores into an
+    integer array (half away from zero, saturating; DESIGN.md D12)."""
+    dt = src.dtype if isinstance(src, torch.Tensor) and src.dtype in MAP_DTYPES else torch.float32
+    p_src = _dev(src, dt, 'src')
+    code = MAP_DTYPES[dt]
     sz_l, sy, sx = src.shape
     sz = int(src_shape[0]) if src_shape is not None else sz_l
     nz, ny, nx = (int(v) for v in out_shape)
     nzl = nz - dst_z0 if dst_nz_local is None else int(dst_nz_local)
     if out is None:
-        out = torch.empty((nzl, ny, nx), dtype=torch.float32, device=src.device)
-    p_out = _dev(out, torch.float32, 'out')
+        out = torch.empty((nzl, ny, nx), dtype=dt, device=src.device)
+    p_out = _dev(out, dt, 'out')
     if tuple(out.shape) != (nzl, ny, nx):
         raise _lib.MicaError(f'out has shape {tuple(out.shape)}, expected {(nzl, ny, nx)}')
     nbytes = lib.mica_resample_workspace_bytes(sz_l, sy, sx, nz, ny, nx, order)
     ws = torch.empty(nbytes, dtype=torch.uint8, device=src.device)
-    check(lib.mica_bspline_resample_f32(p_src, sz, sy, sx, src_z0, sz_l, p_out, nz, ny, nx, dst_z0, nzl,
-                                        C.c_void_p(ws.data_ptr()), nbytes, order, _stream()), 'resample')
+    check(lib.mica_resample(p_src, code, sz, sy, sx, src_z0, sz_l, p_out, code, nz, ny, nx, dst_z0, nzl,
+                            C.c_void_p(ws.data_ptr()), nbytes, order, _stream()), 'resample')
     return out
 
 
@@ -214,9 +225,83 @@ class OrderStats:
         return out
 
 
+class IntOrderStats:
+    """Device-resident state of the exact order statistics of an integer map (int8 / int16 / uint16, DESIGN.md
+    D12): one histogram pass and one pick give the float64 median and 99.9 percentile NumPy computes on the
+    integer array.  Single GPU only."""
+
+    RESULT_BYTES = _lib.INT_STATS_RESULT_BYTES
+
+    def __init__(self, device):
+        self.device = torch.device(device)
+        if self.device.type != 'cuda':
+            raise _lib.MicaError(f'IntOrderStats needs a CUDA device, got {self.device} (mica_b200 has no CPU fallback)')
+        with torch.cuda.device(self.device):
+            self.ws = torch.empty(lib.mica_int_stats_workspace_bytes(), dtype=torch.uint8, device=self.device)
+        self._p = C.c_void_p(self.ws.data_ptr())
+
+    @staticmethod
+    def _int_map(x, name):
+        if isinstance(x, torch.Tensor) and x.dtype not in INT_DTYPES:
+            raise _lib.MicaError(f'{name} must be int8, int16 or uint16, got {x.dtype}')
+        dt = x.dtype if isinstance(x, torch.Tensor) else torch.int16
+        return _dev(x, dt, name), MAP_DTYPES[dt]
+
+    @device_guard
+    def run(self, x: torch.Tensor):
+        p_x, code = self._int_map(x, 'x')
+        check(lib.mica_int_order_stats(p_x, code, x.numel(), self._p, _stream()), 'int_order_stats')
+        return self
+
+    @device_guard
+    def result(self):
+        """(median, p999, n_pos, status), median and p999 as Python floats (float64) -- synchronises the stream."""
+        med, p, npos, status = C.c_double(), C.c_double(), C.c_int64(), C.c_int()
+        check(lib.mica_int_stats_result(self._p, C.byref(med), C.byref(p), C.byref(npos), C.byref(status),
+                                        _stream()), 'int_stats_result')
+        return float(med.value), float(p.value), int(npos.value), int(status.value)
+
+    @device_guard
+    def result_async(self, record: torch.Tensor | None = None) -> torch.Tensor:
+        """Enqueue the copy of the 32-byte result record into pinned host memory (no synchronisation);
+        decode it with ``IntOrderStats.decode`` once the stream has passed this point."""
+        if record is None:
+            record = torch.zeros(self.RESULT_BYTES, dtype=torch.uint8).pin_memory()
+        check(lib.mica_int_stats_result_async(self._p, C.c_void_p(record.data_ptr()), _stream()),
+              'int_stats_result_async')
+        return record
+
+    @staticmethod
+    def decode(record: torch.Tensor):
+        """(median, p999, n_pos, status) from a result record."""
+        raw = record.numpy()
+        med, p = raw[0:16].view(np.float64)
+        return float(med), float(p), int(raw[16:24].view(np.int64)[0]), int(raw[24:28].view(np.int32)[0])
+
+    @device_guard
+    def apply(self, x: torch.Tensor, out: torch.Tensor | None = None) -> torch.Tensor:
+        """The float32 normalised map of ``x`` (a new tensor unless ``out`` is given; left as it was when the
+        status is not NORM_OK)."""
+        p_x, code = self._int_map(x, 'x')
+        if out is None:
+            out = torch.empty(x.shape, dtype=torch.float32, device=x.device)
+        p_y = _dev(out, torch.float32, 'out')
+        if out.numel() != x.numel():
+            raise _lib.MicaError(f'out has {out.numel()} elements, x {x.numel()}')
+        check(lib.mica_normalize_apply_int(p_x, code, p_y, x.numel(), self._p, _stream()), 'normalize_apply_int')
+        return out
+
+
 @device_guard
 def normalize(x: torch.Tensor, inplace: bool = False):
-    """utils/preprocessing.py:122-133 on the device.  Returns (normalised, OrderStats)."""
+    """utils/preprocessing.py:122-133 on the device.  Returns (normalised, OrderStats).  An integer map
+    (int8 / int16 / uint16) gets the float64 statistics of ``IntOrderStats`` and a new float32 volume:
+    ``inplace=True`` raises for it."""
+    if isinstance(x, torch.Tensor) and x.dtype in INT_DTYPES:
+        if inplace:
+            raise _lib.MicaError(f'normalize: a {x.dtype} map cannot be normalised in place (the result is float32)')
+        st = IntOrderStats(x.device).run(x)
+        return st.apply(x, torch.zeros(x.shape, dtype=torch.float32, device=x.device)), st
     st = OrderStats(x.device).run(x)
     return st.apply(x, x if inplace else None), st
 

@@ -211,8 +211,9 @@ class MapPipeline:
         self.header = MapHeader()
         self.normalized = None          # [nz,ny,nx] float32, device
         self.af3 = None                 # [24,nz,ny,nx] float32, device (None -> zero AF3 features)
-        self.stats = None
+        self.stats = None               # OrderStats, or IntOrderStats for an integer map
         self._stats = None
+        self._int_stats = None
         self.norm_status = None
         self._x, self._af, self._nz = [None, None], [None, None], [None, None]
         self.timer = _no_timer      # bench.py swaps in a StageTimer
@@ -266,7 +267,9 @@ class MapPipeline:
         """utils/preprocessing.py:98-133 on the device.  Returns True on success; on the
         reference's two failure modes (:152-157) returns False and leaves ``normalized`` None.
         ``defer_status=True`` skips the host read-back (one stream sync) -- the caller then
-        calls ``check_status()`` once everything is enqueued."""
+        calls ``check_status()`` once everything is enqueued.  An int8 / int16 / uint16 ``src`` is
+        resampled into its own type and normalised in float64 into a new float32 volume (D12); ``median``
+        and ``p999`` are then Python floats."""
         if header is not None:
             self.header = header
         zf = zoom_factors(self.header.voxel_size, self.target_voxel_size)
@@ -276,10 +279,16 @@ class MapPipeline:
                 res = src.clone()
             else:
                 res = ops.resample(src, out_shape, order=self.order)
-        with self.timer('order_stats'):
-            self.stats = self._order_stats().run(res)
-        with self.timer('normalize_apply'):
-            self.normalized = self.stats.apply(res, res)       # in place: the resampled map is not kept
+        if res.dtype in ops.INT_DTYPES:                       # integer map: float64 statistics (D12)
+            with self.timer('order_stats'):
+                self.stats = self._int_order_stats().run(res)
+            with self.timer('normalize_apply'):
+                self.normalized = self.stats.apply(res)        # a new float32 volume
+        else:
+            with self.timer('order_stats'):
+                self.stats = self._order_stats().run(res)
+            with self.timer('normalize_apply'):
+                self.normalized = self.stats.apply(res, res)   # in place: the resampled map is not kept
         self.norm_status = None
         return True if defer_status else self.check_status()
 
@@ -290,6 +299,11 @@ class MapPipeline:
         if self._stats is None:
             self._stats = ops.OrderStats(self.device)
         return self._stats
+
+    def _int_order_stats(self):
+        if self._int_stats is None:
+            self._int_stats = ops.IntOrderStats(self.device)
+        return self._int_stats
 
     @_on_device
     def check_status(self):
@@ -520,10 +534,10 @@ class MapPipeline:
     def finish(self):
         """Wait for every ``run(..., defer_check=True)`` issued so far and raise if one of them failed."""
         pending, self._deferred = self._deferred, []
-        for rec, af, ev in pending:
+        for rec, af, ev, decode in pending:
             ev.synchronize()
             self._pinned_free.append((rec, af))
-            med, p, npos, status = ops.OrderStats.decode(rec)
+            med, p, npos, status = decode(rec)
             self.norm_status, self.median, self.p999, self.n_pos = status, med, p, npos
             if status != NORM_OK:
                 raise MicaError(f'normalisation failed (status {status})')
@@ -564,7 +578,7 @@ class MapPipeline:
                 af[:1].copy_(self._af3_status, non_blocking=True)
             ev = torch.cuda.Event()
             ev.record(torch.cuda.current_stream(self.device))
-            self._deferred.append((rec, af, ev))
+            self._deferred.append((rec, af, ev, self.stats.decode))
             return vols
         # one host read-back for the whole path (the reference reports these per stage)
         if not self.check_status():

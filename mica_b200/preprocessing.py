@@ -21,24 +21,32 @@ from .pipeline import MapHeader, shared_pipeline
 
 
 _STAGING = {}
+#: integer payloads (MRC modes 0, 1, 6) go to the device as they are
+_INT_UPLOAD = {np.dtype(np.int8): torch.int8, np.dtype(np.int16): torch.int16, np.dtype(np.uint16): torch.uint16}
 
 
 def upload_map(data: np.ndarray, device) -> torch.Tensor:
     """Host map (typically the copy-on-write memory map ``mrc.read_mrc`` returns) -> device tensor: the
     planes are copied into a reused pinned staging buffer by a few threads (NumPy releases the GIL) and
-    every finished chunk goes to the GPU at once, instead of one pageable copy of the whole map."""
+    every finished chunk goes to the GPU at once, instead of one pageable copy of the whole map.
+    int8 / int16 / uint16 maps keep their type (an int16 map crosses PCIe at half the float32 bytes);
+    everything else becomes float32."""
     from concurrent.futures import ThreadPoolExecutor
     data = np.asarray(data)
     dev = torch.device(device)
     n = data.size
-    out = torch.empty(data.shape, dtype=torch.float32, device=dev)
-    if n < (1 << 22) or data.dtype != np.float32 or not data.flags.c_contiguous:
-        out.copy_(torch.from_numpy(np.ascontiguousarray(data, dtype=np.float32)))
+    tdt = _INT_UPLOAD.get(data.dtype, torch.float32)
+    ndt = data.dtype if tdt is not torch.float32 else np.dtype(np.float32)
+    out = torch.empty(data.shape, dtype=tdt, device=dev)
+    if n < (1 << 22) or data.dtype != ndt or not data.flags.c_contiguous:
+        out.copy_(torch.from_numpy(np.ascontiguousarray(data, dtype=ndt)))
         return out
-    stage = _STAGING.get('map')
-    if stage is None or stage.numel() < n:
-        stage = _STAGING['map'] = torch.empty(n, dtype=torch.float32).pin_memory()
-    flat_src, flat_dst, flat_out = data.reshape(-1), stage.numpy(), out.view(-1)
+    nbytes = n * ndt.itemsize
+    stage = _STAGING.get('map')                          # bytes: one buffer serves maps of every type
+    if stage is None or stage.numel() < nbytes:
+        stage = _STAGING['map'] = torch.empty(nbytes, dtype=torch.uint8).pin_memory()
+    typed = stage[:nbytes].view(tdt)
+    flat_src, flat_dst, flat_out = data.reshape(-1), stage.numpy()[:nbytes].view(ndt), out.view(-1)
     chunks = 8
     bounds = [n * c // chunks for c in range(chunks + 1)]
     with torch.cuda.device(dev):
@@ -49,7 +57,7 @@ def upload_map(data: np.ndarray, device) -> torch.Tensor:
             return c
         with ThreadPoolExecutor(4) as pool:
             for c in pool.map(fill, range(chunks)):
-                flat_out[bounds[c]:bounds[c + 1]].copy_(stage[bounds[c]:bounds[c + 1]], non_blocking=True)
+                flat_out[bounds[c]:bounds[c + 1]].copy_(typed[bounds[c]:bounds[c + 1]], non_blocking=True)
     return out
 
 
@@ -102,10 +110,9 @@ class DataPreprocessor:
         success = False
         try:
             m = mrc.read_mrc(self.map_path)
-            if m.mode != 2:
-                # the reference would run scipy.zoom and the normalisation on the integer array (rounded
-                # resampling, float64 statistics): a different arithmetic path that is not built here
-                raise ValueError(f'MRC mode {m.mode} maps are not supported (float32 / mode 2 only)')
+            if m.mode not in (0, 1, 2, 6):
+                # float16 (mode 12): scipy.ndimage.zoom refuses the array type, so the reference fails on it too
+                raise ValueError(f'MRC mode {m.mode} maps are not supported (modes 0, 1, 2 and 6 are)')
             header = _header_of(m)
             pipe = shared_pipeline(self.device).configure(order=self.order, target_voxel_size=target_voxel_size)
             src = upload_map(m.data, pipe.device)

@@ -271,6 +271,10 @@ class SlabPipeline(MapPipeline):
     def slab_resample(self, own_src, header=None):
         """Halo exchange + resample of this rank's planes.  Returns (res, owned): the local
         resampled planes [ext_lo, ext_hi) and the view of the owned ones [out_lo, out_hi)."""
+        if getattr(own_src, 'dtype', None) != torch.float32:
+            # integer maps (D12) would need their exact histogram exchanged between the ranks: one GPU only
+            raise MicaError(f'SlabPipeline takes float32 maps only, got {getattr(own_src, "dtype", type(own_src))} '
+                            '(integer maps run on one GPU, MapPipeline)')
         if header is not None:
             self.header = header
         plan = self.make_plan(tuple(own_src.shape), self.header)
