@@ -30,16 +30,14 @@ long long peer_timeout_cycles() {
   return ms * 2000000LL;   // clock64 runs at <= 1.97 GHz on a B200
 }
 TensorMapEncodeFn tensor_map_encode_fn() {
-  static TensorMapEncodeFn fn = nullptr;
-  static bool tried = false;
-  if (!tried) {
-    tried = true;
+  // looked up once; a function-local static is initialised once even when several threads call at the same time
+  static const TensorMapEncodeFn fn = [] {
     void* p = nullptr;
     cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess &&
-        q == cudaDriverEntryPointSuccess)
-      fn = (TensorMapEncodeFn)p;
-  }
+    const bool found = cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess &&
+                       q == cudaDriverEntryPointSuccess;
+    return found ? (TensorMapEncodeFn)p : nullptr;
+  }();
   return fn;
 }
 }  // namespace mica

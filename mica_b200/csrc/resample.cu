@@ -37,6 +37,8 @@
 //   gather3_kernel       one thread per output voxel (axes under 4 samples, strong down-sampling,
 //                        mica_resample_force_generic)
 // Order 1: gather1_kernel, trilinear, one thread per output voxel, no prefilter.
+// Host side: resample_impl checks what every route shares, then hands over to resample_fast or resample_general (or
+// launches gather1_kernel); each path checks its own arguments and encodes its tensor map before the first launch.
 //
 // Integer maps (int8 / int16 / uint16, DESIGN.md D12) always take the general path: its z prefilter reads the
 // map's own type, and its interpolation kernels store with SciPy's integer rule (store_out).  The fast path's
@@ -1206,68 +1208,61 @@ static int g_force_generic = 0;   // tests: run the general kernels on shapes th
 enum { kPassZ = 0, kPassY = 1, kPassX = 2, kPassInterp = 3 };
 static thread_local int g_resample_path[4] = {-1, -1, -1, -1};
 
-constexpr size_t kMaxTileBytes = 200 * 1024;
+// Shared-memory budgets the kernel choices are made against (a B200 block may take up to 227 KiB)
+constexpr size_t kMaxTileBytes = 200 * 1024;  // general path: one prefilter tile of lines (prefilter_cols*, _rows*)
+constexpr size_t kPipeSmemMax = 220 * 1024;   // fast path: the x pass's tile of staged rows (rows_pipe_smem)
+constexpr size_t kSmemPerSm = 225 * 1024;     // fast path: an SM's share for x-pass CTAs, tile + 1 KiB each (rows_grid)
 
-// general path, z and y axes: float32 (z) or float64 (y, in place) in, float64 out; lines that fit no tile are
+// Launches the kernel of one resample pass and records it for mica_last_resample_path.  A kernel that takes dynamic
+// shared memory has its limit raised on every call: the attribute belongs to the current device.
+template <typename... P, typename... A>
+static int launch_pass(int pass, int path, const char* name, void (*kernel)(P...), dim3 grid, int threads,
+                       size_t smem, cudaStream_t st, A... args) {
+  if (smem) MICA_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  kernel<<<grid, threads, smem, st>>>(args...);
+  g_resample_path[pass] = path;
+  MICA_LAUNCH_CHECK(name);
+  return MICA_OK;
+}
+
+// general path, z and y axes: the map's type (z) or float64 (y, in place) in, float64 out; lines that fit no tile are
 // swept in global memory
 template <typename TIn>
 static int launch_cols_f64(const TIn* in, double* out, int n, int64_t line_stride, int n_cols,
                            int64_t outer_stride, int n_outer, cudaStream_t st, int pass) {
-  if (n_cols <= 0 || n_outer <= 0 || n <= 0) return MICA_OK;
   const ColStrides S{line_stride, line_stride, outer_stride, outer_stride};
   const size_t per_col = (size_t)n * sizeof(double);
-  if (!g_force_generic && n >= kMinSegLine && per_col * 32 <= kMaxTileBytes) {
-    const size_t smem = per_col * 16;
-    MICA_CUDA(cudaFuncSetAttribute(prefilter_cols_seg<TIn, 16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    prefilter_cols_seg<TIn, 16><<<dim3((n_cols + 15) / 16, n_outer), 256, smem, st>>>(in, out, n, n_cols, S);
-    g_resample_path[pass] = MICA_RS_COLS_SEG16;
-  } else if (per_col * 32 <= kMaxTileBytes) {
-    const size_t smem = per_col * 32;
-    MICA_CUDA(cudaFuncSetAttribute(prefilter_cols<TIn, 32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    prefilter_cols<TIn, 32><<<dim3((n_cols + 31) / 32, n_outer), 256, smem, st>>>(in, out, n, n_cols, S);
-    g_resample_path[pass] = MICA_RS_COLS32;
-  } else if (per_col * 8 <= kMaxTileBytes) {
-    const size_t smem = per_col * 8;
-    MICA_CUDA(cudaFuncSetAttribute(prefilter_cols<TIn, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    prefilter_cols<TIn, 8><<<dim3((n_cols + 7) / 8, n_outer), 256, smem, st>>>(in, out, n, n_cols, S);
-    g_resample_path[pass] = MICA_RS_COLS8;
-  } else {
-    prefilter_cols_global<TIn><<<dim3((n_cols + 127) / 128, n_outer), 128, 0, st>>>(in, out, n, line_stride, n_cols,
-                                                                                    outer_stride);
-    g_resample_path[pass] = MICA_RS_COLS_GLOBAL;
-  }
-  MICA_LAUNCH_CHECK("prefilter_cols");
-  return MICA_OK;
+  if (!g_force_generic && n >= kMinSegLine && per_col * 32 <= kMaxTileBytes)
+    return launch_pass(pass, MICA_RS_COLS_SEG16, "prefilter_cols", prefilter_cols_seg<TIn, 16>,
+                       dim3((n_cols + 15) / 16, n_outer), 256, per_col * 16, st, in, out, n, n_cols, S);
+  if (per_col * 32 <= kMaxTileBytes)
+    return launch_pass(pass, MICA_RS_COLS32, "prefilter_cols", prefilter_cols<TIn, 32>,
+                       dim3((n_cols + 31) / 32, n_outer), 256, per_col * 32, st, in, out, n, n_cols, S);
+  if (per_col * 8 <= kMaxTileBytes)
+    return launch_pass(pass, MICA_RS_COLS8, "prefilter_cols", prefilter_cols<TIn, 8>,
+                       dim3((n_cols + 7) / 8, n_outer), 256, per_col * 8, st, in, out, n, n_cols, S);
+  return launch_pass(pass, MICA_RS_COLS_GLOBAL, "prefilter_cols", prefilter_cols_global<TIn>,
+                     dim3((n_cols + 127) / 128, n_outer), 128, 0, st, in, out, n, line_stride, n_cols, outer_stride);
 }
 
 // a row that fits no 4-row shared-memory tile is swept in global memory, one row per CTA along grid y
 static bool row_fits_smem(int n) { return (size_t)(n | 1) * sizeof(double) * 4 <= kMaxTileBytes; }
 
+// general path, x axis: contiguous rows, in place
 static int launch_rows(double* data, int n, int64_t n_rows, cudaStream_t st) {
-  if (n <= 0 || n_rows <= 0) return MICA_OK;
-  size_t per_row = (size_t)(n | 1) * sizeof(double);
-  if (!g_force_generic && n >= kMinSegLine && per_row * 32 <= kMaxTileBytes) {
-    size_t smem = per_row * 16;
-    MICA_CUDA(cudaFuncSetAttribute(prefilter_rows_seg<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    prefilter_rows_seg<16><<<(unsigned)ceil_div64(n_rows, 16), 256, smem, st>>>(data, n, n_rows);
-    g_resample_path[kPassX] = MICA_RS_ROWS_SEG16;
-  } else if (per_row * 32 <= kMaxTileBytes) {
-    size_t smem = per_row * 32;
-    MICA_CUDA(cudaFuncSetAttribute(prefilter_rows<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    prefilter_rows<32><<<(unsigned)ceil_div64(n_rows, 32), 256, smem, st>>>(data, n, n_rows);
-    g_resample_path[kPassX] = MICA_RS_ROWS32;
-  } else if (row_fits_smem(n)) {
-    size_t smem = per_row * 4;
-    MICA_CUDA(cudaFuncSetAttribute(prefilter_rows<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    prefilter_rows<4><<<(unsigned)ceil_div64(n_rows, 4), 256, smem, st>>>(data, n, n_rows);
-    g_resample_path[kPassX] = MICA_RS_ROWS4;
-  } else {
-    // a row is a column of a [n_rows x n] matrix with unit line stride
-    prefilter_cols_global<double><<<dim3(1, (unsigned)n_rows), 1, 0, st>>>(data, data, n, 1, 1, n);
-    g_resample_path[kPassX] = MICA_RS_COLS_GLOBAL;
-  }
-  MICA_LAUNCH_CHECK("prefilter_rows");
-  return MICA_OK;
+  const size_t per_row = (size_t)(n | 1) * sizeof(double);
+  if (!g_force_generic && n >= kMinSegLine && per_row * 32 <= kMaxTileBytes)
+    return launch_pass(kPassX, MICA_RS_ROWS_SEG16, "prefilter_rows", prefilter_rows_seg<16>,
+                       (unsigned)ceil_div64(n_rows, 16), 256, per_row * 16, st, data, n, n_rows);
+  if (per_row * 32 <= kMaxTileBytes)
+    return launch_pass(kPassX, MICA_RS_ROWS32, "prefilter_rows", prefilter_rows<32>, (unsigned)ceil_div64(n_rows, 32),
+                       256, per_row * 32, st, data, n, n_rows);
+  if (row_fits_smem(n))
+    return launch_pass(kPassX, MICA_RS_ROWS4, "prefilter_rows", prefilter_rows<4>, (unsigned)ceil_div64(n_rows, 4),
+                       256, per_row * 4, st, data, n, n_rows);
+  // a row is a column of a [n_rows x n] matrix with unit line stride
+  return launch_pass(kPassX, MICA_RS_COLS_GLOBAL, "prefilter_rows", prefilter_cols_global<double>,
+                     dim3(1, (unsigned)n_rows), 1, 0, st, data, data, n, 1, 1, n);
 }
 
 }  // namespace mica
@@ -1291,11 +1286,16 @@ extern "C" int mica_resample_force_generic(int on) {
 
 // The fast order-3 path: z and y prefilters write float32 coefficients (padded row pitch), the x pass
 // prefilters and interpolates rows into a float64 volume [sz_l][sy][nxp], the march interpolates y and z.
-constexpr size_t kPipeSmemMax = 220 * 1024;
 static int64_t pitch_f32(int sx) { return ((int64_t)sx + 3) / 4 * 4; }
 static int64_t pitch_f64(int nx) { return ((int64_t)nx + 1) / 2 * 2; }
 static size_t rows_pipe_smem(int n, int L) {
   return (((size_t)L * (n | 1) * 8 + 15) & ~(size_t)15) + (size_t)kPipeStages * L * pitch_f32(n) * 4;
+}
+
+// source rows that the y taps of an 8-row output tile span: a march stages 12 or 16 rows per source plane
+static int y_span(int sy, int ny) {
+  const double zoom_y = ny > 1 ? (double)(sy - 1) / (double)(ny - 1) : 1.0;
+  return (int)floor(7.0 * zoom_y) + 5;
 }
 
 // Source planes [*c_lo, *c_hi] (global) that hold a z tap of output planes [dst_z0, dst_z0 + dst_nz_local), with
@@ -1312,15 +1312,20 @@ static void needed_planes(int sz, int nz, int dst_z0, int dst_nz_local, int src_
   *c_hi = hi;
 }
 
+// segment length of cols_reg_kernel on a line of ng samples: the line cut into the fewest segments of <= kColLen
+static int cols_reg_seg_len(int ng) {
+  const int n_seg = (ng + kColLen - 1) / kColLen;
+  return (ng + n_seg - 1) / n_seg;
+}
+
 // Block of source planes [*src_lo, *src_hi) a rank must hold so that the z prefilter of output planes
 // [dst_z0, dst_z0 + dst_nz_local) sees the windows the whole map would give it (bit-identical coefficients).
 extern "C" int mica_resample_slab_source_planes(int sz, int nz, int dst_z0, int dst_nz_local, int* src_lo, int* src_hi) {
   MICA_REQUIRE(src_lo && src_hi, "null pointer");
   MICA_REQUIRE(sz > 0 && nz > 0 && dst_z0 >= 0 && dst_nz_local > 0 && dst_z0 + dst_nz_local <= nz, "bad slab");
-  int c_lo, c_hi, n_seg, len;
+  int c_lo, c_hi;
   needed_planes(sz, nz, dst_z0, dst_nz_local, 0, sz, &c_lo, &c_hi);
-  n_seg = (sz + kColLen - 1) / kColLen;
-  len = (sz + n_seg - 1) / n_seg;
+  const int len = cols_reg_seg_len(sz);
   const int lo = c_lo / len * len - kColH, hi = c_hi / len * len + kColLen + kColH;
   *src_lo = lo < 0 ? 0 : lo;
   *src_hi = hi > sz ? sz : hi;
@@ -1330,7 +1335,7 @@ extern "C" int mica_resample_slab_source_planes(int sz, int nz, int dst_z0, int 
 // sz = planes of the whole map, src_nz_local = planes of the block in memory.  The choice follows the WHOLE line,
 // so that every block of a z-slab partition runs the same kernels as the whole map (the z pass numbers its segments
 // on the whole line: the same bits): no bound but the register pass's 8-plane minimum looks at the block.
-static bool fast_path_ok(int sz, int src_nz_local, int sy, int sx, int ny, int nx) {
+static bool fast_path_ok(int sz, int src_nz_local, int sy, int sx, int ny) {
   if (g_force_generic || getenv("MICA_NO_TMA")) return false;
   // No kernel needs this bound (the y pass, cols_reg_kernel, takes lines of any length): it only keeps maps with y
   // lines of more than 1760 samples on the general path they have always taken.
@@ -1338,79 +1343,52 @@ static bool fast_path_ok(int sz, int src_nz_local, int sy, int sx, int ny, int n
   if (sz < kMinSegLine || sy < kMinSegLine || sx < kMinSegLine) return false;             // segment-parallel sweeps
   if (src_nz_local < 8) return false;
   if (rows_pipe_smem(sx, 8) > kPipeSmemMax) return false;            // 8 rows in the x pass's tile: sx <= 1759
-  const double zoom_y = ny > 1 ? (double)(sy - 1) / (double)(ny - 1) : 1.0;
-  if ((int)floor(7.0 * zoom_y) + 5 > 16) return false;                                    // y span of an 8-row tile
+  if (y_span(sy, ny) > 16) return false;
   return tensor_map_encode_fn() != nullptr;
 }
 
 // register-only column pass: 32 columns x 8 segments per CTA, segments of <= kColLen samples.  The line in memory
 // is samples [g0, g0 + n) of a line of ng; the segments of the GLOBAL line that hold samples [need_lo, need_hi]
 // (global numbers) are computed.
-static void cols_reg_geometry(int ng, int* n_seg, int* len) {
-  *n_seg = (ng + kColLen - 1) / kColLen;
-  *len = (ng + *n_seg - 1) / *n_seg;
-}
 static int launch_cols_reg(const float* in, float* out, int n, int n_cols, int n_outer, ColStrides S, cudaStream_t st,
                            int pass, int g0, int ng, int need_lo, int need_hi) {
-  if (n_cols <= 0 || n_outer <= 0 || need_hi < need_lo) return MICA_OK;
-  MICA_REQUIRE(n_outer <= 65535, "too many outer lines for the launch grid");
-  int n_seg_g, len;
-  cols_reg_geometry(ng, &n_seg_g, &len);
+  const int len = cols_reg_seg_len(ng);
   const int seg0 = need_lo / len, n_seg = need_hi / len - seg0 + 1;
-  cols_reg_kernel<<<dim3((n_cols + 31) / 32, (n_seg + 7) / 8, n_outer), 256, 0, st>>>(in, out, n, n_cols, S, len, n_seg,
-                                                                                   g0, ng, seg0);
-  g_resample_path[pass] = MICA_RS_COLS_REG;
-  MICA_LAUNCH_CHECK("cols_reg_kernel");
-  return MICA_OK;
-}
-static int launch_cols_reg(const float* in, float* out, int n, int n_cols, int n_outer, ColStrides S, cudaStream_t st,
-                           int pass) {
-  return launch_cols_reg(in, out, n, n_cols, n_outer, S, st, pass, 0, n, 0, n - 1);
+  return launch_pass(pass, MICA_RS_COLS_REG, "cols_reg_kernel", cols_reg_kernel,
+                     dim3((n_cols + 31) / 32, (n_seg + 7) / 8, n_outer), 256, 0, st, in, out, n, n_cols, S, len,
+                     n_seg, g0, ng, seg0);
 }
 
 // persistent grid of the x pass: as many CTAs as fit an SM's shared memory (at most max_per_sm), no more than there
 // are tiles of L rows; the tiles are dealt round-robin
 static unsigned rows_grid(size_t smem, int max_per_sm, int64_t n_rows, int L) {
-  int per_sm = (int)((size_t)225 * 1024 / (smem + 1024));
+  int per_sm = (int)(kSmemPerSm / (smem + 1024));
   per_sm = per_sm < 1 ? 1 : (per_sm > max_per_sm ? max_per_sm : per_sm);
   const long long tiles = (n_rows + L - 1) / L;
   const long long grid = (long long)kNumSMs * per_sm;
   return (unsigned)(grid < tiles ? grid : tiles);
 }
-template <int L, int THREADS>
-static int launch_rows_pipe_t(const float* in, int64_t in_pitch, double* out, int64_t out_pitch, int n, int nx,
-                              int64_t n_rows, const Tap* tx, cudaStream_t st) {
-  const size_t smem = rows_pipe_smem(n, L);
-  MICA_CUDA(cudaFuncSetAttribute(rows_pipe_interp_kernel<L, THREADS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  rows_pipe_interp_kernel<L, THREADS><<<rows_grid(smem, 2048 / THREADS, n_rows, L), THREADS, smem, st>>>(
-      in, in_pitch, out, out_pitch, n, nx, n_rows, tx);
-  g_resample_path[kPassX] = L == 8 ? MICA_RS_ROWS_PIPE_8_512 : MICA_RS_ROWS_PIPE_16_512;
-  MICA_LAUNCH_CHECK("rows_pipe_interp_kernel");
-  return MICA_OK;
-}
-template <int SEGS>
-static int launch_rows_reg_t(const float* in, int64_t in_pitch, double* out, int64_t out_pitch, int n, int nx,
-                             int64_t n_rows, const Tap* tx, cudaStream_t st) {
-  const size_t smem = rows_pipe_smem(n, 16);
-  MICA_CUDA(cudaFuncSetAttribute(rows_reg_interp_kernel<SEGS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  int len = (n + SEGS - 1) / SEGS;
-  if (len % 2 == 0 && len < kColLen) ++len;      // odd segment length: the lanes of a row hit distinct banks
-  rows_reg_interp_kernel<SEGS><<<rows_grid(smem, 512 / (16 * SEGS), n_rows, 16), 16 * SEGS, smem, st>>>(
-      in, in_pitch, out, out_pitch, n, nx, n_rows, tx, len);
-  g_resample_path[kPassX] = SEGS == 16 ? MICA_RS_ROWS_REG16 : MICA_RS_ROWS_REG32;
-  MICA_LAUNCH_CHECK("rows_reg_interp_kernel");
-  return MICA_OK;
-}
 
-// x pass: the register form for rows of <= 32 segments of kColLen (832 samples), the shared-memory sweep of 16 rows
-// per tile while they fit kPipeSmemMax (879 samples), of 8 rows beyond
+// x pass: the register form for rows of <= 16 or 32 segments of kColLen (832 samples), then the shared-memory sweep
+// of 16 rows per tile while they fit kPipeSmemMax (879 samples), of 8 rows beyond
 static int launch_rows_pipe(const float* in, int64_t in_pitch, double* out, int64_t out_pitch, int n, int nx,
                             int64_t n_rows, const Tap* tx, cudaStream_t st) {
-  if (n_rows <= 0) return MICA_OK;
-  if (n <= 16 * kColLen) return launch_rows_reg_t<16>(in, in_pitch, out, out_pitch, n, nx, n_rows, tx, st);
-  if (n <= 32 * kColLen) return launch_rows_reg_t<32>(in, in_pitch, out, out_pitch, n, nx, n_rows, tx, st);
-  if (rows_pipe_smem(n, 16) <= kPipeSmemMax) return launch_rows_pipe_t<16, 512>(in, in_pitch, out, out_pitch, n, nx, n_rows, tx, st);
-  return launch_rows_pipe_t<8, 512>(in, in_pitch, out, out_pitch, n, nx, n_rows, tx, st);
+  if (n <= 32 * kColLen) {
+    const int segs = n <= 16 * kColLen ? 16 : 32;
+    const size_t smem = rows_pipe_smem(n, 16);
+    int len = (n + segs - 1) / segs;
+    if (len % 2 == 0 && len < kColLen) ++len;      // odd segment length: the lanes of a row hit distinct banks
+    return launch_pass(kPassX, segs == 16 ? MICA_RS_ROWS_REG16 : MICA_RS_ROWS_REG32, "rows_reg_interp_kernel",
+                       segs == 16 ? rows_reg_interp_kernel<16> : rows_reg_interp_kernel<32>,
+                       rows_grid(smem, 512 / (16 * segs), n_rows, 16), 16 * segs, smem, st, in, in_pitch, out,
+                       out_pitch, n, nx, n_rows, tx, len);
+  }
+  const int L = rows_pipe_smem(n, 16) <= kPipeSmemMax ? 16 : 8;
+  const size_t smem = rows_pipe_smem(n, L);
+  return launch_pass(kPassX, L == 16 ? MICA_RS_ROWS_PIPE_16_512 : MICA_RS_ROWS_PIPE_8_512, "rows_pipe_interp_kernel",
+                     L == 16 ? rows_pipe_interp_kernel<16, 512> : rows_pipe_interp_kernel<8, 512>,
+                     rows_grid(smem, 2048 / 512, n_rows, L), 512, smem, st, in, in_pitch, out, out_pitch, n, nx,
+                     n_rows, tx);
 }
 
 extern "C" size_t mica_resample_workspace_bytes(int src_nz_local, int sy, int sx, int nz, int ny, int nx, int order) {
@@ -1425,12 +1403,124 @@ extern "C" size_t mica_resample_workspace_bytes(int src_nz_local, int sy, int sx
   return taps + coeff + 512;
 }
 
+// grid of a march: a CTA owns an [8 y x 64 x] output column and marches zchunk planes of it; the planes are cut into
+// enough chunks of >= 16 for 8 CTAs per SM
+static int march_grid(int ny, int nx, int nz_local, dim3* grid, int* zchunk) {
+  const int xt = (nx + 63) / 64, yt = (ny + 7) / 8;
+  int nzc = (8 * kNumSMs + xt * yt - 1) / (xt * yt);
+  nzc = nzc < 1 ? 1 : nzc;
+  if (nzc > (nz_local + 15) / 16) nzc = (nz_local + 15) / 16;
+  *zchunk = (nz_local + nzc - 1) / nzc;
+  *grid = dim3(xt, yt, (nz_local + *zchunk - 1) / *zchunk);
+  MICA_REQUIRE(yt <= 65535 && grid->z <= 65535, "output too large for the launch grid");
+  return MICA_OK;
+}
+
+// TMA descriptor of the float64 volume [nz][ny][pitch] at base, read in boxes of [box_y][box_x] of one plane
+static CUresult encode_f64_3d(CUtensorMap* map, double* base, int64_t pitch, int ny, int nz, int box_x, int box_y) {
+  const TensorMapEncodeFn enc = tensor_map_encode_fn();
+  if (!enc) return CUDA_ERROR_NOT_SUPPORTED;
+  const cuuint64_t gdim[3] = {(cuuint64_t)pitch, (cuuint64_t)ny, (cuuint64_t)nz};
+  const cuuint64_t gstr[2] = {(cuuint64_t)pitch * 8, (cuuint64_t)ny * pitch * 8};
+  const cuuint32_t box[3] = {(cuuint32_t)box_x, (cuuint32_t)box_y, 1}, estr[3] = {1, 1, 1};
+  return enc(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT64, 3, base, gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+             CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+}
+
+// the fast order-3 path, on a float32 map that fast_path_ok accepts
+template <typename Taps>
+static int resample_fast(const float* src, int sz, int sy, int sx, int src_z0, int src_nz_local, float* dst, int nz,
+                         int ny, int nx, int dst_z0, int dst_nz_local, const Tap* tz, const Tap* ty, const Tap* tx,
+                         ZWin* zw, double* coeff, cudaStream_t st, const Taps& taps) {
+  const int64_t plane = (int64_t)sy * sx;
+  MICA_REQUIRE(plane <= 0x7fffffffLL && src_nz_local <= 65535 && sy <= 65535, "source plane too large");
+  const int64_t p32 = pitch_f32(sx), p64 = pitch_f64(nx);
+  float* c32 = (float*)coeff;
+  float* c32b = c32 + (size_t)src_nz_local * sy * p32;      // second float32 volume (the register pass is not in place)
+  double* xr = (double*)((char*)coeff + align_up((size_t)2 * src_nz_local * sy * p32 * sizeof(float), 256));
+  // source planes whose coefficients the z taps of this output slab can touch (global numbers, one plane of
+  // margin): the whole line for a whole map; for a z-slab the planes beyond them are prefilter horizon only
+  // and take no part in the y and x passes
+  int c_lo, c_hi;
+  needed_planes(sz, nz, dst_z0, dst_nz_local, src_z0, src_nz_local, &c_lo, &c_hi);
+  const int l0 = c_lo - src_z0, cnt = c_hi - c_lo + 1;
+  MICA_REQUIRE(sy <= 65535 && cnt <= 65535, "too many outer lines for the launch grid");   // grid z of cols_reg
+  dim3 mgrid;
+  int zchunk;
+  if (int rc = march_grid(ny, nx, dst_nz_local, &mgrid, &zchunk)) return rc;
+  const int rows = y_span(sy, ny) <= 12 ? 12 : 16;
+  CUtensorMap tmap;
+  const CUresult cr = encode_f64_3d(&tmap, xr, p64, sy, src_nz_local, 64, rows);
+  if (cr != CUDA_SUCCESS) return set_error(MICA_ERR_CUDA, "cuTensorMapEncodeTiled failed (%d)", (int)cr);
+
+  if (int rc = taps()) return rc;
+  const ColStrides Sz{plane, sy * p32, sx, p32}, Sy{p32, p32, sy * p32, sy * p32};
+  const size_t l0_f32 = (size_t)l0 * sy * p32;
+  // axis 0 (z): float32 in (row pitch sx) -> c32b (row pitch p32); axis 1 (y): c32b -> c32
+  if (int rc = launch_cols_reg(src, c32b, src_nz_local, sx, sy, Sz, st, kPassZ, src_z0, sz, c_lo, c_hi)) return rc;
+  if (int rc = launch_cols_reg(c32b + l0_f32, c32 + l0_f32, sy, sx, cnt, Sy, st, kPassY, 0, sy, 0, sy - 1)) return rc;
+  // axis 2 (x): prefilter + interpolate the rows -> x-resampled float64 volume
+  if (int rc = launch_rows_pipe(c32 + l0_f32, p32, xr + (size_t)l0 * sy * p64, p64, sx, nx, (int64_t)cnt * sy, tx, st))
+    return rc;
+  zwin_kernel<<<(dst_nz_local + 127) / 128, 128, 0, st>>>(tz, zw, dst_nz_local, src_nz_local);
+  MICA_LAUNCH_CHECK("zwin_kernel");
+  return launch_pass(kPassInterp, rows == 12 ? MICA_RS_MARCH_YZ_TMA3 : MICA_RS_MARCH_YZ_TMA4, "march_yz_tma_kernel",
+                     rows == 12 ? march_yz_tma_kernel<3> : march_yz_tma_kernel<4>, mgrid, 256,
+                     (size_t)kYzStages * rows * 64 * 8 + 128, st, tmap, zw, ty, dst, ny, nx, dst_nz_local, zchunk);
+}
+
+// general order-3 path: float64 coefficients prefiltered in place along z, y and x; then the marching gather when the
+// y span of an 8-row output tile fits the staged rows and every axis has a full 4-sample window, else one thread per
+// output voxel
+template <typename T, typename Taps>
+static int resample_general(const T* src, int sy, int sx, int src_nz_local, T* dst, int ny, int nx, int dst_nz_local,
+                            const Tap* tz, const Tap* ty, const Tap* tx, ZWin* zw, double* coeff, cudaStream_t st,
+                            const Taps& taps) {
+  const int64_t plane = (int64_t)sy * sx;
+  MICA_REQUIRE(plane <= 0x7fffffffLL && src_nz_local <= 65535, "source plane too large");
+  const int span_y = y_span(sy, ny);
+  const bool march = !g_force_generic && src_nz_local >= 4 && sy >= 4 && sx >= 4 && span_y <= 16;
+  dim3 mgrid;
+  int zchunk = 0;
+  if (march) {
+    if (int rc = march_grid(ny, nx, dst_nz_local, &mgrid, &zchunk)) return rc;
+  }
+  // TMA-fed ring when the coefficient rows are 16-byte multiples and the x span of a 64-wide output tile fits one
+  // box; else the register-prefetch variant
+  const double zoom_x = nx > 1 ? (double)(sx - 1) / (double)(nx - 1) : 1.0;
+  const int xb = (((int)floor(63.0 * zoom_x) + 5) + 1 + 1) & ~1;   // span + 1 (even box start), even width
+  const int rows = span_y <= 12 ? 12 : 16;
+  CUtensorMap tmap;
+  const bool tma = march && sx % 2 == 0 && xb <= 256 && !getenv("MICA_NO_TMA") &&
+                   encode_f64_3d(&tmap, coeff, sx, sy, src_nz_local, xb, rows) == CUDA_SUCCESS;
+
+  if (int rc = taps()) return rc;
+  // axis 0 (z): lines of length src_nz_local, stride plane; reads the map's type, writes float64
+  if (int rc = launch_cols_f64<T>(src, coeff, src_nz_local, plane, (int)plane, 0, 1, st, kPassZ)) return rc;
+  // axis 1 (y): per z plane, lines of length sy, stride sx
+  if (int rc = launch_cols_f64<double>(coeff, coeff, sy, sx, sx, plane, src_nz_local, st, kPassY)) return rc;
+  // axis 2 (x): contiguous rows
+  if (int rc = launch_rows(coeff, sx, (int64_t)src_nz_local * sy, st)) return rc;
+  if (!march)
+    return launch_pass(kPassInterp, MICA_RS_GATHER3, "gather3_kernel", gather3_kernel<T>,
+                       dim3((nx + 127) / 128, ny, dst_nz_local), 128, 0, st, coeff, sy, sx, tz, ty, tx, dst, ny, nx);
+  zwin_kernel<<<(dst_nz_local + 127) / 128, 128, 0, st>>>(tz, zw, dst_nz_local, src_nz_local);
+  MICA_LAUNCH_CHECK("zwin_kernel");
+  if (tma)
+    return launch_pass(kPassInterp, rows == 12 ? MICA_RS_MARCH3_TMA3 : MICA_RS_MARCH3_TMA4, "march3_tma_kernel",
+                       rows == 12 ? march3_tma_kernel<3, T> : march3_tma_kernel<4, T>, mgrid, 256,
+                       (size_t)kMarchStages * (((size_t)rows * xb + 15) / 16 * 16) * 8 + 128, st, tmap, xb, zw, ty, tx,
+                       dst, ny, nx, dst_nz_local, zchunk);
+  return launch_pass(kPassInterp, rows == 12 ? MICA_RS_MARCH3_3 : MICA_RS_MARCH3_4, "march3_kernel",
+                     rows == 12 ? march3_kernel<3, T> : march3_kernel<4, T>, mgrid, 256, 0, st, coeff, sy, sx, zw, ty,
+                     tx, dst, ny, nx, dst_nz_local, zchunk);
+}
+
 // T = the map's sample type, in and out.  Integer maps never take the fast path (see the file header).
 template <typename T>
 static int resample_impl(const T* src, int sz, int sy, int sx, int src_z0, int src_nz_local, T* dst, int nz, int ny,
                          int nx, int dst_z0, int dst_nz_local, void* workspace, size_t workspace_bytes, int order,
                          mica_stream_t stream) {
-  constexpr bool kF32 = std::is_same<T, float>::value;
   cudaStream_t st = (cudaStream_t)stream;
   MICA_REQUIRE(src && dst && workspace, "null pointer");
   MICA_REQUIRE(order == 3 || order == 1, "order must be 3 or 1 (got %d)", order);
@@ -1451,148 +1541,30 @@ static int resample_impl(const T* src, int sz, int sy, int sx, int src_z0, int s
   Tap* tx = ty + ny;
   ZWin* zw = (ZWin*)(ws + align_up((size_t)(nz + ny + nx) * sizeof(Tap), 256));
   double* coeff = (double*)((char*)zw + align_up((size_t)nz * sizeof(ZWin), 256));
+  // each path calls taps() once its own checks have passed and its tensor map is encoded: a refused call launches
+  // nothing
+  auto taps = [&]() -> int {
+    taps_kernel<<<(dst_nz_local + 127) / 128, 128, 0, st>>>(tz, dst_nz_local, dst_z0, sz, nz, order, src_z0,
+                                                             src_nz_local);
+    MICA_LAUNCH_CHECK("taps_kernel(z)");
+    taps_kernel<<<(ny + 127) / 128, 128, 0, st>>>(ty, ny, 0, sy, ny, order, 0, sy);
+    MICA_LAUNCH_CHECK("taps_kernel(y)");
+    taps_kernel<<<(nx + 127) / 128, 128, 0, st>>>(tx, nx, 0, sx, nx, order, 0, sx);
+    MICA_LAUNCH_CHECK("taps_kernel(x)");
+    return MICA_OK;
+  };
 
-  taps_kernel<<<(dst_nz_local + 127) / 128, 128, 0, st>>>(tz, dst_nz_local, dst_z0, sz, nz, order, src_z0, src_nz_local);
-  MICA_LAUNCH_CHECK("taps_kernel(z)");
-  taps_kernel<<<(ny + 127) / 128, 128, 0, st>>>(ty, ny, 0, sy, ny, order, 0, sy);
-  MICA_LAUNCH_CHECK("taps_kernel(y)");
-  taps_kernel<<<(nx + 127) / 128, 128, 0, st>>>(tx, nx, 0, sx, nx, order, 0, sx);
-  MICA_LAUNCH_CHECK("taps_kernel(x)");
-
-  dim3 grid((nx + 127) / 128, ny, dst_nz_local);
-  if (kF32 && order == 3 && fast_path_ok(sz, src_nz_local, sy, sx, ny, nx)) {
-    const float* srcf = (const float*)src;
-    float* dstf = (float*)dst;
-    const int64_t plane = (int64_t)sy * sx;
-    MICA_REQUIRE(plane <= 0x7fffffffLL && src_nz_local <= 65535 && sy <= 65535, "source plane too large");
-    const int64_t p32 = pitch_f32(sx), p64 = pitch_f64(nx);
-    float* c32 = (float*)coeff;
-    double* xr = (double*)((char*)coeff + align_up((size_t)2 * src_nz_local * sy * p32 * sizeof(float), 256));
-    float* c32b = c32 + (size_t)src_nz_local * sy * p32;      // second float32 volume (the register pass is not in place)
-    const ColStrides Sz{plane, sy * p32, sx, p32}, Sy{p32, p32, sy * p32, sy * p32};
-    // source planes whose coefficients the z taps of this output slab can touch (global numbers, one plane of
-    // margin): the whole line for a whole map; for a z-slab the planes beyond them are prefilter horizon only
-    // and take no part in the y and x passes
-    int c_lo, c_hi;
-    needed_planes(sz, nz, dst_z0, dst_nz_local, src_z0, src_nz_local, &c_lo, &c_hi);
-    const int l0 = c_lo - src_z0, cnt = c_hi - c_lo + 1;
-    // axis 0 (z): float32 in (row pitch sx) -> c32b (row pitch p32); axis 1 (y): c32b -> c32
-    int rc = launch_cols_reg(srcf, c32b, src_nz_local, sx, sy, Sz, st, kPassZ, src_z0, sz, c_lo, c_hi);
-    if (rc) return rc;
-    rc = launch_cols_reg(c32b + (size_t)l0 * sy * p32, c32 + (size_t)l0 * sy * p32, sy, sx, cnt, Sy, st, kPassY);
-    if (rc) return rc;
-    // axis 2 (x): prefilter + interpolate the rows -> x-resampled float64 volume
-    rc = launch_rows_pipe(c32 + (size_t)l0 * sy * p32, p32, xr + (size_t)l0 * sy * p64, p64, sx, nx, (int64_t)cnt * sy,
-                          tx, st);
-    if (rc) return rc;
-    zwin_kernel<<<(dst_nz_local + 127) / 128, 128, 0, st>>>(tz, zw, dst_nz_local, src_nz_local);
-    MICA_LAUNCH_CHECK("zwin_kernel");
-    const int xt = (nx + 63) / 64, yt = (ny + 7) / 8;
-    int nzc = (8 * kNumSMs + xt * yt - 1) / (xt * yt);
-    nzc = nzc < 1 ? 1 : nzc;
-    if (nzc > (dst_nz_local + 15) / 16) nzc = (dst_nz_local + 15) / 16;
-    const int zchunk = (dst_nz_local + nzc - 1) / nzc;
-    dim3 mgrid(xt, yt, (dst_nz_local + zchunk - 1) / zchunk);
-    MICA_REQUIRE(yt <= 65535 && mgrid.z <= 65535, "output too large for the launch grid");
-    const double zoom_y = ny > 1 ? (double)(sy - 1) / (double)(ny - 1) : 1.0;
-    const int rows = ((int)floor(7.0 * zoom_y) + 5) <= 12 ? 12 : 16;
-    CUtensorMap tmap;
-    cuuint64_t gdim[3] = {(cuuint64_t)p64, (cuuint64_t)sy, (cuuint64_t)src_nz_local};
-    cuuint64_t gstr[2] = {(cuuint64_t)p64 * 8, (cuuint64_t)sy * p64 * 8};
-    cuuint32_t box[3] = {64, (cuuint32_t)rows, 1};
-    cuuint32_t estr[3] = {1, 1, 1};
-    CUresult cr = tensor_map_encode_fn()(&tmap, CU_TENSOR_MAP_DATA_TYPE_FLOAT64, 3, (void*)xr, gdim, gstr, box, estr,
-                                         CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
-                                         CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (cr != CUDA_SUCCESS) return set_error(MICA_ERR_CUDA, "cuTensorMapEncodeTiled failed (%d)", (int)cr);
-    const size_t smem = (size_t)kYzStages * rows * 64 * 8 + 128;
-    if (rows == 12) {
-      MICA_CUDA(cudaFuncSetAttribute(march_yz_tma_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      march_yz_tma_kernel<3><<<mgrid, 256, smem, st>>>(tmap, zw, ty, dstf, ny, nx, dst_nz_local, zchunk);
-      g_resample_path[kPassInterp] = MICA_RS_MARCH_YZ_TMA3;
-    } else {
-      MICA_CUDA(cudaFuncSetAttribute(march_yz_tma_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      march_yz_tma_kernel<4><<<mgrid, 256, smem, st>>>(tmap, zw, ty, dstf, ny, nx, dst_nz_local, zchunk);
-      g_resample_path[kPassInterp] = MICA_RS_MARCH_YZ_TMA4;
-    }
-    MICA_LAUNCH_CHECK("march_yz_tma_kernel");
-  } else if (order == 3) {
-    const int64_t plane = (int64_t)sy * sx;
-    MICA_REQUIRE(plane <= 0x7fffffffLL && src_nz_local <= 65535, "source plane too large");
-    // axis 0 (z): lines of length src_nz_local, stride plane; reads the map's type, writes float64
-    int rc = launch_cols_f64<T>(src, coeff, src_nz_local, plane, (int)plane, 0, 1, st, kPassZ);
-    if (rc) return rc;
-    // axis 1 (y): per z plane, lines of length sy, stride sx
-    rc = launch_cols_f64<double>(coeff, coeff, sy, sx, sx, plane, src_nz_local, st, kPassY);
-    if (rc) return rc;
-    // axis 2 (x): contiguous rows
-    rc = launch_rows(coeff, sx, (int64_t)src_nz_local * sy, st);
-    if (rc) return rc;
-    // marching gather when the y span of an 8-row output tile fits the staged rows and every
-    // axis has a full 4-sample window; else one thread per output voxel
-    const double zoom_y = ny > 1 ? (double)(sy - 1) / (double)(ny - 1) : 1.0;
-    const int span_y = (int)floor(7.0 * zoom_y) + 5;
-    if (!g_force_generic && src_nz_local >= 4 && sy >= 4 && sx >= 4 && span_y <= 16) {
-      zwin_kernel<<<(dst_nz_local + 127) / 128, 128, 0, st>>>(tz, zw, dst_nz_local, src_nz_local);
-      MICA_LAUNCH_CHECK("zwin_kernel");
-      const int xt = (nx + 63) / 64, yt = (ny + 7) / 8;
-      int nzc = (8 * kNumSMs + xt * yt - 1) / (xt * yt);
-      nzc = nzc < 1 ? 1 : nzc;
-      if (nzc > (dst_nz_local + 15) / 16) nzc = (dst_nz_local + 15) / 16;
-      const int zchunk = (dst_nz_local + nzc - 1) / nzc;
-      dim3 mgrid(xt, yt, (dst_nz_local + zchunk - 1) / zchunk);
-      MICA_REQUIRE(yt <= 65535 && mgrid.z <= 65535, "output too large for the launch grid");
-      // TMA-fed ring when the coefficient rows are 16-byte multiples and the x span of a 64-wide
-      // output tile fits one box; else the register-prefetch variant
-      const double zoom_x = nx > 1 ? (double)(sx - 1) / (double)(nx - 1) : 1.0;
-      const int xb = (((int)floor(63.0 * zoom_x) + 5) + 1 + 1) & ~1;   // span + 1 (even box start), even width
-      const int rows = span_y <= 12 ? 12 : 16;
-      bool tma_ok = false;
-      CUtensorMap tmap;
-      if (sx % 2 == 0 && xb <= 256 && !getenv("MICA_NO_TMA")) {
-        if (TensorMapEncodeFn enc = tensor_map_encode_fn()) {
-          cuuint64_t gdim[3] = {(cuuint64_t)sx, (cuuint64_t)sy, (cuuint64_t)src_nz_local};
-          cuuint64_t gstr[2] = {(cuuint64_t)sx * 8, (cuuint64_t)plane * 8};
-          cuuint32_t box[3] = {(cuuint32_t)xb, (cuuint32_t)rows, 1};
-          cuuint32_t estr[3] = {1, 1, 1};
-          tma_ok = enc(&tmap, CU_TENSOR_MAP_DATA_TYPE_FLOAT64, 3, (void*)coeff, gdim, gstr, box, estr,
-                       CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                       CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
-        }
-      }
-      if (tma_ok) {
-        const size_t smem = (size_t)kMarchStages * (((size_t)rows * xb + 15) / 16 * 16) * 8 + 128;
-        if (rows == 12) {
-          MICA_CUDA(cudaFuncSetAttribute(march3_tma_kernel<3, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-          march3_tma_kernel<3, T><<<mgrid, 256, smem, st>>>(tmap, xb, zw, ty, tx, dst, ny, nx, dst_nz_local, zchunk);
-          g_resample_path[kPassInterp] = MICA_RS_MARCH3_TMA3;
-        } else {
-          MICA_CUDA(cudaFuncSetAttribute(march3_tma_kernel<4, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-          march3_tma_kernel<4, T><<<mgrid, 256, smem, st>>>(tmap, xb, zw, ty, tx, dst, ny, nx, dst_nz_local, zchunk);
-          g_resample_path[kPassInterp] = MICA_RS_MARCH3_TMA4;
-        }
-        MICA_LAUNCH_CHECK("march3_tma_kernel");
-      } else {
-        if (span_y <= 12) {
-          march3_kernel<3, T><<<mgrid, 256, 0, st>>>(coeff, sy, sx, zw, ty, tx, dst, ny, nx, dst_nz_local, zchunk);
-          g_resample_path[kPassInterp] = MICA_RS_MARCH3_3;
-        } else {
-          march3_kernel<4, T><<<mgrid, 256, 0, st>>>(coeff, sy, sx, zw, ty, tx, dst, ny, nx, dst_nz_local, zchunk);
-          g_resample_path[kPassInterp] = MICA_RS_MARCH3_4;
-        }
-        MICA_LAUNCH_CHECK("march3_kernel");
-      }
-    } else {
-      gather3_kernel<T><<<grid, 128, 0, st>>>(coeff, sy, sx, tz, ty, tx, dst, ny, nx);
-      g_resample_path[kPassInterp] = MICA_RS_GATHER3;
-      MICA_LAUNCH_CHECK("gather3_kernel");
-    }
-  } else {
-    gather1_kernel<T, T><<<grid, 128, 0, st>>>(src, sy, sx, tz, ty, tx, dst, ny, nx);
-    g_resample_path[kPassInterp] = MICA_RS_GATHER1;
-    MICA_LAUNCH_CHECK("gather1_kernel");
+  if (order == 1) {
+    if (int rc = taps()) return rc;
+    return launch_pass(kPassInterp, MICA_RS_GATHER1, "gather1_kernel", gather1_kernel<T, T>,
+                       dim3((nx + 127) / 128, ny, dst_nz_local), 128, 0, st, src, sy, sx, tz, ty, tx, dst, ny, nx);
   }
-  return MICA_OK;
+  if constexpr (std::is_same<T, float>::value) {
+    if (fast_path_ok(sz, src_nz_local, sy, sx, ny))
+      return resample_fast(src, sz, sy, sx, src_z0, src_nz_local, dst, nz, ny, nx, dst_z0, dst_nz_local, tz, ty, tx,
+                           zw, coeff, st, taps);
+  }
+  return resample_general(src, sy, sx, src_nz_local, dst, ny, nx, dst_nz_local, tz, ty, tx, zw, coeff, st, taps);
 }
 
 extern "C" int mica_resample(const void* src, int src_dtype, int sz, int sy, int sx, int src_z0, int src_nz_local,

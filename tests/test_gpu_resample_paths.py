@@ -281,3 +281,20 @@ def test_row_fallback_grid_limit_is_reported_before_any_launch(cuda):
         ops.resample(src, (2, 4, 4))
     assert ops.launch_count() == before
     assert route() == (None, None, None, None)
+
+
+def test_refused_call_launches_nothing(cuda):
+    """A call the general path refuses (70000 z lines of one sample: more than the 65535 a launch grid holds)
+    returns MICA_ERR_INVALID before it enqueues anything, the tap tables included."""
+    sz, out_shape = 70000, (8, 8, 8)
+    src = torch.zeros((sz, 1, 1), dtype=torch.float32, device=cuda)
+    dst = torch.empty(out_shape, dtype=torch.float32, device=cuda)
+    nbytes = _lib.lib.mica_resample_workspace_bytes(sz, 1, 1, *out_shape, 3)
+    ws = torch.empty(nbytes, dtype=torch.uint8, device=cuda)
+    before = ops.launch_count()
+    rc = _lib.lib.mica_resample(src.data_ptr(), _lib.DTYPE_F32, sz, 1, 1, 0, sz, dst.data_ptr(), _lib.DTYPE_F32,
+                                *out_shape, 0, out_shape[0], ws.data_ptr(), nbytes, 3,
+                                torch.cuda.current_stream().cuda_stream)
+    assert _lib.ERR_NAMES.get(rc) == 'MICA_ERR_INVALID', rc
+    assert ops.launch_count() == before
+    assert route() == (None, None, None, None)
