@@ -78,6 +78,12 @@ int mica_resample_force_generic(int on);
  * block of it is in memory; with this block every coefficient the slab needs is computed from the same
  * window as on the whole map, so the slab's planes are BIT-IDENTICAL to the whole map's. */
 int mica_resample_slab_source_planes(int sz, int nz, int dst_z0, int dst_nz_local, int* src_lo, int* src_hi);
+/* host: the same for the general path, which integer maps take: the block that holds every raw sample that the z
+ * prefilter segments (16 per line, numbered on the whole line) computed for output planes [dst_z0,
+ * dst_z0+dst_nz_local) read, mirrored reads near plane 0 included.  With that block an integer map's slab is
+ * BIT-IDENTICAL to the whole map.  MICA_ERR_INVALID unless 96 <= sz <= 800: lines outside that range are
+ * prefiltered by one recursion over the whole line, which no block can reproduce bit for bit. */
+int mica_resample_slab_source_planes_general(int sz, int nz, int dst_z0, int dst_nz_local, int* src_lo, int* src_hi);
 
 /* src: device float32 [src_nz_local, sy, sx] = global source planes [src_z0, src_z0+src_nz_local)
  * dst: device float32 [dst_nz_local, ny, nx] = global output planes [dst_z0, dst_z0+dst_nz_local)
@@ -100,7 +106,9 @@ int mica_bspline_resample_f32(const float* src, int sz, int sy, int sx, int src_
  * accepted are float32 -> float32 (the same call as mica_bspline_resample_f32) and an integer type -> the same
  * integer type: scipy.ndimage.zoom on an integer array, which interpolates in float64 and stores into the input's
  * type rounding half away from zero and saturating at the type's range (DESIGN.md D12).  Integer maps always run
- * the float64 general path; zoom == (1,1,1) is again the caller's copy.  Any other pair is MICA_ERR_INVALID. */
+ * the float64 general path; zoom == (1,1,1) is again the caller's copy.  Any other pair is MICA_ERR_INVALID.
+ * An integer block of a longer z line (order 3) must hold the planes mica_resample_slab_source_planes_general
+ * names, and the line must have 96..800 planes; the result is then bit-identical to the whole map's planes. */
 int mica_resample(const void* src, int src_dtype, int sz, int sy, int sx, int src_z0, int src_nz_local,
                   void* dst, int dst_dtype, int nz, int ny, int nx, int dst_z0, int dst_nz_local,
                   void* workspace, size_t workspace_bytes, int order, mica_stream_t stream);
@@ -182,10 +190,33 @@ int mica_normalize_apply_f32(const float* x, float* y, int64_t n, const void* wo
  * float64, np.percentile(pos, 99.9) interpolates in float64 and the normalised map is the float64 expression
  * cast to float32.  Values have at most 16 bits, so one exact histogram of 2^8 / 2^16 bins gives every rank:
  * mica_int_order_stats is one pass over x plus one single-CTA pick that finds the median, count(x <= med),
- * n_pos, the percentile and the status word (MICA_NORM_*) on the device.  Single GPU only. */
+ * n_pos, the percentile and the status word (MICA_NORM_*) on the device.
+ * Several GPUs: init(n_total = voxels of all ranks); hist(this rank's voxels); sum the histograms of all ranks
+ * (2^8 int64 words for int8, 2^16 for int16 / uint16, at mica_int_stats_hist_ptr, or
+ * mica_int_stats_peer_publish + mica_int_stats_peer_sum); pick. */
 size_t mica_int_stats_workspace_bytes(void);
-/* x: device samples of `dtype` (MICA_DTYPE_I8 / I16 / U16), n of them; workspace of the size above */
+/* x: device samples of `dtype` (MICA_DTYPE_I8 / I16 / U16), n of them; workspace of the size above.  The same
+ * launches as init + hist + pick. */
 int mica_int_order_stats(const void* x, int dtype, int64_t n, void* workspace, mica_stream_t stream);
+int mica_int_stats_init(void* workspace, int dtype, int64_t n_total, mica_stream_t stream);
+int mica_int_stats_hist(const void* x, int dtype, int64_t n_local, void* workspace, mica_stream_t stream);
+int64_t* mica_int_stats_hist_ptr(void* workspace);
+/* leaves a state whose status is already final (MICA_NORM_PEER_TIMEOUT) as it is */
+int mica_int_stats_pick(void* workspace, int dtype, mica_stream_t stream);
+/* The histogram sum over NVLink peer memory, on the caller's stream: every rank allocates one buffer of
+ * mica_int_peer_buffer_bytes with mica_ipc_alloc, the ranks open each other's (mica_peer_open) and upload the
+ * table of `world` device pointers.  Per map, after hist:
+ *   mica_int_stats_peer_publish  copies the local histogram into the rank's slot `parity` and raises its flag of
+ *                                `epoch` in every peer's buffer -- it never waits;
+ *   mica_int_stats_peer_sum      waits (bounded: on timeout the status becomes MICA_NORM_PEER_TIMEOUT, which pick
+ *                                leaves alone) for every peer's flag and sums their slots into the local state.
+ * `epoch` = a counter every rank increments once per map (>= 1), `parity` = epoch & 1, as for
+ * mica_select_peer_reduce.  Several ranks driven on ONE GPU must enqueue every publish before any sum. */
+size_t mica_int_peer_buffer_bytes(void);
+int mica_int_stats_peer_publish(const void* workspace, int dtype, void* const* peer_bufs, int rank, int world,
+                                int parity, int epoch, mica_stream_t stream);
+int mica_int_stats_peer_sum(void* workspace, int dtype, void* const* peer_bufs, int rank, int world, int parity,
+                            int epoch, mica_stream_t stream);
 /* synchronises the stream; any out pointer may be NULL */
 int mica_int_stats_result(const void* workspace, double* median, double* p999, int64_t* n_pos, int* norm_status,
                           mica_stream_t stream);
@@ -239,7 +270,9 @@ int mica_select_peer_reduce(void* workspace, void* const* peer_bufs, int rank, i
  *                      of `epoch` and copies the `n_lo` elements the LOWER neighbour published for this rank
  *                      to dst_lo and the `n_hi` elements of the UPPER neighbour to dst_hi, over NVLink.
  * `epoch` increases by one per exchange, `parity` = epoch & 1 (slot reuse is safe because the order-statistics
- * exchange of the map in between synchronises all ranks). */
+ * exchange of the map in between synchronises all ranks).  The _bytes forms count offsets, sizes and the slot
+ * capacity in bytes (planes of any sample type); the float32 forms count float32 elements and forward x 4.
+ * A buffer of mica_halo_buffer_bytes(slot_elems) holds slots of 4 * slot_elems bytes. */
 size_t mica_halo_buffer_bytes(int64_t slot_elems);
 int mica_ipc_alloc(size_t bytes, void** dev_ptr, void* ipc_handle_out /* 64 bytes, nullable */);
 int mica_halo_publish(const float* own, int64_t off_lo, int64_t n_lo, int64_t off_hi, int64_t n_hi,
@@ -247,6 +280,11 @@ int mica_halo_publish(const float* own, int64_t off_lo, int64_t n_lo, int64_t of
                       mica_stream_t stream);
 int mica_halo_pull(float* dst_lo, int64_t n_lo, float* dst_hi, int64_t n_hi, void* const* peer_bufs, int rank,
                    int world, int parity, int epoch, int64_t slot_elems, int* status, mica_stream_t stream);
+int mica_halo_publish_bytes(const void* own, int64_t off_lo, int64_t n_lo, int64_t off_hi, int64_t n_hi,
+                            void* const* peer_bufs, int rank, int world, int parity, int epoch, int64_t slot_bytes,
+                            mica_stream_t stream);
+int mica_halo_pull_bytes(void* dst_lo, int64_t n_lo, void* dst_hi, int64_t n_hi, void* const* peer_bufs, int rank,
+                         int world, int parity, int epoch, int64_t slot_bytes, int* status, mica_stream_t stream);
 
 /* test hooks for the normaliser: (1) evaluate the NumPy expression operation by operation for
  * every voxel instead of the short equivalent path (returns the previous setting); (2) put

@@ -45,6 +45,7 @@ SIGNATURES = {
     'mica_resample_workspace_bytes': (_sz, [_i] * 7),
     'mica_resample_force_generic': (_i, [_i]),
     'mica_resample_slab_source_planes': (_i, [_i, _i, _i, _i, _p, _p]),
+    'mica_resample_slab_source_planes_general': (_i, [_i, _i, _i, _i, _p, _p]),
     'mica_bspline_resample_f32': (_i, [_p, _i, _i, _i, _i, _i, _p, _i, _i, _i, _i, _i, _p, _sz, _i, _p]),
     'mica_resample': (_i, [_p, _i, _i, _i, _i, _i, _i, _p, _i, _i, _i, _i, _i, _i, _p, _sz, _i, _p]),
     'mica_last_resample_path': (_i, [_i]),
@@ -63,6 +64,13 @@ SIGNATURES = {
     'mica_normalize_apply_f32': (_i, [_p, _p, _i64, _p, _p]),
     'mica_int_stats_workspace_bytes': (_sz, []),
     'mica_int_order_stats': (_i, [_p, _i, _i64, _p, _p]),
+    'mica_int_stats_init': (_i, [_p, _i, _i64, _p]),
+    'mica_int_stats_hist': (_i, [_p, _i, _i64, _p, _p]),
+    'mica_int_stats_hist_ptr': (_p, [_p]),
+    'mica_int_stats_pick': (_i, [_p, _i, _p]),
+    'mica_int_peer_buffer_bytes': (_sz, []),
+    'mica_int_stats_peer_publish': (_i, [_p, _i, _p, _i, _i, _i, _i, _p]),
+    'mica_int_stats_peer_sum': (_i, [_p, _i, _p, _i, _i, _i, _i, _p]),
     'mica_int_stats_result': (_i, [_p, C.POINTER(C.c_double), C.POINTER(C.c_double), C.POINTER(_i64), C.POINTER(_i),
                                    _p]),
     'mica_int_stats_result_async': (_i, [_p, _p, _p]),
@@ -80,6 +88,8 @@ SIGNATURES = {
     'mica_ipc_alloc': (_i, [_sz, C.POINTER(_p), _p]),
     'mica_halo_publish': (_i, [_p, _i64, _i64, _i64, _i64, _p, _i, _i, _i, _i, _i64, _p]),
     'mica_halo_pull': (_i, [_p, _i64, _p, _i64, _p, _i, _i, _i, _i, _i64, _p, _p]),
+    'mica_halo_publish_bytes': (_i, [_p, _i64, _i64, _i64, _i64, _p, _i, _i, _i, _i, _i64, _p]),
+    'mica_halo_pull_bytes': (_i, [_p, _i64, _p, _i64, _p, _i, _i, _i, _i, _i64, _p, _p]),
     'mica_af3_encode': (_i, [_p, _p, _p, _i64, _f, _f, _f, _i, _i, _i, _i, _i, _i, _i, _i, _p, _p, _p]),
     'mica_af3_bins_workspace_bytes': (_sz, [_i64, _i, _i, _i, C.POINTER(_i), _i, _i]),
     'mica_af3_bin_atoms': (_i, [_p, _p, _p, _i64, _f, _f, _f, _i, _i, _i, _i, _i, _i, C.POINTER(_i), _i, _i,

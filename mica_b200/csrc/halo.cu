@@ -33,34 +33,48 @@ struct HaloHeader {
 };
 static_assert(sizeof(HaloHeader) == kHaloFlagWords * sizeof(int), "header size");
 
-// buffer layout: HaloHeader | slot[parity 0..1][side 0..1][slot_elems] ; side 0 = planes for the
-// lower neighbour (the low end of my block), side 1 = planes for the upper neighbour
-__host__ __device__ __forceinline__ float* halo_slot(void* buf, int parity, int side, int64_t slot_elems) {
-  return reinterpret_cast<float*>(reinterpret_cast<char*>(buf) + sizeof(HaloHeader)) + (int64_t)(parity * 2 + side) * slot_elems;
+// buffer layout: HaloHeader | slot[parity 0..1][side 0..1][slot_bytes] ; side 0 = planes for the lower neighbour
+// (the low end of my block), side 1 = planes for the upper neighbour.  Slots are counted in bytes, so that planes of
+// any sample type (float32, int16, int8) fit; slot_bytes is a multiple of 16 here.
+__host__ __device__ __forceinline__ char* halo_slot(void* buf, int parity, int side, int64_t slot_bytes) {
+  return reinterpret_cast<char*>(buf) + sizeof(HaloHeader) + (int64_t)(parity * 2 + side) * slot_bytes;
 }
 
-__device__ __forceinline__ void copy_elems(float* __restrict__ dst, const float* __restrict__ src, int64_t n,
+// n bytes in words of W, then the tail bytes
+template <typename W>
+__device__ __forceinline__ void copy_words(char* __restrict__ dst, const char* __restrict__ src, int64_t n,
                                            int64_t tid, int64_t stride, bool remote) {
-  if (((((uintptr_t)dst) | ((uintptr_t)src)) & 15) == 0) {
-    const int64_t n4 = n >> 2;
-    const float4* s4 = reinterpret_cast<const float4*>(src);
-    float4* d4 = reinterpret_cast<float4*>(dst);
-    for (int64_t i = tid; i < n4; i += stride) d4[i] = remote ? __ldcv(s4 + i) : s4[i];
-    for (int64_t i = n4 * 4 + tid; i < n; i += stride) dst[i] = remote ? __ldcv(src + i) : src[i];
-  } else {
-    for (int64_t i = tid; i < n; i += stride) dst[i] = remote ? __ldcv(src + i) : src[i];
-  }
+  const int64_t nw = n / (int64_t)sizeof(W);
+  const W* s = reinterpret_cast<const W*>(src);
+  W* d = reinterpret_cast<W*>(dst);
+  for (int64_t i = tid; i < nw; i += stride) d[i] = remote ? __ldcv(s + i) : s[i];
+  for (int64_t i = nw * (int64_t)sizeof(W) + tid; i < n; i += stride)
+    dst[i] = remote ? (char)__ldcv(reinterpret_cast<const unsigned char*>(src) + i) : src[i];
 }
 
-// own: this rank's block of source planes.  n_lo / n_hi elements go to the lower / upper neighbour
-// from element offsets off_lo / off_hi of the block.
+// 16-byte vectors when both ends are 16-byte aligned (float32 planes always are: the assembled buffers and the slots
+// are), 4-byte words when they are 4-byte aligned, bytes otherwise
+__device__ __forceinline__ void copy_bytes(char* __restrict__ dst, const char* __restrict__ src, int64_t n,
+                                           int64_t tid, int64_t stride, bool remote) {
+  const uintptr_t a = ((uintptr_t)dst) | ((uintptr_t)src);
+  if ((a & 15) == 0)
+    copy_words<uint4>(dst, src, n, tid, stride, remote);
+  else if ((a & 3) == 0)
+    copy_words<unsigned>(dst, src, n, tid, stride, remote);
+  else
+    copy_words<unsigned char>(dst, src, n, tid, stride, remote);
+}
+
+// own: this rank's block of source planes.  n_lo / n_hi bytes go to the lower / upper neighbour from byte offsets
+// off_lo / off_hi of the block.
 __global__ void __launch_bounds__(256)
-halo_publish_kernel(const float* __restrict__ own, int64_t off_lo, int64_t n_lo, int64_t off_hi, int64_t n_hi,
-                    void* const* __restrict__ peers, int rank, int world, int parity, int epoch, int64_t slot_elems) {
+halo_publish_kernel(const char* __restrict__ own, int64_t off_lo, int64_t n_lo, int64_t off_hi, int64_t n_hi,
+                    void* const* __restrict__ peers, int rank, int world, int parity, int epoch, int64_t slot_bytes) {
   void* mine = peers[rank];
   const int64_t tid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x, stride = (int64_t)gridDim.x * blockDim.x;
-  if (rank > 0 && n_lo > 0) copy_elems(halo_slot(mine, parity, 0, slot_elems), own + off_lo, n_lo, tid, stride, false);
-  if (rank + 1 < world && n_hi > 0) copy_elems(halo_slot(mine, parity, 1, slot_elems), own + off_hi, n_hi, tid, stride, false);
+  if (rank > 0 && n_lo > 0) copy_bytes(halo_slot(mine, parity, 0, slot_bytes), own + off_lo, n_lo, tid, stride, false);
+  if (rank + 1 < world && n_hi > 0)
+    copy_bytes(halo_slot(mine, parity, 1, slot_bytes), own + off_hi, n_hi, tid, stride, false);
   __threadfence();
   __syncthreads();
   __shared__ bool last;
@@ -76,11 +90,11 @@ halo_publish_kernel(const float* __restrict__ own, int64_t off_lo, int64_t n_lo,
   }
 }
 
-// dst_lo receives n_lo elements published by the lower neighbour (its side 1), dst_hi n_hi elements
-// published by the upper neighbour (its side 0).  status: set to 1 when a neighbour timed out.
+// dst_lo receives n_lo bytes published by the lower neighbour (its side 1), dst_hi n_hi bytes published by the upper
+// neighbour (its side 0).  status: set to 1 when a neighbour timed out.
 __global__ void __launch_bounds__(256)
-halo_pull_kernel(float* __restrict__ dst_lo, int64_t n_lo, float* __restrict__ dst_hi, int64_t n_hi,
-                 void* const* __restrict__ peers, int rank, int world, int parity, int epoch, int64_t slot_elems,
+halo_pull_kernel(char* __restrict__ dst_lo, int64_t n_lo, char* __restrict__ dst_hi, int64_t n_hi,
+                 void* const* __restrict__ peers, int rank, int world, int parity, int epoch, int64_t slot_bytes,
                  long long timeout_cycles, int* __restrict__ status) {
   __shared__ int ok;
   const HaloHeader* h = reinterpret_cast<const HaloHeader*>(peers[rank]);
@@ -102,8 +116,8 @@ halo_pull_kernel(float* __restrict__ dst_lo, int64_t n_lo, float* __restrict__ d
     return;
   }
   const int64_t tid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x, stride = (int64_t)gridDim.x * blockDim.x;
-  if (want_lo) copy_elems(dst_lo, halo_slot(peers[rank - 1], parity, 1, slot_elems), n_lo, tid, stride, true);
-  if (want_hi) copy_elems(dst_hi, halo_slot(peers[rank + 1], parity, 0, slot_elems), n_hi, tid, stride, true);
+  if (want_lo) copy_bytes(dst_lo, halo_slot(peers[rank - 1], parity, 1, slot_bytes), n_lo, tid, stride, true);
+  if (want_hi) copy_bytes(dst_hi, halo_slot(peers[rank + 1], parity, 0, slot_bytes), n_hi, tid, stride, true);
 }
 
 }  // namespace mica
@@ -132,40 +146,56 @@ extern "C" int mica_ipc_alloc(size_t bytes, void** dev_ptr, void* ipc_handle_out
   return MICA_OK;
 }
 
-static int halo_grid(int64_t elems) {
-  int64_t want = ceil_div64(ceil_div64(elems, 4), 256 * 4);
+// one 16-byte vector per thread and pass, at most two CTAs per SM
+static int halo_grid(int64_t bytes) {
+  int64_t want = ceil_div64(ceil_div64(bytes, 16), 256 * 4);
   if (want < 1) want = 1;
   return (int)(want < 2 * kNumSMs ? want : 2 * kNumSMs);
+}
+
+static int64_t slot_stride(int64_t slot_bytes) { return (slot_bytes + 15) / 16 * 16; }
+
+extern "C" int mica_halo_publish_bytes(const void* own, int64_t off_lo, int64_t n_lo, int64_t off_hi, int64_t n_hi,
+                                       void* const* peer_bufs, int rank, int world, int parity, int epoch,
+                                       int64_t slot_bytes, mica_stream_t stream) {
+  MICA_REQUIRE(peer_bufs && (own || (n_lo == 0 && n_hi == 0)), "null pointer");
+  MICA_REQUIRE(world >= 1 && rank >= 0 && rank < world, "bad rank/world");
+  MICA_REQUIRE(parity == 0 || parity == 1, "parity must be 0 or 1");
+  MICA_REQUIRE(n_lo >= 0 && n_hi >= 0 && n_lo <= slot_bytes && n_hi <= slot_bytes, "halo larger than the slot");
+  if (world == 1) return MICA_OK;
+  halo_publish_kernel<<<halo_grid(n_lo + n_hi), 256, 0, (cudaStream_t)stream>>>(
+      (const char*)own, off_lo, n_lo, off_hi, n_hi, peer_bufs, rank, world, parity, epoch, slot_stride(slot_bytes));
+  MICA_LAUNCH_CHECK("halo_publish_kernel");
+  return MICA_OK;
+}
+
+extern "C" int mica_halo_pull_bytes(void* dst_lo, int64_t n_lo, void* dst_hi, int64_t n_hi, void* const* peer_bufs,
+                                    int rank, int world, int parity, int epoch, int64_t slot_bytes, int* status,
+                                    mica_stream_t stream) {
+  MICA_REQUIRE(peer_bufs && status, "null pointer");
+  MICA_REQUIRE(world >= 1 && rank >= 0 && rank < world, "bad rank/world");
+  MICA_REQUIRE(parity == 0 || parity == 1, "parity must be 0 or 1");
+  MICA_REQUIRE(n_lo >= 0 && n_hi >= 0 && n_lo <= slot_bytes && n_hi <= slot_bytes, "halo larger than the slot");
+  MICA_REQUIRE((n_lo == 0 || dst_lo) && (n_hi == 0 || dst_hi), "null destination");
+  if (world == 1) return MICA_OK;
+  const long long timeout_cycles = mica::peer_timeout_cycles();
+  halo_pull_kernel<<<halo_grid(n_lo + n_hi), 256, 0, (cudaStream_t)stream>>>(
+      (char*)dst_lo, n_lo, (char*)dst_hi, n_hi, peer_bufs, rank, world, parity, epoch, slot_stride(slot_bytes),
+      timeout_cycles, status);
+  MICA_LAUNCH_CHECK("halo_pull_kernel");
+  return MICA_OK;
 }
 
 extern "C" int mica_halo_publish(const float* own, int64_t off_lo, int64_t n_lo, int64_t off_hi, int64_t n_hi,
                                  void* const* peer_bufs, int rank, int world, int parity, int epoch,
                                  int64_t slot_elems, mica_stream_t stream) {
-  MICA_REQUIRE(peer_bufs && (own || (n_lo == 0 && n_hi == 0)), "null pointer");
-  MICA_REQUIRE(world >= 1 && rank >= 0 && rank < world, "bad rank/world");
-  MICA_REQUIRE(parity == 0 || parity == 1, "parity must be 0 or 1");
-  MICA_REQUIRE(n_lo >= 0 && n_hi >= 0 && n_lo <= slot_elems && n_hi <= slot_elems, "halo larger than the slot");
-  if (world == 1) return MICA_OK;
-  const int64_t padded = (slot_elems + 3) / 4 * 4;
-  halo_publish_kernel<<<halo_grid(n_lo + n_hi), 256, 0, (cudaStream_t)stream>>>(
-      own, off_lo, n_lo, off_hi, n_hi, peer_bufs, rank, world, parity, epoch, padded);
-  MICA_LAUNCH_CHECK("halo_publish_kernel");
-  return MICA_OK;
+  return mica_halo_publish_bytes(own, off_lo * 4, n_lo * 4, off_hi * 4, n_hi * 4, peer_bufs, rank, world, parity,
+                                 epoch, slot_elems * 4, stream);
 }
 
 extern "C" int mica_halo_pull(float* dst_lo, int64_t n_lo, float* dst_hi, int64_t n_hi, void* const* peer_bufs,
                               int rank, int world, int parity, int epoch, int64_t slot_elems, int* status,
                               mica_stream_t stream) {
-  MICA_REQUIRE(peer_bufs && status, "null pointer");
-  MICA_REQUIRE(world >= 1 && rank >= 0 && rank < world, "bad rank/world");
-  MICA_REQUIRE(parity == 0 || parity == 1, "parity must be 0 or 1");
-  MICA_REQUIRE(n_lo >= 0 && n_hi >= 0 && n_lo <= slot_elems && n_hi <= slot_elems, "halo larger than the slot");
-  MICA_REQUIRE((n_lo == 0 || dst_lo) && (n_hi == 0 || dst_hi), "null destination");
-  if (world == 1) return MICA_OK;
-  const int64_t padded = (slot_elems + 3) / 4 * 4;
-  const long long timeout_cycles = mica::peer_timeout_cycles();
-  halo_pull_kernel<<<halo_grid(n_lo + n_hi), 256, 0, (cudaStream_t)stream>>>(
-      dst_lo, n_lo, dst_hi, n_hi, peer_bufs, rank, world, parity, epoch, padded, timeout_cycles, status);
-  MICA_LAUNCH_CHECK("halo_pull_kernel");
-  return MICA_OK;
+  return mica_halo_pull_bytes(dst_lo, n_lo * 4, dst_hi, n_hi * 4, peer_bufs, rank, world, parity, epoch,
+                              slot_elems * 4, status, stream);
 }

@@ -16,6 +16,8 @@
 //   int_pick_kernel      one CTA: prefix sums of the histogram, the four order statistics, the float64 median and
 //                        percentile and the status word.
 //   int_normalize_kernel the float64 expression per voxel, float32 out.
+// Several GPUs (a z-slab partition) sum their histograms between hist and pick: over NCCL (mica_int_stats_hist_ptr)
+// or over NVLink peer memory with int_peer_publish_kernel + int_peer_sum_kernel (below).
 #include "common.cuh"
 
 namespace mica {
@@ -146,6 +148,7 @@ int_pick_kernel(IntStatsState* s, int bins, int offset) {
   __shared__ long long pre[kIntPickThreads + 1];
   __shared__ int key[2];
   __shared__ long long cum[2];
+  if (s->status != MICA_NORM_PENDING) return;   // a peer sum that timed out left a partial histogram
   const long long n = s->n_total;
   if (n <= 0) {
     if (threadIdx.x == 0) s->status = MICA_NORM_NO_POSITIVE;
@@ -250,22 +253,103 @@ static bool int_dtype_ok(int dtype) {
 }
 
 template <typename T>
-static int int_order_stats_t(const T* x, int64_t n, IntStatsState* s, cudaStream_t st) {
+static int int_hist_t(const T* x, int64_t n, IntStatsState* s, cudaStream_t st) {
   constexpr int bins = 1 << IntKey<T>::kBits;
-  int_stats_init_kernel<<<(bins + 255) / 256, 256, 0, st>>>(s, bins, (long long)n);
-  MICA_LAUNCH_CHECK("int_stats_init_kernel");
-  if (n > 0) {
-    const size_t smem = (size_t)bins * sizeof(unsigned short);
-    // per device/context attribute: set it on every call
-    MICA_CUDA(cudaFuncSetAttribute(int_hist_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    const int64_t slices = ceil_div64(n, kSlice);
-    const int64_t cap = (int64_t)kNumSMs * (bins > 256 ? 1 : 2);   // 128 KB of counters: one CTA per SM
-    int_hist_kernel<T><<<(unsigned)(slices < cap ? slices : cap), kIntHistThreads, smem, st>>>(x, (long long)n, s);
-    MICA_LAUNCH_CHECK("int_hist_kernel");
-  }
-  int_pick_kernel<<<1, kIntPickThreads, 0, st>>>(s, bins, IntKey<T>::kOffset);
-  MICA_LAUNCH_CHECK("int_pick_kernel");
+  if (n <= 0) return MICA_OK;
+  const size_t smem = (size_t)bins * sizeof(unsigned short);
+  // per device/context attribute: set it on every call
+  MICA_CUDA(cudaFuncSetAttribute(int_hist_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  const int64_t slices = ceil_div64(n, kSlice);
+  const int64_t cap = (int64_t)kNumSMs * (bins > 256 ? 1 : 2);   // 128 KB of counters: one CTA per SM
+  int_hist_kernel<T><<<(unsigned)(slices < cap ? slices : cap), kIntHistThreads, smem, st>>>(x, (long long)n, s);
+  MICA_LAUNCH_CHECK("int_hist_kernel");
   return MICA_OK;
+}
+
+// ---------------------------------------------------- histogram sum over peer memory
+// A z-slab partition needs the SUM of every rank's histogram between hist and pick.  Every rank owns one exported
+// buffer (mica_ipc_alloc of mica_int_peer_buffer_bytes) that all peers have mapped.  Two kernels, so that no kernel
+// waits for a flag another CTA of its own grid raises:
+//   int_peer_publish_kernel  copies the local histogram into this rank's slot `parity`; the last CTA to finish raises
+//                            this rank's epoch flag in every peer's buffer (st.release.sys).  It never waits.
+//   int_peer_sum_kernel      every CTA waits (ld.acquire.sys, bounded) for every peer's flag, then sums its slice of
+//                            bins from every peer's slot into the local state.  A peer that never arrives sets the
+//                            status to MICA_NORM_PEER_TIMEOUT, and int_pick_kernel leaves such a state alone.
+// Only the live bins travel: 2^8 for int8, 2^16 for int16 / uint16.
+// Slots alternate with the call epoch.  Rank r rewrites slot `parity` two calls later, in the publish of epoch e + 2.
+// It gets there only after its sum of epoch e + 1, which waited for every peer's flag of e + 1; a peer raises that
+// flag in its publish of e + 1, which its stream runs after its sum of epoch e has finished reading the slot.
+// The two kernels have entry points of their own: ranks emulated on ONE GPU (tests) must enqueue every rank's
+// publish before any rank's sum, or the spinning sum CTAs of one rank can hold the SMs (or a hardware queue) that
+// another rank's histogram and publish are waiting for.
+constexpr int kIntPeerMaxWorld = 64;
+constexpr int kIntPeerBinsPerCta = 2048;   // 32 CTAs for 2^16 bins: few CTAs spin while the peers publish
+
+struct IntPeerBuffer {
+  unsigned long long slot[2][kIntMaxBins];
+  int flag[kIntPeerMaxWorld];     // flag[p] = last epoch rank p has published
+  unsigned done[2];               // publish bookkeeping: CTAs finished, per parity
+  int pad[kIntPeerMaxWorld - 2];
+};
+
+__global__ void __launch_bounds__(256)
+int_peer_publish_kernel(const IntStatsState* __restrict__ s, IntPeerBuffer* const* __restrict__ peers, int rank,
+                        int world, int parity, int epoch, int bins) {
+  IntPeerBuffer* mine = peers[rank];
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < bins; i += gridDim.x * blockDim.x)
+    mine->slot[parity][i] = s->hist[i];
+  __threadfence();
+  __syncthreads();
+  __shared__ bool last;
+  if (threadIdx.x == 0) last = (atomicAdd(&mine->done[parity], 1u) == gridDim.x - 1);
+  __syncthreads();
+  if (!last) return;
+  if (threadIdx.x == 0) mine->done[parity] = 0;   // ready for this slot's next use (two calls later)
+  __threadfence_system();                         // every CTA's bins (observed through the counter) before the flags
+  __syncthreads();
+  if (threadIdx.x < world) st_release_sys(&peers[threadIdx.x]->flag[rank], epoch);
+}
+
+// grid = ceil(bins / kIntPeerBinsPerCta), block = 256: eight bins per thread
+__global__ void __launch_bounds__(256)
+int_peer_sum_kernel(IntStatsState* __restrict__ s, IntPeerBuffer* const* __restrict__ peers, int rank, int world,
+                    int parity, int epoch, int bins, long long timeout_cycles) {
+  __shared__ int ok;
+  __shared__ const unsigned long long* base[kIntPeerMaxWorld];
+  if (threadIdx.x == 0) ok = 1;
+  __syncthreads();
+  if (threadIdx.x < world) {     // wait for peer threadIdx.x
+    const int* f = &peers[rank]->flag[threadIdx.x];
+    const long long t0 = clock64();
+    while (ld_acquire_sys(f) - epoch < 0) {
+      if (clock64() - t0 > timeout_cycles) {
+        ok = 0;
+        break;
+      }
+    }
+    base[threadIdx.x] = peers[threadIdx.x]->slot[parity];
+  }
+  __threadfence_system();
+  __syncthreads();
+  if (!ok) {
+    if (threadIdx.x == 0) s->status = MICA_NORM_PEER_TIMEOUT;
+    return;
+  }
+  constexpr int kPer = kIntPeerBinsPerCta / 256;
+  const int b0 = blockIdx.x * kIntPeerBinsPerCta + threadIdx.x;
+  unsigned long long sum[kPer];
+#pragma unroll
+  for (int k = 0; k < kPer; ++k) sum[k] = 0ull;
+  for (int p = 0; p < world; ++p) {   // the kPer loads of one peer are issued before they are consumed
+    unsigned long long v[kPer];
+#pragma unroll
+    for (int k = 0; k < kPer; ++k) v[k] = b0 + k * 256 < bins ? __ldcv(base[p] + b0 + k * 256) : 0ull;
+#pragma unroll
+    for (int k = 0; k < kPer; ++k) sum[k] += v[k];
+  }
+#pragma unroll
+  for (int k = 0; k < kPer; ++k)
+    if (b0 + k * 256 < bins) s->hist[b0 + k * 256] = sum[k];
 }
 
 template <typename T>
@@ -283,15 +367,87 @@ using namespace mica;
 
 extern "C" size_t mica_int_stats_workspace_bytes(void) { return sizeof(IntStatsState) + 256; }
 
+static int int_bins(int dtype) { return dtype == MICA_DTYPE_I8 ? 256 : kIntMaxBins; }
+
+extern "C" int mica_int_stats_init(void* workspace, int dtype, int64_t n_total, mica_stream_t stream) {
+  MICA_REQUIRE(workspace, "null pointer");
+  MICA_REQUIRE(n_total >= 0, "negative n");
+  MICA_REQUIRE(int_dtype_ok(dtype), "integer order statistics take MICA_DTYPE_I8 / I16 / U16 (got dtype %d)", dtype);
+  const int bins = int_bins(dtype);
+  int_stats_init_kernel<<<(bins + 255) / 256, 256, 0, (cudaStream_t)stream>>>(int_state_of(workspace), bins,
+                                                                             (long long)n_total);
+  MICA_LAUNCH_CHECK("int_stats_init_kernel");
+  return MICA_OK;
+}
+
+extern "C" int mica_int_stats_hist(const void* x, int dtype, int64_t n_local, void* workspace, mica_stream_t stream) {
+  MICA_REQUIRE(workspace && (x || n_local == 0), "null pointer");
+  MICA_REQUIRE(n_local >= 0, "negative n");
+  MICA_REQUIRE(int_dtype_ok(dtype), "integer order statistics take MICA_DTYPE_I8 / I16 / U16 (got dtype %d)", dtype);
+  IntStatsState* s = int_state_of(workspace);
+  cudaStream_t st = (cudaStream_t)stream;
+  if (dtype == MICA_DTYPE_I8) return int_hist_t((const int8_t*)x, n_local, s, st);
+  if (dtype == MICA_DTYPE_I16) return int_hist_t((const int16_t*)x, n_local, s, st);
+  return int_hist_t((const uint16_t*)x, n_local, s, st);
+}
+
+extern "C" int64_t* mica_int_stats_hist_ptr(void* workspace) {
+  return workspace ? reinterpret_cast<int64_t*>(int_state_of(workspace)->hist) : nullptr;
+}
+
+extern "C" int mica_int_stats_pick(void* workspace, int dtype, mica_stream_t stream) {
+  MICA_REQUIRE(workspace, "null pointer");
+  MICA_REQUIRE(int_dtype_ok(dtype), "integer order statistics take MICA_DTYPE_I8 / I16 / U16 (got dtype %d)", dtype);
+  const int offset = dtype == MICA_DTYPE_I8 ? IntKey<int8_t>::kOffset
+                                            : (dtype == MICA_DTYPE_I16 ? IntKey<int16_t>::kOffset : IntKey<uint16_t>::kOffset);
+  int_pick_kernel<<<1, kIntPickThreads, 0, (cudaStream_t)stream>>>(int_state_of(workspace), int_bins(dtype), offset);
+  MICA_LAUNCH_CHECK("int_pick_kernel");
+  return MICA_OK;
+}
+
 extern "C" int mica_int_order_stats(const void* x, int dtype, int64_t n, void* workspace, mica_stream_t stream) {
   MICA_REQUIRE(workspace && (x || n == 0), "null pointer");
   MICA_REQUIRE(n >= 0, "negative n");
   MICA_REQUIRE(int_dtype_ok(dtype), "integer order statistics take MICA_DTYPE_I8 / I16 / U16 (got dtype %d)", dtype);
-  IntStatsState* s = int_state_of(workspace);
-  cudaStream_t st = (cudaStream_t)stream;
-  if (dtype == MICA_DTYPE_I8) return int_order_stats_t((const int8_t*)x, n, s, st);
-  if (dtype == MICA_DTYPE_I16) return int_order_stats_t((const int16_t*)x, n, s, st);
-  return int_order_stats_t((const uint16_t*)x, n, s, st);
+  if (int rc = mica_int_stats_init(workspace, dtype, n, stream)) return rc;
+  if (int rc = mica_int_stats_hist(x, dtype, n, workspace, stream)) return rc;
+  return mica_int_stats_pick(workspace, dtype, stream);
+}
+
+extern "C" size_t mica_int_peer_buffer_bytes(void) { return sizeof(IntPeerBuffer); }
+
+static int int_peer_args(void* workspace, int dtype, void* const* peer_bufs, int rank, int world, int parity) {
+  MICA_REQUIRE(workspace && peer_bufs, "null pointer");
+  MICA_REQUIRE(int_dtype_ok(dtype), "integer order statistics take MICA_DTYPE_I8 / I16 / U16 (got dtype %d)", dtype);
+  MICA_REQUIRE(world >= 1 && world <= kIntPeerMaxWorld && rank >= 0 && rank < world, "bad rank/world");
+  MICA_REQUIRE(parity == 0 || parity == 1, "parity must be 0 or 1");
+  return MICA_OK;
+}
+
+static unsigned int_peer_grid(int dtype) {
+  return (unsigned)((int_bins(dtype) + kIntPeerBinsPerCta - 1) / kIntPeerBinsPerCta);
+}
+
+extern "C" int mica_int_stats_peer_publish(const void* workspace, int dtype, void* const* peer_bufs, int rank,
+                                           int world, int parity, int epoch, mica_stream_t stream) {
+  if (int rc = int_peer_args((void*)workspace, dtype, peer_bufs, rank, world, parity)) return rc;
+  if (world == 1) return MICA_OK;
+  int_peer_publish_kernel<<<int_peer_grid(dtype), 256, 0, (cudaStream_t)stream>>>(
+      int_state_of(workspace), reinterpret_cast<IntPeerBuffer* const*>(peer_bufs), rank, world, parity, epoch,
+      int_bins(dtype));
+  MICA_LAUNCH_CHECK("int_peer_publish_kernel");
+  return MICA_OK;
+}
+
+extern "C" int mica_int_stats_peer_sum(void* workspace, int dtype, void* const* peer_bufs, int rank, int world,
+                                       int parity, int epoch, mica_stream_t stream) {
+  if (int rc = int_peer_args(workspace, dtype, peer_bufs, rank, world, parity)) return rc;
+  if (world == 1) return MICA_OK;
+  int_peer_sum_kernel<<<int_peer_grid(dtype), 256, 0, (cudaStream_t)stream>>>(
+      int_state_of(workspace), reinterpret_cast<IntPeerBuffer* const*>(peer_bufs), rank, world, parity, epoch,
+      int_bins(dtype), mica::peer_timeout_cycles());
+  MICA_LAUNCH_CHECK("int_peer_sum_kernel");
+  return MICA_OK;
 }
 
 extern "C" int mica_int_stats_result_async(const void* workspace, void* host_record, mica_stream_t stream) {

@@ -42,7 +42,9 @@
 //
 // Integer maps (int8 / int16 / uint16, DESIGN.md D12) always take the general path: its z prefilter reads the
 // map's own type, and its interpolation kernels store with SciPy's integer rule (store_out).  The fast path's
-// float32 coefficients are not exact enough to round to the reference's integers.
+// float32 coefficients are not exact enough to round to the reference's integers.  Given a block of a longer z line
+// (a z-slab), an integer map's z prefilter numbers its segments on the whole line (seg16_plan), so the slab gets the
+// whole map's bits; float32 blocks on the general path are prefiltered as lines of their own.
 #include <cuda.h>
 #include <stdlib.h>
 
@@ -243,54 +245,60 @@ prefilter_rows(double* __restrict__ data, int n, int64_t n_rows) {
 constexpr int kHorizon = 30;
 constexpr int kMinSegLine = 96;     // shorter lines take the one-thread-per-line kernels
 
-// Filters samples [k0, k1) of one line in place; all threads of the block call this together
-// (three block-wide barriers inside).  `line` points at sample 0, `stride` in doubles.
-__device__ __forceinline__ void iir_segment(double* line, int n, int stride, int k0, int k1, bool active) {
+// Filters samples [k0, k1) of one line of n samples in place; all threads of the block call this together (three
+// block-wide barriers inside).  `line` points at sample g0 (a block of a longer line holds samples [g0, ...); g0 = 0
+// for a whole line), `stride` in doubles, k0 / k1 are numbers on the whole line.  `causal` runs the warm-up and the
+// causal sweep (up to sample causal_end, exclusive), `anti` (which implies causal, and causal_end >= k1) the
+// anticausal ones as well: a segment whose causal values another segment's anticausal warm-up reads, but whose own
+// coefficients nobody needs, runs the causal half only, and only as far as those values go.
+__device__ __forceinline__ void iir_segment(double* line, int g0, int n, int stride, int k0, int k1, int causal_end,
+                                            bool causal, bool anti) {
   const double z = kPole;
   double st = 0.0;
-  if (active) {   // causal state entering the segment: sum_j z^j s[k0-1-j], mirrored below 0
+  if (causal) {   // causal state entering the segment: sum_j z^j s[k0-1-j], mirrored below 0
     for (int m = kHorizon - 1; m >= 0; --m) {
       int idx = k0 - 1 - m;
       idx = idx < 0 ? -idx : idx;
-      st = fma(z, st, line[idx * stride]);
+      st = fma(z, st, line[(idx - g0) * stride]);
     }
   }
   __syncthreads();   // every warm-up read of raw samples is done before anyone overwrites them
-  if (active) {
+  if (causal) {
+    const int kc = min(k1, causal_end);
 #pragma unroll 4
-    for (int k = k0; k < k1; ++k) {
-      st = fma(z, st, line[k * stride]);
-      line[k * stride] = st;
+    for (int k = k0; k < kc; ++k) {
+      st = fma(z, st, line[(k - g0) * stride]);
+      line[(k - g0) * stride] = st;
     }
   }
   __syncthreads();
   bool at_end = false;
-  if (active) {   // anticausal state just above the segment
-    if (k1 >= n) {
+  if (anti) {   // anticausal state just above the segment
+    if (k1 >= n) {   // the end initialisation, read here: sample n - 2 may belong to the segment below
       at_end = true;
+      st = (z / (z * z - 1.0)) * (line[(n - 1 - g0) * stride] + z * line[(n - 2 - g0) * stride]);
     } else {
       int kk = k1 + kHorizon;
       int k = kk - 1;
       st = 0.0;
       if (kk >= n) {  // the exact end initialisation is within reach: start from it
-        st = (z / (z * z - 1.0)) * (line[(n - 1) * stride] + z * line[(n - 2) * stride]);
+        st = (z / (z * z - 1.0)) * (line[(n - 1 - g0) * stride] + z * line[(n - 2 - g0) * stride]);
         k = n - 2;
       }
-      for (; k >= k1; --k) st = fma(z, st, -z * line[k * stride]);   // z (st - c): one FMA on the chain
+      for (; k >= k1; --k) st = fma(z, st, -z * line[(k - g0) * stride]);   // z (st - c): one FMA on the chain
     }
   }
   __syncthreads();
-  if (active) {
+  if (anti) {
     int k = k1 - 1;
     if (at_end) {
-      st = (z / (z * z - 1.0)) * (line[(n - 1) * stride] + z * line[(n - 2) * stride]);
-      line[(n - 1) * stride] = st;
+      line[(n - 1 - g0) * stride] = st;
       k = n - 2;
     }
 #pragma unroll 4
     for (; k >= k0; --k) {
-      st = fma(z, st, -z * line[k * stride]);
-      line[k * stride] = st;
+      st = fma(z, st, -z * line[(k - g0) * stride]);
+      line[(k - g0) * stride] = st;
     }
   }
 }
@@ -363,11 +371,14 @@ __device__ __forceinline__ void iir_segment_reg(double* line, int n, int k0, int
   }
 }
 
-// lines along a strided axis.  grid = (ceil(n_cols / L), n_outer), block = 256, tile [n][L],
-// 256 / L segments per line
+// lines along a strided axis.  grid = (ceil(n_cols / L), n_outer), block = 256, tile [n][L], 256 / L segments per
+// line.  The tile holds samples [g0, g0 + n) of lines of ng samples (g0 = 0, ng = n for whole lines); the segments are
+// those of the WHOLE line, seg_lo .. seg_causal_hi run the causal sweep up to causal_end, seg_lo .. seg_out_hi both
+// (seg16_plan).
 template <typename TIn, int L>
 __global__ void __launch_bounds__(256)
-prefilter_cols_seg(const TIn* __restrict__ in, double* __restrict__ out, int n, int n_cols, ColStrides S) {
+prefilter_cols_seg(const TIn* __restrict__ in, double* __restrict__ out, int n, int n_cols, ColStrides S, int g0,
+                   int ng, int seg_lo, int seg_causal_hi, int seg_out_hi, int causal_end) {
   extern __shared__ double tile[];
   constexpr int kSegs = 256 / L;
   const int col0 = blockIdx.x * L;
@@ -380,9 +391,10 @@ prefilter_cols_seg(const TIn* __restrict__ in, double* __restrict__ out, int n, 
     for (int k = seg; k < n; k += kSegs) tile[k * L + j] = (double)p[(int64_t)k * S.line_in] * kGain;
   }
   __syncthreads();
-  const int len = (n + kSegs - 1) / kSegs;
-  const int k0 = seg * len, k1 = min(n, k0 + len);
-  iir_segment(tile + j, n, L, k0, k1, j < ncol && k0 < k1);
+  const int len = (ng + kSegs - 1) / kSegs;
+  const int k0 = seg * len, k1 = min(ng, k0 + len);
+  const bool on = j < ncol && k0 < k1 && seg >= seg_lo;
+  iir_segment(tile + j, g0, ng, L, k0, k1, causal_end, on && seg <= seg_causal_hi, on && seg <= seg_out_hi);
   __syncthreads();
   if (j < ncol) {
     double* q = out + base_out + j;
@@ -407,7 +419,7 @@ prefilter_rows_seg(double* __restrict__ data, int n, int64_t n_rows) {
   const int r = threadIdx.x & (L - 1), seg = threadIdx.x / L;
   const int len = (n + kSegs - 1) / kSegs;
   const int k0 = seg * len, k1 = min(n, k0 + len);
-  iir_segment(tile + r * pitch, n, 1, k0, k1, r < nrow && k0 < k1);
+  iir_segment(tile + r * pitch, 0, n, 1, k0, k1, n, r < nrow && k0 < k1, r < nrow && k0 < k1);
   __syncthreads();
   for (int rr = threadIdx.x >> 5; rr < nrow; rr += 8)
     for (int k = threadIdx.x & 31; k < n; k += 32) g[(int64_t)rr * n + k] = tile[rr * pitch + k];
@@ -1234,7 +1246,8 @@ static int launch_cols_f64(const TIn* in, double* out, int n, int64_t line_strid
   const size_t per_col = (size_t)n * sizeof(double);
   if (!g_force_generic && n >= kMinSegLine && per_col * 32 <= kMaxTileBytes)
     return launch_pass(pass, MICA_RS_COLS_SEG16, "prefilter_cols", prefilter_cols_seg<TIn, 16>,
-                       dim3((n_cols + 15) / 16, n_outer), 256, per_col * 16, st, in, out, n, n_cols, S);
+                       dim3((n_cols + 15) / 16, n_outer), 256, per_col * 16, st, in, out, n, n_cols, S, 0, n, 0, 15,
+                       15, n);
   if (per_col * 32 <= kMaxTileBytes)
     return launch_pass(pass, MICA_RS_COLS32, "prefilter_cols", prefilter_cols<TIn, 32>,
                        dim3((n_cols + 31) / 32, n_outer), 256, per_col * 32, st, in, out, n, n_cols, S);
@@ -1243,6 +1256,51 @@ static int launch_cols_f64(const TIn* in, double* out, int n, int64_t line_strid
                        dim3((n_cols + 7) / 8, n_outer), 256, per_col * 8, st, in, out, n, n_cols, S);
   return launch_pass(pass, MICA_RS_COLS_GLOBAL, "prefilter_cols", prefilter_cols_global<TIn>,
                      dim3((n_cols + 127) / 128, n_outer), 128, 0, st, in, out, n, line_stride, n_cols, outer_stride);
+}
+
+// Lines prefilter_cols_seg<., 16> takes on one GPU (launch_cols_f64): kMinSegLine .. kMaxSeg16Line samples.  Only
+// these can be cut into blocks with the whole line's bits: the kernels of shorter and longer lines (iir_line) run
+// one causal recursion from sample 0 to the end.
+constexpr int kMaxSeg16Line = (int)(kMaxTileBytes / (32 * sizeof(double)));   // 800
+
+// The segments of prefilter_cols_seg<., 16> (16 per line of ng samples, numbered on the whole line) that a block must
+// run so that global samples [need_lo, need_hi] get the whole line's coefficients, and the raw samples
+// [raw_lo, raw_hi) they read.  The segments that hold the needed samples run both sweeps.  The anticausal warm-up of
+// the last of them reads the CAUSAL values of the kHorizon samples above it, or of everything up to the line's end
+// when the exact end initialisation is within reach: the segments that hold those run the causal sweep, up to the
+// last such sample (causal_end).  The last
+// segment's end initialisation reads sample ng - 2, which may lie in the segment below.  Every causal sweep reads
+// the kHorizon raw samples below its segment, mirrored at sample 0.
+struct Seg16Plan {
+  int seg_lo, seg_causal_hi, seg_out_hi, causal_end, raw_lo, raw_hi;
+};
+
+static Seg16Plan seg16_plan(int ng, int need_lo, int need_hi) {
+  const int len = (ng + 15) / 16;
+  Seg16Plan p;
+  p.seg_lo = need_lo / len;
+  p.seg_out_hi = need_hi / len;
+  const int k1 = min(ng, (p.seg_out_hi + 1) * len);
+  int last = k1 - 1;                                   // last sample whose causal value is read
+  if (k1 < ng) last = k1 + kHorizon >= ng ? ng - 1 : k1 + kHorizon - 1;
+  if (k1 >= ng && ng >= 2 && (ng - 2) / len < p.seg_lo) p.seg_lo = (ng - 2) / len;
+  p.seg_causal_hi = last / len;
+  p.causal_end = last + 1;
+  const int k0 = p.seg_lo * len;
+  p.raw_lo = max(0, k0 - kHorizon);
+  p.raw_hi = min(ng, max(p.causal_end, k0 < kHorizon ? kHorizon - k0 + 1 : 0));
+  return p;
+}
+
+// z pass of the general path on a block [g0, g0 + n) of lines of ng samples (an integer map in a z-slab): always
+// prefilter_cols_seg<., 16>, the kernel the whole line takes, with its segments numbered on the whole line
+template <typename TIn>
+static int launch_cols_seg_block(const TIn* in, double* out, int n, int64_t plane, int g0, int ng, const Seg16Plan& p,
+                                 cudaStream_t st) {
+  const ColStrides S{plane, plane, 0, 0};
+  return launch_pass(kPassZ, MICA_RS_COLS_SEG16, "prefilter_cols", prefilter_cols_seg<TIn, 16>,
+                     dim3((unsigned)((plane + 15) / 16), 1), 256, (size_t)n * sizeof(double) * 16, st, in, out, n,
+                     (int)plane, S, g0, ng, p.seg_lo, p.seg_causal_hi, p.seg_out_hi, p.causal_end);
 }
 
 // a row that fits no 4-row shared-memory tile is swept in global memory, one row per CTA along grid y
@@ -1329,6 +1387,23 @@ extern "C" int mica_resample_slab_source_planes(int sz, int nz, int dst_z0, int 
   const int lo = c_lo / len * len - kColH, hi = c_hi / len * len + kColLen + kColH;
   *src_lo = lo < 0 ? 0 : lo;
   *src_hi = hi > sz ? sz : hi;
+  return MICA_OK;
+}
+
+// The general path's counterpart (integer maps): the block that holds every raw sample the segments of
+// prefilter_cols_seg<., 16> that output planes [dst_z0, dst_z0 + dst_nz_local) need read (seg16_plan).
+extern "C" int mica_resample_slab_source_planes_general(int sz, int nz, int dst_z0, int dst_nz_local, int* src_lo,
+                                                        int* src_hi) {
+  MICA_REQUIRE(src_lo && src_hi, "null pointer");
+  MICA_REQUIRE(sz >= kMinSegLine && sz <= kMaxSeg16Line,
+               "a z line of %d samples is prefiltered in one piece on the general path: only lines of %d..%d "
+               "samples can be cut into blocks with the whole line's bits", sz, kMinSegLine, kMaxSeg16Line);
+  MICA_REQUIRE(nz > 0 && dst_z0 >= 0 && dst_nz_local > 0 && dst_z0 + dst_nz_local <= nz, "bad slab");
+  int c_lo, c_hi;
+  needed_planes(sz, nz, dst_z0, dst_nz_local, 0, sz, &c_lo, &c_hi);
+  const Seg16Plan p = seg16_plan(sz, c_lo, c_hi);
+  *src_lo = p.raw_lo;
+  *src_hi = p.raw_hi;
   return MICA_OK;
 }
 
@@ -1471,13 +1546,30 @@ static int resample_fast(const float* src, int sz, int sy, int sx, int src_z0, i
 
 // general order-3 path: float64 coefficients prefiltered in place along z, y and x; then the marching gather when the
 // y span of an 8-row output tile fits the staged rows and every axis has a full 4-sample window, else one thread per
-// output voxel
+// output voxel.  The y and x passes run on the planes the z taps read (needed_planes) only.  An integer map given a
+// block of a longer z line runs its z pass on the whole line's segment grid (seg16_plan): the block's planes come out
+// with the whole map's bits.  A float32 block is prefiltered as a line of its own, as it always has been.
 template <typename T, typename Taps>
-static int resample_general(const T* src, int sy, int sx, int src_nz_local, T* dst, int ny, int nx, int dst_nz_local,
-                            const Tap* tz, const Tap* ty, const Tap* tx, ZWin* zw, double* coeff, cudaStream_t st,
-                            const Taps& taps) {
+static int resample_general(const T* src, int sz, int sy, int sx, int src_z0, int src_nz_local, T* dst, int nz, int ny,
+                            int nx, int dst_z0, int dst_nz_local, const Tap* tz, const Tap* ty, const Tap* tx, ZWin* zw,
+                            double* coeff, cudaStream_t st, const Taps& taps) {
   const int64_t plane = (int64_t)sy * sx;
   MICA_REQUIRE(plane <= 0x7fffffffLL && src_nz_local <= 65535, "source plane too large");
+  int c_lo, c_hi;
+  needed_planes(sz, nz, dst_z0, dst_nz_local, src_z0, src_nz_local, &c_lo, &c_hi);
+  const int l0 = c_lo - src_z0, cnt = c_hi - c_lo + 1;
+  const bool block = !std::is_same<T, float>::value && src_nz_local < sz;
+  Seg16Plan zp{};
+  if (block) {
+    MICA_REQUIRE(sz >= kMinSegLine && sz <= kMaxSeg16Line,
+                 "an integer map's z line of %d samples is prefiltered in one piece: a block of it cannot give the "
+                 "whole map's bits (only lines of %d..%d samples can be cut)", sz, kMinSegLine, kMaxSeg16Line);
+    zp = seg16_plan(sz, c_lo, c_hi);
+    MICA_REQUIRE(src_z0 <= zp.raw_lo && src_z0 + src_nz_local >= zp.raw_hi,
+                 "source planes [%d, %d) do not hold the prefilter windows [%d, %d) of output planes [%d, %d) "
+                 "(mica_resample_slab_source_planes_general)", src_z0, src_z0 + src_nz_local, zp.raw_lo, zp.raw_hi,
+                 dst_z0, dst_z0 + dst_nz_local);
+  }
   const int span_y = y_span(sy, ny);
   const bool march = !g_force_generic && src_nz_local >= 4 && sy >= 4 && sx >= 4 && span_y <= 16;
   dim3 mgrid;
@@ -1496,11 +1588,16 @@ static int resample_general(const T* src, int sy, int sx, int src_nz_local, T* d
 
   if (int rc = taps()) return rc;
   // axis 0 (z): lines of length src_nz_local, stride plane; reads the map's type, writes float64
-  if (int rc = launch_cols_f64<T>(src, coeff, src_nz_local, plane, (int)plane, 0, 1, st, kPassZ)) return rc;
-  // axis 1 (y): per z plane, lines of length sy, stride sx
-  if (int rc = launch_cols_f64<double>(coeff, coeff, sy, sx, sx, plane, src_nz_local, st, kPassY)) return rc;
+  if (block) {
+    if (int rc = launch_cols_seg_block<T>(src, coeff, src_nz_local, plane, src_z0, sz, zp, st)) return rc;
+  } else if (int rc = launch_cols_f64<T>(src, coeff, src_nz_local, plane, (int)plane, 0, 1, st, kPassZ)) {
+    return rc;
+  }
+  // axis 1 (y): per needed z plane, lines of length sy, stride sx
+  double* c0 = coeff + (size_t)l0 * plane;
+  if (int rc = launch_cols_f64<double>(c0, c0, sy, sx, sx, plane, cnt, st, kPassY)) return rc;
   // axis 2 (x): contiguous rows
-  if (int rc = launch_rows(coeff, sx, (int64_t)src_nz_local * sy, st)) return rc;
+  if (int rc = launch_rows(c0, sx, (int64_t)cnt * sy, st)) return rc;
   if (!march)
     return launch_pass(kPassInterp, MICA_RS_GATHER3, "gather3_kernel", gather3_kernel<T>,
                        dim3((nx + 127) / 128, ny, dst_nz_local), 128, 0, st, coeff, sy, sx, tz, ty, tx, dst, ny, nx);
@@ -1564,7 +1661,8 @@ static int resample_impl(const T* src, int sz, int sy, int sx, int src_z0, int s
       return resample_fast(src, sz, sy, sx, src_z0, src_nz_local, dst, nz, ny, nx, dst_z0, dst_nz_local, tz, ty, tx,
                            zw, coeff, st, taps);
   }
-  return resample_general(src, sy, sx, src_nz_local, dst, ny, nx, dst_nz_local, tz, ty, tx, zw, coeff, st, taps);
+  return resample_general(src, sz, sy, sx, src_z0, src_nz_local, dst, nz, ny, nx, dst_z0, dst_nz_local, tz, ty, tx, zw,
+                          coeff, st, taps);
 }
 
 extern "C" int mica_resample(const void* src, int src_dtype, int sz, int sy, int sx, int src_z0, int src_nz_local,

@@ -94,6 +94,15 @@ def resample_slab_source_planes(sz: int, nz: int, dst_z0: int, dst_nz_local: int
     return int(lo.value), int(hi.value)
 
 
+def resample_slab_source_planes_general(sz: int, nz: int, dst_z0: int, dst_nz_local: int):
+    """The same for the general path that integer maps take (16 prefilter segments per z line, numbered on the
+    whole line).  Raises MicaError unless 96 <= sz <= 800."""
+    lo, hi = C.c_int(), C.c_int()
+    check(lib.mica_resample_slab_source_planes_general(int(sz), int(nz), int(dst_z0), int(dst_nz_local),
+                                                       C.byref(lo), C.byref(hi)), 'resample_slab_source_planes_general')
+    return int(lo.value), int(hi.value)
+
+
 #: sample types of the maps resample / normalize take -> MICA_DTYPE_* code
 MAP_DTYPES = {torch.float32: _lib.DTYPE_F32, torch.int8: _lib.DTYPE_I8, torch.int16: _lib.DTYPE_I16,
               torch.uint16: _lib.DTYPE_U16}
@@ -228,7 +237,7 @@ class OrderStats:
 class IntOrderStats:
     """Device-resident state of the exact order statistics of an integer map (int8 / int16 / uint16, DESIGN.md
     D12): one histogram pass and one pick give the float64 median and 99.9 percentile NumPy computes on the
-    integer array.  Single GPU only."""
+    integer array."""
 
     RESULT_BYTES = _lib.INT_STATS_RESULT_BYTES
 
@@ -247,10 +256,31 @@ class IntOrderStats:
         dt = x.dtype if isinstance(x, torch.Tensor) else torch.int16
         return _dev(x, dt, name), MAP_DTYPES[dt]
 
+    def hist_view(self, dtype) -> torch.Tensor:
+        """int64 view of the live histogram bins of a ``dtype`` map (2^8 or 2^16) that a multi-GPU run sums
+        between hist and pick."""
+        bins = 256 if dtype == torch.int8 else 65536
+        off = lib.mica_int_stats_hist_ptr(self._p) - self.ws.data_ptr()
+        return self.ws[off:off + 8 * bins].view(torch.int64)
+
     @device_guard
-    def run(self, x: torch.Tensor):
+    def run(self, x: torch.Tensor, n_total: int | None = None, all_reduce=None, peer=None):
+        """Multi-GPU (``x`` = this rank's voxels, ``n_total`` = all ranks'): the histograms of all ranks are
+        summed between hist and pick, either by ``peer`` (a peer.PeerIntHistogram: over NVLink peer memory) or by
+        ``all_reduce(hist_int64_tensor)`` (torch.distributed.all_reduce over NCCL), both on the current stream."""
         p_x, code = self._int_map(x, 'x')
-        check(lib.mica_int_order_stats(p_x, code, x.numel(), self._p, _stream()), 'int_order_stats')
+        st = _stream()
+        if all_reduce is None and peer is None:
+            check(lib.mica_int_order_stats(p_x, code, x.numel(), self._p, st), 'int_order_stats')
+            return self
+        n_total = x.numel() if n_total is None else int(n_total)
+        check(lib.mica_int_stats_init(self._p, code, n_total, st), 'int_stats_init')
+        check(lib.mica_int_stats_hist(p_x, code, x.numel(), self._p, st), 'int_stats_hist')
+        if peer is not None:
+            peer.reduce(self, code)
+        else:
+            all_reduce(self.hist_view(x.dtype))
+        check(lib.mica_int_stats_pick(self._p, code, st), 'int_stats_pick')
         return self
 
     @device_guard

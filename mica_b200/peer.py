@@ -4,7 +4,8 @@ One buffer per rank, mapped by the other ranks of the box through CUDA IPC, so t
 kernels can publish / signal / wait / read over NVLink inside a kernel instead of an NCCL call:
 
   PeerHistogram   ``mica_select_peer_reduce``: the histogram all-reduce of every radix round;
-  PeerHalo        ``mica_halo_publish`` / ``mica_halo_pull``: the z-halo planes of the source map;
+  PeerIntHistogram ``mica_int_stats_peer_publish`` / ``_sum``: the histogram sum of an integer map's statistics;
+  PeerHalo        ``mica_halo_publish_bytes`` / ``mica_halo_pull_bytes``: the z-halo planes of the source map;
   PeerVolumes     the stitched output volumes of every rank, so that ``postproc_stitch`` can store a
                   core straight into the volumes of the rank that owns it (config 5: cubes dealt out
                   evenly, softmax/argmax + stitch fused with its exchange).
@@ -107,10 +108,48 @@ class PeerHistogram(_IpcGroup):
                   'select_peer_reduce')
 
 
+class PeerIntHistogram(_IpcGroup):
+    """The histogram sum of ``ops.IntOrderStats`` over peer memory: a publish kernel and a sum kernel per map."""
+
+    def __init__(self, device, rank: int, world: int, group=None, _emulated=None):
+        super().__init__(device, rank, world, lib.mica_int_peer_buffer_bytes(), group, _emulated)
+        self.epoch = 0
+
+    @classmethod
+    def emulate(cls, device, world: int):
+        """``world`` groups for ranks 0..world-1 living in this process (tests)."""
+        ptrs = cls._emulate_ptrs(device, world, lib.mica_int_peer_buffer_bytes())
+        groups = [cls(device, r, world, _emulated=ptrs) for r in range(world)]
+        groups[0]._owned_all = ptrs                     # freed with the first group
+        return groups
+
+    def publish(self, stats, dtype_code: int, stream=None):
+        """Step 1 (never waits): make this rank's histogram (``stats``, an ops.IntOrderStats after its hist)
+        available to the peers, for the next epoch."""
+        self.epoch += 1
+        with torch.cuda.device(self.device):
+            check(lib.mica_int_stats_peer_publish(stats._p, int(dtype_code), C.c_void_p(self.table.data_ptr()),
+                                                  self.rank, self.world, self.epoch & 1, self.epoch,
+                                                  self._stream(stream)), 'int_stats_peer_publish')
+
+    def sum(self, stats, dtype_code: int, stream=None):
+        """Step 2: wait for every peer's histogram of the current epoch and sum them into ``stats``."""
+        with torch.cuda.device(self.device):
+            check(lib.mica_int_stats_peer_sum(stats._p, int(dtype_code), C.c_void_p(self.table.data_ptr()),
+                                              self.rank, self.world, self.epoch & 1, self.epoch,
+                                              self._stream(stream)), 'int_stats_peer_sum')
+
+    def reduce(self, stats, dtype_code: int, stream=None):
+        """Both steps, in stream order: one rank per process (the ranks of one GPU must publish first, all of them)."""
+        self.publish(stats, dtype_code, stream)
+        self.sum(stats, dtype_code, stream)
+
+
 class PeerHalo(_IpcGroup):
-    """Source-halo exchange with the two z-neighbours over peer memory.  ``slot_elems``: capacity (float32
-    elements) of one direction's halo; a plan that needs more (or planes from a rank that is not a
-    neighbour) falls back to ``slab.exchange_source_halo`` (NCCL send/recv)."""
+    """Source-halo exchange with the two z-neighbours over peer memory.  ``slot_elems``: capacity of one
+    direction's halo in 4-byte words (float32 elements; planes of a narrower type fill it byte by byte); a plan
+    that needs more (or planes from a rank that is not a neighbour) falls back to ``slab.exchange_source_halo``
+    (NCCL send/recv)."""
 
     def __init__(self, device, rank: int, world: int, slot_elems: int, group=None, _emulated=None):
         self.slot_elems = int(slot_elems)
@@ -139,43 +178,48 @@ class PeerHalo(_IpcGroup):
         return (out['send'].get(rank - 1), out['send'].get(rank + 1), out['recv'].get(rank - 1),
                 out['recv'].get(rank + 1))
 
-    def fits(self, plan, rank):
+    @staticmethod
+    def slot_words(plan, rank_range_planes: int, itemsize: int = 4) -> int:
+        """4-byte words a slot needs for ``rank_range_planes`` source planes of ``itemsize``-byte samples."""
+        return -(-rank_range_planes * plan.src_shape[1] * plan.src_shape[2] * int(itemsize) // 4)
+
+    def fits(self, plan, rank, itemsize: int = 4):
         np_ = self.neighbour_plan(plan, rank)
         if np_ is None:
             return False
-        plane = plan.src_shape[1] * plan.src_shape[2]
-        return all(r is None or (r[1] - r[0]) * plane <= self.slot_elems for r in np_)
+        return all(r is None or self.slot_words(plan, r[1] - r[0], itemsize) <= self.slot_elems for r in np_)
 
     def publish(self, own: torch.Tensor, plan, stream=None):
         """Step 1 (never waits): make the boundary planes of ``own`` (this rank's block) available."""
         me = plan.ranks[self.rank]
         s_lo, s_hi, _, _ = self.neighbour_plan(plan, self.rank)
-        plane = plan.src_shape[1] * plan.src_shape[2]
+        plane = plan.src_shape[1] * plan.src_shape[2] * own.element_size()       # bytes
         self.epoch += 1
         off_lo, n_lo = ((s_lo[0] - me.own_lo) * plane, (s_lo[1] - s_lo[0]) * plane) if s_lo else (0, 0)
         off_hi, n_hi = ((s_hi[0] - me.own_lo) * plane, (s_hi[1] - s_hi[0]) * plane) if s_hi else (0, 0)
         with torch.cuda.device(self.device):
-            check(lib.mica_halo_publish(C.c_void_p(own.data_ptr()), off_lo, n_lo, off_hi, n_hi,
-                                        C.c_void_p(self.table.data_ptr()), self.rank, self.world, self.epoch & 1,
-                                        self.epoch, self.slot_elems, self._stream(stream)), 'halo_publish')
+            check(lib.mica_halo_publish_bytes(C.c_void_p(own.data_ptr()), off_lo, n_lo, off_hi, n_hi,
+                                              C.c_void_p(self.table.data_ptr()), self.rank, self.world,
+                                              self.epoch & 1, self.epoch, 4 * self.slot_elems, self._stream(stream)),
+                  'halo_publish')
 
     def pull(self, buf: torch.Tensor, plan, stream=None):
         """Step 2: wait for the neighbours' planes of the current epoch and copy them into ``buf``
         (global source planes [src_lo, src_hi) of this rank)."""
         me = plan.ranks[self.rank]
         _, _, r_lo, r_hi = self.neighbour_plan(plan, self.rank)
-        plane = plan.src_shape[1] * plan.src_shape[2]
-        flat = buf.view(-1)
+        plane = plan.src_shape[1] * plan.src_shape[2] * buf.element_size()       # bytes
+        flat = buf.view(-1).view(torch.uint8)
         d_lo = flat[(r_lo[0] - me.src_lo) * plane:] if r_lo else None
         d_hi = flat[(r_hi[0] - me.src_lo) * plane:] if r_hi else None
         with torch.cuda.device(self.device):
-            check(lib.mica_halo_pull(C.c_void_p(d_lo.data_ptr()) if r_lo else None,
-                                     (r_lo[1] - r_lo[0]) * plane if r_lo else 0,
-                                     C.c_void_p(d_hi.data_ptr()) if r_hi else None,
-                                     (r_hi[1] - r_hi[0]) * plane if r_hi else 0,
-                                     C.c_void_p(self.table.data_ptr()), self.rank, self.world, self.epoch & 1,
-                                     self.epoch, self.slot_elems, C.c_void_p(self.status.data_ptr()),
-                                     self._stream(stream)), 'halo_pull')
+            check(lib.mica_halo_pull_bytes(C.c_void_p(d_lo.data_ptr()) if r_lo else None,
+                                           (r_lo[1] - r_lo[0]) * plane if r_lo else 0,
+                                           C.c_void_p(d_hi.data_ptr()) if r_hi else None,
+                                           (r_hi[1] - r_hi[0]) * plane if r_hi else 0,
+                                           C.c_void_p(self.table.data_ptr()), self.rank, self.world, self.epoch & 1,
+                                           self.epoch, 4 * self.slot_elems, C.c_void_p(self.status.data_ptr()),
+                                           self._stream(stream)), 'halo_pull')
 
     def exchange(self, own: torch.Tensor, plan, buf: torch.Tensor | None = None) -> torch.Tensor:
         """Assemble source planes [src_lo, src_hi): own part by a device copy, the rest from the neighbours.

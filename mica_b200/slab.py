@@ -11,7 +11,8 @@ every stitched voxel -- has exactly one owner.  Per stage:
                 bit-identical to the one-GPU map); the source halo comes from the two
                 neighbouring ranks over NVLink peer memory (peer.PeerHalo).
   order stats   local histograms over OWNED planes only, all-reduced (int64 sum) between
-                the hist and pick kernels of each of the 5 radix rounds: exact.
+                the hist and pick kernels of each of the 5 radix rounds: exact.  An integer map
+                (int8 / int16 / uint16, DESIGN.md D12) has one exact histogram, summed once.
   AF3 encode    atoms are replicated (a few MB); each rank rasterises its slab + halo.
   extract       a rank's cubes are those whose core lies in its slab; no exchange (the halo
                 planes were resampled and normalised locally).
@@ -52,17 +53,27 @@ class RankSlab:
 
 
 class SlabPlan:
-    """Pure host arithmetic of the partition (unit-tested on CPU)."""
+    """Pure host arithmetic of the partition (unit-tested on CPU).  ``dtype``: the map's sample type.  An integer
+    map resampled at order 3 takes the general path, whose z prefilter gives a block the whole line's bits only for
+    lines of 96..800 planes (``ops.resample_slab_source_planes_general``): other lengths raise MicaError."""
 
     def __init__(self, src_shape, voxel_size_xyz, grid_size, padding, world, target_voxel_size=1.0,
-                 halo_k=16, order=3, aligned=True):
+                 halo_k=16, order=3, aligned=True, dtype=torch.float32):
         self.src_shape = tuple(int(v) for v in src_shape)
         self.world = int(world)
         self.grid_size, self.padding, self.halo_k, self.order = int(grid_size), int(padding), int(halo_k), order
+        self.dtype = dtype
         zf = zoom_factors(voxel_size_xyz, target_voxel_size)
         self.identity = all(float(z) == 1.0 for z in zf)
         self.out_shape = ops.zoom_output_shape(self.src_shape, zf)
         sz, nz = self.src_shape[0], self.out_shape[0]
+        general = dtype in ops.INT_DTYPES and order == 3 and not self.identity
+        if general:
+            try:                                # the library knows which lines the general path can cut
+                ops.resample_slab_source_planes_general(sz, nz, 0, nz)
+            except MicaError as e:
+                raise MicaError(f'a {dtype} map cannot be resampled in z-slabs (run it on one GPU, MapPipeline): '
+                                f'{e}') from None
         layers = -(-nz // self.grid_size)
         lb = _split_even(layers, self.world)
         scale = (sz - 1) / (nz - 1) if nz > 1 else 1.0
@@ -75,7 +86,7 @@ class SlabPlan:
             ob.append(sz if o >= nz else max(ob[-1], min(sz, int(round(o * scale)))))
         ob.append(sz)
         taps_lo, taps_hi = (1, 2) if order == 3 else (0, 1)
-        k = self.halo_k if (order == 3 and not self.identity) else 0
+        k = self.halo_k if (order == 3 and not self.identity and not general) else 0
         self.ranks = []
         for r in range(self.world):
             out_lo, out_hi = min(nz, lb[r] * self.grid_size), min(nz, lb[r + 1] * self.grid_size)
@@ -88,7 +99,11 @@ class SlabPlan:
             else:
                 src_lo = max(0, int(np.floor(ext_lo * scale)) - taps_lo - k)
                 src_hi = min(sz, int(np.floor((ext_hi - 1) * scale)) + taps_hi + k + 1)
-                if order == 3 and aligned:
+                if general:
+                    # the segments of the general path's z prefilter that the slab computes, and their windows
+                    a_lo, a_hi = ops.resample_slab_source_planes_general(sz, nz, ext_lo, ext_hi - ext_lo)
+                    src_lo, src_hi = min(src_lo, a_lo), max(src_hi, a_hi)
+                elif order == 3 and aligned:
                     # whole prefilter segments + their windows: the slab's coefficients are then computed
                     # from the same windows as on one GPU, i.e. the N-rank map is bit-identical to it
                     a_lo, a_hi = ops.resample_slab_source_planes(sz, nz, ext_lo, ext_hi - ext_lo)
@@ -113,7 +128,8 @@ class SlabPlan:
 
 def exchange_source_halo(own: torch.Tensor, plan: SlabPlan, rank: int, group=None) -> torch.Tensor:
     """Assemble the source planes [src_lo, src_hi) this rank needs from its own block
-    ``own`` (= global planes [own_lo, own_hi)) and its neighbours' (send/recv)."""
+    ``own`` (= global planes [own_lo, own_hi)) and its neighbours' (send/recv).  The planes travel as bytes
+    (uint8 views): NCCL has no int16 / uint16 type."""
     import torch.distributed as dist
     me = plan.ranks[rank]
     n = max(0, me.src_hi - me.src_lo)
@@ -122,14 +138,15 @@ def exchange_source_halo(own: torch.Tensor, plan: SlabPlan, rank: int, group=Non
     if hi > lo:
         buf[lo - me.src_lo:hi - me.src_lo].copy_(own[lo - me.own_lo:hi - me.own_lo])
     sends, recvs = plan.transfers(rank)
+    own_b, buf_b = own.contiguous().view(torch.uint8), buf.view(torch.uint8)
     ops_ = []
     keep = []
     for p, a, b in sends:
-        t = own[a - me.own_lo:b - me.own_lo].contiguous()
+        t = own_b[a - me.own_lo:b - me.own_lo].contiguous()
         keep.append(t)
         ops_.append(dist.P2POp(dist.isend, t, p, group))
     for p, a, b in recvs:
-        ops_.append(dist.P2POp(dist.irecv, buf[a - me.src_lo:b - me.src_lo], p, group))
+        ops_.append(dist.P2POp(dist.irecv, buf_b[a - me.src_lo:b - me.src_lo], p, group))
     if ops_:
         for req in dist.batch_isend_irecv(ops_):
             req.wait()
@@ -163,6 +180,7 @@ class SlabPipeline(MapPipeline):
             raise MicaError(f'hist_exchange must be peer or nccl, got {hist_exchange!r}')
         self.hist_exchange = hist_exchange
         self.peer = None
+        self.int_peer = None
 
     def _peer_group(self):
         if self.peer is None:
@@ -170,14 +188,21 @@ class SlabPipeline(MapPipeline):
             self.peer = PeerHistogram(self.device, self.rank, self.world, self.group)
         return self.peer
 
+    def _int_peer_group(self):
+        if self.int_peer is None:
+            from .peer import PeerIntHistogram
+            self.int_peer = PeerIntHistogram(self.device, self.rank, self.world, self.group)
+        return self.int_peer
+
     # -- collectives (torch.distributed over NCCL; injectable for single-process emulation)
     def _all_reduce_hist(self, hist):
         import torch.distributed as dist
         dist.all_reduce(hist, op=dist.ReduceOp.SUM, group=self.group)
 
     def _halo_slot_elems(self, plan):
-        """Largest halo (float32 elements) any rank receives from one neighbour, or None when some rank
-        needs planes from beyond its direct neighbours.  Global: the same answer on every rank."""
+        """Largest halo (in 4-byte words, of planes of the plan's sample type) any rank receives from one
+        neighbour, or None when some rank needs planes from beyond its direct neighbours.  Global: the same
+        answer on every rank."""
         from .peer import PeerHalo
         planes = 0
         for r in range(self.world):
@@ -185,7 +210,8 @@ class SlabPipeline(MapPipeline):
             if np_ is None:
                 return None
             planes = max([planes] + [rng[1] - rng[0] for rng in np_ if rng is not None])
-        return planes * plan.src_shape[1] * plan.src_shape[2]
+        itemsize = torch.empty((), dtype=plan.dtype).element_size()
+        return PeerHalo.slot_words(plan, planes, itemsize)
 
     def prefetch_source(self, next_own, header=None):
         """Exchange the source halo of the NEXT map now, on a side stream, so that it runs under this map's
@@ -198,7 +224,7 @@ class SlabPipeline(MapPipeline):
         if self.world == 1 or self.halo_exchange != 'peer' or self.peer_halo is None:
             return                                    # the first map builds the exchange group (a collective)
         header = self.header if header is None else header
-        if self.plan is None or self._plan_key_of(tuple(next_own.shape), header) != self._plan_key:
+        if self.plan is None or self._plan_key_of(tuple(next_own.shape), header, next_own.dtype) != self._plan_key:
             return                                    # another geometry: this map's plan must stay; exchanged in line
         plan = self.plan
         need = self._halo_slot_elems(plan)
@@ -212,9 +238,10 @@ class SlabPipeline(MapPipeline):
         # pre-phase (no allocator traffic between streams, no record_stream)
         me = plan.ranks[self.rank]
         shape = (max(0, me.src_hi - me.src_lo),) + tuple(next_own.shape[1:])
-        if self._halo_bufs is None or tuple(self._halo_bufs[0].shape) != shape:
+        if self._halo_bufs is None or tuple(self._halo_bufs[0].shape) != shape or \
+                self._halo_bufs[0].dtype != next_own.dtype:
             main.wait_stream(self._halo_stream)        # a dropped prefetch may still be writing the old pair
-            self._halo_bufs = [torch.empty(shape, dtype=torch.float32, device=self.device) for _ in range(2)]
+            self._halo_bufs = [torch.empty(shape, dtype=next_own.dtype, device=self.device) for _ in range(2)]
         self._halo_turn ^= 1
         buf = self._halo_bufs[self._halo_turn]
         self._halo_stream.wait_stream(main)
@@ -251,33 +278,33 @@ class SlabPipeline(MapPipeline):
         from .peer import PeerHalo
         return PeerHalo(self.device, self.rank, self.world, slot_elems, self.group)
 
-    def _plan_key_of(self, own_shape, header):
+    def _plan_key_of(self, own_shape, header, dtype=torch.float32):
         gshape = self.global_src_shape
         if gshape is None:                      # weak-scaling default: equal blocks stacked along z
             gshape = (own_shape[0] * self.world, own_shape[1], own_shape[2])
         return (tuple(gshape), tuple(float(v) for v in header.voxel_size), self.grid_size, self.padding, self.world,
-                float(self.target_voxel_size), self.halo_k, self.order)
+                float(self.target_voxel_size), self.halo_k, self.order, dtype)
 
-    def make_plan(self, own_shape, header):
-        key = self._plan_key_of(own_shape, header)
+    def make_plan(self, own_shape, header, dtype=torch.float32):
+        key = self._plan_key_of(own_shape, header, dtype)
         gshape = key[0]
         if key != self._plan_key:               # host arithmetic only, but it runs once per map otherwise
             self.plan = SlabPlan(gshape, header.voxel_size, self.grid_size, self.padding, self.world,
-                                 self.target_voxel_size, self.halo_k, self.order)
+                                 self.target_voxel_size, self.halo_k, self.order, dtype=dtype)
             self._plan_key = key
         return self.plan
 
     @_on_device
     def slab_resample(self, own_src, header=None):
         """Halo exchange + resample of this rank's planes.  Returns (res, owned): the local
-        resampled planes [ext_lo, ext_hi) and the view of the owned ones [out_lo, out_hi)."""
-        if getattr(own_src, 'dtype', None) != torch.float32:
-            # integer maps (D12) would need their exact histogram exchanged between the ranks: one GPU only
-            raise MicaError(f'SlabPipeline takes float32 maps only, got {getattr(own_src, "dtype", type(own_src))} '
-                            '(integer maps run on one GPU, MapPipeline)')
+        resampled planes [ext_lo, ext_hi) and the view of the owned ones [out_lo, out_hi).  float32, int8,
+        int16 and uint16 maps; the resampled planes have the map's type (D12)."""
+        dtype = getattr(own_src, 'dtype', None)
+        if dtype not in ops.MAP_DTYPES:
+            raise MicaError(f'SlabPipeline takes float32, int8, int16 or uint16 maps, got {dtype or type(own_src)}')
         if header is not None:
             self.header = header
-        plan = self.make_plan(tuple(own_src.shape), self.header)
+        plan = self.make_plan(tuple(own_src.shape), self.header, dtype)
         me = plan.ranks[self.rank]
         nz, ny, nx = plan.out_shape
         with self.timer('halo_exchange'):
@@ -293,21 +320,26 @@ class SlabPipeline(MapPipeline):
         return res, res[me.out_lo - me.ext_lo:me.out_hi - me.ext_lo]
 
     def slab_normalize(self, res):
-        """Apply the (globally agreed) thresholds to the local planes, halo included."""
+        """Apply the (globally agreed) thresholds to the local planes, halo included: in place for a float32
+        map, into a new float32 volume for an integer one."""
         with self.timer('normalize_apply'):
-            self.normalized = self.stats.apply(res, res)
+            self.normalized = self.stats.apply(res) if res.dtype in ops.INT_DTYPES else self.stats.apply(res, res)
         self.norm_status = None
 
     @_on_device
     def resample_and_normalize(self, own_src, header=None, defer_status=False):
+        """As ``MapPipeline.resample_and_normalize`` for this rank's planes; ``median`` and ``p999`` are Python
+        floats for an integer map."""
         res, owned = self.slab_resample(own_src, header)
         nz, ny, nx = self.plan.out_shape
+        integer = res.dtype in ops.INT_DTYPES
+        stats = self._int_order_stats() if integer else self._order_stats()
         with self.timer('order_stats'):
             if self.hist_exchange == 'peer' and self.world > 1:
-                self.stats = self._order_stats().run(owned, n_total=nz * ny * nx, peer=self._peer_group())
+                peer = self._int_peer_group() if integer else self._peer_group()
+                self.stats = stats.run(owned, n_total=nz * ny * nx, peer=peer)
             else:
-                self.stats = self._order_stats().run(owned, n_total=nz * ny * nx,
-                                                             all_reduce=self._all_reduce_hist)
+                self.stats = stats.run(owned, n_total=nz * ny * nx, all_reduce=self._all_reduce_hist)
         self.slab_normalize(res)
         return True if defer_status else self.check_status()
 
