@@ -488,14 +488,29 @@ int mica_zero_around_atoms(const float* xyz, int64_t n_atoms, const float origin
 /* ------------------------------------------- overlap-weighted stitching (BASELINE.json north_star variant)
  * NOT the reference's arithmetic (it pastes disjoint cores, utils/predict.py:494-501): every voxel of every window
  * adds its post-processed probabilities times a separable window weight w1[a] w1[b] w1[c] (window_w1: W = grid_size
- * + 2 padding floats on the HOST) to num [22][X][Y][Z] (backbone, C-alpha, 20 amino-acid probabilities) and the
- * weight to wsum [X][Y][Z]; both zero-initialised by the caller, accumulated over any number of calls.
- * mica_overlap_finalize divides in place and overwrites wsum with amino_acid_prediction (arg-max of the averaged
- * probabilities).  With the core-indicator window the result equals mica_postproc_stitch bit for bit. */
-int mica_overlap_accumulate(const float* bb, const float* ca, const float* aa, const int32_t* ijk, int n_cubes,
-                            int X, int Y, int Z, int grid_size, int padding, const float* window_w1, float* num,
-                            float* wsum, mica_stream_t stream);
-int mica_overlap_finalize(float* num, float* wsum, int64_t n_voxels, mica_stream_t stream);
+ * + 2 padding floats on the HOST, finite, >= 0, at least one > 0), normalised by the weight sum of the full cube
+ * lattice: norm is a DEVICE float64 array [X | Y | Z] of the reciprocals of the three 1-D lattice sums (0 where a
+ * sum is 0).  The contributions are 2^-31 fixed point, added as uint32 into a zero-initialised 23-channel block
+ * laid out [backbone | carbon_alpha | amino_acid_prediction | amino_acid_probability x 20] (the layout of
+ * mica_postproc_stitch_peer), over any number of calls: the sums, and so the result, do not depend on the order,
+ * the batch or the partition.  mica_overlap_finalize_fixed turns a block of n_voxels voxels into the four float32
+ * volumes in place (prediction = arg-max of the 20 sums, first maximum wins).
+ * _peer: the output is owned along cube axis `axis` (0 = x, 2 = k): rank r holds planes [bounds[r], bounds[r+1])
+ * of that axis as such a block at owner_base[r] (a DEVICE array of `world` pointers, local or peer-mapped memory,
+ * which needs native peer atomics: mica_peer_atomics_supported).  Every contribution is added into its owner's
+ * block.  The caller zeroes every block, synchronises all ranks before the first accumulate and after the last,
+ * then each owner finalizes its own block. */
+int mica_overlap_accumulate_fixed(const float* bb, const float* ca, const float* aa, const int32_t* ijk, int n_cubes,
+                                  int X, int Y, int Z, int grid_size, int padding, const float* window_w1,
+                                  const double* norm, void* block, mica_stream_t stream);
+int mica_overlap_accumulate_fixed_peer(const float* bb, const float* ca, const float* aa, const int32_t* ijk,
+                                       int n_cubes, int X, int Y, int Z, int grid_size, int padding,
+                                       const float* window_w1, const double* norm, void* const* owner_base, int axis,
+                                       const int* bounds, int world, mica_stream_t stream);
+int mica_overlap_finalize_fixed(void* block, int64_t n_voxels, mica_stream_t stream);
+/* 1 when `device` can add into the memory of `peer_device` with native atomics over the peer path
+ * (cudaDevP2PAttrNativeAtomicSupported; 1 for device == peer_device), 0 when not, negative MICA_ERR_* on error. */
+int mica_peer_atomics_supported(int device, int peer_device);
 
 /* ------------------------------------------- host I/O helper (SURVEY 8f N2; no device work)
  * Fixed-column PDB reader standing where Bio.PDB.PDBParser stands (utils/preprocessing.py:269,275-298).

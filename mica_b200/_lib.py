@@ -102,8 +102,11 @@ SIGNATURES = {
                                   _p, _p, _p, _p, _p]),
     'mica_stitch_cubes': (_i, [_p, _i, _p, _i, _i, _i, _i, C.POINTER(_i), C.POINTER(_i), _i, _i, _p, _p]),
     'mica_postproc_stitch_peer': (_i, [_p, _p, _p, _p, _i, _i, _i, _i, _i, _i, _p, C.POINTER(_i), _i, _p]),
-    'mica_overlap_accumulate': (_i, [_p, _p, _p, _p, _i, _i, _i, _i, _i, _i, C.POINTER(_f), _p, _p, _p]),
-    'mica_overlap_finalize': (_i, [_p, _p, _i64, _p]),
+    'mica_overlap_accumulate_fixed': (_i, [_p, _p, _p, _p, _i, _i, _i, _i, _i, _i, C.POINTER(_f), _p, _p, _p]),
+    'mica_overlap_accumulate_fixed_peer': (_i, [_p, _p, _p, _p, _i, _i, _i, _i, _i, _i, C.POINTER(_f), _p, _p, _i,
+                                                C.POINTER(_i), _i, _p]),
+    'mica_overlap_finalize_fixed': (_i, [_p, _i64, _p]),
+    'mica_peer_atomics_supported': (_i, [_i, _i]),
     'mica_parse_pdb': (_i64, [C.c_char_p, _i64, _i, _i64, _p, _p, _p, _p, _p, _p, _p]),
     # SURVEY 8(f) N1: candidates
     'mica_cand_threshold_workspace_bytes': (_sz, [_i64]),

@@ -7,6 +7,7 @@ from __future__ import annotations
 
 import ctypes as C
 import functools
+from typing import NamedTuple
 
 import numpy as np
 import torch
@@ -609,12 +610,14 @@ def postproc_stitch_peer(bb: torch.Tensor, ca: torch.Tensor, aa: torch.Tensor, i
 def overlap_window(kind, grid_size: int, padding: int) -> np.ndarray:
     """1-D weights of the overlap-weighted stitch: 'core' (1 on the core, 0 on the halo = the reference's crop),
     'uniform' (plain average of every window covering a voxel), 'triangle' (ramp peaking at the window centre),
-    or an array of W = grid_size + 2 * padding floats."""
+    or an array of W = grid_size + 2 * padding finite weights >= 0, at least one of them > 0."""
     W = int(grid_size) + 2 * int(padding)
     if not isinstance(kind, str):
         w = np.ascontiguousarray(kind, dtype=np.float32)
         if w.shape != (W,):
             raise _lib.MicaError(f'window must have {W} weights, got shape {w.shape}')
+        if not (np.isfinite(w).all() and (w >= 0).all() and (w > 0).any()):
+            raise _lib.MicaError('window weights must be finite and >= 0, with at least one > 0')
         return w
     u = np.arange(W, dtype=np.float64)
     if kind == 'core':
@@ -628,56 +631,145 @@ def overlap_window(kind, grid_size: int, padding: int) -> np.ndarray:
     return w.astype(np.float32)
 
 
-class OverlapStitcher:
-    """The north_star's "stitch with overlap weights": accumulates window-weighted probabilities and the weights
-    themselves over all cubes, then divides (``finalize``).  NOT the reference's arithmetic, which pastes the
-    disjoint cores (``postproc_stitch``; DESIGN.md D2) -- offered as a mode next to it; with ``window='core'`` the
-    two agree bit for bit.  Costs ~8x the reference mode: every voxel of every 64^3 window is post-processed and
-    added atomically, not just the 32^3 (48^3) cores."""
+def is_core_window(w1, grid_size: int, padding: int) -> bool:
+    """True for the 1-on-the-core window: its weighted stitch IS the reference's paste, and runs as one."""
+    return np.array_equal(w1, overlap_window('core', grid_size, padding))
 
-    def __init__(self, cube_shape, device, grid_size: int = 48, padding: int = 8, window='uniform'):
+
+def overlap_norm_tables(w1, cube_shape, grid_size: int, padding: int):
+    """Reciprocals (0 where the sum is 0) of the 1-D weight sums Wx, Wy, Wz of the full cube lattice
+    (``cube_origins``): the weight sum of the overlap-weighted stitch at voxel (x, y, z) is Wx[x] Wy[y] Wz[z], with
+    Wx[x] = sum over the origins i covering x of w1[x - i + padding].  float64, origins added in ascending order.
+    Whatever part of the lattice a run stitches, these come from all of it."""
+    w = np.asarray(w1, dtype=np.float32).astype(np.float64)
+    W = len(w)
+    out = []
+    for n in (int(v) for v in cube_shape):
+        s = np.zeros(n, np.float64)
+        for i in range(0, n, int(grid_size)):
+            lo = i - int(padding)
+            x0, x1 = max(0, lo), min(n, lo + W)
+            s[x0:x1] += w[x0 - lo:x1 - lo]
+        r = np.zeros(n, np.float64)
+        np.divide(1.0, s, out=r, where=s > 0)
+        out.append(r)
+    return out
+
+
+def overlap_owner(coord: int, bounds) -> int:
+    """The rank whose planes [bounds[r], bounds[r+1]) hold ``coord`` -- the lookup of the peer accumulate kernel
+    (empty ranks are skipped)."""
+    r = 0
+    while r + 1 < len(bounds) - 1 and coord >= bounds[r + 1]:
+        r += 1
+    return r
+
+
+def peer_atomics_supported(device: int, peer_device: int) -> bool:
+    """Whether ``device`` can add into ``peer_device``'s memory with native atomics (True for the same device)."""
+    rc = lib.mica_peer_atomics_supported(int(device), int(peer_device))
+    if rc < 0:
+        check(rc, 'peer_atomics_supported')
+    return bool(rc)
+
+
+class OverlapOwners(NamedTuple):
+    """Where the contributions of an overlap-weighted stitch go when the output is split over ranks: rank r owns
+    planes [bounds[r], bounds[r+1]) of cube axis ``axis`` (0 = x, 2 = k) as the 23-channel block at ``table[r]``
+    (int64 device tensor of base pointers, ``peer.PeerVolumes.table``); ``devices``: the CUDA device index of each
+    owner, whose memory the accumulating device must be able to add into atomically."""
+    table: torch.Tensor
+    axis: int
+    bounds: tuple
+    devices: tuple
+
+
+class OverlapStitcher:
+    """The north_star's "stitch with overlap weights": every voxel of every window adds its probabilities times
+    the window weight, normalised by the weight sum of the full cube lattice, in 2^-31 fixed point (uint32), so the
+    result does not depend on the order of the cubes, the batches or the partition; ``finalize`` converts in place.
+    NOT the reference's arithmetic, which pastes the disjoint cores (``postproc_stitch``; DESIGN.md D2) -- offered
+    as a mode next to it; ``window='core'`` runs that paste.  Costs several times the reference mode: every voxel of
+    every 64^3 window is post-processed and added, not just the 32^3 (48^3) cores.
+
+    ``vols``: the volumes (``StitchedVolumes.from_block``, zeroed) this stitcher finalizes; default: a whole-map
+    block of its own.  ``owners``: an ``OverlapOwners`` table -- contributions go to the block of the rank that
+    owns their plane, locally or over NVLink (native peer atomics required); without ``vols`` such a stitcher only
+    accumulates."""
+
+    def __init__(self, cube_shape, device, grid_size: int = 48, padding: int = 8, window='uniform', *, vols=None,
+                 owners: OverlapOwners | None = None):
         self.shape = tuple(int(v) for v in cube_shape)
         self.device = torch.device(device)
+        if self.device.index is None:
+            self.device = torch.device('cuda', torch.cuda.current_device())
         self.grid_size, self.padding = int(grid_size), int(padding)
         self.w1 = overlap_window(window, grid_size, padding)
-        X, Y, Z = self.shape
-        self.block = torch.zeros(23 * X * Y * Z, dtype=torch.float32, device=self.device)
-        n = X * Y * Z
-        self.num, self.wsum = self.block[:22 * n], self.block[22 * n:]
+        self.core = is_core_window(self.w1, self.grid_size, self.padding)
+        self.owners = owners
+        if owners is not None:
+            if owners.axis not in (0, 2) or (self.core and owners.axis != 0):
+                raise _lib.MicaError(f'owners along cube axis {owners.axis}: the weighted stitch splits along 0 or 2, '
+                                     'the core window (the paste) along 0')
+            for d in owners.devices:
+                if not peer_atomics_supported(self.device.index, d):
+                    raise _lib.MicaError(f'overlap-weighted stitching over several GPUs adds into the owners\' '
+                                         f'memory atomically: cuda:{self.device.index} has no native peer atomics '
+                                         f'with cuda:{d}')
+            self._bounds = (C.c_int * len(owners.bounds))(*[int(v) for v in owners.bounds])
+        if vols is None and owners is None:
+            X, Y, Z = self.shape
+            with torch.cuda.device(self.device):
+                vols = StitchedVolumes.from_block(torch.zeros(23 * X * Y * Z, dtype=torch.float32,
+                                                              device=self.device), self.shape, (0, 0, 0), self.shape)
+        if vols is not None and (getattr(vols, 'block', None) is None or vols.device != self.device):
+            raise _lib.MicaError('OverlapStitcher needs volumes of StitchedVolumes.from_block on its own device')
+        self.vols = vols
+        if not self.core:
+            with torch.cuda.device(self.device):
+                self.norm = torch.from_numpy(np.concatenate(
+                    overlap_norm_tables(self.w1, self.shape, self.grid_size, self.padding))).to(self.device)
         self._done = False
 
     @device_guard
     def accumulate(self, bb, ca, aa, ijk, vols=None):
+        if self.core:
+            if self.owners is not None:
+                postproc_stitch_peer(bb, ca, aa, ijk, self.shape, self.owners.table, self.owners.bounds,
+                                     self.grid_size, self.padding)
+            else:
+                postproc_stitch(bb, ca, aa, ijk, self.vols, self.grid_size, self.padding)
+            return
         B = ijk.shape[0]
         W = self.grid_size + 2 * self.padding
         for t, c, name in ((bb, 4, 'bb'), (ca, 4, 'ca'), (aa, 21, 'aa')):
             if tuple(t.shape) != (B, c, W, W, W):
                 raise _lib.MicaError(f'{name} logits must be [{B},{c},{W},{W},{W}], got {tuple(t.shape)}')
         X, Y, Z = self.shape
-        check(lib.mica_overlap_accumulate(
-            _dev(bb, torch.float32, 'bb'), _dev(ca, torch.float32, 'ca'), _dev(aa, torch.float32, 'aa'),
-            _dev(ijk, torch.int32, 'ijk'), B, X, Y, Z, self.grid_size, self.padding,
-            self.w1.ctypes.data_as(C.POINTER(C.c_float)), C.c_void_p(self.num.data_ptr()),
-            C.c_void_p(self.wsum.data_ptr()), _stream()), 'overlap_accumulate')
+        args = (_dev(bb, torch.float32, 'bb'), _dev(ca, torch.float32, 'ca'), _dev(aa, torch.float32, 'aa'),
+                _dev(ijk, torch.int32, 'ijk'), B, X, Y, Z, self.grid_size, self.padding,
+                self.w1.ctypes.data_as(C.POINTER(C.c_float)), C.c_void_p(self.norm.data_ptr()))
+        if self.owners is None:
+            check(lib.mica_overlap_accumulate_fixed(*args, C.c_void_p(self.vols.block.data_ptr()), _stream()),
+                  'overlap_accumulate')
+        else:
+            o = self.owners
+            check(lib.mica_overlap_accumulate_fixed_peer(*args, _dev(o.table, torch.int64, 'owner_table'), int(o.axis),
+                                                         self._bounds, int(o.table.numel()), _stream()),
+                  'overlap_accumulate_peer')
 
     @device_guard
     def finalize(self) -> StitchedVolumes:
-        """Divide by the accumulated weights and return the four volumes (views of the accumulation block, laid
-        out [backbone | carbon_alpha | amino_acid_probability x 20 | amino_acid_prediction])."""
-        X, Y, Z = self.shape
-        n = X * Y * Z
-        if not self._done:
-            check(lib.mica_overlap_finalize(C.c_void_p(self.num.data_ptr()), C.c_void_p(self.wsum.data_ptr()), n,
-                                            _stream()), 'overlap_finalize')
-            self._done = True
-        v = StitchedVolumes.__new__(StitchedVolumes)
-        v.shape, v.device, v.org, v.ext = self.shape, self.device, (0, 0, 0), self.shape
-        v.backbone_probability = self.block[0:n].view(self.shape)
-        v.carbon_alpha_probability = self.block[n:2 * n].view(self.shape)
-        v.amino_acid_probability = self.block[2 * n:22 * n].view((20,) + self.shape)
-        v.amino_acid_prediction = self.block[22 * n:].view(self.shape)
-        v.block = self.block
-        return v
+        """The four volumes (views of the accumulation block, laid out as ``StitchedVolumes.from_block``).  With
+        owners, call it once every rank's contributions have landed (stream sync + barrier)."""
+        if self.vols is None:
+            raise _lib.MicaError('this OverlapStitcher only accumulates into other ranks\' volumes')
+        if not self._done and not self.core:
+            e = self.vols.ext
+            check(lib.mica_overlap_finalize_fixed(C.c_void_p(self.vols.block.data_ptr()), e[0] * e[1] * e[2],
+                                                  _stream()), 'overlap_finalize')
+        self._done = True
+        return self.vols
 
 
 @device_guard

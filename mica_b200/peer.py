@@ -32,6 +32,8 @@ class _IpcGroup:
         self._opened, self._own, self._owned_all = [], None, []
         if _emulated is not None:                       # in-process emulation: pointers are shared directly
             ptrs = _emulated
+            idx = self.device.index if self.device.index is not None else torch.cuda.current_device()
+            self.devices = [idx] * self.world
         else:
             import torch.distributed as dist
             torch.cuda.set_device(self.device)
@@ -43,9 +45,10 @@ class _IpcGroup:
                 check(lib.mica_ipc_alloc(self.nbytes, C.byref(own), handle), 'ipc_alloc')
             self._own = own.value
             gathered = [None] * self.world
-            dist.all_gather_object(gathered, bytes(handle), group=group)
+            dist.all_gather_object(gathered, (bytes(handle), self.device.index), group=group)
+            self.devices = [d for _, d in gathered]       # each rank's CUDA device index
             ptrs = []
-            for r, h in enumerate(gathered):
+            for r, (h, _) in enumerate(gathered):
                 if r == self.rank:
                     ptrs.append(self._own)
                     continue

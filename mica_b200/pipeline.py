@@ -438,19 +438,25 @@ class MapPipeline:
         softmax/argmax + stitch (multi-GPU: cores owned by another rank go to its volumes).
         ``overlap_window`` ('uniform' | 'triangle' | 'core' | W weights): the north_star's overlap-weighted
         stitching instead of the reference's centre-crop paste (``ops.OverlapStitcher``; NOT the reference's
-        arithmetic, see DESIGN.md D2) -- whole map on one GPU only.  ``batches``: the super-batches as
+        arithmetic, see DESIGN.md D2; 'core' is the paste).  Nothing is final before the last batch, so
+        ``on_batch`` is then called once, with the finished volumes.  A split map (subclasses) supplies the owners
+        of the output; its volumes are final after ``finish_map()``.  ``batches``: the super-batches as
         (b0, b1) ranges of the (ordered) cube list, each at most ``batch_cubes`` long, instead of the even cut
         (``worker_batches``: a worker's share of a map dealt over several devices)."""
         if self.normalized is None:
             raise MicaError('no normalised map')
-        self.cube_index()
         overlap = None
         if overlap_window is not None:
-            if stitch_fn is not None or getattr(self, 'box', None) is not None:
-                raise MicaError('overlap-weighted stitching needs the whole map on one GPU')
-            overlap = ops.OverlapStitcher(self.cube_shape, self.device, self.grid_size, self.padding, overlap_window)
-            stitch_fn = overlap.accumulate
-            vols = overlap                                # only a handle for on_batch; finalised at the end
+            w1 = ops.overlap_window(overlap_window, self.grid_size, self.padding)     # refused before any launch
+            if not ops.is_core_window(w1, self.grid_size, self.padding):          # 'core' IS the paste
+                if stitch_fn is not None:
+                    raise MicaError('overlap_window replaces the stitch: pass stitch_fn or overlap_window, not both')
+                overlap = w1
+        self.cube_index()
+        if overlap is not None:
+            overlap = self._overlap_stitcher(overlap, vols)
+            stitch_fn, vols = overlap.accumulate, overlap.vols
+            final_on_batch, on_batch = on_batch, None
         if vols is None:
             vols = self._new_volumes()
         self._custom_order = order is not None
@@ -466,7 +472,7 @@ class MapPipeline:
             if any(not 0 <= b0 < b1 <= n or b1 - b0 > self.batch_cubes for b0, b1 in batches):
                 raise MicaError(f'batches must be non-empty ranges of the {n} cubes, at most {self.batch_cubes} long')
         if not batches:
-            return overlap.finalize() if overlap is not None else vols
+            return self._overlap_done(overlap, final_on_batch, n) if overlap is not None else vols
         want_flags = d8 == 'split' and (model_batch is None or int(model_batch) > 1)
         if stitch_fn is None:
             bound = ops.StitchCall(vols, self.grid_size, self.padding)
@@ -497,7 +503,7 @@ class MapPipeline:
                 consume(self.extract_batch(b0, b1, want_flags=want_flags), b0, b1)
                 if on_batch is not None:
                     on_batch(vols, b1)
-            return overlap.finalize() if overlap is not None else vols
+            return self._overlap_done(overlap, final_on_batch, n) if overlap is not None else vols
 
         t_enqueue = time.perf_counter()
         main = torch.cuda.current_stream(self.device)
@@ -528,7 +534,18 @@ class MapPipeline:
                 on_batch(vols, b1)
             cur = nxt
         self.last_loop_enqueue_ms = (time.perf_counter() - t_enqueue) * 1e3     # host side of the batch loop
-        return overlap.finalize() if overlap is not None else vols
+        return self._overlap_done(overlap, final_on_batch, n) if overlap is not None else vols
+
+    def _overlap_stitcher(self, w1, vols):
+        """The accumulator of an overlap-weighted map: the whole map in one block on this GPU (``vols``, if given,
+        must be ``StitchedVolumes.from_block`` volumes of the whole map, zeroed)."""
+        return ops.OverlapStitcher(self.cube_shape, self.device, self.grid_size, self.padding, w1, vols=vols)
+
+    def _overlap_done(self, overlap, on_batch, n):
+        vols = overlap.finalize()
+        if on_batch is not None:
+            on_batch(vols, n)
+        return vols
 
     @_on_device
     def finish(self):

@@ -158,7 +158,7 @@ class DeviceVolume:
 class CryoEMPredictor:
     def __init__(self, model_path, grids_path, output_path, save_output=True, device='cuda', quiet=False,
                  model=None, keep_on_device=True, host_volumes=None, host_pool=None, reference_batching=False,
-                 super_batch=256, release_inputs=True, devices=None):
+                 super_batch=256, release_inputs=True, devices=None, *, overlap_window=None):
         """Additions to the reference signature (all optional):
 
         ``model``               an already loaded model (callable ``(exp_map, af_features) -> (bb, ca, aa)``).
@@ -185,8 +185,13 @@ class CryoEMPredictor:
                                 own stream.  Every model call sees the cubes, in the order, it sees on one device
                                 with the same options, so the volumes do not depend on the device count.  The
                                 model is loaded once per GPU; an ``nn.Module`` given as ``model`` is deep-copied
-                                to the other GPUs, or ``model`` may be a {device: callable} mapping."""
+                                to the other GPUs, or ``model`` may be a {device: callable} mapping.
+        ``overlap_window``      (keyword only) None: the reference's paste of the cube cores.  'uniform',
+                                'triangle' or W = grid_size + 2 * padding weights: overlap-weighted stitching
+                                (``ops.OverlapStitcher``; NOT the reference's arithmetic, DESIGN.md D2), the same bits
+                                on one device and with ``devices=``.  'core' is the paste."""
         self.devices = devices
+        self.overlap_window = overlap_window
         self.worker_cubes = None                        # cubes each worker ran (several devices only)
         self._workers = None
         self._models = None
@@ -413,11 +418,29 @@ class CryoEMPredictor:
         flags = (af.abs().reshape(B, -1).sum(1) > 0).to(torch.int32)
         return x, af, flags
 
+    def _download(self, vols):
+        """The host volumes of finished device volumes (one synchronisation)."""
+        out_host = self._host_buffers(vols)
+        with torch.cuda.device(vols.device):
+            for k, t in out_host.items():
+                t.copy_(getattr(vols, k), non_blocking=True)
+            torch.cuda.current_stream(vols.device).synchronize()
+        return out_host
+
+    def _overlap_weights(self):
+        """The window of an overlap-weighted map (checked before any launch), or None for the paste."""
+        if self.overlap_window is None:
+            return None
+        gs, pad = self._source['grid_size'], self._source['padding']
+        w1 = ops.overlap_window(self.overlap_window, gs, pad)
+        return None if ops.is_core_window(w1, gs, pad) else w1
+
     def run_inference_and_reconstruct(self):
         """run_inference + reconstruct_volume (utils/predict.py:307-512) fused.  Returns
         (device volumes, {name: pinned host tensor})."""
+        w1 = self._overlap_weights()
         if self._workers:
-            return self._run_on_devices(self._workers)
+            return self._run_on_devices(self._workers, w1)
         dev = torch.device(self.device)
         s = self._source
         gs, pad = s['grid_size'], s['padding']
@@ -429,6 +452,11 @@ class CryoEMPredictor:
             if s['kind'] == 'resident':
                 pipe = self._pipeline(dev)
                 order = self._reference_order() if self.reference_batching else None
+                self._pipe = pipe
+                if w1 is not None:                          # nothing is final before the last cube: no drain
+                    vols = pipe.predict_and_stitch(model, None, model_batch=self._model_batch(), d8=d8, order=order,
+                                                   overlap_window=w1)
+                    return vols, self._download(vols)
                 pipe.cube_index()
                 vols = pipe._new_volumes()
                 out_host = self._host_buffers(vols)
@@ -443,27 +471,33 @@ class CryoEMPredictor:
             if dev.type != 'cuda':
                 raise ops._lib.MicaError('mica_b200 has no CPU path')
             ijk_dev = torch.from_numpy(np.ascontiguousarray(s['ijk'], dtype=np.int32)).to(dev)
-            vols = ops.StitchedVolumes(s['cube_shape'], dev)
+            if w1 is not None:
+                overlap = ops.OverlapStitcher(s['cube_shape'], dev, gs, pad, w1)
+                vols = overlap.vols
+            else:
+                overlap, vols = None, ops.StitchedVolumes(s['cube_shape'], dev)
+
+            def stitch(bb, ca, aa, ijk):
+                bb, ca, aa = bb.contiguous().float(), ca.contiguous().float(), aa.contiguous().float()
+                if overlap is not None:
+                    overlap.accumulate(bb, ca, aa, ijk)
+                else:
+                    ops.postproc_stitch(bb, ca, aa, ijk, vols, gs, pad)
             step = max(self._model_batch(), 1) * 4
             for b0 in range(0, self.sample_count, step):
                 b1 = min(self.sample_count, b0 + step)
                 x, af, flags = self._fetch_files(b0, b1, dev)
-                run_model_chunks(model, x, af, flags.cpu().numpy(), ijk_dev[b0:b1],
-                                 lambda bb, ca, aa, ijk: ops.postproc_stitch(
-                                     bb.contiguous().float(), ca.contiguous().float(), aa.contiguous().float(),
-                                     ijk, vols, gs, pad),
-                                 self._model_batch(), d8)
-            out_host = self._host_buffers(vols)
-            for k, t in out_host.items():
-                t.copy_(getattr(vols, k), non_blocking=True)
-            torch.cuda.synchronize(dev)
-            return vols, out_host
+                run_model_chunks(model, x, af, flags.cpu().numpy(), ijk_dev[b0:b1], stitch, self._model_batch(), d8)
+            if overlap is not None:
+                overlap.finalize()
+            return vols, self._download(vols)
 
-    def _run_on_devices(self, workers):
+    def _run_on_devices(self, workers, w1=None):
         """The map's cubes dealt over ``workers`` (``deal_cubes``), one thread each.  Every worker stores its
-        cores into ONE 23-channel block on workers[0] (``postproc_stitch_peer`` with a one-entry owner table);
-        the host copies run once, after the last worker has finished.  Returns what
-        ``run_inference_and_reconstruct`` returns."""
+        cores into ONE 23-channel block on workers[0] (``postproc_stitch_peer`` with a one-entry owner table) --
+        or, with the window ``w1``, adds its weighted contributions into it (``ops.OverlapStitcher`` with that
+        table), which workers[0] finalises after the last worker has finished; the host copies run once, after
+        that.  Returns what ``run_inference_and_reconstruct`` returns."""
         s = self._source
         gs, pad = s['grid_size'], s['padding']
         primary, n, mb = workers[0], len(s['ijk']), self._model_batch()
@@ -523,6 +557,11 @@ class CryoEMPredictor:
             zeroed.record()
         vols = ops.StitchedVolumes.from_block(block, cube_shape, (0, 0, 0), (X, Y, Z))
         tables = {d: torch.tensor([block.data_ptr()], dtype=torch.int64, device=d) for d in dict.fromkeys(workers)}
+        overlap = None
+        if w1 is not None:
+            overlap = {d: ops.OverlapStitcher(cube_shape, d, gs, pad, w1, vols=vols if d == primary else None,
+                                              owners=ops.OverlapOwners(tables[d], 0, (0, X), (primary.index,)))
+                       for d in dict.fromkeys(workers)}
         for dev, st in zip(workers, streams):
             st.wait_stream(torch.cuda.current_stream(dev))     # inputs copied / binned on the current streams
             st.wait_event(zeroed)
@@ -537,8 +576,11 @@ class CryoEMPredictor:
             dev, table, model = workers[w], tables[workers[w]], self._models[workers[w]]
 
             def stitch(bb, ca, aa, ijk, _vols=None):
-                ops.postproc_stitch_peer(bb.contiguous().float(), ca.contiguous().float(), aa.contiguous().float(),
-                                         ijk, cube_shape, table, (0, X), gs, pad)
+                bb, ca, aa = bb.contiguous().float(), ca.contiguous().float(), aa.contiguous().float()
+                if overlap is not None:
+                    overlap[dev].accumulate(bb, ca, aa, ijk)
+                else:
+                    ops.postproc_stitch_peer(bb, ca, aa, ijk, cube_shape, table, (0, X), gs, pad)
             with torch.cuda.device(dev), torch.cuda.stream(streams[w]), torch.no_grad():
                 if resident:
                     pipes[w].predict_and_stitch(model, vols, model_batch=mb, d8=d8, order=order[lo:hi],
@@ -572,12 +614,9 @@ class CryoEMPredictor:
         for e in errors:
             if e is not None:
                 raise e
-        out_host = self._host_buffers(vols)
-        with torch.cuda.device(primary):
-            for k, t in out_host.items():
-                t.copy_(getattr(vols, k), non_blocking=True)
-            torch.cuda.current_stream(primary).synchronize()
-        return vols, out_host
+        if overlap is not None:
+            overlap[primary].finalize()
+        return vols, self._download(vols)
 
     def _release(self):
         s = self._source or {}

@@ -153,13 +153,93 @@ def exchange_source_halo(own: torch.Tensor, plan: SlabPlan, rank: int, group=Non
     return buf
 
 
-class SlabPipeline(MapPipeline):
+class _SplitMap:
+    """What the pipelines of one map split over ranks share: meeting the other ranks, the exported volume block
+    (peer.PeerVolumes) the other ranks store into, and the overlap-weighted stitch, whose contributions are added
+    into the block of the rank that owns their plane and finalised by ``finish_map``."""
+
+    peer_volumes = None
+    _overlap_pending = None
+
+    def sync_ranks(self):
+        torch.cuda.synchronize(self.device)
+        if self.world > 1 and self.group is not False:
+            import torch.distributed as dist
+            dist.barrier(group=self.group)
+
+    def finish_map(self):
+        """All ranks' contributions have landed: after this every rank may read its own volume block (an
+        overlap-weighted map is finalised here, each owner its own block)."""
+        self.sync_ranks()
+        pending, self._overlap_pending = self._overlap_pending, None
+        if pending is not None:
+            overlap, on_batch, n = pending
+            with torch.cuda.device(self.device):
+                vols = overlap.finalize()
+                if on_batch is not None:
+                    on_batch(vols, n)
+
+    def _exported_volumes(self, n_max):
+        """This rank's box as volumes in its exported block (zeroed): the block other ranks store into."""
+        from .peer import PeerVolumes
+        if self.peer_volumes is None or self.peer_volumes.n_voxels < n_max:
+            if self.peer_volumes is not None:
+                self.peer_volumes.close()
+            if self.world == 1:                   # nothing to map: one local block
+                self.peer_volumes = PeerVolumes.emulate(self.device, 1, n_max)[0]
+            elif self.group is False:
+                raise MicaError('in-process emulation of several ranks: pass _peer_volumes (PeerVolumes.emulate)')
+            else:
+                self.peer_volumes = PeerVolumes(self.device, self.rank, self.world, n_max, self.group)
+        org, ext = self.box
+        n = ext[0] * ext[1] * ext[2]
+        vols = ops.StitchedVolumes.from_block(self.peer_volumes.block(n_elems=23 * n), self.cube_shape, org, ext)
+        vols.block.zero_()
+        return vols
+
+    def _owner_bounds(self):
+        """(cube axis, world + 1 plane bounds) of the output partition."""
+        raise NotImplementedError
+
+    def _overlap_stitcher(self, w1, vols):
+        if vols is None or getattr(vols, 'block', None) is None:
+            raise MicaError('a split map stitches overlap-weighted into its exported volumes (predict_and_stitch '
+                            'builds them when vols is None)')
+        axis, bounds = self._owner_bounds()
+        pv = self.peer_volumes
+        owners = ops.OverlapOwners(pv.table, axis, tuple(bounds), tuple(pv.devices))
+        return ops.OverlapStitcher(self.cube_shape, self.device, self.grid_size, self.padding, w1, vols=vols,
+                                   owners=owners)
+
+    def _overlap_done(self, overlap, on_batch, n):
+        self._overlap_pending = (overlap, on_batch, n)        # finalised by finish_map, once every rank has added
+        return overlap.vols
+
+    def _weighted(self, kw):
+        """True when ``kw`` asks for an overlap-weighted stitch other than 'core' (which is the paste)."""
+        w = kw.get('overlap_window')
+        if w is None or ops.is_core_window(ops.overlap_window(w, self.grid_size, self.padding), self.grid_size,
+                                           self.padding):
+            kw.pop('overlap_window', None)
+            return False
+        return True
+
+    def _predict_overlap(self, model_fn, vols, on_batch, kw):
+        """predict_and_stitch of an overlap-weighted map: owners zero their blocks, ranks meet, then accumulate."""
+        if vols is None:
+            self.cube_index()
+            vols = self._exported_volumes(self._n_max())
+            self.sync_ranks()                     # nobody adds into a block before its owner has cleared it
+        return MapPipeline.predict_and_stitch(self, model_fn, vols, on_batch, **kw)
+
+
+class SlabPipeline(_SplitMap, MapPipeline):
     """One rank's share of a z-slab partitioned map.  ``run`` takes this rank's OWN block
     of source planes (global planes [own_lo, own_hi) of ``global_src_shape``)."""
 
     def __init__(self, device, rank, world, grid_size=48, padding=8, order=3, batch_cubes=16,
                  target_voxel_size=1.0, halo_k=16, global_src_shape=None, group=None, af3_mode='sparse',
-                 hist_exchange='peer', halo_exchange='peer'):
+                 hist_exchange='peer', halo_exchange='peer', _peer_volumes=None):
         super().__init__(device, grid_size, padding, order, batch_cubes, target_voxel_size, af3_mode)
         self.rank, self.world, self.halo_k, self.group = int(rank), int(world), halo_k, group
         self.global_src_shape = global_src_shape
@@ -181,6 +261,7 @@ class SlabPipeline(MapPipeline):
         self.hist_exchange = hist_exchange
         self.peer = None
         self.int_peer = None
+        self.peer_volumes = _peer_volumes         # built on first use by an overlap-weighted map
 
     def _peer_group(self):
         if self.peer is None:
@@ -399,8 +480,23 @@ class SlabPipeline(MapPipeline):
         org, ext = self.box
         return ops.StitchedVolumes(self.cube_shape, self.device, org=org, ext=ext)
 
+    def _owner_bounds(self):
+        return 2, [r.out_lo for r in self.plan.ranks] + [self.plan.ranks[-1].out_hi]
 
-class BalancedCubePipeline(MapPipeline):
+    def _n_max(self):
+        X, Y, _ = self.cube_shape
+        return max(r.out_hi - r.out_lo for r in self.plan.ranks) * X * Y
+
+    def predict_and_stitch(self, model_fn, vols=None, on_batch=None, **kw):
+        """As ``MapPipeline.predict_and_stitch`` for this rank's cubes.  With ``overlap_window`` the windows reach
+        ``padding`` planes into the neighbouring slabs: those contributions are added into the neighbours'
+        exported blocks, and the volumes are final after ``finish_map()`` on every rank."""
+        if self._weighted(kw):
+            return self._predict_overlap(model_fn, vols, on_batch, kw)
+        return super().predict_and_stitch(model_fn, vols, on_batch, **kw)
+
+
+class BalancedCubePipeline(_SplitMap, MapPipeline):
     """One map, its cubes dealt out EVENLY over the ranks (BASELINE configs[4]: the model-bound inference
     loop, where whole cube layers per rank would leave 11 layers / 8 GPUs = 69 % balance).
 
@@ -438,43 +534,28 @@ class BalancedCubePipeline(MapPipeline):
                     (self.x_bounds[self.rank + 1] - self.x_bounds[self.rank], self.cube_shape[1], self.cube_shape[2]))
         return self.ijk_host
 
+    def _n_max(self):
+        _, Y, Z = self.cube_shape
+        return max(self.x_bounds[r + 1] - self.x_bounds[r] for r in range(self.world)) * Y * Z
+
     def _new_volumes(self):
-        from .peer import PeerVolumes
-        X, Y, Z = self.cube_shape
-        n_max = max(self.x_bounds[r + 1] - self.x_bounds[r] for r in range(self.world)) * Y * Z
-        if self.peer_volumes is None or self.peer_volumes.n_voxels < n_max:
-            if self.peer_volumes is not None:
-                self.peer_volumes.close()
-            if self.world == 1:                   # nothing to map: one local block
-                self.peer_volumes = PeerVolumes.emulate(self.device, 1, n_max)[0]
-            elif self.group is False:
-                raise MicaError('in-process emulation of several ranks: pass _peer_volumes (PeerVolumes.emulate)')
-            else:
-                self.peer_volumes = PeerVolumes(self.device, self.rank, self.world, n_max, self.group)
-        org, ext = self.box
-        n = ext[0] * ext[1] * ext[2]
-        vols = ops.StitchedVolumes.from_block(self.peer_volumes.block(n_elems=23 * n), self.cube_shape, org, ext)
-        vols.block.zero_()
-        return vols
+        return self._exported_volumes(self._n_max())
+
+    def _owner_bounds(self):
+        return 0, self.x_bounds
 
     def stitch_fn(self, bb, ca, aa, ijk, vols):
         ops.postproc_stitch_peer(bb, ca, aa, ijk, self.cube_shape, self.peer_volumes.table, self.x_bounds,
                                  self.grid_size, self.padding)
 
     def predict_and_stitch(self, model_fn, vols=None, on_batch=None, **kw):
+        """With ``overlap_window`` every window contribution is added into the block of the rank that owns its x
+        plane; the normaliser comes from the full cube lattice, also under ``cube_subset``."""
+        if self._weighted(kw):
+            return self._predict_overlap(model_fn, vols, on_batch, kw)
         if vols is None:
             self.cube_index()
             vols = self._new_volumes()
             self.sync_ranks()                     # nobody stores into a block before its owner has cleared it
         kw.setdefault('stitch_fn', self.stitch_fn)
         return super().predict_and_stitch(model_fn, vols, on_batch, **kw)
-
-    def sync_ranks(self):
-        torch.cuda.synchronize(self.device)
-        if self.world > 1 and self.group is not False:
-            import torch.distributed as dist
-            dist.barrier(group=self.group)
-
-    def finish_map(self):
-        """All ranks' cores have landed: after this every rank may read its own volume block."""
-        self.sync_ranks()
