@@ -335,6 +335,13 @@ int mica_af3_fill_cubes(const void* workspace, int64_t n_atoms, int nz, int ny, 
                         int grid_size, int padding, const int32_t* ijk_prev, int n_prev,
                         const int32_t* ijk_next, int n_next, float* out, int64_t out_cube_stride,
                         int32_t* nonzero, mica_stream_t stream);
+/* The same with every slot's cube in a test-time-augmentation orientation (0..47, see mica_extract_cubes_oriented):
+ * the slots show the cubes ijk_prev in orientation_prev and are switched to ijk_next in orientation_next.  A slot
+ * that keeps its cube but changes orientation is cleared and set again.  mica_af3_fill_cubes = orientations 0, 0. */
+int mica_af3_fill_cubes_oriented(const void* workspace, int64_t n_atoms, int nz, int ny, int nx, const int perm[3],
+                                 int grid_size, int padding, const int32_t* ijk_prev, int n_prev,
+                                 const int32_t* ijk_next, int n_next, float* out, int64_t out_cube_stride,
+                                 int32_t* nonzero, int orientation_prev, int orientation_next, mica_stream_t stream);
 
 /* --------------------------------------------------------- R5/R6 cube extract
  * Replaces GridCreator.transpose + create_grids_from_mrc (utils/create_grids.py:67-176),
@@ -355,8 +362,20 @@ int mica_extract_cubes(const float* vol, int64_t chan_stride, int n_channels,
                        float* out, int64_t out_cube_stride, int32_t* nonzero, float* cube_max,
                        mica_stream_t stream);
 
+/* Test-time augmentation: every window in one of the 48 orientations of the cube (signed axis permutations).
+ * orientation = 8 p + f: p indexes the permutation pi of the window axes (0,1,2) in lexicographic order, bit a of f
+ * flips output axis a; out[b, c, u] = window[v] with v[pi[a]] = (f_a ? W-1-u_a : u_a), window = what
+ * mica_extract_cubes writes.  Orientation 0 IS mica_extract_cubes (same kernels, same bits); nonzero / cube_max do
+ * not depend on the orientation. */
+int mica_extract_cubes_oriented(const float* vol, int64_t chan_stride, int n_channels,
+                                int nz, int ny, int nx, int z0, int nz_local, const int perm[3],
+                                int grid_size, int padding, const int32_t* ijk, int n_cubes,
+                                float* out, int64_t out_cube_stride, int32_t* nonzero, float* cube_max,
+                                int orientation, mica_stream_t stream);
+
 /* diagnostic: which kernel the last mica_extract_cubes call on this thread used
- * (0 = row copy, 1 = shared-memory tiled transpose, 2 = TMA box loads; -1 = none yet) */
+ * (0 = row copy, 1 = shared-memory tiled transpose, 2 = TMA box loads, 3 = oriented window (orientation != 0);
+ * -1 = none yet) */
 int mica_last_extract_path(void);
 
 /* ------------------------------------------------ R7/R8 post-process + stitch
@@ -507,6 +526,18 @@ int mica_overlap_accumulate_fixed_peer(const float* bb, const float* ca, const f
                                        int n_cubes, int X, int Y, int Z, int grid_size, int padding,
                                        const float* window_w1, const double* norm, void* const* owner_base, int axis,
                                        const int* bounds, int world, mica_stream_t stream);
+/* _oriented: the logits are those of the windows in orientation `orientation` (0..47, mica_extract_cubes_oriented;
+ * test-time augmentation); each voxel's contribution is added at its position in the window itself.  A k-orientation
+ * average folds its 1/k into norm.  Orientation 0 is the plain call. */
+int mica_overlap_accumulate_fixed_oriented(const float* bb, const float* ca, const float* aa, const int32_t* ijk,
+                                           int n_cubes, int X, int Y, int Z, int grid_size, int padding,
+                                           const float* window_w1, const double* norm, int orientation, void* block,
+                                           mica_stream_t stream);
+int mica_overlap_accumulate_fixed_peer_oriented(const float* bb, const float* ca, const float* aa, const int32_t* ijk,
+                                                int n_cubes, int X, int Y, int Z, int grid_size, int padding,
+                                                const float* window_w1, const double* norm, int orientation,
+                                                void* const* owner_base, int axis, const int* bounds, int world,
+                                                mica_stream_t stream);
 int mica_overlap_finalize_fixed(void* block, int64_t n_voxels, mica_stream_t stream);
 /* 1 when `device` can add into the memory of `peer_device` with native atomics over the peer path
  * (cudaDevP2PAttrNativeAtomicSupported; 1 for device == peer_device), 0 when not, negative MICA_ERR_* on error. */

@@ -95,8 +95,12 @@ SIGNATURES = {
     'mica_af3_bin_atoms': (_i, [_p, _p, _p, _i64, _f, _f, _f, _i, _i, _i, _i, _i, _i, C.POINTER(_i), _i, _i,
                                 _p, _sz, _p, _p]),
     'mica_af3_fill_cubes': (_i, [_p, _i64, _i, _i, _i, C.POINTER(_i), _i, _i, _p, _i, _p, _i, _p, _i64, _p, _p]),
+    'mica_af3_fill_cubes_oriented': (_i, [_p, _i64, _i, _i, _i, C.POINTER(_i), _i, _i, _p, _i, _p, _i, _p, _i64, _p,
+                                          _i, _i, _p]),
     'mica_extract_cubes': (_i, [_p, _i64, _i, _i, _i, _i, _i, _i, C.POINTER(_i), _i, _i, _p, _i, _p, _i64,
                                 _p, _p, _p]),
+    'mica_extract_cubes_oriented': (_i, [_p, _i64, _i, _i, _i, _i, _i, _i, C.POINTER(_i), _i, _i, _p, _i, _p, _i64,
+                                         _p, _p, _i, _p]),
     'mica_last_extract_path': (_i, []),
     'mica_postproc_stitch': (_i, [_p, _p, _p, _p, _i, _i, _i, _i, C.POINTER(_i), C.POINTER(_i), _i, _i,
                                   _p, _p, _p, _p, _p]),
@@ -105,6 +109,10 @@ SIGNATURES = {
     'mica_overlap_accumulate_fixed': (_i, [_p, _p, _p, _p, _i, _i, _i, _i, _i, _i, C.POINTER(_f), _p, _p, _p]),
     'mica_overlap_accumulate_fixed_peer': (_i, [_p, _p, _p, _p, _i, _i, _i, _i, _i, _i, C.POINTER(_f), _p, _p, _i,
                                                 C.POINTER(_i), _i, _p]),
+    'mica_overlap_accumulate_fixed_oriented': (_i, [_p, _p, _p, _p, _i, _i, _i, _i, _i, _i, C.POINTER(_f), _p, _i,
+                                                    _p, _p]),
+    'mica_overlap_accumulate_fixed_peer_oriented': (_i, [_p, _p, _p, _p, _i, _i, _i, _i, _i, _i, C.POINTER(_f), _p,
+                                                         _i, _p, _i, C.POINTER(_i), _i, _p]),
     'mica_overlap_finalize_fixed': (_i, [_p, _i64, _p]),
     'mica_peer_atomics_supported': (_i, [_i, _i]),
     'mica_parse_pdb': (_i64, [C.c_char_p, _i64, _i, _i64, _p, _p, _p, _p, _p, _p, _p]),

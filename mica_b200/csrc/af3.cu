@@ -234,26 +234,39 @@ __device__ __forceinline__ int cube_id_of(const BinParams& P, const int32_t* __r
 // ijk_next[b] (b < n_next; left clean otherwise).  A voxel can be in both lists, so "clear, then set"
 // must stay ordered -- the kernel boundary does that, and inside a launch every entry is independent:
 // the entries of a slot spread over kFillBlocks CTAs, which keeps densely populated cubes cheap.
-// Stateless: the caller says what the slots hold.
+// Stateless: the caller says what the slots hold, and in which orientation (test-time augmentation: the slots
+// show every cube of the batch in one orientation, ops.orientation): an entry's window offset v is moved to the
+// oriented offset base + v0 s[0] + v1 s[1] + v2 s[2] (Orientation), the identity for orientation 0.  A slot that
+// keeps its cube but changes orientation is cleared and set again.
+struct FillOrient {
+  int oriented;  // 0: orientation 0, offsets used as binned
+  int base, s[3];
+};
+
 template <bool SET>
 __global__ void __launch_bounds__(256)
 af3_fill_cubes_kernel(BinWorkspace ws, BinParams P, const int32_t* __restrict__ ijk_prev, int n_prev,
                       const int32_t* __restrict__ ijk_next, int n_next, float* __restrict__ out,
-                      int64_t out_cube_stride, int32_t* __restrict__ nonzero) {
+                      int64_t out_cube_stride, int32_t* __restrict__ nonzero, FillOrient o, bool same_orientation) {
   const int slot = blockIdx.y;
   const int prev = slot < n_prev ? cube_id_of(P, ijk_prev, slot) : -1;
   const int next = slot < n_next ? cube_id_of(P, ijk_next, slot) : -1;
   if (SET && blockIdx.x == 0 && threadIdx.x == 0 && nonzero && next >= 0)
     nonzero[slot] = (ws.offsets[next + 1] > ws.offsets[next]) ? 1 : 0;
   const int id = SET ? next : prev;
-  if (id < 0 || prev == next) return;
+  if (id < 0 || (prev == next && same_orientation)) return;
   float* cube = out + (int64_t)slot * out_cube_stride;
   const int64_t W3 = (int64_t)P.W * P.W * P.W;
   const float val = SET ? 1.0f : 0.0f;
   const int e0 = ws.offsets[id], e1 = ws.offsets[id + 1];
   for (int e = e0 + blockIdx.x * 256 + threadIdx.x; e < e1; e += kFillBlocks * 256) {
     const unsigned v = ws.entries[e];
-    const unsigned off = v >> 8, b = v & 7u, r = (v >> 3) & 31u;
+    const unsigned b = v & 7u, r = (v >> 3) & 31u;
+    unsigned off = v >> 8;
+    if (o.oriented) {
+      const int W = P.W, v0 = (int)off / (W * W), v1 = ((int)off / W) % W, v2 = (int)off % W;
+      off = (unsigned)(o.base + v0 * o.s[0] + v1 * o.s[1] + v2 * o.s[2]);
+    }
     if (b) cube[(int64_t)(b - 1) * W3 + off] = val;
     if (r) cube[(int64_t)(r + 3) * W3 + off] = val;
   }
@@ -345,11 +358,25 @@ extern "C" int mica_af3_bin_atoms(const float* xyz, const int8_t* bb_ch, const i
   return MICA_OK;
 }
 
-extern "C" int mica_af3_fill_cubes(const void* workspace, int64_t n_atoms, int nz, int ny, int nx, const int perm[3],
-                                   int grid_size, int padding, const int32_t* ijk_prev, int n_prev,
-                                   const int32_t* ijk_next, int n_next, float* out, int64_t out_cube_stride,
-                                   int32_t* nonzero, mica_stream_t stream) {
+static FillOrient fill_orient(int code, int W) {
+  Orientation ori;
+  orientation_decode(code, W, &ori);
+  FillOrient o;
+  o.oriented = code != 0;
+  o.base = ori.base;
+  for (int m = 0; m < 3; ++m) o.s[m] = ori.s[m];
+  return o;
+}
+
+extern "C" int mica_af3_fill_cubes_oriented(const void* workspace, int64_t n_atoms, int nz, int ny, int nx,
+                                            const int perm[3], int grid_size, int padding, const int32_t* ijk_prev,
+                                            int n_prev, const int32_t* ijk_next, int n_next, float* out,
+                                            int64_t out_cube_stride, int32_t* nonzero, int orientation_prev,
+                                            int orientation_next, mica_stream_t stream) {
   MICA_REQUIRE(workspace && out, "null pointer");
+  Orientation ori;
+  MICA_REQUIRE(orientation_decode(orientation_prev, 1, &ori) && orientation_decode(orientation_next, 1, &ori),
+               "orientations %d, %d: each must be in 0..47", orientation_prev, orientation_next);
   MICA_REQUIRE(n_prev >= 0 && n_next >= 0 && (ijk_prev || n_prev == 0) && (ijk_next || n_next == 0), "bad slot lists");
   BinParams P;
   int rc = make_bin_params(P, nz, ny, nx, perm, grid_size, padding);
@@ -361,13 +388,23 @@ extern "C" int mica_af3_fill_cubes(const void* workspace, int64_t n_atoms, int n
   BinWorkspace ws = carve(const_cast<void*>(workspace), n_cubes, bin_capacity(n_atoms, grid_size, padding));
   if (n_prev > 0) {
     af3_fill_cubes_kernel<false><<<dim3(kFillBlocks, n_prev), 256, 0, (cudaStream_t)stream>>>(
-        ws, P, ijk_prev, n_prev, ijk_next, n_next, out, out_cube_stride, nonzero);
+        ws, P, ijk_prev, n_prev, ijk_next, n_next, out, out_cube_stride, nonzero, fill_orient(orientation_prev, P.W),
+        orientation_prev == orientation_next);
     MICA_LAUNCH_CHECK("af3_fill_cubes_kernel<clear>");
   }
   if (n_next > 0) {
     af3_fill_cubes_kernel<true><<<dim3(kFillBlocks, n_next), 256, 0, (cudaStream_t)stream>>>(
-        ws, P, ijk_prev, n_prev, ijk_next, n_next, out, out_cube_stride, nonzero);
+        ws, P, ijk_prev, n_prev, ijk_next, n_next, out, out_cube_stride, nonzero, fill_orient(orientation_next, P.W),
+        orientation_prev == orientation_next);
     MICA_LAUNCH_CHECK("af3_fill_cubes_kernel<set>");
   }
   return MICA_OK;
+}
+
+extern "C" int mica_af3_fill_cubes(const void* workspace, int64_t n_atoms, int nz, int ny, int nx, const int perm[3],
+                                   int grid_size, int padding, const int32_t* ijk_prev, int n_prev,
+                                   const int32_t* ijk_next, int n_next, float* out, int64_t out_cube_stride,
+                                   int32_t* nonzero, mica_stream_t stream) {
+  return mica_af3_fill_cubes_oriented(workspace, n_atoms, nz, ny, nx, perm, grid_size, padding, ijk_prev, n_prev,
+                                      ijk_next, n_next, out, out_cube_stride, nonzero, 0, 0, stream);
 }

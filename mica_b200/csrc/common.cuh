@@ -82,6 +82,35 @@ __device__ __forceinline__ void st_stream4(float4* p, float4 v) {
                : "memory");
 }
 
+// Test-time-augmentation orientation of a W^3 window (code 0..47, ops.orientation): code = 8 p + f, p the index
+// of the axis permutation pi in lexicographic order, bit a of f flips output axis a.  The oriented window is
+// O[u0,u1,u2] = C[v] with v[pi[a]] = (f_a ? W-1-u_a : u_a).
+constexpr int kNumOrientations = 48;
+struct Orientation {
+  int perm[3];  // pi: output axis a reads window axis perm[a]
+  int flip[3];  // 1 where output axis a is reversed
+  int inv[3];   // pi^-1: window axis m is output axis inv[m]
+  // flat offset of the ORIENTED position of window position v: base + v0 s[0] + v1 s[1] + v2 s[2]
+  int base, s[3];
+};
+static inline bool orientation_decode(int code, int W, Orientation* o) {
+  static const int kPerms[6][3] = {{0, 1, 2}, {0, 2, 1}, {1, 0, 2}, {1, 2, 0}, {2, 0, 1}, {2, 1, 0}};
+  if (code < 0 || code >= kNumOrientations) return false;
+  const int p = code >> 3, f = code & 7;
+  const int pw[3] = {W * W, W, 1};
+  o->base = 0;
+  for (int a = 0; a < 3; ++a) {
+    o->perm[a] = kPerms[p][a];
+    o->flip[a] = (f >> a) & 1;
+    o->inv[kPerms[p][a]] = a;
+  }
+  for (int a = 0; a < 3; ++a) {
+    o->s[o->perm[a]] = o->flip[a] ? -pw[a] : pw[a];
+    if (o->flip[a]) o->base += (W - 1) * pw[a];
+  }
+  return true;
+}
+
 // system-scope release / acquire on a flag word in (possibly peer) global memory: the PTX-model form of
 // "data, fence, flag" between GPUs
 __device__ __forceinline__ void st_release_sys(int* p, int v) {

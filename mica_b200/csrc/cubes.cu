@@ -142,6 +142,84 @@ extract_transpose_kernel(ExtractParams P) {
 }
 
 
+// ---- oriented windows (test-time augmentation, orientation code != 0, ops.orientation): P is expressed in OUTPUT
+// axes -- T, sstride and slab_axis of output axis a are those of window axis pi[a] -- and output axis a starts at
+// cube coordinate ijk[cax[a]] - pad, walked forwards (dir +1) or, flipped, backwards from the far end of the window.
+// MC = the output axis that walks memory x: 2 -> row copy (a flipped row only reverses the lanes: still one
+// 128-byte line per warp); 0 / 1 -> tiled transpose MC <-> 2 through shared memory as extract_transpose_kernel, so
+// loads along x and streaming stores along the output's fastest axis both stay 128-byte coalesced.
+struct OrientAxes {
+  int cax[3];
+  int dir[3];
+};
+
+__device__ __forceinline__ float load_oriented(const ExtractParams& P, const float* src, int p0, int p1, int p2) {
+  if (!in_map(P, p0, p1, p2)) return 0.f;
+  const int q0 = p0 - (P.slab_axis == 0 ? P.z0 : 0), q1 = p1 - (P.slab_axis == 1 ? P.z0 : 0),
+            q2 = p2 - (P.slab_axis == 2 ? P.z0 : 0);
+  const int qs = P.slab_axis == 0 ? q0 : (P.slab_axis == 1 ? q1 : q2);
+  if ((unsigned)qs >= (unsigned)P.nzl) return 0.f;
+  return __ldg(src + q0 * P.sstride[0] + q1 * P.sstride[1] + q2 * P.sstride[2]);
+}
+
+// grid = (W [output axis 0 for MC == 2, else the slow output axis that is not MC], B, C), block = (32, 8)
+template <int MC>
+__global__ void __launch_bounds__(256)
+extract_oriented_kernel(ExtractParams P, OrientAxes A) {
+  __shared__ float tile[32][33];
+  const int uo = blockIdx.x, c = blockIdx.z, b = blockIdx.y;
+  const int W = P.W;
+  int org[3];
+#pragma unroll
+  for (int a = 0; a < 3; ++a) org[a] = P.ijk[3 * b + A.cax[a]] - P.pad + (A.dir[a] < 0 ? W - 1 : 0);
+  const float* src = P.vol + (int64_t)c * P.chan_stride;
+  float* dst = P.out + (int64_t)b * P.out_cube_stride + (int64_t)c * W * W * W;
+  const int tx = threadIdx.x, ty = threadIdx.y;
+  bool any_nz = false;
+  float vmax = -CUDART_INF_F;
+  if (MC == 2) {
+    const int p0 = org[0] + A.dir[0] * uo;
+    for (int u1 = ty; u1 < W; u1 += 8) {
+      const int p1 = org[1] + A.dir[1] * u1;
+      for (int u2 = tx; u2 < W; u2 += 32) {
+        const float v = load_oriented(P, src, p0, p1, org[2] + A.dir[2] * u2);
+        any_nz |= (v != 0.f);
+        vmax = fmaxf(vmax, v);
+        st_stream(dst + ((int64_t)uo * W + u1) * W + u2, v);
+      }
+    }
+  } else {
+    constexpr int OA = 1 - (MC & 1);
+    const int64_t out_mc = (MC == 0) ? (int64_t)W * W : W;
+    const int64_t out_oa = (MC == 0) ? W : (int64_t)W * W;
+    const int po = org[OA] + A.dir[OA] * uo;
+    for (int t2 = 0; t2 < W; t2 += 32) {
+      for (int tc = 0; tc < W; tc += 32) {
+#pragma unroll
+        for (int r = 0; r < 4; ++r) {
+          const int u2 = t2 + ty + 8 * r, uc = tc + tx;
+          float v = 0.f;
+          if (u2 < W && uc < W) {
+            const int p2 = org[2] + A.dir[2] * u2, pc = org[MC] + A.dir[MC] * uc;
+            v = MC == 0 ? load_oriented(P, src, pc, po, p2) : load_oriented(P, src, po, pc, p2);
+          }
+          any_nz |= (v != 0.f);
+          vmax = fmaxf(vmax, v);
+          tile[ty + 8 * r][tx] = v;
+        }
+        __syncthreads();
+#pragma unroll
+        for (int r = 0; r < 4; ++r) {
+          const int uc = tc + ty + 8 * r, u2 = t2 + tx;
+          if (uc < W && u2 < W) st_stream(dst + uc * out_mc + uo * out_oa + u2, tile[tx][ty + 8 * r]);
+        }
+        __syncthreads();
+      }
+    }
+  }
+  block_flags(P, b, any_nz, vmax);
+}
+
 // ---- TMA path for the standard layout (cube axis 0 is memory-contiguous, W % 32 == 0,
 // 16-byte aligned rows): one CTA = one [32 a] x [BT b] x [W c] tile of one (cube, channel).
 // A single elected thread issues ONE cp.async.bulk.tensor box load of a rank-4 tensor map
@@ -245,12 +323,14 @@ using namespace mica;
 static thread_local int g_last_extract_path = -1;
 extern "C" int mica_last_extract_path(void) { return g_last_extract_path; }
 
-extern "C" int mica_extract_cubes(const float* vol, int64_t chan_stride, int n_channels,
-                                  int nz, int ny, int nx, int z0, int nz_local, const int perm[3],
-                                  int grid_size, int padding, const int32_t* ijk, int n_cubes,
-                                  float* out, int64_t out_cube_stride, int32_t* nonzero, float* cube_max,
-                                  mica_stream_t stream) {
+extern "C" int mica_extract_cubes_oriented(const float* vol, int64_t chan_stride, int n_channels,
+                                           int nz, int ny, int nx, int z0, int nz_local, const int perm[3],
+                                           int grid_size, int padding, const int32_t* ijk, int n_cubes,
+                                           float* out, int64_t out_cube_stride, int32_t* nonzero, float* cube_max,
+                                           int orientation, mica_stream_t stream) {
   cudaStream_t st = (cudaStream_t)stream;
+  Orientation ori;
+  MICA_REQUIRE(orientation_decode(orientation, 1, &ori), "orientation %d is not in 0..47", orientation);
   MICA_REQUIRE(vol && perm && out && (ijk || n_cubes == 0), "null pointer");
   MICA_REQUIRE(n_channels > 0 && n_channels <= 65535, "bad channel count %d", n_channels);
   MICA_REQUIRE(nz > 0 && ny > 0 && nx > 0, "empty volume");
@@ -287,6 +367,40 @@ extern "C" int mica_extract_cubes(const float* vol, int64_t chan_stride, int n_c
   P.cube_max = cube_max;
 
   const int contiguous_axis = perm[0] == 2 ? 0 : (perm[1] == 2 ? 1 : 2);
+  if (orientation != 0) {
+    ExtractParams Q = P;  // in output axes: output axis a walks window axis ori.perm[a]
+    OrientAxes A;
+    for (int a = 0; a < 3; ++a) {
+      Q.T[a] = P.T[ori.perm[a]];
+      Q.sstride[a] = P.sstride[ori.perm[a]];
+      A.cax[a] = ori.perm[a];
+      A.dir[a] = ori.flip[a] ? -1 : 1;
+    }
+    Q.slab_axis = ori.inv[P.slab_axis];
+    const int mc = ori.inv[contiguous_axis];
+    const int kMaxZ = 32768;
+    for (int b0 = 0; b0 < n_cubes; b0 += kMaxZ) {
+      const int nb = (n_cubes - b0 < kMaxZ) ? n_cubes - b0 : kMaxZ;
+      Q.ijk = ijk + 3 * (int64_t)b0;
+      Q.out = out + (int64_t)b0 * out_cube_stride;
+      Q.nonzero = nonzero ? nonzero + b0 : nullptr;
+      Q.cube_max = cube_max ? cube_max + b0 : nullptr;
+      if (nonzero || cube_max) {
+        init_flags_kernel<<<(nb + 255) / 256, 256, 0, st>>>(Q.nonzero, Q.cube_max, nb);
+        MICA_LAUNCH_CHECK("init_flags_kernel");
+      }
+      dim3 grid(W, nb, n_channels), block(32, 8);
+      if (mc == 2)
+        extract_oriented_kernel<2><<<grid, block, 0, st>>>(Q, A);
+      else if (mc == 0)
+        extract_oriented_kernel<0><<<grid, block, 0, st>>>(Q, A);
+      else
+        extract_oriented_kernel<1><<<grid, block, 0, st>>>(Q, A);
+      g_last_extract_path = 3;
+      MICA_LAUNCH_CHECK("extract_oriented_kernel");
+    }
+    return MICA_OK;
+  }
 
   // TMA path: standard layout, window a multiple of 32, 16-byte aligned base / rows / channels
   CUtensorMap tmap;
@@ -350,4 +464,13 @@ extern "C" int mica_extract_cubes(const float* vol, int64_t chan_stride, int n_c
     MICA_LAUNCH_CHECK("extract_cubes kernel");
   }
   return MICA_OK;
+}
+
+extern "C" int mica_extract_cubes(const float* vol, int64_t chan_stride, int n_channels,
+                                  int nz, int ny, int nx, int z0, int nz_local, const int perm[3],
+                                  int grid_size, int padding, const int32_t* ijk, int n_cubes,
+                                  float* out, int64_t out_cube_stride, int32_t* nonzero, float* cube_max,
+                                  mica_stream_t stream) {
+  return mica_extract_cubes_oriented(vol, chan_stride, n_channels, nz, ny, nx, z0, nz_local, perm, grid_size,
+                                     padding, ijk, n_cubes, out, out_cube_stride, nonzero, cube_max, 0, stream);
 }

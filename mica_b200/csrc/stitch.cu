@@ -161,6 +161,7 @@ struct OverlapParams {
   int X, Y, Z, pad, W;
   const double* norm;  // [X | Y | Z] reciprocals of the lattice weight sums
   uint32_t* block;     // local destination: 23 channels of [X, Y, Z]
+  int obase, os[3];    // logits of window voxel v at obase + v . os (Orientation; W^2, W, 1 for orientation 0)
 };
 
 // owners of the output along one cube axis (0 = x, 2 = k): rank r holds planes [bounds[r], bounds[r+1]) of that
@@ -187,7 +188,66 @@ __device__ __forceinline__ void red_add_u32(uint32_t* p, uint32_t v) {
   if (v) asm volatile("red.global.add.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
 }
 
-// grid = (B, W [window plane a] * ceil(W*W / 256)), block = 256: one window voxel per thread
+// where the contributions of window voxel (gx, gy, gz) go: the local block, or (PEER) the block of the rank that
+// owns its plane along O.axis.  Returns the channel-0 address; channels are vol_n apart.
+template <bool PEER>
+__device__ __forceinline__ uint32_t* overlap_dest(const OverlapParams& P, const OverlapOwners& O, int gx, int gy,
+                                                  int gz, int64_t* vol_n) {
+  if (!PEER) {
+    *vol_n = (int64_t)P.X * P.Y * P.Z;
+    return P.block + ((int64_t)gx * P.Y + gy) * P.Z + gz;
+  }
+  const int g = O.axis == 0 ? gx : gz;
+  int r = 0;
+  while (r + 1 < O.world && g >= O.bounds[r + 1]) ++r;
+  const int lo = O.bounds[r], n = O.bounds[r + 1] - lo;
+  if (O.axis == 0) {
+    *vol_n = (int64_t)n * P.Y * P.Z;
+    return O.base[r] + ((int64_t)(gx - lo) * P.Y + gy) * P.Z + gz;
+  }
+  *vol_n = (int64_t)P.X * P.Y * n;
+  return O.base[r] + ((int64_t)gx * P.Y + gy) * n + (gz - lo);
+}
+
+// the 22 contributions (backbone, carbon_alpha, amino_acid_probability x 20) of the logits at offset src of cube
+// b's [4 | 4 | 21] x W^3 channels: the softmax of the paste (postproc_stitch_kernel), maximum taken the same way
+constexpr int kOverlapQ = 22;
+__device__ __forceinline__ void overlap_contrib(const OverlapParams& P, int b, int64_t src, double scale,
+                                                uint32_t q[kOverlapQ]) {
+  const int64_t W3 = (int64_t)P.W * P.W * P.W;
+  const float* bb = P.bb + (int64_t)b * 4 * W3;
+  const float* ca = P.ca + (int64_t)b * 4 * W3;
+  const float* aa = P.aa + (int64_t)b * 21 * W3;
+  const float b0 = ld_stream(bb + src), b2 = ld_stream(bb + 2 * W3 + src), b3 = ld_stream(bb + 3 * W3 + src);
+  const float c0 = ld_stream(ca + src), c2 = ld_stream(ca + 2 * W3 + src), c3 = ld_stream(ca + 3 * W3 + src);
+  float l[20];
+#pragma unroll
+  for (int t = 0; t < 20; ++t) l[t] = ld_stream(aa + (int64_t)(t + 1) * W3 + src);
+  q[0] = overlap_fixed(softmax3_last(b0, b2, b3), scale);
+  q[1] = overlap_fixed(softmax3_last(c0, c2, c3), scale);
+  float m = l[0];
+#pragma unroll
+  for (int t = 1; t < 20; ++t) {
+    if (l[t] > m) m = l[t];
+  }
+  float s = 0.f;
+#pragma unroll
+  for (int t = 0; t < 20; ++t) {
+    l[t] = exp_neg(l[t] - m);
+    s += l[t];
+  }
+  const float rs = __frcp_rn(s);
+#pragma unroll
+  for (int t = 0; t < 20; ++t) q[2 + t] = overlap_fixed(l[t] * rs, scale);
+}
+
+// block channel of contribution ch: [backbone | carbon_alpha | (prediction) | probability x 20]
+__device__ __forceinline__ int64_t overlap_channel(int ch, int64_t vol_n) { return (ch < 2 ? ch : ch + 1) * vol_n; }
+
+// grid = (B, W [window plane a] * ceil(W*W / 256)), block = 256: one window voxel per thread, lanes along window
+// axis 2.  The logits are those of the window in orientation P.orient (test-time augmentation; orientation 0 = the
+// window itself): window voxel v reads them at the oriented offset obase + v . os, which for the orientations
+// run here (|os[2]| == 1: the fastest axis stays, possibly reversed) keeps the reads coalesced.
 // PEER: each contribution goes to the block of the rank that owns its plane along O.axis, locally or over NVLink
 template <bool PEER>
 __global__ void __launch_bounds__(256)
@@ -208,50 +268,64 @@ overlap_accumulate_kernel(OverlapParams P, OverlapWindow Wn, OverlapOwners O) {
   const float wb = Wn.w1[bj], wc = Wn.w1[c];
   if (wb == 0.f || wc == 0.f) return;
   const double scale = overlap_scale(wa, wb, wc, P.norm[gx], P.norm[P.X + gy], P.norm[P.X + P.Y + gz]);
-  uint32_t* base = P.block;
-  int64_t vol_n = (int64_t)P.X * P.Y * P.Z;
-  int64_t dst = ((int64_t)gx * P.Y + gy) * P.Z + gz;
-  if (PEER) {
-    const int g = O.axis == 0 ? gx : gz;
-    int r = 0;
-    while (r + 1 < O.world && g >= O.bounds[r + 1]) ++r;
-    const int lo = O.bounds[r], n = O.bounds[r + 1] - lo;
-    base = O.base[r];
-    if (O.axis == 0) {
-      vol_n = (int64_t)n * P.Y * P.Z;
-      dst = ((int64_t)(gx - lo) * P.Y + gy) * P.Z + gz;
-    } else {
-      vol_n = (int64_t)P.X * P.Y * n;
-      dst = ((int64_t)gx * P.Y + gy) * n + (gz - lo);
+  int64_t vol_n;
+  uint32_t* dst = overlap_dest<PEER>(P, O, gx, gy, gz, &vol_n);
+  const int64_t src = P.obase + (int64_t)a * P.os[0] + (int64_t)bj * P.os[1] + (int64_t)c * P.os[2];
+  uint32_t q[kOverlapQ];
+  overlap_contrib(P, b, src, scale, q);
+#pragma unroll
+  for (int t = 0; t < kOverlapQ; ++t) red_add_u32(dst + overlap_channel(t, vol_n), q[t]);
+}
+
+// The orientations that move the fastest axis (|os[2]| != 1): the logits are contiguous along window axis K (0 or 1),
+// the block along window axis 2.  One CTA = a 32 (axis K) x 32 (axis 2) tile of one plane of the remaining window
+// axis L: the 22 contributions are computed with lanes along K (coalesced logit reads), parked in shared memory
+// ([22][32][33] uint32, conflict-free both ways) and added with lanes along axis 2 (coalesced red.global.add).
+// grid = (B, W [plane of L] * ceil(W/32)^2), block = 256
+constexpr int kOverlapTileSmem = kOverlapQ * 32 * 33 * 4;
+template <bool PEER>
+__global__ void __launch_bounds__(256)
+overlap_accumulate_tiled_kernel(OverlapParams P, OverlapWindow Wn, OverlapOwners O, int K) {
+  extern __shared__ uint32_t tq[];
+  const int W = P.W, nt = (W + 31) >> 5;
+  const int b = blockIdx.x, l = blockIdx.y / (nt * nt), t = blockIdx.y - l * nt * nt;
+  if (Wn.w1[l] == 0.f) return;  // uniform over the CTA
+  const int tk = (t / nt) << 5, t2 = (t % nt) << 5;
+  const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
+  const int i0 = P.ijk[3 * b + 0] - P.pad, j0 = P.ijk[3 * b + 1] - P.pad, k0 = P.ijk[3 * b + 2] - P.pad;
+#pragma unroll 1
+  for (int r = 0; r < 4; ++r) {
+    const int vk = tk + tx, v2 = t2 + ty + 8 * r;
+    uint32_t q[kOverlapQ];
+#pragma unroll
+    for (int c = 0; c < kOverlapQ; ++c) q[c] = 0u;
+    if (vk < W && v2 < W) {
+      const int v0 = K == 0 ? vk : l, v1 = K == 0 ? l : vk;
+      const int gx = i0 + v0, gy = j0 + v1, gz = k0 + v2;
+      const float w0 = Wn.w1[v0], w1 = Wn.w1[v1], w2 = Wn.w1[v2];
+      if ((unsigned)gx < (unsigned)P.X && (unsigned)gy < (unsigned)P.Y && (unsigned)gz < (unsigned)P.Z &&
+          w0 != 0.f && w1 != 0.f && w2 != 0.f) {
+        const double scale = overlap_scale(w0, w1, w2, P.norm[gx], P.norm[P.X + gy], P.norm[P.X + P.Y + gz]);
+        const int64_t src = P.obase + (int64_t)v0 * P.os[0] + (int64_t)v1 * P.os[1] + (int64_t)v2 * P.os[2];
+        overlap_contrib(P, b, src, scale, q);
+      }
     }
+#pragma unroll
+    for (int c = 0; c < kOverlapQ; ++c) tq[(c * 32 + ty + 8 * r) * 33 + tx] = q[c];
   }
-  const int64_t W3 = (int64_t)W * W * W;
-  const float* bb = P.bb + (int64_t)b * 4 * W3;
-  const float* ca = P.ca + (int64_t)b * 4 * W3;
-  const float* aa = P.aa + (int64_t)b * 21 * W3;
-  const int64_t src = ((int64_t)a * W + bj) * W + c;
-  const float b0 = ld_stream(bb + src), b2 = ld_stream(bb + 2 * W3 + src), b3 = ld_stream(bb + 3 * W3 + src);
-  const float c0 = ld_stream(ca + src), c2 = ld_stream(ca + 2 * W3 + src), c3 = ld_stream(ca + 3 * W3 + src);
-  float l[20];
+  __syncthreads();
+#pragma unroll 1
+  for (int r = 0; r < 4; ++r) {
+    const int v2 = t2 + tx, vk = tk + ty + 8 * r;
+    if (vk >= W || v2 >= W) continue;
+    const int v0 = K == 0 ? vk : l, v1 = K == 0 ? l : vk;
+    const int gx = i0 + v0, gy = j0 + v1, gz = k0 + v2;
+    if ((unsigned)gx >= (unsigned)P.X || (unsigned)gy >= (unsigned)P.Y || (unsigned)gz >= (unsigned)P.Z) continue;
+    int64_t vol_n;
+    uint32_t* dst = overlap_dest<PEER>(P, O, gx, gy, gz, &vol_n);
 #pragma unroll
-  for (int t = 0; t < 20; ++t) l[t] = ld_stream(aa + (int64_t)(t + 1) * W3 + src);
-  red_add_u32(base + dst, overlap_fixed(softmax3_last(b0, b2, b3), scale));
-  red_add_u32(base + vol_n + dst, overlap_fixed(softmax3_last(c0, c2, c3), scale));
-  // the softmax of the paste (postproc_stitch_kernel), maximum taken the same way
-  float m = l[0];
-#pragma unroll
-  for (int t = 1; t < 20; ++t) {
-    if (l[t] > m) m = l[t];
+    for (int c = 0; c < kOverlapQ; ++c) red_add_u32(dst + overlap_channel(c, vol_n), tq[(c * 32 + tx) * 33 + ty + 8 * r]);
   }
-  float s = 0.f;
-#pragma unroll
-  for (int t = 0; t < 20; ++t) {
-    l[t] = exp_neg(l[t] - m);
-    s += l[t];
-  }
-  const float rs = __frcp_rn(s);
-#pragma unroll
-  for (int t = 0; t < 20; ++t) red_add_u32(base + (int64_t)(3 + t) * vol_n + dst, overlap_fixed(l[t] * rs, scale));
 }
 
 // in place over one 23-channel block of n voxels: sums -> float(s) 2^-31, arg-max of the 20 amino-acid sums
@@ -426,8 +500,13 @@ extern "C" int mica_stitch_cubes(const float* cubes, int n_ch, const int32_t* ij
 
 static int overlap_setup(const float* bb, const float* ca, const float* aa, const int32_t* ijk, int n_cubes, int X,
                          int Y, int Z, int grid_size, int padding, const float* window_w1, const double* norm,
-                         OverlapParams* P, OverlapWindow* Wn) {
+                         int orientation, OverlapParams* P, OverlapWindow* Wn) {
   MICA_REQUIRE(window_w1 && norm, "null pointer");
+  Orientation ori;
+  MICA_REQUIRE(orientation_decode(orientation, grid_size + 2 * padding, &ori), "orientation %d is not in 0..47",
+               orientation);
+  P->obase = ori.base;
+  for (int m = 0; m < 3; ++m) P->os[m] = ori.s[m];
   MICA_REQUIRE(n_cubes == 0 || (bb && ca && aa && ijk), "null input");
   MICA_REQUIRE(grid_size > 0 && padding >= 0 && X > 0 && Y > 0 && Z > 0, "bad geometry");
   const int W = grid_size + 2 * padding;
@@ -468,21 +547,31 @@ static int overlap_launch(OverlapParams P, const OverlapWindow& Wn, const Overla
     P.ca = ca + (int64_t)b0 * 4 * W3;
     P.aa = aa + (int64_t)b0 * 21 * W3;
     P.ijk = ijk + 3 * (int64_t)b0;
-    const int chunks = (P.W * P.W + 255) / 256;
-    overlap_accumulate_kernel<PEER><<<dim3(nb, P.W * chunks), 256, 0, stream>>>(P, Wn, O);
-    MICA_LAUNCH_CHECK(PEER ? "overlap_accumulate_kernel<peer>" : "overlap_accumulate_kernel");
+    if (P.os[2] == 1 || P.os[2] == -1) {
+      const int chunks = (P.W * P.W + 255) / 256;
+      overlap_accumulate_kernel<PEER><<<dim3(nb, P.W * chunks), 256, 0, stream>>>(P, Wn, O);
+      MICA_LAUNCH_CHECK(PEER ? "overlap_accumulate_kernel<peer>" : "overlap_accumulate_kernel");
+    } else {
+      const int nt = (P.W + 31) / 32, K = (P.os[0] == 1 || P.os[0] == -1) ? 0 : 1;
+      MICA_CUDA(cudaFuncSetAttribute(overlap_accumulate_tiled_kernel<PEER>,
+                                     cudaFuncAttributeMaxDynamicSharedMemorySize, kOverlapTileSmem));
+      overlap_accumulate_tiled_kernel<PEER><<<dim3(nb, P.W * nt * nt), 256, kOverlapTileSmem, stream>>>(P, Wn, O, K);
+      MICA_LAUNCH_CHECK(PEER ? "overlap_accumulate_tiled_kernel<peer>" : "overlap_accumulate_tiled_kernel");
+    }
   }
   return MICA_OK;
 }
 
-extern "C" int mica_overlap_accumulate_fixed(const float* bb, const float* ca, const float* aa, const int32_t* ijk,
-                                             int n_cubes, int X, int Y, int Z, int grid_size, int padding,
-                                             const float* window_w1, const double* norm, void* block,
-                                             mica_stream_t stream) {
+extern "C" int mica_overlap_accumulate_fixed_oriented(const float* bb, const float* ca, const float* aa,
+                                                      const int32_t* ijk, int n_cubes, int X, int Y, int Z,
+                                                      int grid_size, int padding, const float* window_w1,
+                                                      const double* norm, int orientation, void* block,
+                                                      mica_stream_t stream) {
   MICA_REQUIRE(block, "null block");
   OverlapParams P;
   OverlapWindow Wn;
-  int rc = overlap_setup(bb, ca, aa, ijk, n_cubes, X, Y, Z, grid_size, padding, window_w1, norm, &P, &Wn);
+  int rc = overlap_setup(bb, ca, aa, ijk, n_cubes, X, Y, Z, grid_size, padding, window_w1, norm, orientation, &P,
+                         &Wn);
   if (rc) return rc;
   if (n_cubes <= 0) return MICA_OK;
   P.block = static_cast<uint32_t*>(block);
@@ -493,17 +582,19 @@ extern "C" int mica_overlap_accumulate_fixed(const float* bb, const float* ca, c
   return overlap_launch<false>(P, Wn, O, n_cubes, (cudaStream_t)stream);
 }
 
-extern "C" int mica_overlap_accumulate_fixed_peer(const float* bb, const float* ca, const float* aa,
-                                                  const int32_t* ijk, int n_cubes, int X, int Y, int Z,
-                                                  int grid_size, int padding, const float* window_w1,
-                                                  const double* norm, void* const* owner_base, int axis,
-                                                  const int* bounds, int world, mica_stream_t stream) {
+extern "C" int mica_overlap_accumulate_fixed_peer_oriented(const float* bb, const float* ca, const float* aa,
+                                                           const int32_t* ijk, int n_cubes, int X, int Y, int Z,
+                                                           int grid_size, int padding, const float* window_w1,
+                                                           const double* norm, int orientation,
+                                                           void* const* owner_base, int axis, const int* bounds,
+                                                           int world, mica_stream_t stream) {
   MICA_REQUIRE(owner_base && bounds, "null owner table");
   MICA_REQUIRE(world >= 1 && world <= kStitchMaxWorld, "bad world size %d", world);
   MICA_REQUIRE(axis == 0 || axis == 2, "owner axis must be 0 (x) or 2 (k), got %d", axis);
   OverlapParams P;
   OverlapWindow Wn;
-  int rc = overlap_setup(bb, ca, aa, ijk, n_cubes, X, Y, Z, grid_size, padding, window_w1, norm, &P, &Wn);
+  int rc = overlap_setup(bb, ca, aa, ijk, n_cubes, X, Y, Z, grid_size, padding, window_w1, norm, orientation, &P,
+                         &Wn);
   if (rc) return rc;
   const int G = axis == 0 ? X : Z;
   MICA_REQUIRE(bounds[0] == 0 && bounds[world] == G, "bounds must run from 0 to %d", G);
@@ -516,6 +607,23 @@ extern "C" int mica_overlap_accumulate_fixed_peer(const float* bb, const float* 
   for (int r = 0; r <= world; ++r) O.bounds[r] = bounds[r];
   for (int r = world + 1; r <= kStitchMaxWorld; ++r) O.bounds[r] = G;
   return overlap_launch<true>(P, Wn, O, n_cubes, (cudaStream_t)stream);
+}
+
+extern "C" int mica_overlap_accumulate_fixed(const float* bb, const float* ca, const float* aa, const int32_t* ijk,
+                                             int n_cubes, int X, int Y, int Z, int grid_size, int padding,
+                                             const float* window_w1, const double* norm, void* block,
+                                             mica_stream_t stream) {
+  return mica_overlap_accumulate_fixed_oriented(bb, ca, aa, ijk, n_cubes, X, Y, Z, grid_size, padding, window_w1, norm,
+                                                0, block, stream);
+}
+
+extern "C" int mica_overlap_accumulate_fixed_peer(const float* bb, const float* ca, const float* aa,
+                                                  const int32_t* ijk, int n_cubes, int X, int Y, int Z,
+                                                  int grid_size, int padding, const float* window_w1,
+                                                  const double* norm, void* const* owner_base, int axis,
+                                                  const int* bounds, int world, mica_stream_t stream) {
+  return mica_overlap_accumulate_fixed_peer_oriented(bb, ca, aa, ijk, n_cubes, X, Y, Z, grid_size, padding, window_w1,
+                                                     norm, 0, owner_base, axis, bounds, world, stream);
 }
 
 extern "C" int mica_overlap_finalize_fixed(void* block, int64_t n_voxels, mica_stream_t stream) {

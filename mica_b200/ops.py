@@ -7,6 +7,7 @@ from __future__ import annotations
 
 import ctypes as C
 import functools
+import itertools
 from typing import NamedTuple
 
 import numpy as np
@@ -377,20 +378,21 @@ class Af3CubeFiller:
         self.ws = None
         self._geom = None
         self._shown = None          # the ijk tensor whose cubes the slots currently show (kept alive)
+        self._shown_orient = 0      # ... and the orientation they show them in
 
     @device_guard
-    def _fill(self, ijk, nonzero_ptr):
+    def _fill(self, ijk, nonzero_ptr, orient=0):
         n_atoms, (nz, ny, nx) = self._geom
         prev = self._shown
-        check(lib.mica_af3_fill_cubes(C.c_void_p(self.ws.data_ptr()), n_atoms, nz, ny, nx, _lib.int3(self.perm),
-                                      self.grid_size, self.padding,
-                                      C.c_void_p(prev.data_ptr()) if prev is not None else None,
-                                      int(prev.shape[0]) if prev is not None else 0,
-                                      C.c_void_p(ijk.data_ptr()) if ijk is not None else None,
-                                      int(ijk.shape[0]) if ijk is not None else 0,
-                                      C.c_void_p(self.buffer.data_ptr()), self.buffer.stride(0),
-                                      nonzero_ptr, _stream()), 'af3_fill_cubes')
-        self._shown = ijk
+        check(lib.mica_af3_fill_cubes_oriented(C.c_void_p(self.ws.data_ptr()), n_atoms, nz, ny, nx,
+                                               _lib.int3(self.perm), self.grid_size, self.padding,
+                                               C.c_void_p(prev.data_ptr()) if prev is not None else None,
+                                               int(prev.shape[0]) if prev is not None else 0,
+                                               C.c_void_p(ijk.data_ptr()) if ijk is not None else None,
+                                               int(ijk.shape[0]) if ijk is not None else 0,
+                                               C.c_void_p(self.buffer.data_ptr()), self.buffer.stride(0),
+                                               nonzero_ptr, self._shown_orient, orient, _stream()), 'af3_fill_cubes')
+        self._shown, self._shown_orient = ijk, orient
 
     def clear(self):
         """Un-scatter every slot (buffer back to all zeros)."""
@@ -428,8 +430,10 @@ class Af3CubeFiller:
         self.clear()
         self.ws, self._geom, self.status = other.ws, other._geom, other.status
 
-    def fill(self, ijk: torch.Tensor, nonzero: torch.Tensor | None = None) -> torch.Tensor:
-        """AF3 channels of the cubes ``ijk`` (int32 [B,3], B <= n_slots) -> view [B,24,W,W,W]."""
+    def fill(self, ijk: torch.Tensor, nonzero: torch.Tensor | None = None, orient: int = 0) -> torch.Tensor:
+        """AF3 channels of the cubes ``ijk`` (int32 [B,3], B <= n_slots) -> view [B,24,W,W,W], every cube in
+        orientation ``orient`` (``orientation``; ``nonzero`` does not depend on it)."""
+        orient = _orientation_arg(orient)
         B = int(ijk.shape[0])
         if B > self.n_slots:
             raise _lib.MicaError(f'batch of {B} cubes exceeds the {self.n_slots} slots')
@@ -440,8 +444,105 @@ class Af3CubeFiller:
         if self.buffer is None:
             W = self.grid_size + 2 * self.padding
             self.buffer = torch.zeros((self.n_slots, 24, W, W, W), dtype=torch.float32, device=self.device)
-        self._fill(ijk, p_nz)
+        self._fill(ijk, p_nz, orient)
         return self.buffer[:B]
+
+
+# ------------------------------------------------- test-time augmentation: orientations of the window
+#: the permutations of the window axes (0, 1, 2) in lexicographic order (the p of an orientation code)
+_AXIS_PERMS = tuple(itertools.permutations(range(3)))
+N_ORIENTATIONS = 48
+#: the named orientation sets of ``tta_orientations``
+TTA_SETS = ('flips', 'rot90', 'all')
+
+
+def _orientation_arg(code) -> int:
+    if isinstance(code, (bool, np.bool_)) or not isinstance(code, (int, np.integer)):
+        raise _lib.MicaError(f'an orientation is an int in 0..{N_ORIENTATIONS - 1}, got {code!r}')
+    if not 0 <= int(code) < N_ORIENTATIONS:
+        raise _lib.MicaError(f'orientation {int(code)} is not in 0..{N_ORIENTATIONS - 1}')
+    return int(code)
+
+
+def orientation(code):
+    """(perm, flips) of an orientation code 0..47 of the W^3 model-input window: ``code = 8 p + f``, ``perm`` the
+    p-th permutation of the axes (0, 1, 2) in lexicographic order, ``flips[a]`` = bit a of f.  The oriented window is
+    ``O[u0, u1, u2] = C[v]`` with ``v[perm[a]] = W-1-u_a if flips[a] else u_a``, i.e. ``np.transpose(C, perm)``
+    then ``np.flip`` along every output axis a with ``flips[a]`` (``orient_array``).  Code 0 is the identity.
+
+    The axes are those of the model input ``[B, C, u0, u1, u2]`` -- the window AFTER the D6 axis permutation of the
+    map (``perm`` of ``extract_cubes``), not the map's (z, y, x)."""
+    code = _orientation_arg(code)
+    return _AXIS_PERMS[code >> 3], tuple(bool((code >> a) & 1) for a in range(3))
+
+
+def orientation_code(perm, flips) -> int:
+    """The code of (perm, flips): inverse of ``orientation``."""
+    return 8 * _AXIS_PERMS.index(tuple(int(a) for a in perm)) + sum(1 << a for a in range(3) if flips[a])
+
+
+def orientation_det(code) -> int:
+    """+1 for a proper rotation (keeps chirality), -1 for a mirror image."""
+    perm, flips = orientation(code)
+    inversions = sum(1 for a in range(3) for b in range(a + 1, 3) if perm[a] > perm[b])
+    return (-1) ** (inversions + sum(flips))
+
+
+def orient_array(a: np.ndarray, code) -> np.ndarray:
+    """The window(s) ``a`` (the last three axes) in orientation ``code`` (a view)."""
+    perm, flips = orientation(code)
+    lead = a.ndim - 3
+    out = np.transpose(a, tuple(range(lead)) + tuple(lead + p for p in perm))
+    for ax in range(3):
+        if flips[ax]:
+            out = np.flip(out, lead + ax)
+    return out
+
+
+@functools.lru_cache(maxsize=None)
+def _orientation_table():
+    """compose[g][h] = code of orienting by h, then by g; every orientation acts faithfully on the 8 corners."""
+    probe = np.arange(8).reshape(2, 2, 2)
+    key = {orient_array(probe, c).tobytes(): c for c in range(N_ORIENTATIONS)}
+    return tuple(tuple(key[orient_array(orient_array(probe, h), g).tobytes()] for h in range(N_ORIENTATIONS))
+                 for g in range(N_ORIENTATIONS))
+
+
+def compose_orientations(g, h) -> int:
+    """The code of ``orient_array(orient_array(C, h), g)``."""
+    return _orientation_table()[_orientation_arg(g)][_orientation_arg(h)]
+
+
+def inverse_orientation(code) -> int:
+    """The code that maps ``orient_array(C, code)`` back to ``C``."""
+    return _orientation_table()[_orientation_arg(code)].index(0)
+
+
+def tta_orientations(tta):
+    """The orientation codes of a test-time augmentation, validated: None (no augmentation) -> None;
+    'flips' -> the 8 mirrorings of the axes (p = 0); 'rot90' -> the 24 proper rotations (det +1: they keep the
+    chirality of a protein); 'all' -> the 48; or a non-empty sequence of distinct codes 0..47, kept in its order.
+    Raises MicaError otherwise."""
+    if tta is None:
+        return None
+    if isinstance(tta, str):
+        if tta == 'flips':
+            return tuple(range(8))
+        if tta == 'rot90':
+            return tuple(c for c in range(N_ORIENTATIONS) if orientation_det(c) == 1)
+        if tta == 'all':
+            return tuple(range(N_ORIENTATIONS))
+        raise _lib.MicaError(f"tta must be one of {TTA_SETS}, a sequence of orientation codes or None, got {tta!r}")
+    try:
+        codes = tuple(_orientation_arg(c) for c in tta)
+    except TypeError:
+        raise _lib.MicaError(f'tta must be one of {TTA_SETS}, a sequence of orientation codes or None, '
+                             f'got {tta!r}') from None
+    if not codes:
+        raise _lib.MicaError('tta: an empty list of orientations')
+    if len(set(codes)) != len(codes):
+        raise _lib.MicaError(f'tta: orientation codes must be distinct, got {list(codes)}')
+    return codes
 
 
 # ------------------------------------------------------------ R5/R6 cube extract
@@ -459,10 +560,12 @@ def cube_origins(cube_shape, grid_size):
 @device_guard
 def extract_cubes(vol: torch.Tensor, ijk: torch.Tensor, grid_size: int = 48, padding: int = 8,
                   perm=STANDARD_PERM, *, global_nz=None, z0: int = 0, out: torch.Tensor | None = None,
-                  nonzero: torch.Tensor | None = None, cube_max: torch.Tensor | None = None):
+                  nonzero: torch.Tensor | None = None, cube_max: torch.Tensor | None = None, orient: int = 0):
     """vol [C,nz_local,ny,nx] (or [nz,ny,nx]) -> out [B,C,W,W,W] for the cube origins ``ijk``
     (int32 [B,3], cube space).  ``out`` may be a channel slice of a larger [B,Ctot,W,W,W]
-    buffer (only the batch stride may be non-dense)."""
+    buffer (only the batch stride may be non-dense).  ``orient``: every window in that orientation
+    (``orientation``; test-time augmentation), cut straight from the map; 0 = the windows as they are."""
+    orient = _orientation_arg(orient)
     if vol.dim() == 3:
         vol = vol.unsqueeze(0)
     p_vol = _dev(vol, torch.float32, 'vol')
@@ -480,9 +583,9 @@ def extract_cubes(vol: torch.Tensor, ijk: torch.Tensor, grid_size: int = 48, pad
     cube_stride = out.stride(0) if B else Cn * W ** 3
     p_nz = _dev(nonzero, torch.int32, 'nonzero') if nonzero is not None else None
     p_mx = _dev(cube_max, torch.float32, 'cube_max') if cube_max is not None else None
-    check(lib.mica_extract_cubes(p_vol, vol.stride(0), Cn, nz, ny, nx, z0, nzl, _lib.int3(perm), grid_size,
-                                 padding, p_ijk, B, C.c_void_p(out.data_ptr()), cube_stride, p_nz, p_mx,
-                                 _stream()), 'extract_cubes')
+    check(lib.mica_extract_cubes_oriented(p_vol, vol.stride(0), Cn, nz, ny, nx, z0, nzl, _lib.int3(perm), grid_size,
+                                          padding, p_ijk, B, C.c_void_p(out.data_ptr()), cube_stride, p_nz, p_mx,
+                                          orient, _stream()), 'extract_cubes')
     return out
 
 
@@ -636,22 +739,23 @@ def is_core_window(w1, grid_size: int, padding: int) -> bool:
     return np.array_equal(w1, overlap_window('core', grid_size, padding))
 
 
-def overlap_norm_tables(w1, cube_shape, grid_size: int, padding: int):
+def overlap_norm_tables(w1, cube_shape, grid_size: int, padding: int, tta_k: int = 1):
     """Reciprocals (0 where the sum is 0) of the 1-D weight sums Wx, Wy, Wz of the full cube lattice
     (``cube_origins``): the weight sum of the overlap-weighted stitch at voxel (x, y, z) is Wx[x] Wy[y] Wz[z], with
     Wx[x] = sum over the origins i covering x of w1[x - i + padding].  float64, origins added in ascending order.
-    Whatever part of the lattice a run stitches, these come from all of it."""
+    Whatever part of the lattice a run stitches, these come from all of it.  ``tta_k``: the number of orientations
+    of a test-time augmentation, every window then contributing k times; the x table holds 1 / (k Wx)."""
     w = np.asarray(w1, dtype=np.float32).astype(np.float64)
     W = len(w)
     out = []
-    for n in (int(v) for v in cube_shape):
+    for axis, n in enumerate(int(v) for v in cube_shape):
         s = np.zeros(n, np.float64)
         for i in range(0, n, int(grid_size)):
             lo = i - int(padding)
             x0, x1 = max(0, lo), min(n, lo + W)
             s[x0:x1] += w[x0 - lo:x1 - lo]
         r = np.zeros(n, np.float64)
-        np.divide(1.0, s, out=r, where=s > 0)
+        np.divide(1.0, s * int(tta_k) if axis == 0 else s, out=r, where=s > 0)
         out.append(r)
     return out
 
@@ -695,17 +799,23 @@ class OverlapStitcher:
     ``vols``: the volumes (``StitchedVolumes.from_block``, zeroed) this stitcher finalizes; default: a whole-map
     block of its own.  ``owners``: an ``OverlapOwners`` table -- contributions go to the block of the rank that
     owns their plane, locally or over NVLink (native peer atomics required); without ``vols`` such a stitcher only
-    accumulates."""
+    accumulates.
+
+    ``tta``: test-time augmentation (``tta_orientations``): every window is accumulated once per orientation, from
+    the logits of the model run on the window in that orientation (``accumulate(..., orient=)``), and the result is
+    the average over the k orientations -- the 1/k is in the normaliser tables.  Any window, 'core' included, then
+    runs in fixed point (orientations (0,) alone are the plain stitch).  NOT the reference's arithmetic either."""
 
     def __init__(self, cube_shape, device, grid_size: int = 48, padding: int = 8, window='uniform', *, vols=None,
-                 owners: OverlapOwners | None = None):
+                 owners: OverlapOwners | None = None, tta=None):
         self.shape = tuple(int(v) for v in cube_shape)
         self.device = torch.device(device)
         if self.device.index is None:
             self.device = torch.device('cuda', torch.cuda.current_device())
         self.grid_size, self.padding = int(grid_size), int(padding)
         self.w1 = overlap_window(window, grid_size, padding)
-        self.core = is_core_window(self.w1, self.grid_size, self.padding)
+        self.orientations = tta_orientations(tta) or (0,)
+        self.core = is_core_window(self.w1, self.grid_size, self.padding) and self.orientations == (0,)
         self.owners = owners
         if owners is not None:
             if owners.axis not in (0, 2) or (self.core and owners.axis != 0):
@@ -728,11 +838,15 @@ class OverlapStitcher:
         if not self.core:
             with torch.cuda.device(self.device):
                 self.norm = torch.from_numpy(np.concatenate(
-                    overlap_norm_tables(self.w1, self.shape, self.grid_size, self.padding))).to(self.device)
+                    overlap_norm_tables(self.w1, self.shape, self.grid_size, self.padding,
+                                        len(self.orientations)))).to(self.device)
         self._done = False
 
     @device_guard
-    def accumulate(self, bb, ca, aa, ijk, vols=None):
+    def accumulate(self, bb, ca, aa, ijk, vols=None, orient: int = 0):
+        """Add one batch of logits, those of the windows ``ijk`` in orientation ``orient`` (one of ``tta``)."""
+        if _orientation_arg(orient) not in self.orientations:
+            raise _lib.MicaError(f'orientation {orient} is not one of this stitcher\'s {list(self.orientations)}')
         if self.core:
             if self.owners is not None:
                 postproc_stitch_peer(bb, ca, aa, ijk, self.shape, self.owners.table, self.owners.bounds,
@@ -748,15 +862,15 @@ class OverlapStitcher:
         X, Y, Z = self.shape
         args = (_dev(bb, torch.float32, 'bb'), _dev(ca, torch.float32, 'ca'), _dev(aa, torch.float32, 'aa'),
                 _dev(ijk, torch.int32, 'ijk'), B, X, Y, Z, self.grid_size, self.padding,
-                self.w1.ctypes.data_as(C.POINTER(C.c_float)), C.c_void_p(self.norm.data_ptr()))
+                self.w1.ctypes.data_as(C.POINTER(C.c_float)), C.c_void_p(self.norm.data_ptr()), int(orient))
         if self.owners is None:
-            check(lib.mica_overlap_accumulate_fixed(*args, C.c_void_p(self.vols.block.data_ptr()), _stream()),
+            check(lib.mica_overlap_accumulate_fixed_oriented(*args, C.c_void_p(self.vols.block.data_ptr()), _stream()),
                   'overlap_accumulate')
         else:
             o = self.owners
-            check(lib.mica_overlap_accumulate_fixed_peer(*args, _dev(o.table, torch.int64, 'owner_table'), int(o.axis),
-                                                         self._bounds, int(o.table.numel()), _stream()),
-                  'overlap_accumulate_peer')
+            check(lib.mica_overlap_accumulate_fixed_peer_oriented(
+                *args, _dev(o.table, torch.int64, 'owner_table'), int(o.axis), self._bounds, int(o.table.numel()),
+                _stream()), 'overlap_accumulate_peer')
 
     @device_guard
     def finalize(self) -> StitchedVolumes:

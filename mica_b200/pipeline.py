@@ -386,28 +386,30 @@ class MapPipeline:
             self._af[slot] = torch.empty((B, 24, W, W, W), dtype=torch.float32, device=self.device)
         return self._af[slot][:B]
 
-    def _extract_map(self, ijk, x):
-        ops.extract_cubes(self.normalized, ijk, self.grid_size, self.padding, self.perm, out=x)
+    def _extract_map(self, ijk, x, orient=0):
+        ops.extract_cubes(self.normalized, ijk, self.grid_size, self.padding, self.perm, out=x, orient=orient)
 
-    def _extract_af3(self, ijk, af, nonzero):
-        ops.extract_cubes(self.af3, ijk, self.grid_size, self.padding, self.perm, out=af, nonzero=nonzero)
+    def _extract_af3(self, ijk, af, nonzero, orient=0):
+        ops.extract_cubes(self.af3, ijk, self.grid_size, self.padding, self.perm, out=af, nonzero=nonzero,
+                          orient=orient)
 
     @_on_device
-    def extract_batch(self, b0: int, b1: int, want_flags: bool = False, slot: int = 0):
+    def extract_batch(self, b0: int, b1: int, want_flags: bool = False, slot: int = 0, orient: int = 0):
         """Cubes [b0,b1) -> (exp_map [B,1,W,W,W], af_features [B,24,W,W,W][, nonzero flags])
         -- the two tensors MICA.forward takes (models/model.py:331).  ``slot`` picks one of
-        the two input buffers (the prefetch of batch n+1 must not overwrite batch n)."""
+        the two input buffers (the prefetch of batch n+1 must not overwrite batch n).  ``orient``: both
+        tensors in that orientation (``ops.orientation``; the flags do not depend on it)."""
         x, nzf = self._buffers(b1 - b0, slot)
         ijk = self.ijk[b0:b1]
         with self.timer('extract_map'):
-            self._extract_map(ijk, x)
+            self._extract_map(ijk, x, orient)
         if self._atoms_binned:
             with self.timer('af3_fill_cubes'):
-                af = self._fillers[slot].fill(ijk, nzf if want_flags else None)
+                af = self._fillers[slot].fill(ijk, nzf if want_flags else None, orient)
         elif self.af3 is not None:
             af = self._af_buffer(b1 - b0, slot)
             with self.timer('extract_af3'):
-                self._extract_af3(ijk, af, nzf if want_flags else None)
+                self._extract_af3(ijk, af, nzf if want_flags else None, orient)
         else:
             af = self._af_buffer(b1 - b0, slot)
             af.zero_()                                         # dataset/dataset.py:218-219
@@ -422,7 +424,7 @@ class MapPipeline:
     @_on_device
     def predict_and_stitch(self, model_fn, vols: ops.StitchedVolumes | None = None, on_batch=None, *,
                            model_batch=None, d8='none', order=None, stitch_fn=None, overlap_window=None,
-                           batches=None):
+                           batches=None, tta=None):
         """run_inference + reconstruct_volume (utils/predict.py:307-587) without the
         per-cube files.  ``model_fn(exp_map, af_features) -> (bb, ca, aa)`` logits, enqueued
         on the current stream.  With ``prefetch`` the cubes of batch n+1 are cut on a side
@@ -442,20 +444,33 @@ class MapPipeline:
         ``on_batch`` is then called once, with the finished volumes.  A split map (subclasses) supplies the owners
         of the output; its volumes are final after ``finish_map()``.  ``batches``: the super-batches as
         (b0, b1) ranges of the (ordered) cube list, each at most ``batch_cubes`` long, instead of the even cut
-        (``worker_batches``: a worker's share of a map dealt over several devices)."""
+        (``worker_batches``: a worker's share of a map dealt over several devices).
+
+        ``tta`` ('flips' | 'rot90' | 'all' | orientation codes, ``ops.tta_orientations``): test-time augmentation.
+        Every super-batch is cut, run through the model and accumulated once per orientation, and the volumes are
+        the average of the k orientations' probabilities (window weights ``overlap_window``, default 'core'), always
+        in the order-free fixed point of ``ops.OverlapStitcher`` -- NOT the reference's arithmetic.  The work list is
+        the (super-batch, orientation) pairs, fed through the same two-slot prefetch.  ``on_batch`` is called once,
+        with the finished volumes.  A ``stitch_fn`` then takes a sixth argument, the orientation of the logits.
+        ``tta=[0]`` is ``tta=None``."""
         if self.normalized is None:
             raise MicaError('no normalised map')
+        codes = ops.tta_orientations(tta)                                          # refused before any launch
+        if codes == (0,):
+            codes = None
         overlap = None
-        if overlap_window is not None:
-            w1 = ops.overlap_window(overlap_window, self.grid_size, self.padding)     # refused before any launch
-            if not ops.is_core_window(w1, self.grid_size, self.padding):          # 'core' IS the paste
-                if stitch_fn is not None:
+        if overlap_window is not None or codes is not None:
+            w1 = ops.overlap_window('core' if overlap_window is None else overlap_window, self.grid_size, self.padding)
+            if codes is not None or not ops.is_core_window(w1, self.grid_size, self.padding):    # 'core' IS the paste
+                if stitch_fn is not None and codes is None:
                     raise MicaError('overlap_window replaces the stitch: pass stitch_fn or overlap_window, not both')
-                overlap = w1
+                overlap = w1 if stitch_fn is None else None
         self.cube_index()
+        final_on_batch = None
         if overlap is not None:
-            overlap = self._overlap_stitcher(overlap, vols)
+            overlap = self._overlap_stitcher(overlap, vols, codes)
             stitch_fn, vols = overlap.accumulate, overlap.vols
+        if overlap is not None or codes is not None:
             final_on_batch, on_batch = on_batch, None
         if vols is None:
             vols = self._new_volumes()
@@ -472,7 +487,9 @@ class MapPipeline:
             if any(not 0 <= b0 < b1 <= n or b1 - b0 > self.batch_cubes for b0, b1 in batches):
                 raise MicaError(f'batches must be non-empty ranges of the {n} cubes, at most {self.batch_cubes} long')
         if not batches:
-            return self._overlap_done(overlap, final_on_batch, n) if overlap is not None else vols
+            return self._predict_done(overlap, final_on_batch, vols, n)
+        work = [(b0, b1, 0) for b0, b1 in batches] if codes is None else \
+            [(b0, b1, g) for b0, b1 in batches for g in codes]
         want_flags = d8 == 'split' and (model_batch is None or int(model_batch) > 1)
         if stitch_fn is None:
             bound = ops.StitchCall(vols, self.grid_size, self.padding)
@@ -481,15 +498,18 @@ class MapPipeline:
                 bound(bb, ca, aa, ijk)
         timed = self.timer is not _no_timer
 
-        def stitch(bb, ca, aa, ijk):
-            bb, ca, aa = _f32c(bb), _f32c(ca), _f32c(aa)
-            if timed:
-                with self.timer('postproc_stitch'):
-                    stitch_fn(bb, ca, aa, ijk, vols)
-            else:
-                stitch_fn(bb, ca, aa, ijk, vols)
+        orient_arg = () if codes is None else (0,)
 
-        def consume(cur, b0, b1):
+        def consume(cur, b0, b1, g):
+            extra = orient_arg and (g,)
+
+            def stitch(bb, ca, aa, ijk):
+                bb, ca, aa = _f32c(bb), _f32c(ca), _f32c(aa)
+                if timed:
+                    with self.timer('postproc_stitch'):
+                        stitch_fn(bb, ca, aa, ijk, vols, *extra)
+                else:
+                    stitch_fn(bb, ca, aa, ijk, vols, *extra)
             flags = None
             if want_flags:
                 x, af, nzf = cur
@@ -498,12 +518,12 @@ class MapPipeline:
                 x, af = cur[0], cur[1]
             run_model_chunks(model_fn, x, af, flags, self.ijk[b0:b1], stitch, model_batch, d8)
 
-        if not self.prefetch or len(batches) == 1:
-            for b0, b1 in batches:
-                consume(self.extract_batch(b0, b1, want_flags=want_flags), b0, b1)
+        if not self.prefetch or len(work) == 1:
+            for b0, b1, g in work:
+                consume(self.extract_batch(b0, b1, want_flags=want_flags, orient=g), b0, b1, g)
                 if on_batch is not None:
                     on_batch(vols, b1)
-            return self._overlap_done(overlap, final_on_batch, n) if overlap is not None else vols
+            return self._predict_done(overlap, final_on_batch, vols, n)
 
         t_enqueue = time.perf_counter()
         main = torch.cuda.current_stream(self.device)
@@ -518,28 +538,36 @@ class MapPipeline:
             with torch.cuda.stream(pre):
                 if consumed[slot] is not None:
                     pre.wait_event(consumed[slot])           # the model has read this buffer's last batch
-                out = self.extract_batch(*batches[i], want_flags=want_flags, slot=slot)
+                b0, b1, g = work[i]
+                out = self.extract_batch(b0, b1, want_flags=want_flags, slot=slot, orient=g)
                 ready[slot] = torch.cuda.Event()
                 ready[slot].record(pre)
             return out
 
         cur = cut(0)
-        for i, (b0, b1) in enumerate(batches):
-            nxt = cut(i + 1) if i + 1 < len(batches) else None
+        for i, (b0, b1, g) in enumerate(work):
+            nxt = cut(i + 1) if i + 1 < len(work) else None
             main.wait_event(ready[i & 1])
-            consume(cur, b0, b1)
+            consume(cur, b0, b1, g)
             consumed[i & 1] = torch.cuda.Event()
             consumed[i & 1].record(main)
             if on_batch is not None:
                 on_batch(vols, b1)
             cur = nxt
         self.last_loop_enqueue_ms = (time.perf_counter() - t_enqueue) * 1e3     # host side of the batch loop
-        return self._overlap_done(overlap, final_on_batch, n) if overlap is not None else vols
+        return self._predict_done(overlap, final_on_batch, vols, n)
 
-    def _overlap_stitcher(self, w1, vols):
+    def _predict_done(self, overlap, on_batch, vols, n):
+        if overlap is not None:
+            return self._overlap_done(overlap, on_batch, n)
+        if on_batch is not None:              # test-time augmentation into a caller's stitch_fn
+            on_batch(vols, n)
+        return vols
+
+    def _overlap_stitcher(self, w1, vols, tta=None):
         """The accumulator of an overlap-weighted map: the whole map in one block on this GPU (``vols``, if given,
         must be ``StitchedVolumes.from_block`` volumes of the whole map, zeroed)."""
-        return ops.OverlapStitcher(self.cube_shape, self.device, self.grid_size, self.padding, w1, vols=vols)
+        return ops.OverlapStitcher(self.cube_shape, self.device, self.grid_size, self.padding, w1, vols=vols, tta=tta)
 
     def _overlap_done(self, overlap, on_batch, n):
         vols = overlap.finalize()

@@ -158,7 +158,7 @@ class DeviceVolume:
 class CryoEMPredictor:
     def __init__(self, model_path, grids_path, output_path, save_output=True, device='cuda', quiet=False,
                  model=None, keep_on_device=True, host_volumes=None, host_pool=None, reference_batching=False,
-                 super_batch=256, release_inputs=True, devices=None, *, overlap_window=None):
+                 super_batch=256, release_inputs=True, devices=None, *, overlap_window=None, tta=None):
         """Additions to the reference signature (all optional):
 
         ``model``               an already loaded model (callable ``(exp_map, af_features) -> (bb, ca, aa)``).
@@ -189,9 +189,17 @@ class CryoEMPredictor:
         ``overlap_window``      (keyword only) None: the reference's paste of the cube cores.  'uniform',
                                 'triangle' or W = grid_size + 2 * padding weights: overlap-weighted stitching
                                 (``ops.OverlapStitcher``; NOT the reference's arithmetic, DESIGN.md D2), the same bits
-                                on one device and with ``devices=``.  'core' is the paste."""
+                                on one device and with ``devices=``.  'core' is the paste.
+        ``tta``                 (keyword only) test-time augmentation: 'flips' (8 mirrorings), 'rot90' (the 24
+                                rotations), 'all' (48) or a list of orientation codes (``ops.orientation``).  The
+                                model runs on every cube in each orientation and the probabilities are averaged
+                                (window ``overlap_window``, default 'core'; NOT the reference's arithmetic), the same
+                                bits on one device and with ``devices=``.  Needs the resident map GridCreator
+                                registers: with the reference's per-cube files it is logged and (False, {}) returned.
+                                A bad value is refused before any launch."""
         self.devices = devices
         self.overlap_window = overlap_window
+        self.tta = tta
         self.worker_cubes = None                        # cubes each worker ran (several devices only)
         self._workers = None
         self._models = None
@@ -435,9 +443,22 @@ class CryoEMPredictor:
         w1 = ops.overlap_window(self.overlap_window, gs, pad)
         return None if ops.is_core_window(w1, gs, pad) else w1
 
+    def _tta_codes(self):
+        """The orientations of a test-time-augmented map, or None (orientation 0 alone is no augmentation)."""
+        codes = ops.tta_orientations(self.tta)
+        return None if codes in (None, (0,)) else codes
+
     def run_inference_and_reconstruct(self):
         """run_inference + reconstruct_volume (utils/predict.py:307-512) fused.  Returns
         (device volumes, {name: pinned host tensor})."""
+        codes = self._tta_codes()
+        if codes is not None and self._source['kind'] != 'resident':
+            raise ops._lib.MicaError('tta cuts each cube in every orientation from the resident map: the per-cube '
+                                     'grid files hold no volume to cut them from')
+        if codes is not None and self._workers:
+            gs, pad = self._source['grid_size'], self._source['padding']
+            return self._run_on_devices(self._workers, ops.overlap_window(
+                'core' if self.overlap_window is None else self.overlap_window, gs, pad), codes)
         w1 = self._overlap_weights()
         if self._workers:
             return self._run_on_devices(self._workers, w1)
@@ -453,9 +474,10 @@ class CryoEMPredictor:
                 pipe = self._pipeline(dev)
                 order = self._reference_order() if self.reference_batching else None
                 self._pipe = pipe
-                if w1 is not None:                          # nothing is final before the last cube: no drain
+                if w1 is not None or codes is not None:     # nothing is final before the last cube: no drain
                     vols = pipe.predict_and_stitch(model, None, model_batch=self._model_batch(), d8=d8, order=order,
-                                                   overlap_window=w1)
+                                                   overlap_window=self.overlap_window if codes is not None else w1,
+                                                   tta=codes)
                     return vols, self._download(vols)
                 pipe.cube_index()
                 vols = pipe._new_volumes()
@@ -492,12 +514,13 @@ class CryoEMPredictor:
                 overlap.finalize()
             return vols, self._download(vols)
 
-    def _run_on_devices(self, workers, w1=None):
+    def _run_on_devices(self, workers, w1=None, tta=None):
         """The map's cubes dealt over ``workers`` (``deal_cubes``), one thread each.  Every worker stores its
         cores into ONE 23-channel block on workers[0] (``postproc_stitch_peer`` with a one-entry owner table) --
         or, with the window ``w1``, adds its weighted contributions into it (``ops.OverlapStitcher`` with that
         table), which workers[0] finalises after the last worker has finished; the host copies run once, after
-        that.  Returns what ``run_inference_and_reconstruct`` returns."""
+        that.  ``tta``: the orientations of a test-time augmentation (with ``w1``; every worker runs its cubes in
+        all of them).  Returns what ``run_inference_and_reconstruct`` returns."""
         s = self._source
         gs, pad = s['grid_size'], s['padding']
         primary, n, mb = workers[0], len(s['ijk']), self._model_batch()
@@ -560,7 +583,8 @@ class CryoEMPredictor:
         overlap = None
         if w1 is not None:
             overlap = {d: ops.OverlapStitcher(cube_shape, d, gs, pad, w1, vols=vols if d == primary else None,
-                                              owners=ops.OverlapOwners(tables[d], 0, (0, X), (primary.index,)))
+                                              owners=ops.OverlapOwners(tables[d], 0, (0, X), (primary.index,)),
+                                              tta=tta)
                        for d in dict.fromkeys(workers)}
         for dev, st in zip(workers, streams):
             st.wait_stream(torch.cuda.current_stream(dev))     # inputs copied / binned on the current streams
@@ -575,16 +599,17 @@ class CryoEMPredictor:
                 return
             dev, table, model = workers[w], tables[workers[w]], self._models[workers[w]]
 
-            def stitch(bb, ca, aa, ijk, _vols=None):
+            def stitch(bb, ca, aa, ijk, _vols=None, orient=0):
                 bb, ca, aa = bb.contiguous().float(), ca.contiguous().float(), aa.contiguous().float()
                 if overlap is not None:
-                    overlap[dev].accumulate(bb, ca, aa, ijk)
+                    overlap[dev].accumulate(bb, ca, aa, ijk, orient=orient)
                 else:
                     ops.postproc_stitch_peer(bb, ca, aa, ijk, cube_shape, table, (0, X), gs, pad)
             with torch.cuda.device(dev), torch.cuda.stream(streams[w]), torch.no_grad():
                 if resident:
                     pipes[w].predict_and_stitch(model, vols, model_batch=mb, d8=d8, order=order[lo:hi],
-                                                batches=worker_batches(lo, hi, super_batch), stitch_fn=stitch)
+                                                batches=worker_batches(lo, hi, super_batch), stitch_fn=stitch,
+                                                tta=tta)
                     return
                 for b0, b1 in worker_batches(lo, hi, super_batch):
                     x, af, flags = self._fetch_files(lo + b0, lo + b1, dev)
@@ -635,6 +660,7 @@ class CryoEMPredictor:
     def run_prediction(self):
         t_total = time.time()
         try:
+            self._tta_codes()                                    # a bad tta is refused before any launch
             self._workers = self._resolve_workers()
             if not self.select_processing_strategy():
                 return False, {}

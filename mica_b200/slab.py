@@ -201,7 +201,7 @@ class _SplitMap:
         """(cube axis, world + 1 plane bounds) of the output partition."""
         raise NotImplementedError
 
-    def _overlap_stitcher(self, w1, vols):
+    def _overlap_stitcher(self, w1, vols, tta=None):
         if vols is None or getattr(vols, 'block', None) is None:
             raise MicaError('a split map stitches overlap-weighted into its exported volumes (predict_and_stitch '
                             'builds them when vols is None)')
@@ -209,14 +209,18 @@ class _SplitMap:
         pv = self.peer_volumes
         owners = ops.OverlapOwners(pv.table, axis, tuple(bounds), tuple(pv.devices))
         return ops.OverlapStitcher(self.cube_shape, self.device, self.grid_size, self.padding, w1, vols=vols,
-                                   owners=owners)
+                                   owners=owners, tta=tta)
 
     def _overlap_done(self, overlap, on_batch, n):
         self._overlap_pending = (overlap, on_batch, n)        # finalised by finish_map, once every rank has added
         return overlap.vols
 
     def _weighted(self, kw):
-        """True when ``kw`` asks for an overlap-weighted stitch other than 'core' (which is the paste)."""
+        """True when ``kw`` asks for an overlap-weighted stitch other than 'core' (which is the paste), or for a
+        test-time augmentation (other than orientation 0 alone), which always accumulates."""
+        if ops.tta_orientations(kw.get('tta')) not in (None, (0,)):
+            return True
+        kw.pop('tta', None)
         w = kw.get('overlap_window')
         if w is None or ops.is_core_window(ops.overlap_window(w, self.grid_size, self.padding), self.grid_size,
                                            self.padding):
@@ -468,13 +472,13 @@ class SlabPipeline(_SplitMap, MapPipeline):
         self.box = ((0, 0, me.out_lo), (self.cube_shape[0], self.cube_shape[1], me.out_hi - me.out_lo))
         return self.ijk_host
 
-    def _extract_map(self, ijk, x):
+    def _extract_map(self, ijk, x, orient=0):
         ops.extract_cubes(self.normalized, ijk, self.grid_size, self.padding, self.perm, out=x,
-                          global_nz=self.global_nz, z0=self.z0)
+                          global_nz=self.global_nz, z0=self.z0, orient=orient)
 
-    def _extract_af3(self, ijk, af, nonzero):
+    def _extract_af3(self, ijk, af, nonzero, orient=0):
         ops.extract_cubes(self.af3, ijk, self.grid_size, self.padding, self.perm, out=af,
-                          global_nz=self.global_nz, z0=self.z0, nonzero=nonzero)
+                          global_nz=self.global_nz, z0=self.z0, nonzero=nonzero, orient=orient)
 
     def _new_volumes(self):
         org, ext = self.box
@@ -488,9 +492,9 @@ class SlabPipeline(_SplitMap, MapPipeline):
         return max(r.out_hi - r.out_lo for r in self.plan.ranks) * X * Y
 
     def predict_and_stitch(self, model_fn, vols=None, on_batch=None, **kw):
-        """As ``MapPipeline.predict_and_stitch`` for this rank's cubes.  With ``overlap_window`` the windows reach
-        ``padding`` planes into the neighbouring slabs: those contributions are added into the neighbours'
-        exported blocks, and the volumes are final after ``finish_map()`` on every rank."""
+        """As ``MapPipeline.predict_and_stitch`` for this rank's cubes.  With ``overlap_window`` (or ``tta``) the
+        windows reach ``padding`` planes into the neighbouring slabs: those contributions are added into the
+        neighbours' exported blocks, and the volumes are final after ``finish_map()`` on every rank."""
         if self._weighted(kw):
             return self._predict_overlap(model_fn, vols, on_batch, kw)
         return super().predict_and_stitch(model_fn, vols, on_batch, **kw)
@@ -549,8 +553,8 @@ class BalancedCubePipeline(_SplitMap, MapPipeline):
                                  self.grid_size, self.padding)
 
     def predict_and_stitch(self, model_fn, vols=None, on_batch=None, **kw):
-        """With ``overlap_window`` every window contribution is added into the block of the rank that owns its x
-        plane; the normaliser comes from the full cube lattice, also under ``cube_subset``."""
+        """With ``overlap_window`` (or ``tta``) every window contribution is added into the block of the rank that
+        owns its x plane; the normaliser comes from the full cube lattice, also under ``cube_subset``."""
         if self._weighted(kw):
             return self._predict_overlap(model_fn, vols, on_batch, kw)
         if vols is None:
