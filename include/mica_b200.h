@@ -373,6 +373,16 @@ int mica_extract_cubes_oriented(const float* vol, int64_t chan_stride, int n_cha
                                 float* out, int64_t out_cube_stride, int32_t* nonzero, float* cube_max,
                                 int orientation, mica_stream_t stream);
 
+/* Window maximum of every cube, for the inference keep rule of the reference's training grids
+ * (create_grids_for_normalized_map.py:78: a window whose max is below min_max is not written).
+ * out[b] (device float32 [n_cubes]) = the maximum of the W^3 window mica_extract_cubes cuts for cube b from vol
+ * (one channel, [nz_local, ny, nx] holding global planes [z0, z0+nz_local)), zeros standing for the parts outside
+ * the map or the slab; NaN if the window holds a NaN (np.max; the extract's cube_max ignores NaN).  Read-only: no
+ * per-voxel output. */
+int mica_cube_window_max(const float* vol, int nz, int ny, int nx, int z0, int nz_local, const int perm[3],
+                         int grid_size, int padding, const int32_t* ijk, int n_cubes, float* out,
+                         mica_stream_t stream);
+
 /* diagnostic: which kernel the last mica_extract_cubes call on this thread used
  * (0 = row copy, 1 = shared-memory tiled transpose, 2 = TMA box loads, 3 = oriented window (orientation != 0);
  * -1 = none yet) */
@@ -393,6 +403,13 @@ int mica_postproc_stitch(const float* bb, const float* ca, const float* aa,
                          const int org[3], const int ext[3], int grid_size, int padding,
                          float* bb_vol, float* ca_vol, float* aa_prob_vol, float* aa_pred_vol,
                          mica_stream_t stream);
+
+/* The cores of the cubes ijk (device int32 [B,3]) the model did not run on -- skipped by the inference keep rule --
+ * set to 0 in all four volumes (box and layout as mica_postproc_stitch): what the reference's stitcher leaves where a
+ * cube has no grid file.  Needed only for volumes that held an earlier map; fresh volumes are zero. */
+int mica_zero_cores(const int32_t* ijk, int n_cubes, int X, int Y, int Z, const int org[3], const int ext[3],
+                    int grid_size, float* bb_vol, float* ca_vol, float* aa_prob_vol, float* aa_pred_vol,
+                    mica_stream_t stream);
 
 /* plain centre-crop paste of already post-processed cubes (reconstruct_volume on
  * its own, utils/predict.py:494-501): cubes device [B, n_ch, W^3] -> vol [n_ch, ext...] */

@@ -102,8 +102,10 @@ SIGNATURES = {
     'mica_extract_cubes_oriented': (_i, [_p, _i64, _i, _i, _i, _i, _i, _i, C.POINTER(_i), _i, _i, _p, _i, _p, _i64,
                                          _p, _p, _i, _p]),
     'mica_last_extract_path': (_i, []),
+    'mica_cube_window_max': (_i, [_p, _i, _i, _i, _i, _i, C.POINTER(_i), _i, _i, _p, _i, _p, _p]),
     'mica_postproc_stitch': (_i, [_p, _p, _p, _p, _i, _i, _i, _i, C.POINTER(_i), C.POINTER(_i), _i, _i,
                                   _p, _p, _p, _p, _p]),
+    'mica_zero_cores': (_i, [_p, _i, _i, _i, _i, C.POINTER(_i), C.POINTER(_i), _i, _p, _p, _p, _p, _p]),
     'mica_stitch_cubes': (_i, [_p, _i, _p, _i, _i, _i, _i, C.POINTER(_i), C.POINTER(_i), _i, _i, _p, _p]),
     'mica_postproc_stitch_peer': (_i, [_p, _p, _p, _p, _i, _i, _i, _i, _i, _i, _p, C.POINTER(_i), _i, _p]),
     'mica_overlap_accumulate_fixed': (_i, [_p, _p, _p, _p, _i, _i, _i, _i, _i, _i, C.POINTER(_f), _p, _p, _p]),

@@ -5,7 +5,12 @@ By default no per-cube ``.npz`` file is written: the cube index (origins, window
 axis permutation) and the resident volume -- or, for the AF3 channels, just the atoms --
 are registered under ``output_dir`` for CryoEMPredictor, which cuts the cubes on the GPU
 straight into the model batch on the pipeline DataPreprocessor started.
-``materialize=True`` also writes the reference's files (same names and keys)."""
+``materialize=True`` also writes the reference's files (same names and keys).
+
+``min_max`` (or the ``MICA_MIN_MAX`` environment variable): register -- and write -- only the cubes of the
+normalised map whose window maximum is not below it, the rule the reference applies to its training grids
+(create_grids_for_normalized_map.py:78).  CryoEMPredictor then predicts exactly those cubes; the cores of the
+others stay 0, as in the reference's stitcher when a grid file is absent."""
 from __future__ import annotations
 
 import glob
@@ -17,14 +22,31 @@ import numpy as np
 import torch
 
 from . import mrc, ops, pdb, session
+from ._lib import MicaError
 from .pipeline import MapHeader
 
 
+def env_min_max():
+    """``MICA_MIN_MAX`` as a finite float, None when unset or empty; MicaError for anything else."""
+    text = os.environ.get('MICA_MIN_MAX', '').strip()
+    if not text:
+        return None
+    try:
+        v = float(text)
+    except ValueError:
+        raise MicaError(f'MICA_MIN_MAX={text!r} is not a number') from None
+    return ops.check_min_max(v)
+
+
 class GridCreator:
-    def __init__(self, quiet=False, device='cuda', materialize=False):
+    def __init__(self, quiet=False, device='cuda', materialize=False, min_max=None):
+        """``min_max``: keep only the normalised map's cubes whose window maximum is not below this finite number
+        (ties and windows holding a NaN are kept); None reads ``MICA_MIN_MAX`` (unset or empty: every cube).  A bad
+        value is logged and the grid creation fails before any launch."""
         self.quiet = quiet
         self.device = torch.device(device)
         self.materialize = materialize
+        self.min_max = min_max
         self.logger = logging.getLogger(__name__)
         self.processed_count = 0
         self.failed_count = 0
@@ -80,13 +102,19 @@ class GridCreator:
                          mapc=header.mapc, mapr=header.mapr, maps=header.maps)
 
     # utils/create_grids.py:89-184
-    def create_grids_from_mrc(self, mrc_file, output_dir, grid_size=48, padding=8, file_prefix='grid'):
+    def create_grids_from_mrc(self, mrc_file, output_dir, grid_size=48, padding=8, file_prefix='grid', *,
+                              min_max=None):
+        """``min_max``: only the cubes the keep rule keeps (``ops.select_cubes``) are registered and written."""
         try:
+            min_max = ops.check_min_max(min_max)                  # refused before any launch
             vol, header = self._load(mrc_file)
             perm, offset, cube_shape, ijk = self._index(tuple(vol.shape), header, grid_size)
+            if min_max is not None:
+                maxima = ops.cube_window_max(vol, torch.from_numpy(ijk).to(vol.device), grid_size, padding, perm)
+                ijk = np.ascontiguousarray(ijk[ops.select_cubes(maxima, min_max)])
             session.put(output_dir, kind='cubes', volume=vol, header=header, perm=perm, offset=offset,
                         cube_shape=cube_shape, ijk=ijk, grid_size=grid_size, padding=padding, prefix=file_prefix,
-                        pipe=self._pipe, source=mrc_file)
+                        pipe=self._pipe, source=mrc_file, min_max=min_max)
             if self.materialize:
                 self._write_npz(vol, header, perm, cube_shape, ijk, output_dir, grid_size, padding, file_prefix)
             return len(ijk), offset
@@ -101,8 +129,13 @@ class GridCreator:
             error_msg = f'Normalized map not found: {normalized_map_path}'
             self.logger.error(error_msg)
             return {'success': False, 'error': error_msg}
+        try:
+            min_max = ops.check_min_max(self.min_max) if self.min_max is not None else env_min_max()
+        except MicaError as e:
+            self.logger.error(f'Grid creation refused: {e}')
+            return {'success': False, 'error': str(e)}
         grid_count, offset = self.create_grids_from_mrc(normalized_map_path, output_dir, grid_size, padding,
-                                                        'normalized_map_grid')
+                                                        'normalized_map_grid', min_max=min_max)
         return {'success': grid_count > 0, 'grid_count': grid_count, 'offset': offset,
                 'output_directory': output_dir, 'processing_time': time.time() - start_time,
                 'input_file': normalized_map_path}

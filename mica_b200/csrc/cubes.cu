@@ -309,6 +309,68 @@ extract_tma_kernel(const __grid_constant__ CUtensorMap tmap, TmaExtractParams P)
 
 constexpr int kTmaBT = 4;  // b-rows per tile: 4 * 64 * 128 B = 32 KB of shared memory per CTA
 
+// ---- window maximum (inference keep rule, ops.select_cubes): out[b] = max of cube b's W^3 window, zeros standing
+// for the parts outside the map (np.pad), NaN if the window holds one (np.max).  The maximum does not depend on the
+// element order, so the window is walked as the axis-aligned box it covers in MEMORY order, whatever the perm: rows
+// along x stay coalesced, and nothing is written per voxel.  One CTA per cube; warps take (z, y, 32-wide x chunk)
+// items, four independent loads in flight per thread.
+struct WindowMaxParams {
+  const float* vol;     // [nz_local, ny, nx]
+  int ny, nx;
+  int lo_z, hi_z;       // the planes the block holds, global: [z0, z0 + nz_local)
+  int z0;
+  int inv[3];           // inv[a] = cube axis that walks memory axis a (0 = z, 1 = y, 2 = x)
+  int W, pad;
+  const int32_t* ijk;
+  float* out;
+};
+
+__global__ void __launch_bounds__(256)
+cube_window_max_kernel(WindowMaxParams P) {
+  const int b = blockIdx.x;
+  int lo[3], n[3];
+  bool clipped = false;
+  const int dim_lo[3] = {P.lo_z, 0, 0}, dim_hi[3] = {P.hi_z, P.ny, P.nx};
+#pragma unroll
+  for (int a = 0; a < 3; ++a) {
+    const int w0 = P.ijk[3 * b + P.inv[a]] - P.pad;
+    const int a0 = max(w0, dim_lo[a]), a1 = min(w0 + P.W, dim_hi[a]);
+    lo[a] = a0;
+    n[a] = max(0, a1 - a0);
+    clipped |= n[a] < P.W;
+  }
+  float vmax = clipped ? 0.f : -CUDART_INF_F;
+  bool nan = false;
+  const int chunks = (n[2] + 31) >> 5;
+  const int items = n[0] * n[1] * chunks;
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const float* base = P.vol + ((int64_t)(lo[0] - P.z0) * P.ny + lo[1]) * P.nx + lo[2];
+#pragma unroll 4
+  for (int it = warp; it < items; it += 8) {
+    const int c = it % chunks, row = it / chunks;
+    const int x = (c << 5) + lane;
+    if (x < n[2]) {
+      const int y = row % n[1], z = row / n[1];
+      const float v = __ldg(base + ((int64_t)z * P.ny + y) * P.nx + x);
+      nan |= v != v;
+      vmax = fmaxf(vmax, v);
+    }
+  }
+  __shared__ float red[8];
+  __shared__ int any_nan;
+  if (threadIdx.x == 0) any_nan = 0;
+  for (int o = 16; o > 0; o >>= 1) vmax = fmaxf(vmax, __shfl_xor_sync(0xffffffffu, vmax, o));
+  if (lane == 0) red[warp] = vmax;
+  __syncthreads();
+  if (nan) any_nan = 1;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    float m = red[0];
+    for (int w = 1; w < 8; ++w) m = fmaxf(m, red[w]);
+    P.out[b] = any_nan ? CUDART_NAN_F : m;
+  }
+}
+
 __global__ void init_flags_kernel(int32_t* nonzero, float* cube_max, int n) {
   int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
@@ -463,6 +525,40 @@ extern "C" int mica_extract_cubes_oriented(const float* vol, int64_t chan_stride
     g_last_extract_path = use_tma ? 2 : (contiguous_axis == 2 ? 0 : 1);
     MICA_LAUNCH_CHECK("extract_cubes kernel");
   }
+  return MICA_OK;
+}
+
+extern "C" int mica_cube_window_max(const float* vol, int nz, int ny, int nx, int z0, int nz_local,
+                                    const int perm[3], int grid_size, int padding, const int32_t* ijk, int n_cubes,
+                                    float* out, mica_stream_t stream) {
+  MICA_REQUIRE(vol && perm && (out || n_cubes == 0) && (ijk || n_cubes == 0), "null pointer");
+  MICA_REQUIRE(nz > 0 && ny > 0 && nx > 0, "empty volume");
+  MICA_REQUIRE(z0 >= 0 && nz_local > 0 && z0 + nz_local <= nz, "bad slab");
+  MICA_REQUIRE(grid_size > 0 && padding >= 0, "bad grid_size/padding");
+  MICA_REQUIRE(n_cubes >= 0, "bad cube count %d", n_cubes);
+  WindowMaxParams P;
+  int seen = 0;
+  for (int m = 0; m < 3; ++m) {
+    MICA_REQUIRE(perm[m] >= 0 && perm[m] < 3, "perm must be a permutation of 0,1,2");
+    seen |= 1 << perm[m];
+    P.inv[perm[m]] = m;
+  }
+  MICA_REQUIRE(seen == 7, "perm must be a permutation of 0,1,2");
+  const int64_t W = (int64_t)grid_size + 2 * (int64_t)padding;
+  MICA_REQUIRE(W <= 65535, "window too large");
+  if (n_cubes == 0) return MICA_OK;
+  P.vol = vol;
+  P.ny = ny;
+  P.nx = nx;
+  P.lo_z = z0;
+  P.hi_z = z0 + nz_local;
+  P.z0 = z0;
+  P.W = (int)W;
+  P.pad = padding;
+  P.ijk = ijk;
+  P.out = out;
+  cube_window_max_kernel<<<n_cubes, 256, 0, (cudaStream_t)stream>>>(P);
+  MICA_LAUNCH_CHECK("cube_window_max_kernel");
   return MICA_OK;
 }
 

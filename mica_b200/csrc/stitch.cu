@@ -432,6 +432,58 @@ extern "C" int mica_postproc_stitch(const float* bb, const float* ca, const floa
   return MICA_OK;
 }
 
+// the paste of cubes the model did not run on (the keep rule of ops.select_cubes): their cores, clipped to the box,
+// become 0 in all 23 channels -- what the reference's stitcher leaves where a cube has no grid file.
+// grid = (n_cubes, grid_size [core plane a]), block = 256 over the (b, c) plane of the core.
+__global__ void __launch_bounds__(256)
+zero_cores_kernel(StitchParams P) {
+  const int S = P.S, b = blockIdx.x, a = blockIdx.y;
+  const int gx = P.ijk[3 * b + 0] + a, j = P.ijk[3 * b + 1], k = P.ijk[3 * b + 2];
+  if (gx >= P.X || gx < P.org[0] || gx >= P.org[0] + P.ext[0]) return;
+  const int64_t vol_n = (int64_t)P.ext[0] * P.ext[1] * P.ext[2];
+  for (int e = threadIdx.x; e < S * S; e += blockDim.x) {
+    const int gy = j + e / S, gz = k + e % S;
+    if (gy >= P.Y || gz >= P.Z) continue;
+    const int ly = gy - P.org[1], lz = gz - P.org[2];
+    if (ly < 0 || ly >= P.ext[1] || lz < 0 || lz >= P.ext[2]) continue;
+    const int64_t o = ((int64_t)(gx - P.org[0]) * P.ext[1] + ly) * P.ext[2] + lz;
+    P.bb_vol[o] = 0.f;
+    P.ca_vol[o] = 0.f;
+    P.aa_pred_vol[o] = 0.f;
+#pragma unroll 4
+    for (int t = 0; t < 20; ++t) P.aa_prob_vol[t * vol_n + o] = 0.f;
+  }
+}
+
+extern "C" int mica_zero_cores(const int32_t* ijk, int n_cubes, int X, int Y, int Z, const int org[3],
+                               const int ext[3], int grid_size, float* bb_vol, float* ca_vol, float* aa_prob_vol,
+                               float* aa_pred_vol, mica_stream_t stream) {
+  MICA_REQUIRE(bb_vol && ca_vol && aa_prob_vol && aa_pred_vol, "null output volume");
+  MICA_REQUIRE(n_cubes == 0 || ijk, "null input");
+  MICA_REQUIRE(grid_size > 0 && grid_size <= 65535, "bad grid_size");
+  MICA_REQUIRE(n_cubes >= 0, "bad cube count %d", n_cubes);
+  int rc = check_box(X, Y, Z, org, ext);
+  if (rc) return rc;
+  if (n_cubes == 0) return MICA_OK;
+  StitchParams P = {};
+  P.ijk = ijk;
+  P.X = X;
+  P.Y = Y;
+  P.Z = Z;
+  for (int m = 0; m < 3; ++m) {
+    P.org[m] = org[m];
+    P.ext[m] = ext[m];
+  }
+  P.S = grid_size;
+  P.bb_vol = bb_vol;
+  P.ca_vol = ca_vol;
+  P.aa_prob_vol = aa_prob_vol;
+  P.aa_pred_vol = aa_pred_vol;
+  zero_cores_kernel<<<dim3(n_cubes, grid_size), 256, 0, (cudaStream_t)stream>>>(P);
+  MICA_LAUNCH_CHECK("zero_cores_kernel");
+  return MICA_OK;
+}
+
 extern "C" int mica_postproc_stitch_peer(const float* bb, const float* ca, const float* aa, const int32_t* ijk,
                                          int n_cubes, int X, int Y, int Z, int grid_size, int padding,
                                          void* const* owner_base, const int* x_bounds, int world,

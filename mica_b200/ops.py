@@ -589,6 +589,55 @@ def extract_cubes(vol: torch.Tensor, ijk: torch.Tensor, grid_size: int = 48, pad
     return out
 
 
+def check_min_max(min_max):
+    """``min_max`` as a float, or None.  A finite number is the only other thing accepted (refused before any launch)."""
+    if min_max is None:
+        return None
+    if isinstance(min_max, (bool, np.bool_)) or not isinstance(min_max, (int, float, np.integer, np.floating)):
+        raise _lib.MicaError(f'min_max must be a finite number or None, got {min_max!r}')
+    v = float(min_max)
+    if not np.isfinite(v):
+        raise _lib.MicaError(f'min_max must be a finite number or None, got {min_max!r}')
+    return v
+
+
+@device_guard
+def cube_window_max(vol: torch.Tensor, ijk: torch.Tensor, grid_size: int = 48, padding: int = 8,
+                    perm=STANDARD_PERM, *, global_nz=None, z0: int = 0, out: torch.Tensor | None = None):
+    """float32 [B] device tensor: the maximum of every cube's W^3 window (the one ``extract_cubes`` cuts from ``vol``,
+    [nz_local, ny, nx] holding global planes [z0, z0 + nz_local) of ``global_nz``), zeros standing for the parts
+    outside the map, NaN if the window holds a NaN -- ``np.max`` over the reference's ``np.pad``-ed window."""
+    p_vol = _dev(vol, torch.float32, 'vol')
+    if vol.dim() != 3:
+        raise _lib.MicaError(f'vol must be [nz, ny, nx], got shape {tuple(vol.shape)}')
+    nzl, ny, nx = vol.shape
+    nz = nzl if global_nz is None else int(global_nz)
+    p_ijk = _dev(ijk, torch.int32, 'ijk')
+    B = int(ijk.shape[0])
+    if out is None:
+        out = torch.empty(B, dtype=torch.float32, device=vol.device)
+    p_out = _dev(out, torch.float32, 'out')
+    if tuple(out.shape) != (B,):
+        raise _lib.MicaError(f'out must be [{B}], got {tuple(out.shape)}')
+    check(lib.mica_cube_window_max(p_vol, nz, ny, nx, int(z0), nzl, _lib.int3(perm), int(grid_size), int(padding),
+                                   p_ijk, B, p_out, _stream()), 'cube_window_max')
+    return out
+
+
+def select_cubes(maxima: torch.Tensor, min_max) -> np.ndarray:
+    """The cubes the reference's training-grid rule keeps (create_grids_for_normalized_map.py:78, negated):
+    ``not (window.max() < min_max)`` in float32 -- a tie and a NaN window are kept.  Returns the kept indices into
+    ``maxima`` (int64, ascending) after one device-to-host copy of the maxima."""
+    t = check_min_max(min_max)
+    if t is None:
+        raise _lib.MicaError('select_cubes needs a finite min_max')
+    m = maxima.detach().to('cpu').numpy()
+    if m.dtype != np.float32:
+        raise _lib.MicaError(f'maxima must be float32, got {m.dtype}')
+    with np.errstate(over='ignore', invalid='ignore'):      # a threshold beyond float32's range; NaN compares False
+        return np.flatnonzero(~(m < np.float32(t))).astype(np.int64)
+
+
 # ------------------------------------------------------ R7/R8 post-process + stitch
 class StitchedVolumes:
     """The four volumes CryoEMPredictor.run_prediction returns (utils/predict.py:526-531),
@@ -647,6 +696,20 @@ def postproc_stitch(bb: torch.Tensor, ca: torch.Tensor, aa: torch.Tensor, ijk: t
         _dev(vols.carbon_alpha_probability, torch.float32, 'ca_vol'),
         _dev(vols.amino_acid_probability, torch.float32, 'aa_prob_vol'),
         _dev(vols.amino_acid_prediction, torch.float32, 'aa_pred_vol'), _stream()), 'postproc_stitch')
+    return vols
+
+
+@device_guard
+def zero_cores(ijk: torch.Tensor, vols: StitchedVolumes, grid_size: int = 48):
+    """The cores of the cubes ``ijk`` (int32 [B,3]) set to 0 in all four volumes, clipped to their box: the cubes a
+    keep rule skipped (``select_cubes``), in volumes that held an earlier map."""
+    X, Y, Z = vols.shape
+    check(lib.mica_zero_cores(_dev(ijk, torch.int32, 'ijk'), int(ijk.shape[0]), X, Y, Z, _lib.int3(vols.org),
+                              _lib.int3(vols.ext), int(grid_size),
+                              _dev(vols.backbone_probability, torch.float32, 'bb_vol'),
+                              _dev(vols.carbon_alpha_probability, torch.float32, 'ca_vol'),
+                              _dev(vols.amino_acid_probability, torch.float32, 'aa_prob_vol'),
+                              _dev(vols.amino_acid_prediction, torch.float32, 'aa_pred_vol'), _stream()), 'zero_cores')
     return vols
 
 

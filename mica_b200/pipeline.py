@@ -424,7 +424,7 @@ class MapPipeline:
     @_on_device
     def predict_and_stitch(self, model_fn, vols: ops.StitchedVolumes | None = None, on_batch=None, *,
                            model_batch=None, d8='none', order=None, stitch_fn=None, overlap_window=None,
-                           batches=None, tta=None):
+                           batches=None, tta=None, min_max=None):
         """run_inference + reconstruct_volume (utils/predict.py:307-587) without the
         per-cube files.  ``model_fn(exp_map, af_features) -> (bb, ca, aa)`` logits, enqueued
         on the current stream.  With ``prefetch`` the cubes of batch n+1 are cut on a side
@@ -452,10 +452,19 @@ class MapPipeline:
         in the order-free fixed point of ``ops.OverlapStitcher`` -- NOT the reference's arithmetic.  The work list is
         the (super-batch, orientation) pairs, fed through the same two-slot prefetch.  ``on_batch`` is called once,
         with the finished volumes.  A ``stitch_fn`` then takes a sixth argument, the orientation of the logits.
-        ``tta=[0]`` is ``tta=None``."""
+        ``tta=[0]`` is ``tta=None``.
+
+        ``min_max`` (a finite number; None = every cube): the keep rule of the reference's training grids
+        (create_grids_for_normalized_map.py:78) at inference -- only cubes whose window maximum is not below it
+        (``ops.cube_window_max`` / ``ops.select_cubes``: ties and NaN windows are kept) reach the model, in the
+        relative order they have in ``order`` (or the loop order).  A skipped cube's core is 0 in all four volumes
+        (the reference's stitcher where a grid file is absent): caller-given ``vols`` get those cores cleared.  With
+        ``overlap_window`` / ``tta`` a skipped window adds nothing and the normaliser stays the full lattice's.  No
+        cube kept: zero volumes, the model is not called."""
         if self.normalized is None:
             raise MicaError('no normalised map')
         codes = ops.tta_orientations(tta)                                          # refused before any launch
+        min_max = ops.check_min_max(min_max)
         if codes == (0,):
             codes = None
         overlap = None
@@ -466,6 +475,11 @@ class MapPipeline:
                     raise MicaError('overlap_window replaces the stitch: pass stitch_fn or overlap_window, not both')
                 overlap = w1 if stitch_fn is None else None
         self.cube_index()
+        # an ascending order is a subsequence of the loop order: finished layers can still be drained (_SlabDrain)
+        self._custom_order = order is not None and not bool(np.all(np.diff(np.asarray(order, dtype=np.int64)) > 0))
+        skipped = None
+        if min_max is not None:
+            order, skipped = self._keep_rule(min_max, order)
         final_on_batch = None
         if overlap is not None:
             overlap = self._overlap_stitcher(overlap, vols, codes)
@@ -473,8 +487,9 @@ class MapPipeline:
         if overlap is not None or codes is not None:
             final_on_batch, on_batch = on_batch, None
         if vols is None:
-            vols = self._new_volumes()
-        self._custom_order = order is not None
+            vols = self._new_volumes()                    # zero: skipped cores need nothing
+        elif skipped is not None and overlap is None and len(skipped):
+            ops.zero_cores(torch.from_numpy(skipped).to(self.device), vols, self.grid_size)
         if order is not None:
             order = np.asarray(order, dtype=np.int64)
             self._set_cube_origins(self.ijk_host[order], ('ordered', id(order), len(order)))
@@ -486,7 +501,9 @@ class MapPipeline:
             batches = [(int(b0), int(b1)) for b0, b1 in batches]
             if any(not 0 <= b0 < b1 <= n or b1 - b0 > self.batch_cubes for b0, b1 in batches):
                 raise MicaError(f'batches must be non-empty ranges of the {n} cubes, at most {self.batch_cubes} long')
-        if not batches:
+        if not batches:                                   # no cube kept (min_max)
+            if on_batch is not None:
+                on_batch(vols, n)
             return self._predict_done(overlap, final_on_batch, vols, n)
         work = [(b0, b1, 0) for b0, b1 in batches] if codes is None else \
             [(b0, b1, g) for b0, b1 in batches for g in codes]
@@ -556,6 +573,23 @@ class MapPipeline:
             cur = nxt
         self.last_loop_enqueue_ms = (time.perf_counter() - t_enqueue) * 1e3     # host side of the batch loop
         return self._predict_done(overlap, final_on_batch, vols, n)
+
+    def _window_max(self, ijk):
+        """Window maxima of the cubes ``ijk`` (device int32 [B,3]) on this pipeline's normalised map."""
+        return ops.cube_window_max(self.normalized, ijk, self.grid_size, self.padding, self.perm)
+
+    def _keep_rule(self, min_max, order):
+        """(order, skipped) under the keep rule: ``order`` = the kept indices of ``ijk_host`` in ``order``'s relative
+        sequence (ascending = the loop order when ``order`` is None); ``skipped`` = origins (int32 [n,3]) of the cubes
+        whose cores this pipeline's volumes must show as 0."""
+        kept = ops.select_cubes(self._window_max(self.ijk), min_max)
+        mask = np.zeros(len(self.ijk_host), dtype=bool)
+        mask[kept] = True
+        skipped = np.ascontiguousarray(self.ijk_host[~mask])
+        if order is None:
+            return kept, skipped
+        order = np.asarray(order, dtype=np.int64)
+        return order[mask[order]], skipped
 
     def _predict_done(self, overlap, on_batch, vols, n):
         if overlap is not None:

@@ -397,6 +397,29 @@ class CryoEMPredictor:
             pipe.af3, pipe._atoms_binned = None, False      # dataset/dataset.py:218-219: zeros
         return pipe
 
+    def _lattice_subset(self, pipe):
+        """The registered cubes (``GridCreator(min_max=)`` may have kept only some) as indices into the pipeline's
+        loop-order cube list, ascending; None when every cube of the lattice is registered."""
+        ijk = np.asarray(self._source['ijk'], dtype=np.int64).reshape(-1, 3)
+        full = pipe.cube_index()
+        if len(ijk) == len(full) and np.array_equal(ijk, full):
+            return None
+        gs = pipe.grid_size
+        n = np.array([-(-int(v) // gs) for v in pipe.cube_shape], dtype=np.int64)
+        q = ijk // gs
+        if (ijk % gs).any() or (q < 0).any() or (q >= n).any():
+            raise ops._lib.MicaError('the registered cubes are not origins of the map\'s cube lattice')
+        return (q[:, 0] * n[1] + q[:, 1]) * n[2] + q[:, 2]
+
+    def _pipeline_order(self, pipe):
+        """The ``order=`` of the registered cubes on ``pipe`` (reference order with ``reference_batching``), or None
+        for the whole lattice in loop order."""
+        order = self._reference_order() if self.reference_batching else None
+        sub = self._lattice_subset(pipe)
+        if sub is None:
+            return order
+        return sub if order is None else sub[np.asarray(order, dtype=np.int64)]
+
     def _host_buffers(self, vols):
         out = {}
         for k, v in vols.as_dict().items():
@@ -472,7 +495,7 @@ class CryoEMPredictor:
         with torch.no_grad():
             if s['kind'] == 'resident':
                 pipe = self._pipeline(dev)
-                order = self._reference_order() if self.reference_batching else None
+                order = self._pipeline_order(pipe)
                 self._pipe = pipe
                 if w1 is not None or codes is not None:     # nothing is final before the last cube: no drain
                     vols = pipe.predict_and_stitch(model, None, model_batch=self._model_batch(), d8=d8, order=order,
@@ -556,7 +579,7 @@ class CryoEMPredictor:
                 else:
                     pipe.af3, pipe._atoms_binned = af3, False
                 pipes[w] = pipe
-            order = self._reference_order() if self.reference_batching else None
+            order = self._pipeline_order(pipes[0])
             order = np.arange(n, dtype=np.int64) if order is None else np.asarray(order, dtype=np.int64)
             pipes[0].cube_index()
             cube_shape = pipes[0].cube_shape

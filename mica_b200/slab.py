@@ -480,6 +480,11 @@ class SlabPipeline(_SplitMap, MapPipeline):
         ops.extract_cubes(self.af3, ijk, self.grid_size, self.padding, self.perm, out=af,
                           global_nz=self.global_nz, z0=self.z0, nonzero=nonzero, orient=orient)
 
+    def _window_max(self, ijk):
+        # this rank's cubes on its block, halo included: the planes are the whole map's bits, so are the decisions
+        return ops.cube_window_max(self.normalized, ijk, self.grid_size, self.padding, self.perm,
+                                   global_nz=self.global_nz, z0=self.z0)
+
     def _new_volumes(self):
         org, ext = self.box
         return ops.StitchedVolumes(self.cube_shape, self.device, org=org, ext=ext)
@@ -494,7 +499,8 @@ class SlabPipeline(_SplitMap, MapPipeline):
     def predict_and_stitch(self, model_fn, vols=None, on_batch=None, **kw):
         """As ``MapPipeline.predict_and_stitch`` for this rank's cubes.  With ``overlap_window`` (or ``tta``) the
         windows reach ``padding`` planes into the neighbouring slabs: those contributions are added into the
-        neighbours' exported blocks, and the volumes are final after ``finish_map()`` on every rank."""
+        neighbours' exported blocks, and the volumes are final after ``finish_map()`` on every rank.  ``min_max``: each
+        rank measures its own cubes on its normalised block (halo included), so the decisions are the one-GPU map's."""
         if self._weighted(kw):
             return self._predict_overlap(model_fn, vols, on_batch, kw)
         return super().predict_and_stitch(model_fn, vols, on_batch, **kw)
@@ -520,23 +526,41 @@ class BalancedCubePipeline(_SplitMap, MapPipeline):
         self.peer_volumes = _peer_volumes
         self.x_bounds = None
 
-    def cube_index(self):
+    def cube_index(self, subset=None):
+        """Deal ``subset`` (indices into the loop-order cube list; default ``cube_subset``, None = all) over the ranks."""
         perm, offset = self.header.transpose_order()
         self.perm, self.offset = perm, offset
         self.cube_shape = ops.cube_space_shape(self.normalized.shape, perm)
         ijk = ops.cube_origins(self.cube_shape, self.grid_size)
-        if self.cube_subset is not None:
-            ijk = ijk[np.asarray(self.cube_subset, dtype=np.int64)]
+        if subset is None:
+            subset = self.cube_subset
+        if subset is not None:
+            subset = np.asarray(subset, dtype=np.int64)
+            ijk = ijk[subset]
         b = _split_even(len(ijk), self.world)
         self.cube_range = (b[self.rank], b[self.rank + 1])
         self.cubes_per_rank = [b[r + 1] - b[r] for r in range(self.world)]
         self._set_cube_origins(ijk[b[self.rank]:b[self.rank + 1]],
                                (self.cube_shape, self.grid_size, self.rank, self.world, len(ijk),
-                                None if self.cube_subset is None else hash(tuple(self.cube_subset))))
+                                None if subset is None else hash(subset.tobytes())))
         self.x_bounds = _split_even(self.cube_shape[0], self.world)
         self.box = ((self.x_bounds[self.rank], 0, 0),
                     (self.x_bounds[self.rank + 1] - self.x_bounds[self.rank], self.cube_shape[1], self.cube_shape[2]))
         return self.ijk_host
+
+    def _keep_rule(self, min_max, order):
+        """Every rank measures the whole map (``cube_subset``, if set, in its order) and deals the kept cubes -- the
+        same list on every rank; every owner clears the skipped cores in its own box (nobody stores there)."""
+        if order is not None:
+            raise MicaError('BalancedCubePipeline deals the cubes itself: pass cube_subset, not order, with min_max')
+        idx = np.arange(len(ops.cube_origins(self.cube_shape, self.grid_size)), dtype=np.int64) \
+            if self.cube_subset is None else np.asarray(self.cube_subset, dtype=np.int64)
+        cand = ops.cube_origins(self.cube_shape, self.grid_size)[idx]
+        kept = ops.select_cubes(self._window_max(torch.from_numpy(cand).to(self.device)), min_max)
+        mask = np.zeros(len(idx), dtype=bool)
+        mask[kept] = True
+        self.cube_index(idx[kept])
+        return None, np.ascontiguousarray(cand[~mask])
 
     def _n_max(self):
         _, Y, Z = self.cube_shape
@@ -554,7 +578,8 @@ class BalancedCubePipeline(_SplitMap, MapPipeline):
 
     def predict_and_stitch(self, model_fn, vols=None, on_batch=None, **kw):
         """With ``overlap_window`` (or ``tta``) every window contribution is added into the block of the rank that
-        owns its x plane; the normaliser comes from the full cube lattice, also under ``cube_subset``."""
+        owns its x plane; the normaliser comes from the full cube lattice, also under ``cube_subset``.  ``min_max``: every
+        rank measures the whole map and deals the kept cubes as ``cube_subset`` (``cubes_per_rank``)."""
         if self._weighted(kw):
             return self._predict_overlap(model_fn, vols, on_batch, kw)
         if vols is None:
