@@ -101,6 +101,9 @@ int mica_bspline_resample_f32(const float* src, int sz, int sy, int sx, int src_
 #define MICA_DTYPE_I16 1 /* int16, MRC mode 1 */
 #define MICA_DTYPE_F32 2 /* float32, MRC mode 2 */
 #define MICA_DTYPE_U16 6 /* uint16, MRC mode 6 */
+/* bfloat16: no MRC mode carries it, and no map is read in it.  Only the model-facing buffers take it (the cube
+ * batches of the *_as extract / AF3 fill, the logits of the *_as stitches); mica_resample refuses it. */
+#define MICA_DTYPE_BF16 16
 
 /* mica_bspline_resample_f32 for any of these types: src and dst hold samples of src_dtype / dst_dtype.  The pairs
  * accepted are float32 -> float32 (the same call as mica_bspline_resample_f32) and an integer type -> the same
@@ -342,6 +345,13 @@ int mica_af3_fill_cubes_oriented(const void* workspace, int64_t n_atoms, int nz,
                                  int grid_size, int padding, const int32_t* ijk_prev, int n_prev,
                                  const int32_t* ijk_next, int n_next, float* out, int64_t out_cube_stride,
                                  int32_t* nonzero, int orientation_prev, int orientation_next, mica_stream_t stream);
+/* The same into an `out` of out_dtype elements (MICA_DTYPE_F32 or MICA_DTYPE_BF16; out_cube_stride in elements):
+ * bf16 1.0 / 0.0 are exact, so a bf16 buffer holds the float32 one's values.  mica_af3_fill_cubes_oriented =
+ * out_dtype MICA_DTYPE_F32.  Any other dtype is MICA_ERR_INVALID before any launch. */
+int mica_af3_fill_cubes_as(const void* workspace, int64_t n_atoms, int nz, int ny, int nx, const int perm[3],
+                           int grid_size, int padding, const int32_t* ijk_prev, int n_prev, const int32_t* ijk_next,
+                           int n_next, void* out, int out_dtype, int64_t out_cube_stride, int32_t* nonzero,
+                           int orientation_prev, int orientation_next, mica_stream_t stream);
 
 /* --------------------------------------------------------- R5/R6 cube extract
  * Replaces GridCreator.transpose + create_grids_from_mrc (utils/create_grids.py:67-176),
@@ -372,6 +382,15 @@ int mica_extract_cubes_oriented(const float* vol, int64_t chan_stride, int n_cha
                                 int grid_size, int padding, const int32_t* ijk, int n_cubes,
                                 float* out, int64_t out_cube_stride, int32_t* nonzero, float* cube_max,
                                 int orientation, mica_stream_t stream);
+/* The same into an `out` of out_dtype elements (MICA_DTYPE_F32 or MICA_DTYPE_BF16; out_cube_stride in elements), the
+ * map itself float32.  bf16: every voxel is rounded once to nearest even; nonzero and cube_max come from the float32
+ * values before rounding, so they are those of the float32 call.  The same kernel routes as the float32 call
+ * (mica_last_extract_path).  mica_extract_cubes_oriented = out_dtype MICA_DTYPE_F32.  Any other dtype is
+ * MICA_ERR_INVALID before any launch. */
+int mica_extract_cubes_as(const float* vol, int64_t chan_stride, int n_channels, int nz, int ny, int nx, int z0,
+                          int nz_local, const int perm[3], int grid_size, int padding, const int32_t* ijk, int n_cubes,
+                          void* out, int out_dtype, int64_t out_cube_stride, int32_t* nonzero, float* cube_max,
+                          int orientation, mica_stream_t stream);
 
 /* Window maximum of every cube, for the inference keep rule of the reference's training grids
  * (create_grids_for_normalized_map.py:78: a window whose max is below min_max is not written).
@@ -427,6 +446,17 @@ int mica_stitch_cubes(const float* cubes, int n_ch, const int32_t* ijk, int n_cu
 int mica_postproc_stitch_peer(const float* bb, const float* ca, const float* aa, const int32_t* ijk, int n_cubes,
                               int X, int Y, int Z, int grid_size, int padding, void* const* owner_base,
                               const int* x_bounds, int world, mica_stream_t stream);
+/* mica_postproc_stitch / mica_postproc_stitch_peer with logits of logit_dtype (MICA_DTYPE_F32 or MICA_DTYPE_BF16,
+ * all three the same).  bf16 logits are widened exactly to float32 on load; everything after is the float32
+ * arithmetic, so the volumes equal the float32 call on the widened logits bit for bit.  The volumes stay float32.
+ * Any other dtype is MICA_ERR_INVALID before any launch. */
+int mica_postproc_stitch_as(const void* bb, const void* ca, const void* aa, int logit_dtype, const int32_t* ijk,
+                            int n_cubes, int X, int Y, int Z, const int org[3], const int ext[3], int grid_size,
+                            int padding, float* bb_vol, float* ca_vol, float* aa_prob_vol, float* aa_pred_vol,
+                            mica_stream_t stream);
+int mica_postproc_stitch_peer_as(const void* bb, const void* ca, const void* aa, int logit_dtype, const int32_t* ijk,
+                                 int n_cubes, int X, int Y, int Z, int grid_size, int padding, void* const* owner_base,
+                                 const int* x_bounds, int world, mica_stream_t stream);
 
 /* ===================================================================================
  * SURVEY.md section 8(f) "next" rows, built to the same bar as R1-R8.
@@ -555,6 +585,18 @@ int mica_overlap_accumulate_fixed_peer_oriented(const float* bb, const float* ca
                                                 const float* window_w1, const double* norm, int orientation,
                                                 void* const* owner_base, int axis, const int* bounds, int world,
                                                 mica_stream_t stream);
+/* The _oriented calls with logits of logit_dtype (MICA_DTYPE_F32 or MICA_DTYPE_BF16, all three the same): bf16 logits
+ * are widened exactly on load, then the same fixed-point recipe, so the sums equal the float32 call on the widened
+ * logits bit for bit, on every partition.  Any other dtype is MICA_ERR_INVALID before any launch. */
+int mica_overlap_accumulate_fixed_as(const void* bb, const void* ca, const void* aa, int logit_dtype,
+                                     const int32_t* ijk, int n_cubes, int X, int Y, int Z, int grid_size, int padding,
+                                     const float* window_w1, const double* norm, int orientation, void* block,
+                                     mica_stream_t stream);
+int mica_overlap_accumulate_fixed_peer_as(const void* bb, const void* ca, const void* aa, int logit_dtype,
+                                          const int32_t* ijk, int n_cubes, int X, int Y, int Z, int grid_size,
+                                          int padding, const float* window_w1, const double* norm, int orientation,
+                                          void* const* owner_base, int axis, const int* bounds, int world,
+                                          mica_stream_t stream);
 int mica_overlap_finalize_fixed(void* block, int64_t n_voxels, mica_stream_t stream);
 /* 1 when `device` can add into the memory of `peer_device` with native atomics over the peer path
  * (cudaDevP2PAttrNativeAtomicSupported; 1 for device == peer_device), 0 when not, negative MICA_ERR_* on error. */

@@ -15,6 +15,7 @@ MICA_OK = 0
 ERR_NAMES = {-1: 'MICA_ERR_INVALID', -2: 'MICA_ERR_CUDA', -3: 'MICA_ERR_WORKSPACE', -4: 'MICA_ERR_NO_DEVICE'}
 NORM_OK, NORM_NO_POSITIVE, NORM_ZERO_PCTL, NORM_PENDING, NORM_PEER_TIMEOUT = 0, 1, 2, 3, 4
 DTYPE_I8, DTYPE_I16, DTYPE_F32, DTYPE_U16 = 0, 1, 2, 6      # MICA_DTYPE_*: the MRC modes of these sample types
+DTYPE_BF16 = 16                                             # MICA_DTYPE_BF16: model-facing buffers only, no MRC mode
 INT_STATS_RESULT_BYTES = 32
 SELECT_HIST_WORDS = 4096
 SELECT_PASSES = 7
@@ -97,10 +98,14 @@ SIGNATURES = {
     'mica_af3_fill_cubes': (_i, [_p, _i64, _i, _i, _i, C.POINTER(_i), _i, _i, _p, _i, _p, _i, _p, _i64, _p, _p]),
     'mica_af3_fill_cubes_oriented': (_i, [_p, _i64, _i, _i, _i, C.POINTER(_i), _i, _i, _p, _i, _p, _i, _p, _i64, _p,
                                           _i, _i, _p]),
+    'mica_af3_fill_cubes_as': (_i, [_p, _i64, _i, _i, _i, C.POINTER(_i), _i, _i, _p, _i, _p, _i, _p, _i, _i64, _p,
+                                    _i, _i, _p]),
     'mica_extract_cubes': (_i, [_p, _i64, _i, _i, _i, _i, _i, _i, C.POINTER(_i), _i, _i, _p, _i, _p, _i64,
                                 _p, _p, _p]),
     'mica_extract_cubes_oriented': (_i, [_p, _i64, _i, _i, _i, _i, _i, _i, C.POINTER(_i), _i, _i, _p, _i, _p, _i64,
                                          _p, _p, _i, _p]),
+    'mica_extract_cubes_as': (_i, [_p, _i64, _i, _i, _i, _i, _i, _i, C.POINTER(_i), _i, _i, _p, _i, _p, _i, _i64,
+                                   _p, _p, _i, _p]),
     'mica_last_extract_path': (_i, []),
     'mica_cube_window_max': (_i, [_p, _i, _i, _i, _i, _i, C.POINTER(_i), _i, _i, _p, _i, _p, _p]),
     'mica_postproc_stitch': (_i, [_p, _p, _p, _p, _i, _i, _i, _i, C.POINTER(_i), C.POINTER(_i), _i, _i,
@@ -108,6 +113,9 @@ SIGNATURES = {
     'mica_zero_cores': (_i, [_p, _i, _i, _i, _i, C.POINTER(_i), C.POINTER(_i), _i, _p, _p, _p, _p, _p]),
     'mica_stitch_cubes': (_i, [_p, _i, _p, _i, _i, _i, _i, C.POINTER(_i), C.POINTER(_i), _i, _i, _p, _p]),
     'mica_postproc_stitch_peer': (_i, [_p, _p, _p, _p, _i, _i, _i, _i, _i, _i, _p, C.POINTER(_i), _i, _p]),
+    'mica_postproc_stitch_as': (_i, [_p, _p, _p, _i, _p, _i, _i, _i, _i, C.POINTER(_i), C.POINTER(_i), _i, _i,
+                                     _p, _p, _p, _p, _p]),
+    'mica_postproc_stitch_peer_as': (_i, [_p, _p, _p, _i, _p, _i, _i, _i, _i, _i, _i, _p, C.POINTER(_i), _i, _p]),
     'mica_overlap_accumulate_fixed': (_i, [_p, _p, _p, _p, _i, _i, _i, _i, _i, _i, C.POINTER(_f), _p, _p, _p]),
     'mica_overlap_accumulate_fixed_peer': (_i, [_p, _p, _p, _p, _i, _i, _i, _i, _i, _i, C.POINTER(_f), _p, _p, _i,
                                                 C.POINTER(_i), _i, _p]),
@@ -115,6 +123,10 @@ SIGNATURES = {
                                                     _p, _p]),
     'mica_overlap_accumulate_fixed_peer_oriented': (_i, [_p, _p, _p, _p, _i, _i, _i, _i, _i, _i, C.POINTER(_f), _p,
                                                          _i, _p, _i, C.POINTER(_i), _i, _p]),
+    'mica_overlap_accumulate_fixed_as': (_i, [_p, _p, _p, _i, _p, _i, _i, _i, _i, _i, _i, C.POINTER(_f), _p, _i,
+                                              _p, _p]),
+    'mica_overlap_accumulate_fixed_peer_as': (_i, [_p, _p, _p, _i, _p, _i, _i, _i, _i, _i, _i, C.POINTER(_f), _p,
+                                                   _i, _p, _i, C.POINTER(_i), _i, _p]),
     'mica_overlap_finalize_fixed': (_i, [_p, _i64, _p]),
     'mica_peer_atomics_supported': (_i, [_i, _i]),
     'mica_parse_pdb': (_i64, [C.c_char_p, _i64, _i, _i64, _p, _p, _p, _p, _p, _p, _p]),

@@ -243,10 +243,11 @@ struct FillOrient {
   int base, s[3];
 };
 
-template <bool SET>
+// T: the buffer's element type, float or __nv_bfloat16 (1.0 and 0.0 are exact in both)
+template <bool SET, typename T>
 __global__ void __launch_bounds__(256)
 af3_fill_cubes_kernel(BinWorkspace ws, BinParams P, const int32_t* __restrict__ ijk_prev, int n_prev,
-                      const int32_t* __restrict__ ijk_next, int n_next, float* __restrict__ out,
+                      const int32_t* __restrict__ ijk_next, int n_next, T* __restrict__ out,
                       int64_t out_cube_stride, int32_t* __restrict__ nonzero, FillOrient o, bool same_orientation) {
   const int slot = blockIdx.y;
   const int prev = slot < n_prev ? cube_id_of(P, ijk_prev, slot) : -1;
@@ -255,7 +256,7 @@ af3_fill_cubes_kernel(BinWorkspace ws, BinParams P, const int32_t* __restrict__ 
     nonzero[slot] = (ws.offsets[next + 1] > ws.offsets[next]) ? 1 : 0;
   const int id = SET ? next : prev;
   if (id < 0 || (prev == next && same_orientation)) return;
-  float* cube = out + (int64_t)slot * out_cube_stride;
+  T* cube = out + (int64_t)slot * out_cube_stride;
   const int64_t W3 = (int64_t)P.W * P.W * P.W;
   const float val = SET ? 1.0f : 0.0f;
   const int e0 = ws.offsets[id], e1 = ws.offsets[id + 1];
@@ -267,8 +268,8 @@ af3_fill_cubes_kernel(BinWorkspace ws, BinParams P, const int32_t* __restrict__ 
       const int W = P.W, v0 = (int)off / (W * W), v1 = ((int)off / W) % W, v2 = (int)off % W;
       off = (unsigned)(o.base + v0 * o.s[0] + v1 * o.s[1] + v2 * o.s[2]);
     }
-    if (b) cube[(int64_t)(b - 1) * W3 + off] = val;
-    if (r) cube[(int64_t)(r + 3) * W3 + off] = val;
+    if (b) st_plain_el(cube + (int64_t)(b - 1) * W3 + off, val);
+    if (r) st_plain_el(cube + (int64_t)(r + 3) * W3 + off, val);
   }
 }
 
@@ -368,11 +369,11 @@ static FillOrient fill_orient(int code, int W) {
   return o;
 }
 
-extern "C" int mica_af3_fill_cubes_oriented(const void* workspace, int64_t n_atoms, int nz, int ny, int nx,
-                                            const int perm[3], int grid_size, int padding, const int32_t* ijk_prev,
-                                            int n_prev, const int32_t* ijk_next, int n_next, float* out,
-                                            int64_t out_cube_stride, int32_t* nonzero, int orientation_prev,
-                                            int orientation_next, mica_stream_t stream) {
+template <typename T>
+static int af3_fill_cubes_impl(const void* workspace, int64_t n_atoms, int nz, int ny, int nx, const int perm[3],
+                               int grid_size, int padding, const int32_t* ijk_prev, int n_prev,
+                               const int32_t* ijk_next, int n_next, T* out, int64_t out_cube_stride,
+                               int32_t* nonzero, int orientation_prev, int orientation_next, cudaStream_t stream) {
   MICA_REQUIRE(workspace && out, "null pointer");
   Orientation ori;
   MICA_REQUIRE(orientation_decode(orientation_prev, 1, &ori) && orientation_decode(orientation_next, 1, &ori),
@@ -387,18 +388,44 @@ extern "C" int mica_af3_fill_cubes_oriented(const void* workspace, int64_t n_ato
   const int n_cubes = P.ncube[0] * P.ncube[1] * P.ncube[2];
   BinWorkspace ws = carve(const_cast<void*>(workspace), n_cubes, bin_capacity(n_atoms, grid_size, padding));
   if (n_prev > 0) {
-    af3_fill_cubes_kernel<false><<<dim3(kFillBlocks, n_prev), 256, 0, (cudaStream_t)stream>>>(
+    af3_fill_cubes_kernel<false, T><<<dim3(kFillBlocks, n_prev), 256, 0, stream>>>(
         ws, P, ijk_prev, n_prev, ijk_next, n_next, out, out_cube_stride, nonzero, fill_orient(orientation_prev, P.W),
         orientation_prev == orientation_next);
     MICA_LAUNCH_CHECK("af3_fill_cubes_kernel<clear>");
   }
   if (n_next > 0) {
-    af3_fill_cubes_kernel<true><<<dim3(kFillBlocks, n_next), 256, 0, (cudaStream_t)stream>>>(
+    af3_fill_cubes_kernel<true, T><<<dim3(kFillBlocks, n_next), 256, 0, stream>>>(
         ws, P, ijk_prev, n_prev, ijk_next, n_next, out, out_cube_stride, nonzero, fill_orient(orientation_next, P.W),
         orientation_prev == orientation_next);
     MICA_LAUNCH_CHECK("af3_fill_cubes_kernel<set>");
   }
   return MICA_OK;
+}
+
+extern "C" int mica_af3_fill_cubes_as(const void* workspace, int64_t n_atoms, int nz, int ny, int nx,
+                                      const int perm[3], int grid_size, int padding, const int32_t* ijk_prev,
+                                      int n_prev, const int32_t* ijk_next, int n_next, void* out, int out_dtype,
+                                      int64_t out_cube_stride, int32_t* nonzero, int orientation_prev,
+                                      int orientation_next, mica_stream_t stream) {
+  MICA_REQUIRE(model_dtype_bytes(out_dtype), "AF3 cube dtype %d: must be MICA_DTYPE_F32 or MICA_DTYPE_BF16",
+               out_dtype);
+  if (out_dtype == MICA_DTYPE_BF16)
+    return af3_fill_cubes_impl(workspace, n_atoms, nz, ny, nx, perm, grid_size, padding, ijk_prev, n_prev, ijk_next,
+                               n_next, static_cast<__nv_bfloat16*>(out), out_cube_stride, nonzero, orientation_prev,
+                               orientation_next, (cudaStream_t)stream);
+  return af3_fill_cubes_impl(workspace, n_atoms, nz, ny, nx, perm, grid_size, padding, ijk_prev, n_prev, ijk_next,
+                             n_next, static_cast<float*>(out), out_cube_stride, nonzero, orientation_prev,
+                             orientation_next, (cudaStream_t)stream);
+}
+
+extern "C" int mica_af3_fill_cubes_oriented(const void* workspace, int64_t n_atoms, int nz, int ny, int nx,
+                                            const int perm[3], int grid_size, int padding, const int32_t* ijk_prev,
+                                            int n_prev, const int32_t* ijk_next, int n_next, float* out,
+                                            int64_t out_cube_stride, int32_t* nonzero, int orientation_prev,
+                                            int orientation_next, mica_stream_t stream) {
+  return mica_af3_fill_cubes_as(workspace, n_atoms, nz, ny, nx, perm, grid_size, padding, ijk_prev, n_prev, ijk_next,
+                                n_next, out, MICA_DTYPE_F32, out_cube_stride, nonzero, orientation_prev,
+                                orientation_next, stream);
 }
 
 extern "C" int mica_af3_fill_cubes(const void* workspace, int64_t n_atoms, int nz, int ny, int nx, const int perm[3],

@@ -1,6 +1,7 @@
 // Shared helpers for the mica_b200 kernels (sm_100a only).
 #pragma once
 #include <cuda.h>
+#include <cuda_bf16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdio.h>
@@ -80,6 +81,35 @@ __device__ __forceinline__ void st_stream(float* p, float v) {
 __device__ __forceinline__ void st_stream4(float4* p, float4 v) {
   asm volatile("st.global.cs.v4.f32 [%0], {%1,%2,%3,%4};" ::"l"(p), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w)
                : "memory");
+}
+
+// Model-facing buffers (cube batches, logits) are float32 or bfloat16 (MICA_DTYPE_F32 / MICA_DTYPE_BF16); source
+// maps and output volumes are always float32.  A bf16 store rounds the float32 value once, to nearest even; a bf16
+// load widens exactly (the 16 bits become the high half of the float32).
+__device__ __forceinline__ void st_stream_el(float* p, float v) { st_stream(p, v); }
+__device__ __forceinline__ void st_stream_el(__nv_bfloat16* p, float v) {
+  const unsigned short h = __bfloat16_as_ushort(__float2bfloat16_rn(v));
+  asm volatile("st.global.cs.b16 [%0], %1;" ::"l"(p), "h"(h) : "memory");
+}
+__device__ __forceinline__ void st_plain_el(float* p, float v) { *p = v; }
+__device__ __forceinline__ void st_plain_el(__nv_bfloat16* p, float v) { *p = __float2bfloat16_rn(v); }
+__device__ __forceinline__ float bf16_bits_to_float(unsigned short h) { return __uint_as_float((unsigned)h << 16); }
+__device__ __forceinline__ float ld_stream_el(const float* p) { return ld_stream(p); }
+__device__ __forceinline__ float ld_stream_el(const __nv_bfloat16* p) {
+  unsigned short h;
+  asm volatile("ld.global.nc.L1::no_allocate.b16 %0, [%1];" : "=h"(h) : "l"(p));
+  return bf16_bits_to_float(h);
+}
+// ld_stream_half_line for bf16 logits: at stride 32 a bf16 core row is the 64 bytes [32, 96) of a 128-byte line,
+// which straddles both 64-byte halves, so the float32 helper's .L2::64B cap does not apply.  No L2 prefetch-size
+// qualifier: on B200 none / 64B / 128B / 256B read these cores within 0.4 % of each other, none marginally fastest
+// (tools/micro/bf16_core_read.cu, profiles/bf16_core_read_microbench.txt).
+__device__ __forceinline__ float ld_stream_core_el(const float* p) { return ld_stream_half_line(p); }
+__device__ __forceinline__ float ld_stream_core_el(const __nv_bfloat16* p) { return ld_stream_el(p); }
+
+// host side: the element size of a model-facing dtype code, 0 if the code is not one of them
+static inline int model_dtype_bytes(int dtype) {
+  return dtype == MICA_DTYPE_F32 ? 4 : (dtype == MICA_DTYPE_BF16 ? 2 : 0);
 }
 
 // Test-time-augmentation orientation of a W^3 window (code 0..47, ops.orientation): code = 8 p + f, p the index

@@ -30,7 +30,7 @@ struct ExtractParams {
   int z0, nzl;         // slab: memory planes [z0, z0 + nzl)
   int W, pad;
   const int32_t* ijk;
-  float* out;
+  void* out;               // float or __nv_bfloat16 (the kernels' T), out_cube_stride in elements
   int64_t out_cube_stride;
   int32_t* nonzero;
   float* cube_max;
@@ -60,13 +60,16 @@ __device__ __forceinline__ bool in_map(const ExtractParams& P, int p0, int p1, i
 
 // ---- cube's fastest axis (2) is the memory-contiguous one: row copy.
 // grid = (W [u0], B, C), block = (32, 8)
+// T (here and in the other extract kernels): the element type of the output, float or __nv_bfloat16; the flags are
+// taken on the float32 values before st_stream_el rounds them
+template <typename T>
 __global__ void __launch_bounds__(256)
 extract_rows_kernel(ExtractParams P) {
   const int u0 = blockIdx.x, c = blockIdx.z, b = blockIdx.y;
   const int W = P.W;
   const int i0 = P.ijk[3 * b + 0] - P.pad, j0 = P.ijk[3 * b + 1] - P.pad, k0 = P.ijk[3 * b + 2] - P.pad;
   const float* src = P.vol + (int64_t)c * P.chan_stride;
-  float* dst = P.out + (int64_t)b * P.out_cube_stride + (int64_t)c * W * W * W + (int64_t)u0 * W * W;
+  T* dst = static_cast<T*>(P.out) + (int64_t)b * P.out_cube_stride + (int64_t)c * W * W * W + (int64_t)u0 * W * W;
   const int p0 = i0 + u0;
   const int zsub[3] = {P.slab_axis == 0 ? P.z0 : 0, P.slab_axis == 1 ? P.z0 : 0, P.slab_axis == 2 ? P.z0 : 0};
   bool any_nz = false;
@@ -83,7 +86,7 @@ extract_rows_kernel(ExtractParams P) {
       }
       any_nz |= (v != 0.f);
       vmax = fmaxf(vmax, v);
-      st_stream(dst + (int64_t)u1 * W + u2, v);
+      st_stream_el(dst + (int64_t)u1 * W + u2, v);
     }
   }
   block_flags(P, b, any_nz, vmax);
@@ -91,7 +94,7 @@ extract_rows_kernel(ExtractParams P) {
 
 // ---- cube axis MC (0 or 1) is memory-contiguous: tiled transpose MC <-> 2.
 // grid = (W [u_o, the other slow axis], B, C), block = (32, 8)
-template <int MC>
+template <int MC, typename T>
 __global__ void __launch_bounds__(256)
 extract_transpose_kernel(ExtractParams P) {
   __shared__ float tile[32][33];
@@ -100,7 +103,7 @@ extract_transpose_kernel(ExtractParams P) {
   const int W = P.W;
   int org[3] = {P.ijk[3 * b + 0] - P.pad, P.ijk[3 * b + 1] - P.pad, P.ijk[3 * b + 2] - P.pad};
   const float* src = P.vol + (int64_t)c * P.chan_stride;
-  float* dst = P.out + (int64_t)b * P.out_cube_stride + (int64_t)c * W * W * W;
+  T* dst = static_cast<T*>(P.out) + (int64_t)b * P.out_cube_stride + (int64_t)c * W * W * W;
   const int64_t out_mc = (MC == 0) ? (int64_t)W * W : W;   // output stride of cube axis MC
   const int64_t out_oa = (MC == 0) ? W : (int64_t)W * W;   // output stride of the other slow axis
   const int po = org[OA] + uo;
@@ -133,7 +136,7 @@ extract_transpose_kernel(ExtractParams P) {
 #pragma unroll
       for (int r = 0; r < 4; ++r) {
         const int uc = tc + ty + 8 * r, u2 = t2 + tx;
-        if (uc < W && u2 < W) st_stream(dst + uc * out_mc + uo * out_oa + u2, tile[tx][ty + 8 * r]);
+        if (uc < W && u2 < W) st_stream_el(dst + uc * out_mc + uo * out_oa + u2, tile[tx][ty + 8 * r]);
       }
       __syncthreads();
     }
@@ -163,7 +166,7 @@ __device__ __forceinline__ float load_oriented(const ExtractParams& P, const flo
 }
 
 // grid = (W [output axis 0 for MC == 2, else the slow output axis that is not MC], B, C), block = (32, 8)
-template <int MC>
+template <int MC, typename T>
 __global__ void __launch_bounds__(256)
 extract_oriented_kernel(ExtractParams P, OrientAxes A) {
   __shared__ float tile[32][33];
@@ -173,7 +176,7 @@ extract_oriented_kernel(ExtractParams P, OrientAxes A) {
 #pragma unroll
   for (int a = 0; a < 3; ++a) org[a] = P.ijk[3 * b + A.cax[a]] - P.pad + (A.dir[a] < 0 ? W - 1 : 0);
   const float* src = P.vol + (int64_t)c * P.chan_stride;
-  float* dst = P.out + (int64_t)b * P.out_cube_stride + (int64_t)c * W * W * W;
+  T* dst = static_cast<T*>(P.out) + (int64_t)b * P.out_cube_stride + (int64_t)c * W * W * W;
   const int tx = threadIdx.x, ty = threadIdx.y;
   bool any_nz = false;
   float vmax = -CUDART_INF_F;
@@ -185,7 +188,7 @@ extract_oriented_kernel(ExtractParams P, OrientAxes A) {
         const float v = load_oriented(P, src, p0, p1, org[2] + A.dir[2] * u2);
         any_nz |= (v != 0.f);
         vmax = fmaxf(vmax, v);
-        st_stream(dst + ((int64_t)uo * W + u1) * W + u2, v);
+        st_stream_el(dst + ((int64_t)uo * W + u1) * W + u2, v);
       }
     }
   } else {
@@ -211,7 +214,7 @@ extract_oriented_kernel(ExtractParams P, OrientAxes A) {
 #pragma unroll
         for (int r = 0; r < 4; ++r) {
           const int uc = tc + ty + 8 * r, u2 = t2 + tx;
-          if (uc < W && u2 < W) st_stream(dst + uc * out_mc + uo * out_oa + u2, tile[tx][ty + 8 * r]);
+          if (uc < W && u2 < W) st_stream_el(dst + uc * out_mc + uo * out_oa + u2, tile[tx][ty + 8 * r]);
         }
         __syncthreads();
       }
@@ -234,7 +237,7 @@ __device__ __forceinline__ uint32_t smem_u32(const void* p) {
 
 struct TmaExtractParams {
   const int32_t* ijk;
-  float* out;
+  void* out;
   int64_t out_cube_stride;
   int32_t* nonzero;
   float* cube_max;
@@ -242,7 +245,7 @@ struct TmaExtractParams {
   int off_c, off_b;  // slab offsets subtracted from the tensor-map coordinates of dims 1 and 2
 };
 
-template <int BT>
+template <int BT, typename T>
 __global__ void __launch_bounds__(256)
 extract_tma_kernel(const __grid_constant__ CUtensorMap tmap, TmaExtractParams P) {
   extern __shared__ uint8_t smem_raw[];
@@ -280,7 +283,8 @@ extract_tma_kernel(const __grid_constant__ CUtensorMap tmap, TmaExtractParams P)
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int c_groups = W >> 5;
   const int64_t W2 = (int64_t)W * W;
-  float* dst = P.out + (int64_t)cube * P.out_cube_stride + (int64_t)ch * W2 * W + (int64_t)a0 * W2 + (int64_t)b0 * W;
+  T* dst = static_cast<T*>(P.out) + (int64_t)cube * P.out_cube_stride + (int64_t)ch * W2 * W + (int64_t)a0 * W2 +
+           (int64_t)b0 * W;
   bool any_nz = false;
   float vmax = -CUDART_INF_F;
   const int items = BT * c_groups * 8;
@@ -290,11 +294,11 @@ extract_tma_kernel(const __grid_constant__ CUtensorMap tmap, TmaExtractParams P)
     const int z = (cg << 5) + lane;
     const int R = y * W + z;
     const float4 v = *reinterpret_cast<const float4*>(tile + (size_t)R * 128 + (((j ^ (R & 7))) << 4));
-    float* o = dst + (int64_t)(4 * j) * W2 + (int64_t)y * W + z;
-    st_stream(o, v.x);
-    st_stream(o + W2, v.y);
-    st_stream(o + 2 * W2, v.z);
-    st_stream(o + 3 * W2, v.w);
+    T* o = dst + (int64_t)(4 * j) * W2 + (int64_t)y * W + z;
+    st_stream_el(o, v.x);
+    st_stream_el(o + W2, v.y);
+    st_stream_el(o + 2 * W2, v.z);
+    st_stream_el(o + 3 * W2, v.w);
     any_nz |= (v.x != 0.f) | (v.y != 0.f) | (v.z != 0.f) | (v.w != 0.f);
     vmax = fmaxf(fmaxf(vmax, fmaxf(v.x, v.y)), fmaxf(v.z, v.w));
   }
@@ -385,12 +389,11 @@ using namespace mica;
 static thread_local int g_last_extract_path = -1;
 extern "C" int mica_last_extract_path(void) { return g_last_extract_path; }
 
-extern "C" int mica_extract_cubes_oriented(const float* vol, int64_t chan_stride, int n_channels,
-                                           int nz, int ny, int nx, int z0, int nz_local, const int perm[3],
-                                           int grid_size, int padding, const int32_t* ijk, int n_cubes,
-                                           float* out, int64_t out_cube_stride, int32_t* nonzero, float* cube_max,
-                                           int orientation, mica_stream_t stream) {
-  cudaStream_t st = (cudaStream_t)stream;
+template <typename T>
+static int extract_cubes_impl(const float* vol, int64_t chan_stride, int n_channels, int nz, int ny, int nx, int z0,
+                              int nz_local, const int perm[3], int grid_size, int padding, const int32_t* ijk,
+                              int n_cubes, T* out, int64_t out_cube_stride, int32_t* nonzero, float* cube_max,
+                              int orientation, cudaStream_t st) {
   Orientation ori;
   MICA_REQUIRE(orientation_decode(orientation, 1, &ori), "orientation %d is not in 0..47", orientation);
   MICA_REQUIRE(vol && perm && out && (ijk || n_cubes == 0), "null pointer");
@@ -453,11 +456,11 @@ extern "C" int mica_extract_cubes_oriented(const float* vol, int64_t chan_stride
       }
       dim3 grid(W, nb, n_channels), block(32, 8);
       if (mc == 2)
-        extract_oriented_kernel<2><<<grid, block, 0, st>>>(Q, A);
+        extract_oriented_kernel<2, T><<<grid, block, 0, st>>>(Q, A);
       else if (mc == 0)
-        extract_oriented_kernel<0><<<grid, block, 0, st>>>(Q, A);
+        extract_oriented_kernel<0, T><<<grid, block, 0, st>>>(Q, A);
       else
-        extract_oriented_kernel<1><<<grid, block, 0, st>>>(Q, A);
+        extract_oriented_kernel<1, T><<<grid, block, 0, st>>>(Q, A);
       g_last_extract_path = 3;
       MICA_LAUNCH_CHECK("extract_oriented_kernel");
     }
@@ -486,7 +489,7 @@ extern "C" int mica_extract_cubes_oriented(const float* vol, int64_t chan_stride
                        CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
       if (r == CUDA_SUCCESS) {
         use_tma = true;
-        MICA_CUDA(cudaFuncSetAttribute(extract_tma_kernel<kTmaBT>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+        MICA_CUDA(cudaFuncSetAttribute(extract_tma_kernel<kTmaBT, T>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                        (int)tma_smem));
       }
     }
@@ -504,28 +507,53 @@ extern "C" int mica_extract_cubes_oriented(const float* vol, int64_t chan_stride
     }
     dim3 grid(W, nb, n_channels), block(32, 8);
     if (use_tma) {
-      TmaExtractParams T;
-      T.ijk = P.ijk;
-      T.out = P.out;
-      T.out_cube_stride = out_cube_stride;
-      T.nonzero = P.nonzero;
-      T.cube_max = P.cube_max;
-      T.W = W;
-      T.pad = padding;
-      T.off_c = perm[2] == 0 ? z0 : 0;
-      T.off_b = perm[1] == 0 ? z0 : 0;
+      TmaExtractParams TP;
+      TP.ijk = P.ijk;
+      TP.out = P.out;
+      TP.out_cube_stride = out_cube_stride;
+      TP.nonzero = P.nonzero;
+      TP.cube_max = P.cube_max;
+      TP.W = W;
+      TP.pad = padding;
+      TP.off_c = perm[2] == 0 ? z0 : 0;
+      TP.off_b = perm[1] == 0 ? z0 : 0;
       dim3 tgrid((W / 32) * (W / kTmaBT), nb, n_channels);
-      extract_tma_kernel<kTmaBT><<<tgrid, 256, tma_smem, st>>>(tmap, T);
+      extract_tma_kernel<kTmaBT, T><<<tgrid, 256, tma_smem, st>>>(tmap, TP);
     } else if (contiguous_axis == 2)
-      extract_rows_kernel<<<grid, block, 0, st>>>(P);
+      extract_rows_kernel<T><<<grid, block, 0, st>>>(P);
     else if (contiguous_axis == 0)
-      extract_transpose_kernel<0><<<grid, block, 0, st>>>(P);
+      extract_transpose_kernel<0, T><<<grid, block, 0, st>>>(P);
     else
-      extract_transpose_kernel<1><<<grid, block, 0, st>>>(P);
+      extract_transpose_kernel<1, T><<<grid, block, 0, st>>>(P);
     g_last_extract_path = use_tma ? 2 : (contiguous_axis == 2 ? 0 : 1);
     MICA_LAUNCH_CHECK("extract_cubes kernel");
   }
   return MICA_OK;
+}
+
+extern "C" int mica_extract_cubes_as(const float* vol, int64_t chan_stride, int n_channels, int nz, int ny, int nx,
+                                     int z0, int nz_local, const int perm[3], int grid_size, int padding,
+                                     const int32_t* ijk, int n_cubes, void* out, int out_dtype,
+                                     int64_t out_cube_stride, int32_t* nonzero, float* cube_max, int orientation,
+                                     mica_stream_t stream) {
+  MICA_REQUIRE(model_dtype_bytes(out_dtype), "cube output dtype %d: must be MICA_DTYPE_F32 or MICA_DTYPE_BF16",
+               out_dtype);
+  if (out_dtype == MICA_DTYPE_BF16)
+    return extract_cubes_impl(vol, chan_stride, n_channels, nz, ny, nx, z0, nz_local, perm, grid_size, padding, ijk,
+                              n_cubes, static_cast<__nv_bfloat16*>(out), out_cube_stride, nonzero, cube_max,
+                              orientation, (cudaStream_t)stream);
+  return extract_cubes_impl(vol, chan_stride, n_channels, nz, ny, nx, z0, nz_local, perm, grid_size, padding, ijk,
+                            n_cubes, static_cast<float*>(out), out_cube_stride, nonzero, cube_max, orientation,
+                            (cudaStream_t)stream);
+}
+
+extern "C" int mica_extract_cubes_oriented(const float* vol, int64_t chan_stride, int n_channels,
+                                           int nz, int ny, int nx, int z0, int nz_local, const int perm[3],
+                                           int grid_size, int padding, const int32_t* ijk, int n_cubes,
+                                           float* out, int64_t out_cube_stride, int32_t* nonzero, float* cube_max,
+                                           int orientation, mica_stream_t stream) {
+  return mica_extract_cubes_as(vol, chan_stride, n_channels, nz, ny, nx, z0, nz_local, perm, grid_size, padding, ijk,
+                               n_cubes, out, MICA_DTYPE_F32, out_cube_stride, nonzero, cube_max, orientation, stream);
 }
 
 extern "C" int mica_cube_window_max(const float* vol, int nz, int ny, int nx, int z0, int nz_local,

@@ -27,9 +27,9 @@ struct StitchOwners {
 };
 
 struct StitchParams {
-  const float* bb;
-  const float* ca;
-  const float* aa;
+  const void* bb;  // logits of the kernels' element type T (float or __nv_bfloat16)
+  const void* ca;
+  const void* aa;
   const int32_t* ijk;
   int X, Y, Z;
   int org[3], ext[3];
@@ -62,7 +62,8 @@ __device__ __forceinline__ float softmax3_last(float l0, float l1, float l2) {
 // PEER: the destination of a core plane is the volume block of the rank that owns its x plane -- the
 // local one or a peer's, written over NVLink (coalesced 128-byte runs, fire and forget).  The owner is
 // uniform per CTA (a CTA handles one core plane), so the lookup costs nothing per voxel.
-template <bool PEER>
+// T: the logits' element type, float or __nv_bfloat16 -- bf16 is widened exactly on load, the rest is the same
+template <bool PEER, typename T>
 __global__ void __launch_bounds__(256)
 postproc_stitch_kernel(StitchParams P, StitchOwners O) {
   const int S = P.S, W = P.W;
@@ -72,9 +73,9 @@ postproc_stitch_kernel(StitchParams P, StitchOwners O) {
   const int gx = i + a;
   if (gx >= P.X || gx < P.org[0] || gx >= P.org[0] + P.ext[0]) return;
   const int64_t W3 = (int64_t)W * W * W;
-  const float* bb = P.bb + (int64_t)b * 4 * W3;
-  const float* ca = P.ca + (int64_t)b * 4 * W3;
-  const float* aa = P.aa + (int64_t)b * 21 * W3;
+  const T* bb = static_cast<const T*>(P.bb) + (int64_t)b * 4 * W3;
+  const T* ca = static_cast<const T*>(P.ca) + (int64_t)b * 4 * W3;
+  const T* aa = static_cast<const T*>(P.aa) + (int64_t)b * 21 * W3;
   int64_t vol_n = (int64_t)P.ext[0] * P.ext[1] * P.ext[2];
   int x_org = P.org[0];
   if (PEER) {
@@ -99,11 +100,11 @@ postproc_stitch_kernel(StitchParams P, StitchOwners O) {
     const int64_t src = ((int64_t)(a + P.pad) * W + (bj + P.pad)) * W + (c + P.pad);
     const int64_t dst = ((int64_t)(gx - x_org) * P.ext[1] + ly) * P.ext[2] + lz;
     // issue every load before the math: 26 independent requests in flight per thread
-    const float b0 = ld_stream_half_line(bb + src), b2 = ld_stream_half_line(bb + 2 * W3 + src), b3 = ld_stream_half_line(bb + 3 * W3 + src);
-    const float c0 = ld_stream_half_line(ca + src), c2 = ld_stream_half_line(ca + 2 * W3 + src), c3 = ld_stream_half_line(ca + 3 * W3 + src);
+    const float b0 = ld_stream_core_el(bb + src), b2 = ld_stream_core_el(bb + 2 * W3 + src), b3 = ld_stream_core_el(bb + 3 * W3 + src);
+    const float c0 = ld_stream_core_el(ca + src), c2 = ld_stream_core_el(ca + 2 * W3 + src), c3 = ld_stream_core_el(ca + 3 * W3 + src);
     float l[20];
 #pragma unroll
-    for (int t = 0; t < 20; ++t) l[t] = ld_stream_half_line(aa + (int64_t)(t + 1) * W3 + src);
+    for (int t = 0; t < 20; ++t) l[t] = ld_stream_core_el(aa + (int64_t)(t + 1) * W3 + src);
     st_stream(P.bb_vol + dst, softmax3_last(b0, b2, b3));
     st_stream(P.ca_vol + dst, softmax3_last(c0, c2, c3));
     // argmax on the logits (softmax is monotone); first maximum wins, as torch.max
@@ -154,9 +155,9 @@ struct OverlapWindow {
 };
 
 struct OverlapParams {
-  const float* bb;
-  const float* ca;
-  const float* aa;
+  const void* bb;  // logits of the kernels' element type T (float or __nv_bfloat16)
+  const void* ca;
+  const void* aa;
   const int32_t* ijk;
   int X, Y, Z, pad, W;
   const double* norm;  // [X | Y | Z] reciprocals of the lattice weight sums
@@ -210,19 +211,21 @@ __device__ __forceinline__ uint32_t* overlap_dest(const OverlapParams& P, const 
 }
 
 // the 22 contributions (backbone, carbon_alpha, amino_acid_probability x 20) of the logits at offset src of cube
-// b's [4 | 4 | 21] x W^3 channels: the softmax of the paste (postproc_stitch_kernel), maximum taken the same way
+// b's [4 | 4 | 21] x W^3 channels: the softmax of the paste (postproc_stitch_kernel), maximum taken the same way.
+// T: the logits' element type (bf16 widened exactly on load)
 constexpr int kOverlapQ = 22;
+template <typename T>
 __device__ __forceinline__ void overlap_contrib(const OverlapParams& P, int b, int64_t src, double scale,
                                                 uint32_t q[kOverlapQ]) {
   const int64_t W3 = (int64_t)P.W * P.W * P.W;
-  const float* bb = P.bb + (int64_t)b * 4 * W3;
-  const float* ca = P.ca + (int64_t)b * 4 * W3;
-  const float* aa = P.aa + (int64_t)b * 21 * W3;
-  const float b0 = ld_stream(bb + src), b2 = ld_stream(bb + 2 * W3 + src), b3 = ld_stream(bb + 3 * W3 + src);
-  const float c0 = ld_stream(ca + src), c2 = ld_stream(ca + 2 * W3 + src), c3 = ld_stream(ca + 3 * W3 + src);
+  const T* bb = static_cast<const T*>(P.bb) + (int64_t)b * 4 * W3;
+  const T* ca = static_cast<const T*>(P.ca) + (int64_t)b * 4 * W3;
+  const T* aa = static_cast<const T*>(P.aa) + (int64_t)b * 21 * W3;
+  const float b0 = ld_stream_el(bb + src), b2 = ld_stream_el(bb + 2 * W3 + src), b3 = ld_stream_el(bb + 3 * W3 + src);
+  const float c0 = ld_stream_el(ca + src), c2 = ld_stream_el(ca + 2 * W3 + src), c3 = ld_stream_el(ca + 3 * W3 + src);
   float l[20];
 #pragma unroll
-  for (int t = 0; t < 20; ++t) l[t] = ld_stream(aa + (int64_t)(t + 1) * W3 + src);
+  for (int t = 0; t < 20; ++t) l[t] = ld_stream_el(aa + (int64_t)(t + 1) * W3 + src);
   q[0] = overlap_fixed(softmax3_last(b0, b2, b3), scale);
   q[1] = overlap_fixed(softmax3_last(c0, c2, c3), scale);
   float m = l[0];
@@ -249,7 +252,7 @@ __device__ __forceinline__ int64_t overlap_channel(int ch, int64_t vol_n) { retu
 // window itself): window voxel v reads them at the oriented offset obase + v . os, which for the orientations
 // run here (|os[2]| == 1: the fastest axis stays, possibly reversed) keeps the reads coalesced.
 // PEER: each contribution goes to the block of the rank that owns its plane along O.axis, locally or over NVLink
-template <bool PEER>
+template <bool PEER, typename T>
 __global__ void __launch_bounds__(256)
 overlap_accumulate_kernel(OverlapParams P, OverlapWindow Wn, OverlapOwners O) {
   const int W = P.W;
@@ -272,7 +275,7 @@ overlap_accumulate_kernel(OverlapParams P, OverlapWindow Wn, OverlapOwners O) {
   uint32_t* dst = overlap_dest<PEER>(P, O, gx, gy, gz, &vol_n);
   const int64_t src = P.obase + (int64_t)a * P.os[0] + (int64_t)bj * P.os[1] + (int64_t)c * P.os[2];
   uint32_t q[kOverlapQ];
-  overlap_contrib(P, b, src, scale, q);
+  overlap_contrib<T>(P, b, src, scale, q);
 #pragma unroll
   for (int t = 0; t < kOverlapQ; ++t) red_add_u32(dst + overlap_channel(t, vol_n), q[t]);
 }
@@ -283,7 +286,7 @@ overlap_accumulate_kernel(OverlapParams P, OverlapWindow Wn, OverlapOwners O) {
 // ([22][32][33] uint32, conflict-free both ways) and added with lanes along axis 2 (coalesced red.global.add).
 // grid = (B, W [plane of L] * ceil(W/32)^2), block = 256
 constexpr int kOverlapTileSmem = kOverlapQ * 32 * 33 * 4;
-template <bool PEER>
+template <bool PEER, typename T>
 __global__ void __launch_bounds__(256)
 overlap_accumulate_tiled_kernel(OverlapParams P, OverlapWindow Wn, OverlapOwners O, int K) {
   extern __shared__ uint32_t tq[];
@@ -307,7 +310,7 @@ overlap_accumulate_tiled_kernel(OverlapParams P, OverlapWindow Wn, OverlapOwners
           w0 != 0.f && w1 != 0.f && w2 != 0.f) {
         const double scale = overlap_scale(w0, w1, w2, P.norm[gx], P.norm[P.X + gy], P.norm[P.X + P.Y + gz]);
         const int64_t src = P.obase + (int64_t)v0 * P.os[0] + (int64_t)v1 * P.os[1] + (int64_t)v2 * P.os[2];
-        overlap_contrib(P, b, src, scale, q);
+        overlap_contrib<T>(P, b, src, scale, q);
       }
     }
 #pragma unroll
@@ -388,11 +391,17 @@ static int check_box(int X, int Y, int Z, const int org[3], const int ext[3]) {
   return MICA_OK;
 }
 
-extern "C" int mica_postproc_stitch(const float* bb, const float* ca, const float* aa,
-                                    const int32_t* ijk, int n_cubes, int X, int Y, int Z,
-                                    const int org[3], const int ext[3], int grid_size, int padding,
-                                    float* bb_vol, float* ca_vol, float* aa_prob_vol, float* aa_pred_vol,
-                                    mica_stream_t stream) {
+// byte offset of cube b0's logits in a [B, n_ch, W^3] batch of `esize`-byte elements
+static inline const void* cube_offset(const void* p, int64_t b0, int n_ch, int64_t W3, int esize) {
+  return static_cast<const char*>(p) + b0 * n_ch * W3 * esize;
+}
+
+extern "C" int mica_postproc_stitch_as(const void* bb, const void* ca, const void* aa, int logit_dtype,
+                                       const int32_t* ijk, int n_cubes, int X, int Y, int Z, const int org[3],
+                                       const int ext[3], int grid_size, int padding, float* bb_vol, float* ca_vol,
+                                       float* aa_prob_vol, float* aa_pred_vol, mica_stream_t stream) {
+  const int esize = model_dtype_bytes(logit_dtype);
+  MICA_REQUIRE(esize, "logit dtype %d: must be MICA_DTYPE_F32 or MICA_DTYPE_BF16", logit_dtype);
   MICA_REQUIRE(bb_vol && ca_vol && aa_prob_vol && aa_pred_vol, "null output volume");
   MICA_REQUIRE(n_cubes == 0 || (bb && ca && aa && ijk), "null input");
   MICA_REQUIRE(grid_size > 0 && padding >= 0, "bad grid_size/padding");
@@ -421,15 +430,28 @@ extern "C" int mica_postproc_stitch(const float* bb, const float* ca, const floa
   const int kMaxY = 32768;
   for (int b0 = 0; b0 < n_cubes; b0 += kMaxY) {
     const int nb = (n_cubes - b0 < kMaxY) ? n_cubes - b0 : kMaxY;
-    P.bb = bb + (int64_t)b0 * 4 * W3;
-    P.ca = ca + (int64_t)b0 * 4 * W3;
-    P.aa = aa + (int64_t)b0 * 21 * W3;
+    P.bb = cube_offset(bb, b0, 4, W3, esize);
+    P.ca = cube_offset(ca, b0, 4, W3, esize);
+    P.aa = cube_offset(aa, b0, 21, W3, esize);
     P.ijk = ijk + 3 * (int64_t)b0;
     const int chunks = (grid_size * grid_size + 255) / 256;
-    postproc_stitch_kernel<false><<<dim3(nb, grid_size * chunks), 256, 0, (cudaStream_t)stream>>>(P, StitchOwners());
+    const dim3 grid(nb, grid_size * chunks);
+    if (logit_dtype == MICA_DTYPE_BF16)
+      postproc_stitch_kernel<false, __nv_bfloat16><<<grid, 256, 0, (cudaStream_t)stream>>>(P, StitchOwners());
+    else
+      postproc_stitch_kernel<false, float><<<grid, 256, 0, (cudaStream_t)stream>>>(P, StitchOwners());
     MICA_LAUNCH_CHECK("postproc_stitch_kernel");
   }
   return MICA_OK;
+}
+
+extern "C" int mica_postproc_stitch(const float* bb, const float* ca, const float* aa,
+                                    const int32_t* ijk, int n_cubes, int X, int Y, int Z,
+                                    const int org[3], const int ext[3], int grid_size, int padding,
+                                    float* bb_vol, float* ca_vol, float* aa_prob_vol, float* aa_pred_vol,
+                                    mica_stream_t stream) {
+  return mica_postproc_stitch_as(bb, ca, aa, MICA_DTYPE_F32, ijk, n_cubes, X, Y, Z, org, ext, grid_size, padding,
+                                 bb_vol, ca_vol, aa_prob_vol, aa_pred_vol, stream);
 }
 
 // the paste of cubes the model did not run on (the keep rule of ops.select_cubes): their cores, clipped to the box,
@@ -484,10 +506,12 @@ extern "C" int mica_zero_cores(const int32_t* ijk, int n_cubes, int X, int Y, in
   return MICA_OK;
 }
 
-extern "C" int mica_postproc_stitch_peer(const float* bb, const float* ca, const float* aa, const int32_t* ijk,
-                                         int n_cubes, int X, int Y, int Z, int grid_size, int padding,
-                                         void* const* owner_base, const int* x_bounds, int world,
-                                         mica_stream_t stream) {
+extern "C" int mica_postproc_stitch_peer_as(const void* bb, const void* ca, const void* aa, int logit_dtype,
+                                            const int32_t* ijk, int n_cubes, int X, int Y, int Z, int grid_size,
+                                            int padding, void* const* owner_base, const int* x_bounds, int world,
+                                            mica_stream_t stream) {
+  const int esize = model_dtype_bytes(logit_dtype);
+  MICA_REQUIRE(esize, "logit dtype %d: must be MICA_DTYPE_F32 or MICA_DTYPE_BF16", logit_dtype);
   MICA_REQUIRE(owner_base && x_bounds, "null owner table");
   MICA_REQUIRE(world >= 1 && world <= kStitchMaxWorld, "bad world size %d", world);
   MICA_REQUIRE(n_cubes == 0 || (bb && ca && aa && ijk), "null input");
@@ -516,15 +540,27 @@ extern "C" int mica_postproc_stitch_peer(const float* bb, const float* ca, const
   const int kMaxY = 32768;
   for (int b0 = 0; b0 < n_cubes; b0 += kMaxY) {
     const int nb = (n_cubes - b0 < kMaxY) ? n_cubes - b0 : kMaxY;
-    P.bb = bb + (int64_t)b0 * 4 * W3;
-    P.ca = ca + (int64_t)b0 * 4 * W3;
-    P.aa = aa + (int64_t)b0 * 21 * W3;
+    P.bb = cube_offset(bb, b0, 4, W3, esize);
+    P.ca = cube_offset(ca, b0, 4, W3, esize);
+    P.aa = cube_offset(aa, b0, 21, W3, esize);
     P.ijk = ijk + 3 * (int64_t)b0;
     const int chunks = (grid_size * grid_size + 255) / 256;
-    postproc_stitch_kernel<true><<<dim3(nb, grid_size * chunks), 256, 0, (cudaStream_t)stream>>>(P, O);
+    const dim3 grid(nb, grid_size * chunks);
+    if (logit_dtype == MICA_DTYPE_BF16)
+      postproc_stitch_kernel<true, __nv_bfloat16><<<grid, 256, 0, (cudaStream_t)stream>>>(P, O);
+    else
+      postproc_stitch_kernel<true, float><<<grid, 256, 0, (cudaStream_t)stream>>>(P, O);
     MICA_LAUNCH_CHECK("postproc_stitch_kernel<peer>");
   }
   return MICA_OK;
+}
+
+extern "C" int mica_postproc_stitch_peer(const float* bb, const float* ca, const float* aa, const int32_t* ijk,
+                                         int n_cubes, int X, int Y, int Z, int grid_size, int padding,
+                                         void* const* owner_base, const int* x_bounds, int world,
+                                         mica_stream_t stream) {
+  return mica_postproc_stitch_peer_as(bb, ca, aa, MICA_DTYPE_F32, ijk, n_cubes, X, Y, Z, grid_size, padding,
+                                      owner_base, x_bounds, world, stream);
 }
 
 extern "C" int mica_stitch_cubes(const float* cubes, int n_ch, const int32_t* ijk, int n_cubes,
@@ -550,7 +586,7 @@ extern "C" int mica_stitch_cubes(const float* cubes, int n_ch, const int32_t* ij
   return MICA_OK;
 }
 
-static int overlap_setup(const float* bb, const float* ca, const float* aa, const int32_t* ijk, int n_cubes, int X,
+static int overlap_setup(const void* bb, const void* ca, const void* aa, const int32_t* ijk, int n_cubes, int X,
                          int Y, int Z, int grid_size, int padding, const float* window_w1, const double* norm,
                          int orientation, OverlapParams* P, OverlapWindow* Wn) {
   MICA_REQUIRE(window_w1 && norm, "null pointer");
@@ -586,39 +622,40 @@ static int overlap_setup(const float* bb, const float* ca, const float* aa, cons
   return MICA_OK;
 }
 
-template <bool PEER>
+template <bool PEER, typename T>
 static int overlap_launch(OverlapParams P, const OverlapWindow& Wn, const OverlapOwners& O, int n_cubes,
                           cudaStream_t stream) {
   const int64_t W3 = (int64_t)P.W * P.W * P.W;
-  const float *bb = P.bb, *ca = P.ca, *aa = P.aa;
+  const void *bb = P.bb, *ca = P.ca, *aa = P.aa;
   const int32_t* ijk = P.ijk;
   const int kMaxX = 32768;
   for (int b0 = 0; b0 < n_cubes; b0 += kMaxX) {
     const int nb = (n_cubes - b0 < kMaxX) ? n_cubes - b0 : kMaxX;
-    P.bb = bb + (int64_t)b0 * 4 * W3;
-    P.ca = ca + (int64_t)b0 * 4 * W3;
-    P.aa = aa + (int64_t)b0 * 21 * W3;
+    P.bb = cube_offset(bb, b0, 4, W3, sizeof(T));
+    P.ca = cube_offset(ca, b0, 4, W3, sizeof(T));
+    P.aa = cube_offset(aa, b0, 21, W3, sizeof(T));
     P.ijk = ijk + 3 * (int64_t)b0;
     if (P.os[2] == 1 || P.os[2] == -1) {
       const int chunks = (P.W * P.W + 255) / 256;
-      overlap_accumulate_kernel<PEER><<<dim3(nb, P.W * chunks), 256, 0, stream>>>(P, Wn, O);
+      overlap_accumulate_kernel<PEER, T><<<dim3(nb, P.W * chunks), 256, 0, stream>>>(P, Wn, O);
       MICA_LAUNCH_CHECK(PEER ? "overlap_accumulate_kernel<peer>" : "overlap_accumulate_kernel");
     } else {
       const int nt = (P.W + 31) / 32, K = (P.os[0] == 1 || P.os[0] == -1) ? 0 : 1;
-      MICA_CUDA(cudaFuncSetAttribute(overlap_accumulate_tiled_kernel<PEER>,
+      MICA_CUDA(cudaFuncSetAttribute(overlap_accumulate_tiled_kernel<PEER, T>,
                                      cudaFuncAttributeMaxDynamicSharedMemorySize, kOverlapTileSmem));
-      overlap_accumulate_tiled_kernel<PEER><<<dim3(nb, P.W * nt * nt), 256, kOverlapTileSmem, stream>>>(P, Wn, O, K);
+      overlap_accumulate_tiled_kernel<PEER, T><<<dim3(nb, P.W * nt * nt), 256, kOverlapTileSmem, stream>>>(P, Wn, O, K);
       MICA_LAUNCH_CHECK(PEER ? "overlap_accumulate_tiled_kernel<peer>" : "overlap_accumulate_tiled_kernel");
     }
   }
   return MICA_OK;
 }
 
-extern "C" int mica_overlap_accumulate_fixed_oriented(const float* bb, const float* ca, const float* aa,
-                                                      const int32_t* ijk, int n_cubes, int X, int Y, int Z,
-                                                      int grid_size, int padding, const float* window_w1,
-                                                      const double* norm, int orientation, void* block,
-                                                      mica_stream_t stream) {
+extern "C" int mica_overlap_accumulate_fixed_as(const void* bb, const void* ca, const void* aa, int logit_dtype,
+                                                const int32_t* ijk, int n_cubes, int X, int Y, int Z, int grid_size,
+                                                int padding, const float* window_w1, const double* norm,
+                                                int orientation, void* block, mica_stream_t stream) {
+  MICA_REQUIRE(model_dtype_bytes(logit_dtype), "logit dtype %d: must be MICA_DTYPE_F32 or MICA_DTYPE_BF16",
+               logit_dtype);
   MICA_REQUIRE(block, "null block");
   OverlapParams P;
   OverlapWindow Wn;
@@ -631,15 +668,18 @@ extern "C" int mica_overlap_accumulate_fixed_oriented(const float* bb, const flo
   O.base = nullptr;
   O.axis = 0;
   O.world = 1;
-  return overlap_launch<false>(P, Wn, O, n_cubes, (cudaStream_t)stream);
+  if (logit_dtype == MICA_DTYPE_BF16)
+    return overlap_launch<false, __nv_bfloat16>(P, Wn, O, n_cubes, (cudaStream_t)stream);
+  return overlap_launch<false, float>(P, Wn, O, n_cubes, (cudaStream_t)stream);
 }
 
-extern "C" int mica_overlap_accumulate_fixed_peer_oriented(const float* bb, const float* ca, const float* aa,
-                                                           const int32_t* ijk, int n_cubes, int X, int Y, int Z,
-                                                           int grid_size, int padding, const float* window_w1,
-                                                           const double* norm, int orientation,
-                                                           void* const* owner_base, int axis, const int* bounds,
-                                                           int world, mica_stream_t stream) {
+extern "C" int mica_overlap_accumulate_fixed_peer_as(const void* bb, const void* ca, const void* aa, int logit_dtype,
+                                                     const int32_t* ijk, int n_cubes, int X, int Y, int Z,
+                                                     int grid_size, int padding, const float* window_w1,
+                                                     const double* norm, int orientation, void* const* owner_base,
+                                                     int axis, const int* bounds, int world, mica_stream_t stream) {
+  MICA_REQUIRE(model_dtype_bytes(logit_dtype), "logit dtype %d: must be MICA_DTYPE_F32 or MICA_DTYPE_BF16",
+               logit_dtype);
   MICA_REQUIRE(owner_base && bounds, "null owner table");
   MICA_REQUIRE(world >= 1 && world <= kStitchMaxWorld, "bad world size %d", world);
   MICA_REQUIRE(axis == 0 || axis == 2, "owner axis must be 0 (x) or 2 (k), got %d", axis);
@@ -658,7 +698,28 @@ extern "C" int mica_overlap_accumulate_fixed_peer_oriented(const float* bb, cons
   O.world = world;
   for (int r = 0; r <= world; ++r) O.bounds[r] = bounds[r];
   for (int r = world + 1; r <= kStitchMaxWorld; ++r) O.bounds[r] = G;
-  return overlap_launch<true>(P, Wn, O, n_cubes, (cudaStream_t)stream);
+  if (logit_dtype == MICA_DTYPE_BF16)
+    return overlap_launch<true, __nv_bfloat16>(P, Wn, O, n_cubes, (cudaStream_t)stream);
+  return overlap_launch<true, float>(P, Wn, O, n_cubes, (cudaStream_t)stream);
+}
+
+extern "C" int mica_overlap_accumulate_fixed_oriented(const float* bb, const float* ca, const float* aa,
+                                                      const int32_t* ijk, int n_cubes, int X, int Y, int Z,
+                                                      int grid_size, int padding, const float* window_w1,
+                                                      const double* norm, int orientation, void* block,
+                                                      mica_stream_t stream) {
+  return mica_overlap_accumulate_fixed_as(bb, ca, aa, MICA_DTYPE_F32, ijk, n_cubes, X, Y, Z, grid_size, padding,
+                                          window_w1, norm, orientation, block, stream);
+}
+
+extern "C" int mica_overlap_accumulate_fixed_peer_oriented(const float* bb, const float* ca, const float* aa,
+                                                           const int32_t* ijk, int n_cubes, int X, int Y, int Z,
+                                                           int grid_size, int padding, const float* window_w1,
+                                                           const double* norm, int orientation,
+                                                           void* const* owner_base, int axis, const int* bounds,
+                                                           int world, mica_stream_t stream) {
+  return mica_overlap_accumulate_fixed_peer_as(bb, ca, aa, MICA_DTYPE_F32, ijk, n_cubes, X, Y, Z, grid_size, padding,
+                                               window_w1, norm, orientation, owner_base, axis, bounds, world, stream);
 }
 
 extern "C" int mica_overlap_accumulate_fixed(const float* bb, const float* ca, const float* aa, const int32_t* ijk,

@@ -68,6 +68,29 @@ def _dev(t: torch.Tensor, dtype, name: str):
     return C.c_void_p(t.data_ptr())
 
 
+#: element types of the model-facing buffers (cube batches, logits) -> MICA_DTYPE_* code; maps and volumes are float32
+MODEL_DTYPES = {torch.float32: _lib.DTYPE_F32, torch.bfloat16: _lib.DTYPE_BF16}
+
+
+def model_dtype(dtype) -> torch.dtype:
+    """``dtype`` if it is a dtype the cube batches and logits can have (float32, bfloat16); MicaError otherwise."""
+    if dtype not in MODEL_DTYPES:
+        raise _lib.MicaError(f'model inputs and logits are torch.float32 or torch.bfloat16, got {dtype!r}')
+    return dtype
+
+
+def _logits(bb, ca, aa, B, W):
+    """(pointers, MICA_DTYPE code) of one batch of logits: [B,4|4|21,W,W,W] CUDA tensors, contiguous, all float32 or
+    all bfloat16."""
+    for t, c, name in ((bb, 4, 'bb'), (ca, 4, 'ca'), (aa, 21, 'aa')):
+        if tuple(t.shape) != (B, c, W, W, W):
+            raise _lib.MicaError(f'{name} logits must be [{B},{c},{W},{W},{W}], got {tuple(t.shape)}')
+    dt = bb.dtype
+    if dt not in MODEL_DTYPES or ca.dtype != dt or aa.dtype != dt:
+        raise _lib.MicaError(f'logits must be all float32 or all bfloat16, got {bb.dtype}, {ca.dtype}, {aa.dtype}')
+    return (_dev(bb, dt, 'bb'), _dev(ca, dt, 'ca'), _dev(aa, dt, 'aa')), MODEL_DTYPES[dt]
+
+
 def require_gpu():
     n = lib.mica_device_count()
     if n < 0:
@@ -368,9 +391,11 @@ def af3_encode(coords: torch.Tensor, bb_ch: torch.Tensor, aa_ch: torch.Tensor, o
 class Af3CubeFiller:
     """Sparse AF3 path (R4 + R5 fused): keeps a [n_slots,24,W,W,W] model-input buffer equal to
     "zeros + the atoms of the cube currently in each slot" without ever building the dense
-    24-channel volume.  ``bin`` once per map, ``fill`` once per batch."""
+    24-channel volume.  ``bin`` once per map, ``fill`` once per batch.  ``dtype``: the buffer's element
+    type, float32 or bfloat16 (1.0 and 0.0 are exact in both)."""
 
-    def __init__(self, device, n_slots, grid_size=48, padding=8, perm=(2, 1, 0)):
+    def __init__(self, device, n_slots, grid_size=48, padding=8, perm=(2, 1, 0), dtype=torch.float32):
+        self.dtype = model_dtype(dtype)
         self.device, self.n_slots = device, int(n_slots)
         self.grid_size, self.padding, self.perm = int(grid_size), int(padding), tuple(perm)
         self.buffer = None          # [n_slots,24,W,W,W], allocated (zeroed) by the first fill
@@ -384,15 +409,22 @@ class Af3CubeFiller:
     def _fill(self, ijk, nonzero_ptr, orient=0):
         n_atoms, (nz, ny, nx) = self._geom
         prev = self._shown
-        check(lib.mica_af3_fill_cubes_oriented(C.c_void_p(self.ws.data_ptr()), n_atoms, nz, ny, nx,
-                                               _lib.int3(self.perm), self.grid_size, self.padding,
-                                               C.c_void_p(prev.data_ptr()) if prev is not None else None,
-                                               int(prev.shape[0]) if prev is not None else 0,
-                                               C.c_void_p(ijk.data_ptr()) if ijk is not None else None,
-                                               int(ijk.shape[0]) if ijk is not None else 0,
-                                               C.c_void_p(self.buffer.data_ptr()), self.buffer.stride(0),
-                                               nonzero_ptr, self._shown_orient, orient, _stream()), 'af3_fill_cubes')
+        check(lib.mica_af3_fill_cubes_as(C.c_void_p(self.ws.data_ptr()), n_atoms, nz, ny, nx,
+                                         _lib.int3(self.perm), self.grid_size, self.padding,
+                                         C.c_void_p(prev.data_ptr()) if prev is not None else None,
+                                         int(prev.shape[0]) if prev is not None else 0,
+                                         C.c_void_p(ijk.data_ptr()) if ijk is not None else None,
+                                         int(ijk.shape[0]) if ijk is not None else 0,
+                                         C.c_void_p(self.buffer.data_ptr()), MODEL_DTYPES[self.dtype],
+                                         self.buffer.stride(0), nonzero_ptr, self._shown_orient, orient, _stream()),
+              'af3_fill_cubes')
         self._shown, self._shown_orient = ijk, orient
+
+    def retype(self, dtype):
+        """Give the slot buffer element type ``dtype`` (float32 or bfloat16): the buffer is dropped and the next
+        ``fill`` allocates a clean one.  The atom bins stay."""
+        self.dtype = model_dtype(dtype)
+        self.buffer, self._shown, self._shown_orient = None, None, 0
 
     def clear(self):
         """Un-scatter every slot (buffer back to all zeros)."""
@@ -443,7 +475,7 @@ class Af3CubeFiller:
         _dev(ijk, torch.int32, 'ijk')
         if self.buffer is None:
             W = self.grid_size + 2 * self.padding
-            self.buffer = torch.zeros((self.n_slots, 24, W, W, W), dtype=torch.float32, device=self.device)
+            self.buffer = torch.zeros((self.n_slots, 24, W, W, W), dtype=self.dtype, device=self.device)
         self._fill(ijk, p_nz, orient)
         return self.buffer[:B]
 
@@ -564,7 +596,9 @@ def extract_cubes(vol: torch.Tensor, ijk: torch.Tensor, grid_size: int = 48, pad
     """vol [C,nz_local,ny,nx] (or [nz,ny,nx]) -> out [B,C,W,W,W] for the cube origins ``ijk``
     (int32 [B,3], cube space).  ``out`` may be a channel slice of a larger [B,Ctot,W,W,W]
     buffer (only the batch stride may be non-dense).  ``orient``: every window in that orientation
-    (``orientation``; test-time augmentation), cut straight from the map; 0 = the windows as they are."""
+    (``orientation``; test-time augmentation), cut straight from the map; 0 = the windows as they are.
+    ``out`` may be float32 (default) or bfloat16: every voxel is then rounded once to nearest even, and ``nonzero`` /
+    ``cube_max`` are taken on the float32 values, so they are those of a float32 ``out``."""
     orient = _orientation_arg(orient)
     if vol.dim() == 3:
         vol = vol.unsqueeze(0)
@@ -576,16 +610,16 @@ def extract_cubes(vol: torch.Tensor, ijk: torch.Tensor, grid_size: int = 48, pad
     W = grid_size + 2 * padding
     if out is None:
         out = torch.empty((B, Cn, W, W, W), dtype=torch.float32, device=vol.device)
-    if not out.is_cuda or out.dtype != torch.float32 or tuple(out.shape) != (B, Cn, W, W, W):
-        raise _lib.MicaError(f'out must be a CUDA float32 [{B},{Cn},{W},{W},{W}] tensor')
+    if not out.is_cuda or out.dtype not in MODEL_DTYPES or tuple(out.shape) != (B, Cn, W, W, W):
+        raise _lib.MicaError(f'out must be a CUDA float32 or bfloat16 [{B},{Cn},{W},{W},{W}] tensor')
     if B and out.stride()[1:] != (W ** 3, W * W, W, 1):
         raise _lib.MicaError('out must be dense in every axis but the batch')
     cube_stride = out.stride(0) if B else Cn * W ** 3
     p_nz = _dev(nonzero, torch.int32, 'nonzero') if nonzero is not None else None
     p_mx = _dev(cube_max, torch.float32, 'cube_max') if cube_max is not None else None
-    check(lib.mica_extract_cubes_oriented(p_vol, vol.stride(0), Cn, nz, ny, nx, z0, nzl, _lib.int3(perm), grid_size,
-                                          padding, p_ijk, B, C.c_void_p(out.data_ptr()), cube_stride, p_nz, p_mx,
-                                          orient, _stream()), 'extract_cubes')
+    check(lib.mica_extract_cubes_as(p_vol, vol.stride(0), Cn, nz, ny, nx, z0, nzl, _lib.int3(perm), grid_size,
+                                    padding, p_ijk, B, C.c_void_p(out.data_ptr()), MODEL_DTYPES[out.dtype], cube_stride,
+                                    p_nz, p_mx, orient, _stream()), 'extract_cubes')
     return out
 
 
@@ -682,16 +716,14 @@ class StitchedVolumes:
 @device_guard
 def postproc_stitch(bb: torch.Tensor, ca: torch.Tensor, aa: torch.Tensor, ijk: torch.Tensor,
                     vols: StitchedVolumes, grid_size: int = 48, padding: int = 8):
-    """Fused utils/predict.py:342-349 + :494-501 for one batch of cubes."""
+    """Fused utils/predict.py:342-349 + :494-501 for one batch of cubes.  The logits are all float32 or all bfloat16
+    (widened exactly on load: the volumes equal the float32 call on ``logits.float()``)."""
     B = ijk.shape[0]
     W = grid_size + 2 * padding
-    for t, c, name in ((bb, 4, 'bb'), (ca, 4, 'ca'), (aa, 21, 'aa')):
-        if tuple(t.shape) != (B, c, W, W, W):
-            raise _lib.MicaError(f'{name} logits must be [{B},{c},{W},{W},{W}], got {tuple(t.shape)}')
+    ptrs, code = _logits(bb, ca, aa, B, W)
     X, Y, Z = vols.shape
-    check(lib.mica_postproc_stitch(
-        _dev(bb, torch.float32, 'bb'), _dev(ca, torch.float32, 'ca'), _dev(aa, torch.float32, 'aa'),
-        _dev(ijk, torch.int32, 'ijk'), B, X, Y, Z, _lib.int3(vols.org), _lib.int3(vols.ext), grid_size, padding,
+    check(lib.mica_postproc_stitch_as(
+        *ptrs, code, _dev(ijk, torch.int32, 'ijk'), B, X, Y, Z, _lib.int3(vols.org), _lib.int3(vols.ext), grid_size, padding,
         _dev(vols.backbone_probability, torch.float32, 'bb_vol'),
         _dev(vols.carbon_alpha_probability, torch.float32, 'ca_vol'),
         _dev(vols.amino_acid_probability, torch.float32, 'aa_prob_vol'),
@@ -717,8 +749,8 @@ class StitchCall:
     """``postproc_stitch`` bound to one set of volumes and one geometry: everything that does not change from
     batch to batch (volume pointers, box, shapes) is converted to ctypes once, so the per-call host cost is a
     handful of microseconds -- the drop-in feeds the model in the reference's batches of <= 8 cubes, i.e.
-    hundreds of stitch calls per map.  The caller guarantees CUDA float32 contiguous logits on the volumes'
-    device (checked on the first call and whenever the batch size changes)."""
+    hundreds of stitch calls per map.  The caller guarantees CUDA contiguous logits, all float32 or all bfloat16, on
+    the volumes' device (checked on the first call and whenever the batch size or the dtype changes)."""
 
     def __init__(self, vols: 'StitchedVolumes', grid_size: int = 48, padding: int = 8):
         self.vols, self.grid_size, self.padding = vols, int(grid_size), int(padding)
@@ -729,28 +761,26 @@ class StitchCall:
                        _dev(vols.carbon_alpha_probability, torch.float32, 'ca_vol'),
                        _dev(vols.amino_acid_probability, torch.float32, 'aa_prob_vol'),
                        _dev(vols.amino_acid_prediction, torch.float32, 'aa_pred_vol'))
-        self._checked_B = -1
+        self._checked = None            # (B, dtype) of the last checked call
+        self._code = _lib.DTYPE_F32
         self._dev_index = vols.device.index
 
     def __call__(self, bb, ca, aa, ijk):
         B = ijk.shape[0]
-        if B != self._checked_B:
-            W = self.W
-            for t, c, name in ((bb, 4, 'bb'), (ca, 4, 'ca'), (aa, 21, 'aa')):
-                if tuple(t.shape) != (B, c, W, W, W):
-                    raise _lib.MicaError(f'{name} logits must be [{B},{c},{W},{W},{W}], got {tuple(t.shape)}')
-                _dev(t, torch.float32, name)
+        if (B, bb.dtype) != self._checked:
+            _, self._code = _logits(bb, ca, aa, B, self.W)
+            for t, name in ((bb, 'bb'), (ca, 'ca'), (aa, 'aa')):
                 if t.device != self.vols.device:
                     raise _lib.MicaError(f'{name} logits live on {t.device}, the volumes on {self.vols.device}')
             _dev(ijk, torch.int32, 'ijk')
-            self._checked_B = B
+            self._checked = (B, bb.dtype)
         if torch.cuda.current_device() != self._dev_index:
             with torch.cuda.device(self._dev_index):
                 return self(bb, ca, aa, ijk)
         X, Y, Z, org, ext, gs, pad, p_bb, p_ca, p_aap, p_aapred = self._fixed
-        check(lib.mica_postproc_stitch(bb.data_ptr(), ca.data_ptr(), aa.data_ptr(), ijk.data_ptr(), B, X, Y, Z, org,
-                                       ext, gs, pad, p_bb, p_ca, p_aap, p_aapred,
-                                       torch.cuda.current_stream().cuda_stream), 'postproc_stitch')
+        check(lib.mica_postproc_stitch_as(bb.data_ptr(), ca.data_ptr(), aa.data_ptr(), self._code, ijk.data_ptr(), B,
+                                          X, Y, Z, org, ext, gs, pad, p_bb, p_ca, p_aap, p_aapred,
+                                          torch.cuda.current_stream().cuda_stream), 'postproc_stitch')
 
 
 @device_guard
@@ -758,18 +788,16 @@ def postproc_stitch_peer(bb: torch.Tensor, ca: torch.Tensor, aa: torch.Tensor, i
                          owner_table: torch.Tensor, x_bounds, grid_size: int = 48, padding: int = 8):
     """``postproc_stitch`` for one map whose cubes are dealt out over several GPUs: every core plane goes to
     the volume block of the rank that owns its x range (``owner_table``: int64 device tensor of ``world``
-    base pointers, ``peer.PeerVolumes.table``; ``x_bounds``: world + 1 plane bounds), local or over NVLink."""
+    base pointers, ``peer.PeerVolumes.table``; ``x_bounds``: world + 1 plane bounds), local or over NVLink.  Logits as
+    ``postproc_stitch``: all float32 or all bfloat16."""
     B = ijk.shape[0]
     W = grid_size + 2 * padding
-    for t, c, name in ((bb, 4, 'bb'), (ca, 4, 'ca'), (aa, 21, 'aa')):
-        if tuple(t.shape) != (B, c, W, W, W):
-            raise _lib.MicaError(f'{name} logits must be [{B},{c},{W},{W},{W}], got {tuple(t.shape)}')
+    ptrs, code = _logits(bb, ca, aa, B, W)
     X, Y, Z = (int(v) for v in cube_shape)
     world = int(owner_table.numel())
     bounds = (C.c_int * (world + 1))(*[int(v) for v in x_bounds])
-    check(lib.mica_postproc_stitch_peer(
-        _dev(bb, torch.float32, 'bb'), _dev(ca, torch.float32, 'ca'), _dev(aa, torch.float32, 'aa'),
-        _dev(ijk, torch.int32, 'ijk'), B, X, Y, Z, grid_size, padding,
+    check(lib.mica_postproc_stitch_peer_as(
+        *ptrs, code, _dev(ijk, torch.int32, 'ijk'), B, X, Y, Z, grid_size, padding,
         _dev(owner_table, torch.int64, 'owner_table'), bounds, world, _stream()), 'postproc_stitch_peer')
 
 
@@ -907,7 +935,8 @@ class OverlapStitcher:
 
     @device_guard
     def accumulate(self, bb, ca, aa, ijk, vols=None, orient: int = 0):
-        """Add one batch of logits, those of the windows ``ijk`` in orientation ``orient`` (one of ``tta``)."""
+        """Add one batch of logits, those of the windows ``ijk`` in orientation ``orient`` (one of ``tta``); all float32
+        or all bfloat16 (widened exactly on load: the sums equal the float32 call on ``logits.float()``)."""
         if _orientation_arg(orient) not in self.orientations:
             raise _lib.MicaError(f'orientation {orient} is not one of this stitcher\'s {list(self.orientations)}')
         if self.core:
@@ -919,19 +948,16 @@ class OverlapStitcher:
             return
         B = ijk.shape[0]
         W = self.grid_size + 2 * self.padding
-        for t, c, name in ((bb, 4, 'bb'), (ca, 4, 'ca'), (aa, 21, 'aa')):
-            if tuple(t.shape) != (B, c, W, W, W):
-                raise _lib.MicaError(f'{name} logits must be [{B},{c},{W},{W},{W}], got {tuple(t.shape)}')
+        ptrs, code = _logits(bb, ca, aa, B, W)
         X, Y, Z = self.shape
-        args = (_dev(bb, torch.float32, 'bb'), _dev(ca, torch.float32, 'ca'), _dev(aa, torch.float32, 'aa'),
-                _dev(ijk, torch.int32, 'ijk'), B, X, Y, Z, self.grid_size, self.padding,
+        args = (*ptrs, code, _dev(ijk, torch.int32, 'ijk'), B, X, Y, Z, self.grid_size, self.padding,
                 self.w1.ctypes.data_as(C.POINTER(C.c_float)), C.c_void_p(self.norm.data_ptr()), int(orient))
         if self.owners is None:
-            check(lib.mica_overlap_accumulate_fixed_oriented(*args, C.c_void_p(self.vols.block.data_ptr()), _stream()),
+            check(lib.mica_overlap_accumulate_fixed_as(*args, C.c_void_p(self.vols.block.data_ptr()), _stream()),
                   'overlap_accumulate')
         else:
             o = self.owners
-            check(lib.mica_overlap_accumulate_fixed_peer_oriented(
+            check(lib.mica_overlap_accumulate_fixed_peer_as(
                 *args, _dev(o.table, torch.int64, 'owner_table'), int(o.axis), self._bounds, int(o.table.numel()),
                 _stream()), 'overlap_accumulate_peer')
 

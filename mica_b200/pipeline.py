@@ -110,11 +110,13 @@ def _on_device(method):
 D8_MODES = ('none', 'split', 'reference')
 
 
-def _f32c(t):
-    """Logits as the stitch kernel wants them (contiguous float32); a no-op for tensors that already are."""
-    if t.dtype != torch.float32:
-        t = t.float()
-    return t if t.is_contiguous() else t.contiguous()
+def _f32c(*logits):
+    """Logits as the stitch kernels take them: contiguous, all float32 or all bfloat16.  Float32 and bfloat16 pass
+    through (the kernels widen bfloat16 exactly); any other dtype, or a mix, becomes float32.  A no-op for tensors that
+    already are what the kernels take."""
+    dt = logits[0].dtype
+    keep = dt in ops.MODEL_DTYPES and all(t.dtype == dt for t in logits)
+    return tuple((t if keep else t.float()).contiguous() for t in logits)
 
 
 def run_model_chunks(model_fn, x, af, flags_host, ijk, stitch, model_batch=None, d8='none'):
@@ -201,7 +203,12 @@ class MapPipeline:
     """One GPU's share of the hot path.  With ``slab`` left None it owns the whole map."""
 
     def __init__(self, device, grid_size: int = 48, padding: int = 8, order: int = 3,
-                 batch_cubes: int = 16, target_voxel_size: float = 1.0, af3_mode: str = 'sparse'):
+                 batch_cubes: int = 16, target_voxel_size: float = 1.0, af3_mode: str = 'sparse',
+                 cube_dtype=torch.float32):
+        #: element type of the cube batches handed to ``model_fn`` (map and AF3 channels): torch.float32 or
+        #: torch.bfloat16 (each voxel rounded once to nearest even; the AF3 channels' 1 / 0 are exact).  Running the
+        #: model in a matching precision is the caller's job; the stitch takes float32 or bfloat16 logits.
+        self.cube_dtype = ops.model_dtype(cube_dtype)
         ops.require_gpu()
         self.device = torch.device(device)
         self.grid_size, self.padding, self.order = int(grid_size), int(padding), int(order)
@@ -234,10 +241,18 @@ class MapPipeline:
         self._pinned_free = []          # (order-stats record, AF3 status word) pairs in pinned memory, reused:
         self._pre_stream = None         # cudaHostAlloc synchronises the device, so never allocate per step
 
-    def configure(self, grid_size=None, padding=None, batch_cubes=None, order=None, target_voxel_size=None):
-        """Change the cube geometry / batch size of a live pipeline (the drop-in classes learn them stage
-        by stage: ``GridCreator`` is told grid_size and padding after ``DataPreprocessor`` has already
-        normalised the map).  Buffers that depend on what changed are dropped and rebuilt on demand."""
+    def configure(self, grid_size=None, padding=None, batch_cubes=None, order=None, target_voxel_size=None,
+                  cube_dtype=None):
+        """Change the cube geometry / batch size / ``cube_dtype`` of a live pipeline (the drop-in classes learn them
+        stage by stage: ``GridCreator`` is told grid_size and padding after ``DataPreprocessor`` has already
+        normalised the map).  Buffers that depend on what changed are dropped and rebuilt on demand (a new
+        ``cube_dtype`` drops the slot buffers of the cubes and of the AF3 fillers; the atom bins stay)."""
+        if cube_dtype is not None and ops.model_dtype(cube_dtype) != self.cube_dtype:
+            self.cube_dtype = cube_dtype
+            self._x, self._af, self._nz = [None, None], [None, None], [None, None]
+            for f in self._fillers:
+                if f is not None:
+                    f.retype(cube_dtype)
         gs = self.grid_size if grid_size is None else int(grid_size)
         pad = self.padding if padding is None else int(padding)
         bc = self.batch_cubes if batch_cubes is None else int(batch_cubes)
@@ -332,7 +347,7 @@ class MapPipeline:
                 f = self._fillers[i]
                 if f is None or f.perm != tuple(perm) or f.n_slots < self.batch_cubes:
                     self._fillers[i] = ops.Af3CubeFiller(self.device, self.batch_cubes, self.grid_size,
-                                                         self.padding, perm)
+                                                         self.padding, perm, dtype=self.cube_dtype)
                 else:
                     f.clear()                         # with the OLD bins, before they are rebuilt
             f = self._fillers[0]
@@ -376,14 +391,14 @@ class MapPipeline:
     def _buffers(self, B, slot=0):
         W = self.window
         if self._x[slot] is None or self._x[slot].shape[0] < B:
-            self._x[slot] = torch.empty((B, 1, W, W, W), dtype=torch.float32, device=self.device)
+            self._x[slot] = torch.empty((B, 1, W, W, W), dtype=self.cube_dtype, device=self.device)
             self._nz[slot] = torch.empty(B, dtype=torch.int32, device=self.device)
         return self._x[slot][:B], self._nz[slot][:B]
 
     def _af_buffer(self, B, slot=0):
         W = self.window
         if self._af[slot] is None or self._af[slot].shape[0] < B:
-            self._af[slot] = torch.empty((B, 24, W, W, W), dtype=torch.float32, device=self.device)
+            self._af[slot] = torch.empty((B, 24, W, W, W), dtype=self.cube_dtype, device=self.device)
         return self._af[slot][:B]
 
     def _extract_map(self, ijk, x, orient=0):
@@ -395,8 +410,8 @@ class MapPipeline:
 
     @_on_device
     def extract_batch(self, b0: int, b1: int, want_flags: bool = False, slot: int = 0, orient: int = 0):
-        """Cubes [b0,b1) -> (exp_map [B,1,W,W,W], af_features [B,24,W,W,W][, nonzero flags])
-        -- the two tensors MICA.forward takes (models/model.py:331).  ``slot`` picks one of
+        """Cubes [b0,b1) -> (exp_map [B,1,W,W,W], af_features [B,24,W,W,W][, nonzero flags]), both of
+        ``cube_dtype`` -- the two tensors MICA.forward takes (models/model.py:331).  ``slot`` picks one of
         the two input buffers (the prefetch of batch n+1 must not overwrite batch n).  ``orient``: both
         tensors in that orientation (``ops.orientation``; the flags do not depend on it)."""
         x, nzf = self._buffers(b1 - b0, slot)
@@ -521,7 +536,7 @@ class MapPipeline:
             extra = orient_arg and (g,)
 
             def stitch(bb, ca, aa, ijk):
-                bb, ca, aa = _f32c(bb), _f32c(ca), _f32c(aa)
+                bb, ca, aa = _f32c(bb, ca, aa)
                 if timed:
                     with self.timer('postproc_stitch'):
                         stitch_fn(bb, ca, aa, ijk, vols, *extra)

@@ -31,12 +31,28 @@ import torch
 
 from . import ops, pdb, session
 from ._lib import check, lib
-from .pipeline import (MapPipeline, _SlabDrain, deal_cubes, run_model_chunks, shared_pipeline, worker_batches,
-                       worker_pipeline)
+from .pipeline import (MapPipeline, _f32c, _SlabDrain, deal_cubes, run_model_chunks, shared_pipeline,
+                       worker_batches, worker_pipeline)
 
 MAP_TYPES = ('backbone_probability', 'carbon_alpha_probability', 'amino_acid_prediction',
              'amino_acid_probability')
 SMALL_VOLUMES = MAP_TYPES[:3]
+#: ``precision=`` / ``MICA_PRECISION`` -> the dtype of the cubes the model is given (None: float32)
+PRECISIONS = {'fp32': torch.float32, 'bf16': torch.bfloat16}
+
+
+def parse_precision(spec):
+    """``precision=`` / ``MICA_PRECISION`` -> torch.float32 or torch.bfloat16.  None or '' -> float32 (today's path);
+    'fp32' / 'bf16' (any case, surrounding blanks ignored).  Anything else raises ValueError."""
+    if spec is None:
+        return torch.float32
+    if isinstance(spec, str):
+        key = spec.strip().lower()
+        if not key:
+            return torch.float32
+        if key in PRECISIONS:
+            return PRECISIONS[key]
+    raise ValueError(f"precision must be None, 'fp32' or 'bf16', got {spec!r}")
 
 
 def parse_devices(spec, n_visible: int, allow_repeats: bool = True):
@@ -158,7 +174,8 @@ class DeviceVolume:
 class CryoEMPredictor:
     def __init__(self, model_path, grids_path, output_path, save_output=True, device='cuda', quiet=False,
                  model=None, keep_on_device=True, host_volumes=None, host_pool=None, reference_batching=False,
-                 super_batch=256, release_inputs=True, devices=None, *, overlap_window=None, tta=None):
+                 super_batch=256, release_inputs=True, devices=None, *, overlap_window=None, tta=None,
+                 precision=None):
         """Additions to the reference signature (all optional):
 
         ``model``               an already loaded model (callable ``(exp_map, af_features) -> (bb, ca, aa)``).
@@ -196,8 +213,18 @@ class CryoEMPredictor:
                                 (window ``overlap_window``, default 'core'; NOT the reference's arithmetic), the same
                                 bits on one device and with ``devices=``.  Needs the resident map GridCreator
                                 registers: with the reference's per-cube files it is logged and (False, {}) returned.
-                                A bad value is refused before any launch."""
+                                A bad value is refused before any launch.
+        ``precision``           (keyword only) None reads ``MICA_PRECISION`` when ``run_prediction`` is called (unset or
+                                empty: 'fp32').  'fp32': today's path.  'bf16': the cubes are cut straight into
+                                bfloat16 model inputs (every voxel rounded once to nearest even; the AF3 channels'
+                                1 / 0 are exact, so MICA's zero-AF3 test takes the same branch), the model runs under
+                                ``torch.autocast('cuda', dtype=torch.bfloat16)``, and its bfloat16 logits go to the
+                                stitch, which widens them exactly.  The volumes stay float32.  On every device of
+                                ``devices=``, with ``tta``, ``overlap_window`` and the per-cube files.  A bad value is
+                                logged and (False, {}) returned before any launch."""
         self.devices = devices
+        self.precision = precision
+        self._cube_dtype = torch.float32                # resolved from precision / MICA_PRECISION by run_prediction
         self.overlap_window = overlap_window
         self.tta = tta
         self.worker_cubes = None                        # cubes each worker ran (several devices only)
@@ -359,6 +386,19 @@ class CryoEMPredictor:
         return model
 
     # ------------------------------------------------------------------ inference + stitch
+    def _resolve_precision(self):
+        return parse_precision(os.environ.get('MICA_PRECISION') if self.precision is None else self.precision)
+
+    def _model_fn(self, model):
+        """``model`` as the pipelines call it: itself in float32; under bfloat16 autocast with ``precision='bf16'``."""
+        if self._cube_dtype == torch.float32:
+            return model
+
+        def call(exp_map, af_features):
+            with torch.autocast('cuda', dtype=torch.bfloat16):
+                return model(exp_map, af_features)
+        return call
+
     def _model_batch(self):
         return self.optimal_batch_size if self.use_optimized_batching else 1
 
@@ -385,7 +425,8 @@ class CryoEMPredictor:
         m, a = s['map'], s['af3']
         pipe = m.get('pipe') or shared_pipeline(m['volume'].device)
         n = len(s['ijk'])
-        pipe.configure(grid_size=s['grid_size'], padding=s['padding'], batch_cubes=max(1, min(self.super_batch, n)))
+        pipe.configure(grid_size=s['grid_size'], padding=s['padding'], batch_cubes=max(1, min(self.super_batch, n)),
+                       cube_dtype=self._cube_dtype)
         pipe.set_normalized(m['volume'], m['header'])
         if a is not None and a.get('atoms') is not None:
             if not pipe.encode_af3(*a['atoms']):            # bins for the final geometry; cannot fail if
@@ -444,8 +485,8 @@ class CryoEMPredictor:
                 afs.append(np.stack(feats))
             except Exception:
                 afs.append(np.zeros((24, W, W, W), np.float32))
-        x = torch.from_numpy(np.stack(xs)[:, None].astype(np.float32)).to(dev)
-        af = torch.from_numpy(np.stack(afs).astype(np.float32)).to(dev)
+        x = torch.from_numpy(np.stack(xs)[:, None].astype(np.float32)).to(dev).to(self._cube_dtype)
+        af = torch.from_numpy(np.stack(afs).astype(np.float32)).to(dev).to(self._cube_dtype)
         flags = (af.abs().reshape(B, -1).sum(1) > 0).to(torch.int32)
         return x, af, flags
 
@@ -491,6 +532,7 @@ class CryoEMPredictor:
         model = self.model
         if hasattr(model, 'eval'):
             model.eval()
+        model = self._model_fn(model)
         d8 = 'reference' if self.reference_batching else 'split'
         with torch.no_grad():
             if s['kind'] == 'resident':
@@ -523,7 +565,7 @@ class CryoEMPredictor:
                 overlap, vols = None, ops.StitchedVolumes(s['cube_shape'], dev)
 
             def stitch(bb, ca, aa, ijk):
-                bb, ca, aa = bb.contiguous().float(), ca.contiguous().float(), aa.contiguous().float()
+                bb, ca, aa = _f32c(bb, ca, aa)
                 if overlap is not None:
                     overlap.accumulate(bb, ca, aa, ijk)
                 else:
@@ -571,7 +613,8 @@ class CryoEMPredictor:
                                    else None, af3)
                 norm, atoms, af3 = inputs[dev]
                 pipe = worker_pipeline(dev, slot)[0]
-                pipe.configure(grid_size=gs, padding=pad, batch_cubes=max(1, min(self.super_batch, n)))
+                pipe.configure(grid_size=gs, padding=pad, batch_cubes=max(1, min(self.super_batch, n)),
+                               cube_dtype=self._cube_dtype)
                 pipe.set_normalized(norm, m['header'])
                 if atoms is not None:
                     if not pipe.encode_af3(*atoms):
@@ -620,10 +663,10 @@ class CryoEMPredictor:
             lo, hi = ranges[w]
             if hi <= lo:
                 return
-            dev, table, model = workers[w], tables[workers[w]], self._models[workers[w]]
+            dev, table, model = workers[w], tables[workers[w]], self._model_fn(self._models[workers[w]])
 
             def stitch(bb, ca, aa, ijk, _vols=None, orient=0):
-                bb, ca, aa = bb.contiguous().float(), ca.contiguous().float(), aa.contiguous().float()
+                bb, ca, aa = _f32c(bb, ca, aa)
                 if overlap is not None:
                     overlap[dev].accumulate(bb, ca, aa, ijk, orient=orient)
                 else:
@@ -684,6 +727,7 @@ class CryoEMPredictor:
         t_total = time.time()
         try:
             self._tta_codes()                                    # a bad tta is refused before any launch
+            self._cube_dtype = self._resolve_precision()         # so is a bad precision
             self._workers = self._resolve_workers()
             if not self.select_processing_strategy():
                 return False, {}
