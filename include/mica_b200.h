@@ -614,6 +614,21 @@ int64_t mica_parse_pdb(const char* text, int64_t nbytes, int with_hetatm, int64_
                        uint8_t* fields, float* occupancy, int32_t* model, int8_t* bb_ch, int8_t* aa_ch,
                        int64_t* info);
 
+/* Prediction maps (oracle/prediction_maps_oracle.py): the four stitched volumes resampled onto a target grid in its
+ * memory order, one launch.  bb, ca, aa_pred, aa_prob: device float32 volumes in cube space [X,Y,Z] (aa_prob
+ * [20][X,Y,Z]), the working map's memory axes permuted by perm (cube axis a walks memory axis perm[a], any of the 6
+ * permutations); aa_pred is not read.  They must cover the whole cube space (org 0, ext (X, Y, Z)), and (X, Y, Z) must
+ * be working_zyx permuted by perm.  working_zyx / target_zyx: memory shapes (nz, ny, nx) of the working grid and of the
+ * target grid.  Per memory axis target index s reads the working coordinate float64(s (n_w - 1)) / float64(n_s - 1);
+ * each of the 22 probability channels is interpolated trilinearly with float64 weights (products and sums rounded in
+ * the oracle's order) and rounded to float32.  out_bb, out_ca, out_pred: device float32 [nz,ny,nx]; out_prob
+ * [20][nz,ny,nx].  out_pred is the index of the first largest of the 20 resampled probabilities (a NaN counts as the
+ * largest), as float32.  Bad arguments are MICA_ERR_INVALID before any launch. */
+int mica_volumes_to_grid(const float* bb, const float* ca, const float* aa_pred, const float* aa_prob, int X, int Y,
+                         int Z, const int org[3], const int ext[3], const int perm[3], const int working_zyx[3],
+                         const int target_zyx[3], float* out_bb, float* out_ca, float* out_pred, float* out_prob,
+                         mica_stream_t stream);
+
 #ifdef __cplusplus
 }
 #endif

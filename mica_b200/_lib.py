@@ -153,6 +153,9 @@ SIGNATURES = {
     'mica_label_aa_mask': (_i, [_p, _p, _i64, _f, _f, _f, _i, _i, _i, _i, _i, _i, _p, _sz, _p, _p, _p]),
     'mica_contour_threshold_f32': (_i, [_p, _p, _i64, _f, _p]),
     'mica_zero_around_atoms': (_i, [_p, _i64, C.POINTER(_f), C.POINTER(_f), C.c_double, _i, _i, _i, _p, _p, _p]),
+    # prediction maps on the input map's grid
+    'mica_volumes_to_grid': (_i, [_p, _p, _p, _p, _i, _i, _i, C.POINTER(_i), C.POINTER(_i), C.POINTER(_i),
+                                  C.POINTER(_i), C.POINTER(_i), _p, _p, _p, _p, _p]),
 }
 
 for _name, (_res, _args) in SIGNATURES.items():

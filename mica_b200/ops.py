@@ -989,3 +989,60 @@ def stitch_cubes(cubes: torch.Tensor, ijk: torch.Tensor, cube_shape, grid_size: 
                                 X, Y, Z, _lib.int3(org), _lib.int3(ext), grid_size, padding,
                                 _dev(out, torch.float32, 'out'), _stream()), 'stitch_cubes')
     return out
+
+
+# ------------------------------------------------------------------ prediction maps
+#: the four volumes of ``StitchedVolumes.as_dict`` / ``CryoEMPredictor.run_prediction``
+VOLUME_KEYS = ('backbone_probability', 'carbon_alpha_probability', 'amino_acid_prediction', 'amino_acid_probability')
+
+
+def volumes_to_grid(vols, perm, working_shape, target_shape) -> dict:
+    """The four stitched volumes resampled onto a target grid (oracle/prediction_maps_oracle.py), in its memory order.
+
+    ``vols``: a ``StitchedVolumes`` or a mapping with the ``VOLUME_KEYS`` -- float32 CUDA tensors in cube space
+    ``[X, Y, Z]`` (``[20, X, Y, Z]`` for ``amino_acid_probability``) covering the whole cube space; the stitched
+    ``amino_acid_prediction`` is not read.  ``perm``: the map's ``MapHeader.transpose_order()[0]`` (cube axis a walks
+    memory axis perm[a]).  ``working_shape`` / ``target_shape``: memory shapes (nz, ny, nx) of the normalised map and of
+    the target grid (the input map's, or ``working_shape`` itself).  Returns float32 tensors ``[nz, ny, nx]`` (``[20,
+    nz, ny, nx]`` for ``amino_acid_probability``), views of one new 23-channel block laid out as ``StitchedVolumes``;
+    ``amino_acid_prediction`` is the arg-max of the 20 resampled probabilities.  One launch."""
+    org = ext = None
+    if isinstance(vols, StitchedVolumes):
+        org, ext = vols.org, vols.ext
+        cube_shape = vols.shape
+        vols = vols.as_dict()
+    missing = [k for k in VOLUME_KEYS if k not in vols]
+    if missing:
+        raise _lib.MicaError(f'volumes_to_grid: missing volumes {missing}')
+    bb = vols['backbone_probability']
+    if org is None:
+        cube_shape = tuple(bb.shape)
+    return _volumes_to_grid(bb, vols['carbon_alpha_probability'], vols['amino_acid_prediction'],
+                            vols['amino_acid_probability'], cube_shape, org, ext, perm, working_shape, target_shape)
+
+
+@device_guard
+def _volumes_to_grid(bb, ca, pred, prob, cube_shape, org, ext, perm, working_shape, target_shape):
+    ptrs = [_dev(t, torch.float32, name) for t, name in ((bb, 'backbone_probability'), (ca, 'carbon_alpha_probability'),
+                                                         (pred, 'amino_acid_prediction'),
+                                                         (prob, 'amino_acid_probability'))]
+    if len(cube_shape) != 3:
+        raise _lib.MicaError(f'volumes_to_grid: volumes must be [X, Y, Z], got {tuple(cube_shape)}')
+    X, Y, Z = (int(v) for v in cube_shape)
+    org = (0, 0, 0) if org is None else tuple(int(v) for v in org)
+    ext = (X, Y, Z) if ext is None else tuple(int(v) for v in ext)
+    for t, want, name in ((bb, ext, 'backbone_probability'), (ca, ext, 'carbon_alpha_probability'),
+                          (pred, ext, 'amino_acid_prediction'), (prob, (20,) + ext, 'amino_acid_probability')):
+        if tuple(t.shape) != want:
+            raise _lib.MicaError(f'volumes_to_grid: {name} has shape {tuple(t.shape)}, expected {want}')
+    target = tuple(int(v) for v in target_shape)
+    working = tuple(int(v) for v in working_shape)
+    if len(target) != 3 or min(target) < 1 or len(working) != 3:
+        raise _lib.MicaError(f'volumes_to_grid: bad target shape {tuple(target_shape)}')
+    n = target[0] * target[1] * target[2]
+    block = torch.empty(23 * n, dtype=torch.float32, device=bb.device)
+    out = StitchedVolumes.from_block(block, target, (0, 0, 0), target).as_dict()
+    check(lib.mica_volumes_to_grid(*ptrs, X, Y, Z, _lib.int3(org), _lib.int3(ext), _lib.int3(perm),
+                                   _lib.int3(working), _lib.int3(target),
+                                   *(C.c_void_p(out[k].data_ptr()) for k in VOLUME_KEYS), _stream()), 'volumes_to_grid')
+    return out

@@ -29,7 +29,7 @@ from collections.abc import Mapping
 import numpy as np
 import torch
 
-from . import ops, pdb, session
+from . import mrc, ops, pdb, session
 from ._lib import check, lib
 from .pipeline import (MapPipeline, _f32c, _SlabDrain, deal_cubes, run_model_chunks, shared_pipeline,
                        worker_batches, worker_pipeline)
@@ -39,6 +39,22 @@ MAP_TYPES = ('backbone_probability', 'carbon_alpha_probability', 'amino_acid_pre
 SMALL_VOLUMES = MAP_TYPES[:3]
 #: ``precision=`` / ``MICA_PRECISION`` -> the dtype of the cubes the model is given (None: float32)
 PRECISIONS = {'fp32': torch.float32, 'bf16': torch.bfloat16}
+#: ``save_maps=`` / ``MICA_SAVE_MAPS``: the grid the MRC prediction maps are written on
+SAVE_MAPS = ('input', 'working')
+
+
+def parse_save_maps(spec):
+    """``save_maps=`` / ``MICA_SAVE_MAPS`` -> 'input', 'working' or None (no maps).  None or '' -> None; 'input' /
+    'working' (any case, surrounding blanks ignored).  Anything else raises ValueError."""
+    if spec is None:
+        return None
+    if isinstance(spec, str):
+        key = spec.strip().lower()
+        if not key:
+            return None
+        if key in SAVE_MAPS:
+            return key
+    raise ValueError(f"save_maps must be None, 'input' or 'working', got {spec!r}")
 
 
 def parse_precision(spec):
@@ -97,6 +113,30 @@ def parse_devices(spec, n_visible: int, allow_repeats: bool = True):
     if not allow_repeats and len(set(out)) != len(out):
         raise ValueError(f'devices: {spec!r} lists a device twice')
     return out
+
+
+def map_file_names(kind):
+    """The MRC files ``save_maps`` writes for one of the ``MAP_TYPES``."""
+    if kind == 'amino_acid_probability':
+        return [f'{kind}_{c:02d}.mrc' for c in range(20)]
+    return [f'{kind}.mrc']
+
+
+def write_map_files(directory, kind, data, header):
+    """One kind of prediction map (host float32, target memory order; [20, nz, ny, nx] for the probabilities) as MRC
+    files in ``directory`` with the fields of ``header`` (a ``MapHeader``).  ``amino_acid_prediction`` is mode 0 (its
+    labels 0..19 are exact in int8), everything else mode 2."""
+    kw = dict(voxel_size=tuple(np.float32(v) for v in header.voxel_size),
+              origin=tuple(np.float32(v) for v in header.origin), mapc=int(header.mapc), mapr=int(header.mapr),
+              maps=int(header.maps), nxstart=int(header.nxstart), nystart=int(header.nystart),
+              nzstart=int(header.nzstart))
+    names = map_file_names(kind)
+    planes = data if kind == 'amino_acid_probability' else [data]
+    if len(planes) != len(names):
+        raise ValueError(f'{kind}: expected {len(names)} channel(s), got {len(planes)}')
+    dtype = np.int8 if kind == 'amino_acid_prediction' else np.float32
+    for name, plane in zip(names, planes):
+        mrc.write_mrc(os.path.join(directory, name), mrc.MrcMap(data=plane, **kw), dtype=dtype)
 
 
 class HostPool:
@@ -175,7 +215,7 @@ class CryoEMPredictor:
     def __init__(self, model_path, grids_path, output_path, save_output=True, device='cuda', quiet=False,
                  model=None, keep_on_device=True, host_volumes=None, host_pool=None, reference_batching=False,
                  super_batch=256, release_inputs=True, devices=None, *, overlap_window=None, tta=None,
-                 precision=None):
+                 precision=None, save_maps=None):
         """Additions to the reference signature (all optional):
 
         ``model``               an already loaded model (callable ``(exp_map, af_features) -> (bb, ca, aa)``).
@@ -221,7 +261,22 @@ class CryoEMPredictor:
                                 ``torch.autocast('cuda', dtype=torch.bfloat16)``, and its bfloat16 logits go to the
                                 stitch, which widens them exactly.  The volumes stay float32.  On every device of
                                 ``devices=``, with ``tta``, ``overlap_window`` and the per-cube files.  A bad value is
-                                logged and (False, {}) returned before any launch."""
+                                logged and (False, {}) returned before any launch.
+        ``save_maps``           (keyword only) None reads ``MICA_SAVE_MAPS`` when ``run_prediction`` is called (unset or
+                                empty: no maps).  'input': the four volumes are also written as MRC maps on the input
+                                map's grid -- its shape, voxel size, origin, mapc/mapr/maps and n*start -- so they
+                                overlay it voxel for voxel; 'working': on the 1 A working grid, with the header of
+                                ``resampled_normalized_map.mrc``.  Resampled trilinearly on the device
+                                (``ops.volumes_to_grid``; the label is the arg-max of the resampled probabilities) and
+                                written to ``reconstruction_path`` whatever ``save_output`` says:
+                                ``backbone_probability.mrc``, ``carbon_alpha_probability.mrc``,
+                                ``amino_acid_probability_00.mrc`` .. ``_19.mrc`` (mode 2) and ``amino_acid_prediction.mrc``
+                                (mode 0).  Needs the resident map GridCreator registers ('input': one that came through
+                                DataPreprocessor); otherwise, or for a bad value, it is logged and (False, {}) returned
+                                before any launch."""
+        self.save_maps = save_maps
+        self._maps_target = None                        # resolved by run_prediction: what the maps are written on
+        self.maps_timing = {}                           # seconds of the last map writing: kernel, download, write
         self.devices = devices
         self.precision = precision
         self._cube_dtype = torch.float32                # resolved from precision / MICA_PRECISION by run_prediction
@@ -709,6 +764,48 @@ class CryoEMPredictor:
             overlap[primary].finalize()
         return vols, self._download(vols)
 
+    # ------------------------------------------------------------------ prediction maps
+    def _resolve_maps_target(self):
+        """None when no maps are wanted, else (mode, perm, working shape, target shape, header) of the maps; MicaError
+        when they cannot be written (checked before any launch)."""
+        mode = parse_save_maps(os.environ.get('MICA_SAVE_MAPS') if self.save_maps is None else self.save_maps)
+        if mode is None:
+            return None
+        s = self._source
+        if s['kind'] != 'resident':
+            raise ops._lib.MicaError(f'save_maps={mode!r} needs the resident map GridCreator registers: the per-cube '
+                                     'grid files carry no map header')
+        m = s['map']
+        perm = tuple(int(v) for v in m['perm'])
+        working = tuple(int(v) for v in m['volume'].shape)
+        if mode == 'working':
+            return mode, perm, working, working, m['header']
+        src = session.get(m['source']) if m.get('source') is not None else None
+        if src is None or src.get('source_shape') is None:
+            raise ops._lib.MicaError("save_maps='input' needs the map to come through DataPreprocessor, which keeps the "
+                                     "input map's shape and header")
+        return mode, perm, working, tuple(src['source_shape']), src['source_header']
+
+    def _write_maps(self, vols):
+        """The MRC prediction maps of ``vols`` on the grid ``_maps_target`` names, one kind of volume in host memory at
+        a time.  Extra HBM: the 23 target-grid channels."""
+        _, perm, working, target, h = self._maps_target
+        t0 = time.time()
+        maps = ops.volumes_to_grid(vols, perm, working, target)
+        torch.cuda.synchronize(vols.device)
+        t1 = time.time()
+        os.makedirs(self.reconstruction_path, exist_ok=True)
+        down = write = 0.0
+        for k in MAP_TYPES:
+            ta = time.time()
+            host = maps.pop(k).cpu().numpy()
+            tb = time.time()
+            write_map_files(self.reconstruction_path, k, host, h)
+            down += tb - ta
+            write += time.time() - tb
+            del host
+        self.maps_timing = {'kernel': t1 - t0, 'download': down, 'write': write}
+
     def _release(self):
         s = self._source or {}
         if s.get('kind') != 'resident':
@@ -729,8 +826,10 @@ class CryoEMPredictor:
             self._tta_codes()                                    # a bad tta is refused before any launch
             self._cube_dtype = self._resolve_precision()         # so is a bad precision
             self._workers = self._resolve_workers()
+            parse_save_maps(os.environ.get('MICA_SAVE_MAPS') if self.save_maps is None else self.save_maps)
             if not self.select_processing_strategy():
                 return False, {}
+            self._maps_target = self._resolve_maps_target()      # refused before any launch
             if not self.load_model():
                 return False, {}
             t0 = time.time()
@@ -744,11 +843,14 @@ class CryoEMPredictor:
             for k, v in vols.as_dict().items():
                 volumes[k] = out_host[k].numpy() if k in out_host else DeviceVolume(v)
             self.timing_stats['reconstruction'] = time.time() - t0
+            t0 = time.time()
             if self.save_output:
-                t0 = time.time()
                 os.makedirs(self.reconstruction_path, exist_ok=True)
                 for k in MAP_TYPES:
                     np.save(f'{self.reconstruction_path}/{k}.npy', np.asarray(volumes[k]))
+            if self._maps_target is not None:
+                self._write_maps(vols)
+            if self.save_output or self._maps_target is not None:
                 self.timing_stats['saving'] = time.time() - t0
             if self.release_inputs:
                 self._release()

@@ -127,7 +127,8 @@ class DataPreprocessor:
                         nzstart=m.nzstart))
                 pipe.header = out_header
                 session.put(out_path, kind='normalized_map', volume=pipe.normalized, header=out_header,
-                            median=pipe.median, p999=pipe.p999, pipe=pipe)
+                            median=pipe.median, p999=pipe.p999, pipe=pipe,
+                            source_shape=tuple(int(v) for v in m.data.shape), source_header=header)
                 self.normalized_map_path = out_path
                 success = True
             else:
