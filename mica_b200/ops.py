@@ -745,44 +745,6 @@ def zero_cores(ijk: torch.Tensor, vols: StitchedVolumes, grid_size: int = 48):
     return vols
 
 
-class StitchCall:
-    """``postproc_stitch`` bound to one set of volumes and one geometry: everything that does not change from
-    batch to batch (volume pointers, box, shapes) is converted to ctypes once, so the per-call host cost is a
-    handful of microseconds -- the drop-in feeds the model in the reference's batches of <= 8 cubes, i.e.
-    hundreds of stitch calls per map.  The caller guarantees CUDA contiguous logits, all float32 or all bfloat16, on
-    the volumes' device (checked on the first call and whenever the batch size or the dtype changes)."""
-
-    def __init__(self, vols: 'StitchedVolumes', grid_size: int = 48, padding: int = 8):
-        self.vols, self.grid_size, self.padding = vols, int(grid_size), int(padding)
-        self.W = self.grid_size + 2 * self.padding
-        X, Y, Z = vols.shape
-        self._fixed = (X, Y, Z, _lib.int3(vols.org), _lib.int3(vols.ext), self.grid_size, self.padding,
-                       _dev(vols.backbone_probability, torch.float32, 'bb_vol'),
-                       _dev(vols.carbon_alpha_probability, torch.float32, 'ca_vol'),
-                       _dev(vols.amino_acid_probability, torch.float32, 'aa_prob_vol'),
-                       _dev(vols.amino_acid_prediction, torch.float32, 'aa_pred_vol'))
-        self._checked = None            # (B, dtype) of the last checked call
-        self._code = _lib.DTYPE_F32
-        self._dev_index = vols.device.index
-
-    def __call__(self, bb, ca, aa, ijk):
-        B = ijk.shape[0]
-        if (B, bb.dtype) != self._checked:
-            _, self._code = _logits(bb, ca, aa, B, self.W)
-            for t, name in ((bb, 'bb'), (ca, 'ca'), (aa, 'aa')):
-                if t.device != self.vols.device:
-                    raise _lib.MicaError(f'{name} logits live on {t.device}, the volumes on {self.vols.device}')
-            _dev(ijk, torch.int32, 'ijk')
-            self._checked = (B, bb.dtype)
-        if torch.cuda.current_device() != self._dev_index:
-            with torch.cuda.device(self._dev_index):
-                return self(bb, ca, aa, ijk)
-        X, Y, Z, org, ext, gs, pad, p_bb, p_ca, p_aap, p_aapred = self._fixed
-        check(lib.mica_postproc_stitch_as(bb.data_ptr(), ca.data_ptr(), aa.data_ptr(), self._code, ijk.data_ptr(), B,
-                                          X, Y, Z, org, ext, gs, pad, p_bb, p_ca, p_aap, p_aapred,
-                                          torch.cuda.current_stream().cuda_stream), 'postproc_stitch')
-
-
 @device_guard
 def postproc_stitch_peer(bb: torch.Tensor, ca: torch.Tensor, aa: torch.Tensor, ijk: torch.Tensor, cube_shape,
                          owner_table: torch.Tensor, x_bounds, grid_size: int = 48, padding: int = 8):
@@ -823,6 +785,23 @@ def overlap_window(kind, grid_size: int, padding: int) -> np.ndarray:
     else:
         raise _lib.MicaError(f"window must be 'core', 'uniform', 'triangle' or an array, got {kind!r}")
     return w.astype(np.float32)
+
+
+def stitch_mode(window, tta, grid_size: int, padding: int):
+    """(w1, codes) of a stitch, every argument validated before any launch.  ``w1``: the weights of the overlap-weighted
+    stitch (``overlap_window``), or None for the reference's paste of the cube cores; ``codes``: the orientations of a
+    test-time augmentation (``tta_orientations``), or None.  ``tta`` None or (0,) is no augmentation.  Without it,
+    ``window`` None or 'core' is the paste (the 1-on-the-core weighted stitch IS the paste, and runs as one).  Under it
+    the window defaults to 'core' and every window, 'core' included, runs in fixed point."""
+    codes = tta_orientations(tta)
+    if codes == (0,):
+        codes = None
+    if window is None and codes is None:
+        return None, None
+    w1 = overlap_window('core' if window is None else window, grid_size, padding)
+    if codes is None and is_core_window(w1, grid_size, padding):
+        return None, None
+    return w1, codes
 
 
 def is_core_window(w1, grid_size: int, padding: int) -> bool:
@@ -869,106 +848,149 @@ def peer_atomics_supported(device: int, peer_device: int) -> bool:
 
 
 class OverlapOwners(NamedTuple):
-    """Where the contributions of an overlap-weighted stitch go when the output is split over ranks: rank r owns
-    planes [bounds[r], bounds[r+1]) of cube axis ``axis`` (0 = x, 2 = k) as the 23-channel block at ``table[r]``
-    (int64 device tensor of base pointers, ``peer.PeerVolumes.table``); ``devices``: the CUDA device index of each
-    owner, whose memory the accumulating device must be able to add into atomically."""
+    """Where a stitch (paste or weighted) stores when the output is split over ranks: rank r owns planes
+    [bounds[r], bounds[r+1]) of cube axis ``axis`` (0 = x, 2 = k) as the 23-channel block at ``table[r]`` (int64 device
+    tensor of base pointers, ``peer.PeerVolumes.table``); ``devices``: the CUDA device index of each owner, whose
+    memory the weighted stitch must be able to add into atomically."""
     table: torch.Tensor
     axis: int
     bounds: tuple
     devices: tuple
 
 
-class OverlapStitcher:
-    """The north_star's "stitch with overlap weights": every voxel of every window adds its probabilities times
-    the window weight, normalised by the weight sum of the full cube lattice, in 2^-31 fixed point (uint32), so the
-    result does not depend on the order of the cubes, the batches or the partition; ``finalize`` converts in place.
-    NOT the reference's arithmetic, which pastes the disjoint cores (``postproc_stitch``; DESIGN.md D2) -- offered
-    as a mode next to it; ``window='core'`` runs that paste.  Costs several times the reference mode: every voxel of
-    every 64^3 window is post-processed and added, not just the 32^3 (48^3) cores.
+class Stitcher:
+    """The stitch of one map's batches of logits, its mode and destination bound once (``stitch_mode``).
 
-    ``vols``: the volumes (``StitchedVolumes.from_block``, zeroed) this stitcher finalizes; default: a whole-map
-    block of its own.  ``owners``: an ``OverlapOwners`` table -- contributions go to the block of the rank that
-    owns their plane, locally or over NVLink (native peer atomics required); without ``vols`` such a stitcher only
-    accumulates.
+    The paste: the reference's softmax/argmax and paste of the disjoint cube cores (``postproc_stitch``), final batch
+    by batch (``per_batch``).  The weighted stitch, the north_star's "stitch with overlap weights": every voxel of every
+    window adds its probabilities times the window weight, normalised by the weight sum of the full cube lattice, in
+    2^-31 fixed point (uint32), so the result does not depend on the order of the cubes, the batches or the partition;
+    ``finalize`` converts in place.  NOT the reference's arithmetic (DESIGN.md D2), and several times its cost: every
+    voxel of every 64^3 window is post-processed and added, not just the 32^3 (48^3) cores.  ``tta``: test-time
+    augmentation; every window is stitched once per orientation (``orientations``), from the logits of the model run on
+    the window in that orientation, and the result is the average over the k orientations (the 1/k is in the
+    normaliser tables) -- always the weighted stitch.
 
-    ``tta``: test-time augmentation (``tta_orientations``): every window is accumulated once per orientation, from
-    the logits of the model run on the window in that orientation (``accumulate(..., orient=)``), and the result is
-    the average over the k orientations -- the 1/k is in the normaliser tables.  Any window, 'core' included, then
-    runs in fixed point (orientations (0,) alone are the plain stitch).  NOT the reference's arithmetic either."""
+    ``vols``: the volumes on ``device`` it stores into; the weighted stitch needs ``StitchedVolumes.from_block``
+    volumes, zeroed.  ``owners``: a ``OverlapOwners`` table -- every core plane (paste, along cube axis 0, plain stores)
+    or window contribution (weighted, along axis 0 or 2, native peer atomics required) goes to the block of the rank
+    that owns its plane, locally or over NVLink; ``vols`` is then this rank's own box, if any.  Default: a zeroed
+    whole-map block of its own."""
 
-    def __init__(self, cube_shape, device, grid_size: int = 48, padding: int = 8, window='uniform', *, vols=None,
-                 owners: OverlapOwners | None = None, tta=None):
+    def __init__(self, cube_shape, device, grid_size: int = 48, padding: int = 8, window=None, *, tta=None, vols=None,
+                 owners: OverlapOwners | None = None):
         self.shape = tuple(int(v) for v in cube_shape)
         self.device = torch.device(device)
         if self.device.index is None:
             self.device = torch.device('cuda', torch.cuda.current_device())
         self.grid_size, self.padding = int(grid_size), int(padding)
-        self.w1 = overlap_window(window, grid_size, padding)
-        self.orientations = tta_orientations(tta) or (0,)
-        self.core = is_core_window(self.w1, self.grid_size, self.padding) and self.orientations == (0,)
-        self.owners = owners
+        self.w1, codes = stitch_mode(window, tta, grid_size, padding)
+        #: the paste: the volumes are final batch by batch; the weighted stitch: after ``finalize``
+        self.per_batch = self.w1 is None
+        #: the orientations the batches come in: (0,) without test-time augmentation
+        self.orientations = codes or (0,)
         if owners is not None:
-            if owners.axis not in (0, 2) or (self.core and owners.axis != 0):
+            if owners.axis not in ((0,) if self.per_batch else (0, 2)):
                 raise _lib.MicaError(f'owners along cube axis {owners.axis}: the weighted stitch splits along 0 or 2, '
-                                     'the core window (the paste) along 0')
-            for d in owners.devices:
+                                     'the paste along 0')
+            for d in () if self.per_batch else owners.devices:
                 if not peer_atomics_supported(self.device.index, d):
                     raise _lib.MicaError(f'overlap-weighted stitching over several GPUs adds into the owners\' '
                                          f'memory atomically: cuda:{self.device.index} has no native peer atomics '
                                          f'with cuda:{d}')
-            self._bounds = (C.c_int * len(owners.bounds))(*[int(v) for v in owners.bounds])
+        X, Y, Z = self.shape
         if vols is None and owners is None:
-            X, Y, Z = self.shape
             with torch.cuda.device(self.device):
-                vols = StitchedVolumes.from_block(torch.zeros(23 * X * Y * Z, dtype=torch.float32,
-                                                              device=self.device), self.shape, (0, 0, 0), self.shape)
-        if vols is not None and (getattr(vols, 'block', None) is None or vols.device != self.device):
-            raise _lib.MicaError('OverlapStitcher needs volumes of StitchedVolumes.from_block on its own device')
+                vols = StitchedVolumes.from_block(torch.zeros(23 * X * Y * Z, dtype=torch.float32, device=self.device),
+                                                  self.shape, (0, 0, 0), self.shape)
+        if vols is not None and _cuda_device_of(vols) != self.device:
+            raise _lib.MicaError(f'the volumes live on {vols.device}, the stitcher on {self.device}')
+        if vols is not None and not self.per_batch and getattr(vols, 'block', None) is None:
+            raise _lib.MicaError('the weighted stitch needs volumes of StitchedVolumes.from_block')
         self.vols = vols
-        if not self.core:
+        # the arguments that do not change from batch to batch, converted to ctypes once: the drop-in feeds the model
+        # in the reference's batches of <= 8 cubes, i.e. hundreds of stitch calls per map
+        gs, pad = self.grid_size, self.padding
+        if owners is not None:
+            table = _dev(owners.table, torch.int64, 'owner_table')
+            bounds = (C.c_int * len(owners.bounds))(*[int(v) for v in owners.bounds])
+            world = int(owners.table.numel())
+        if self.per_batch and owners is None:
+            self._fn, self._what = lib.mica_postproc_stitch_as, 'postproc_stitch'
+            self._head, self._tail = (X, Y, Z, _lib.int3(vols.org), _lib.int3(vols.ext), gs, pad,
+                                      _dev(vols.backbone_probability, torch.float32, 'bb_vol'),
+                                      _dev(vols.carbon_alpha_probability, torch.float32, 'ca_vol'),
+                                      _dev(vols.amino_acid_probability, torch.float32, 'aa_prob_vol'),
+                                      _dev(vols.amino_acid_prediction, torch.float32, 'aa_pred_vol')), ()
+        elif self.per_batch:
+            self._fn, self._what = lib.mica_postproc_stitch_peer_as, 'postproc_stitch_peer'
+            self._head, self._tail = (X, Y, Z, gs, pad, table, bounds, world), ()
+        else:
             with torch.cuda.device(self.device):
                 self.norm = torch.from_numpy(np.concatenate(
-                    overlap_norm_tables(self.w1, self.shape, self.grid_size, self.padding,
-                                        len(self.orientations)))).to(self.device)
+                    overlap_norm_tables(self.w1, self.shape, gs, pad, len(self.orientations)))).to(self.device)
+            self._head = (X, Y, Z, gs, pad, self.w1.ctypes.data_as(C.POINTER(C.c_float)),
+                          C.c_void_p(self.norm.data_ptr()))
+            if owners is None:
+                self._fn, self._what = lib.mica_overlap_accumulate_fixed_as, 'overlap_accumulate'
+                self._tail = (C.c_void_p(vols.block.data_ptr()),)
+            else:
+                self._fn, self._what = lib.mica_overlap_accumulate_fixed_peer_as, 'overlap_accumulate_peer'
+                self._tail = (table, int(owners.axis), bounds, world)
+        self._checked = None            # (B, dtype) of the last checked call
+        self._code = _lib.DTYPE_F32
         self._done = False
 
-    @device_guard
-    def accumulate(self, bb, ca, aa, ijk, vols=None, orient: int = 0):
-        """Add one batch of logits, those of the windows ``ijk`` in orientation ``orient`` (one of ``tta``); all float32
-        or all bfloat16 (widened exactly on load: the sums equal the float32 call on ``logits.float()``)."""
-        if _orientation_arg(orient) not in self.orientations:
-            raise _lib.MicaError(f'orientation {orient} is not one of this stitcher\'s {list(self.orientations)}')
-        if self.core:
-            if self.owners is not None:
-                postproc_stitch_peer(bb, ca, aa, ijk, self.shape, self.owners.table, self.owners.bounds,
-                                     self.grid_size, self.padding)
-            else:
-                postproc_stitch(bb, ca, aa, ijk, self.vols, self.grid_size, self.padding)
-            return
-        B = ijk.shape[0]
-        W = self.grid_size + 2 * self.padding
-        ptrs, code = _logits(bb, ca, aa, B, W)
-        X, Y, Z = self.shape
-        args = (*ptrs, code, _dev(ijk, torch.int32, 'ijk'), B, X, Y, Z, self.grid_size, self.padding,
-                self.w1.ctypes.data_as(C.POINTER(C.c_float)), C.c_void_p(self.norm.data_ptr()), int(orient))
-        if self.owners is None:
-            check(lib.mica_overlap_accumulate_fixed_as(*args, C.c_void_p(self.vols.block.data_ptr()), _stream()),
-                  'overlap_accumulate')
-        else:
-            o = self.owners
-            check(lib.mica_overlap_accumulate_fixed_peer_as(
-                *args, _dev(o.table, torch.int64, 'owner_table'), int(o.axis), self._bounds, int(o.table.numel()),
-                _stream()), 'overlap_accumulate_peer')
+    @staticmethod
+    def kernel_logits(bb, ca, aa):
+        """Logits as the stitch kernels take them: contiguous, all float32 or all bfloat16.  Float32 and bfloat16 pass
+        through (the kernels widen bfloat16 exactly); any other dtype, or a mix, becomes float32."""
+        dt = bb.dtype
+        if dt not in MODEL_DTYPES or ca.dtype != dt or aa.dtype != dt:
+            bb, ca, aa = bb.float(), ca.float(), aa.float()
+        return bb.contiguous(), ca.contiguous(), aa.contiguous()
 
-    @device_guard
+    def __call__(self, bb, ca, aa, ijk, orient=0):
+        """Stitch one batch of logits, those of the windows ``ijk`` (int32 [B,3]) in orientation ``orient`` (one of
+        ``orientations``), as the model gives them (``kernel_logits``).  The logits and ``ijk`` are checked on the
+        first call and whenever the batch size or the dtype changes."""
+        if self.per_batch:
+            if orient:
+                raise _lib.MicaError(f'the paste stitches orientation 0 only, got {orient!r}')
+        elif _orientation_arg(orient) not in self.orientations:
+            raise _lib.MicaError(f'orientation {orient} is not one of this stitcher\'s {list(self.orientations)}')
+        bb, ca, aa = self.kernel_logits(bb, ca, aa)
+        B = ijk.shape[0]
+        if (B, bb.dtype) != self._checked:
+            _, self._code = _logits(bb, ca, aa, B, self.grid_size + 2 * self.padding)
+            _dev(ijk, torch.int32, 'ijk')
+            for t, name in ((bb, 'bb'), (ca, 'ca'), (aa, 'aa'), (ijk, 'ijk')):
+                if t.device != self.device:
+                    raise _lib.MicaError(f'{name} lives on {t.device}, the stitcher on {self.device}')
+            self._checked = (B, bb.dtype)
+        if torch.cuda.current_device() != self.device.index:
+            with torch.cuda.device(self.device):
+                return self(bb, ca, aa, ijk, orient)
+        args = (bb.data_ptr(), ca.data_ptr(), aa.data_ptr(), self._code, ijk.data_ptr(), B, *self._head)
+        if not self.per_batch:
+            args += (int(orient), *self._tail)
+        check(self._fn(*args, torch.cuda.current_stream().cuda_stream), self._what)
+
+    def clear_cores(self, ijk):
+        """The cubes ``ijk`` (int32 [n,3]) a keep rule skipped (``select_cubes``): the paste sets their cores to 0 in
+        ``vols``, which may hold an earlier map; the weighted stitch adds nothing for them."""
+        if self.per_batch and self.vols is not None and len(ijk):
+            zero_cores(torch.as_tensor(ijk).to(self.device), self.vols, self.grid_size)
+
     def finalize(self) -> StitchedVolumes:
-        """The four volumes (views of the accumulation block, laid out as ``StitchedVolumes.from_block``).  With
-        owners, call it once every rank's contributions have landed (stream sync + barrier)."""
+        """The four volumes: ``vols`` (for the weighted stitch, converted in place from fixed point).  With owners,
+        call it once every rank's contributions have landed (stream sync + barrier)."""
+        if self.per_batch or self._done:
+            return self.vols
         if self.vols is None:
-            raise _lib.MicaError('this OverlapStitcher only accumulates into other ranks\' volumes')
-        if not self._done and not self.core:
-            e = self.vols.ext
+            raise _lib.MicaError('this Stitcher only adds into other ranks\' volumes')
+        e = self.vols.ext
+        with torch.cuda.device(self.device):
             check(lib.mica_overlap_finalize_fixed(C.c_void_p(self.vols.block.data_ptr()), e[0] * e[1] * e[2],
                                                   _stream()), 'overlap_finalize')
         self._done = True

@@ -109,19 +109,13 @@ def _on_device(method):
 
 D8_MODES = ('none', 'split', 'reference')
 
-
-def _f32c(*logits):
-    """Logits as the stitch kernels take them: contiguous, all float32 or all bfloat16.  Float32 and bfloat16 pass
-    through (the kernels widen bfloat16 exactly); any other dtype, or a mix, becomes float32.  A no-op for tensors that
-    already are what the kernels take."""
-    dt = logits[0].dtype
-    keep = dt in ops.MODEL_DTYPES and all(t.dtype == dt for t in logits)
-    return tuple((t if keep else t.float()).contiguous() for t in logits)
+#: the logits hand-off of the stitch (``ops.Stitcher.kernel_logits``), importable from here as before
+_f32c = ops.Stitcher.kernel_logits
 
 
 def run_model_chunks(model_fn, x, af, flags_host, ijk, stitch, model_batch=None, d8='none'):
     """Feed one super-batch of cubes to ``model_fn`` the way the reference feeds MICA.forward, and hand
-    every result to ``stitch(bb, ca, aa, ijk_chunk)``.
+    every result to ``stitch(bb, ca, aa, ijk_chunk)`` (an ``ops.Stitcher``, or a function calling one).
 
     ``model_batch``: cubes per model call (the reference: 1 up to 200 cubes, else <= 8,
     utils/predict.py:156-215); None = the whole super-batch in one call.
@@ -438,8 +432,8 @@ class MapPipeline:
     # ---------------------------------------------------------------- stage 5 (+model)
     @_on_device
     def predict_and_stitch(self, model_fn, vols: ops.StitchedVolumes | None = None, on_batch=None, *,
-                           model_batch=None, d8='none', order=None, stitch_fn=None, overlap_window=None,
-                           batches=None, tta=None, min_max=None):
+                           model_batch=None, d8='none', order=None, overlap_window=None, batches=None, tta=None,
+                           min_max=None, stitcher: ops.Stitcher | None = None):
         """run_inference + reconstruct_volume (utils/predict.py:307-587) without the
         per-cube files.  ``model_fn(exp_map, af_features) -> (bb, ca, aa)`` logits, enqueued
         on the current stream.  With ``prefetch`` the cubes of batch n+1 are cut on a side
@@ -451,11 +445,9 @@ class MapPipeline:
         such a super-batch is fed to the model (``run_model_chunks``: the reference's batches of <= 8 and
         its whole-batch zero-AF3 test, D8).  ``order``: a permutation of the cube indices (the reference
         visits cubes in ``glob`` order, utils/predict.py:269); default = the i-major loop order of
-        utils/create_grids.py:143-145.  ``stitch_fn(bb, ca, aa, ijk, vols)`` replaces the local
-        softmax/argmax + stitch (multi-GPU: cores owned by another rank go to its volumes).
-        ``overlap_window`` ('uniform' | 'triangle' | 'core' | W weights): the north_star's overlap-weighted
-        stitching instead of the reference's centre-crop paste (``ops.OverlapStitcher``; NOT the reference's
-        arithmetic, see DESIGN.md D2; 'core' is the paste).  Nothing is final before the last batch, so
+        utils/create_grids.py:143-145.  ``overlap_window`` ('uniform' | 'triangle' | 'core' | W weights): the
+        north_star's overlap-weighted stitching instead of the reference's centre-crop paste (``ops.Stitcher``; NOT
+        the reference's arithmetic, see DESIGN.md D2; 'core' is the paste).  Nothing is final before the last batch, so
         ``on_batch`` is then called once, with the finished volumes.  A split map (subclasses) supplies the owners
         of the output; its volumes are final after ``finish_map()``.  ``batches``: the super-batches as
         (b0, b1) ranges of the (ordered) cube list, each at most ``batch_cubes`` long, instead of the even cut
@@ -464,10 +456,13 @@ class MapPipeline:
         ``tta`` ('flips' | 'rot90' | 'all' | orientation codes, ``ops.tta_orientations``): test-time augmentation.
         Every super-batch is cut, run through the model and accumulated once per orientation, and the volumes are
         the average of the k orientations' probabilities (window weights ``overlap_window``, default 'core'), always
-        in the order-free fixed point of ``ops.OverlapStitcher`` -- NOT the reference's arithmetic.  The work list is
+        in the order-free fixed point of ``ops.Stitcher`` -- NOT the reference's arithmetic.  The work list is
         the (super-batch, orientation) pairs, fed through the same two-slot prefetch.  ``on_batch`` is called once,
-        with the finished volumes.  A ``stitch_fn`` then takes a sixth argument, the orientation of the logits.
-        ``tta=[0]`` is ``tta=None``.
+        with the finished volumes.  ``tta=[0]`` is ``tta=None``.
+
+        ``stitcher``: an ``ops.Stitcher`` whose destination the caller owns (several workers adding into one map),
+        instead of ``vols`` / ``overlap_window`` / ``tta``; the caller finalizes it, and ``on_batch`` runs only for the
+        paste.  Returns its ``vols``.
 
         ``min_max`` (a finite number; None = every cube): the keep rule of the reference's training grids
         (create_grids_for_normalized_map.py:78) at inference -- only cubes whose window maximum is not below it
@@ -478,33 +473,20 @@ class MapPipeline:
         cube kept: zero volumes, the model is not called."""
         if self.normalized is None:
             raise MicaError('no normalised map')
-        codes = ops.tta_orientations(tta)                                          # refused before any launch
+        if stitcher is not None and (vols is not None or overlap_window is not None or tta is not None):
+            raise MicaError('a stitcher brings its own volumes, window and orientations: pass it alone')
+        w1, codes = ops.stitch_mode(overlap_window, tta, self.grid_size, self.padding)   # refused before any launch
         min_max = ops.check_min_max(min_max)
-        if codes == (0,):
-            codes = None
-        overlap = None
-        if overlap_window is not None or codes is not None:
-            w1 = ops.overlap_window('core' if overlap_window is None else overlap_window, self.grid_size, self.padding)
-            if codes is not None or not ops.is_core_window(w1, self.grid_size, self.padding):    # 'core' IS the paste
-                if stitch_fn is not None and codes is None:
-                    raise MicaError('overlap_window replaces the stitch: pass stitch_fn or overlap_window, not both')
-                overlap = w1 if stitch_fn is None else None
         self.cube_index()
         # an ascending order is a subsequence of the loop order: finished layers can still be drained (_SlabDrain)
         self._custom_order = order is not None and not bool(np.all(np.diff(np.asarray(order, dtype=np.int64)) > 0))
         skipped = None
         if min_max is not None:
             order, skipped = self._keep_rule(min_max, order)
-        final_on_batch = None
-        if overlap is not None:
-            overlap = self._overlap_stitcher(overlap, vols, codes)
-            stitch_fn, vols = overlap.accumulate, overlap.vols
-        if overlap is not None or codes is not None:
-            final_on_batch, on_batch = on_batch, None
-        if vols is None:
-            vols = self._new_volumes()                    # zero: skipped cores need nothing
-        elif skipped is not None and overlap is None and len(skipped):
-            ops.zero_cores(torch.from_numpy(skipped).to(self.device), vols, self.grid_size)
+        st = self._make_stitcher(w1, codes, vols) if stitcher is None else stitcher
+        if skipped is not None and vols is not None:      # new volumes are zero: skipped cores need nothing
+            st.clear_cores(skipped)
+        vols = st.vols
         if order is not None:
             order = np.asarray(order, dtype=np.int64)
             self._set_cube_origins(self.ijk_host[order], ('ordered', id(order), len(order)))
@@ -516,32 +498,18 @@ class MapPipeline:
             batches = [(int(b0), int(b1)) for b0, b1 in batches]
             if any(not 0 <= b0 < b1 <= n or b1 - b0 > self.batch_cubes for b0, b1 in batches):
                 raise MicaError(f'batches must be non-empty ranges of the {n} cubes, at most {self.batch_cubes} long')
-        if not batches:                                   # no cube kept (min_max)
-            if on_batch is not None:
-                on_batch(vols, n)
-            return self._predict_done(overlap, final_on_batch, vols, n)
-        work = [(b0, b1, 0) for b0, b1 in batches] if codes is None else \
-            [(b0, b1, g) for b0, b1 in batches for g in codes]
+        work = [(b0, b1, g) for b0, b1 in batches for g in st.orientations]
+        per_batch = on_batch if st.per_batch else None
         want_flags = d8 == 'split' and (model_batch is None or int(model_batch) > 1)
-        if stitch_fn is None:
-            bound = ops.StitchCall(vols, self.grid_size, self.padding)
-
-            def stitch_fn(bb, ca, aa, ijk, vols_):
-                bound(bb, ca, aa, ijk)
         timed = self.timer is not _no_timer
 
-        orient_arg = () if codes is None else (0,)
-
         def consume(cur, b0, b1, g):
-            extra = orient_arg and (g,)
-
             def stitch(bb, ca, aa, ijk):
-                bb, ca, aa = _f32c(bb, ca, aa)
                 if timed:
                     with self.timer('postproc_stitch'):
-                        stitch_fn(bb, ca, aa, ijk, vols, *extra)
+                        st(bb, ca, aa, ijk, g)
                 else:
-                    stitch_fn(bb, ca, aa, ijk, vols, *extra)
+                    st(bb, ca, aa, ijk, g)
             flags = None
             if want_flags:
                 x, af, nzf = cur
@@ -550,44 +518,46 @@ class MapPipeline:
                 x, af = cur[0], cur[1]
             run_model_chunks(model_fn, x, af, flags, self.ijk[b0:b1], stitch, model_batch, d8)
 
-        if not self.prefetch or len(work) == 1:
+        if not work:                                      # no cube kept (min_max)
+            if per_batch is not None:
+                per_batch(vols, n)
+        elif not self.prefetch or len(work) == 1:
             for b0, b1, g in work:
                 consume(self.extract_batch(b0, b1, want_flags=want_flags, orient=g), b0, b1, g)
-                if on_batch is not None:
-                    on_batch(vols, b1)
-            return self._predict_done(overlap, final_on_batch, vols, n)
+                if per_batch is not None:
+                    per_batch(vols, b1)
+        else:
+            t_enqueue = time.perf_counter()
+            main = torch.cuda.current_stream(self.device)
+            if self._pre_stream is None:
+                self._pre_stream = torch.cuda.Stream(self.device)
+            pre = self._pre_stream
+            pre.wait_stream(main)                    # normalised map, atom bins, ijk are produced on `main`
+            ready, consumed = [None, None], [None, None]
 
-        t_enqueue = time.perf_counter()
-        main = torch.cuda.current_stream(self.device)
-        if self._pre_stream is None:
-            self._pre_stream = torch.cuda.Stream(self.device)
-        pre = self._pre_stream
-        pre.wait_stream(main)                    # normalised map, atom bins, ijk are produced on `main`
-        ready, consumed = [None, None], [None, None]
+            def cut(i):
+                slot = i & 1
+                with torch.cuda.stream(pre):
+                    if consumed[slot] is not None:
+                        pre.wait_event(consumed[slot])           # the model has read this buffer's last batch
+                    b0, b1, g = work[i]
+                    out = self.extract_batch(b0, b1, want_flags=want_flags, slot=slot, orient=g)
+                    ready[slot] = torch.cuda.Event()
+                    ready[slot].record(pre)
+                return out
 
-        def cut(i):
-            slot = i & 1
-            with torch.cuda.stream(pre):
-                if consumed[slot] is not None:
-                    pre.wait_event(consumed[slot])           # the model has read this buffer's last batch
-                b0, b1, g = work[i]
-                out = self.extract_batch(b0, b1, want_flags=want_flags, slot=slot, orient=g)
-                ready[slot] = torch.cuda.Event()
-                ready[slot].record(pre)
-            return out
-
-        cur = cut(0)
-        for i, (b0, b1, g) in enumerate(work):
-            nxt = cut(i + 1) if i + 1 < len(work) else None
-            main.wait_event(ready[i & 1])
-            consume(cur, b0, b1, g)
-            consumed[i & 1] = torch.cuda.Event()
-            consumed[i & 1].record(main)
-            if on_batch is not None:
-                on_batch(vols, b1)
-            cur = nxt
-        self.last_loop_enqueue_ms = (time.perf_counter() - t_enqueue) * 1e3     # host side of the batch loop
-        return self._predict_done(overlap, final_on_batch, vols, n)
+            cur = cut(0)
+            for i, (b0, b1, g) in enumerate(work):
+                nxt = cut(i + 1) if i + 1 < len(work) else None
+                main.wait_event(ready[i & 1])
+                consume(cur, b0, b1, g)
+                consumed[i & 1] = torch.cuda.Event()
+                consumed[i & 1].record(main)
+                if per_batch is not None:
+                    per_batch(vols, b1)
+                cur = nxt
+            self.last_loop_enqueue_ms = (time.perf_counter() - t_enqueue) * 1e3     # host side of the batch loop
+        return vols if stitcher is not None else self._stitch_done(st, on_batch, n)
 
     def _window_max(self, ijk):
         """Window maxima of the cubes ``ijk`` (device int32 [B,3]) on this pipeline's normalised map."""
@@ -606,21 +576,18 @@ class MapPipeline:
         order = np.asarray(order, dtype=np.int64)
         return order[mask[order]], skipped
 
-    def _predict_done(self, overlap, on_batch, vols, n):
-        if overlap is not None:
-            return self._overlap_done(overlap, on_batch, n)
-        if on_batch is not None:              # test-time augmentation into a caller's stitch_fn
-            on_batch(vols, n)
-        return vols
+    def _make_stitcher(self, w1, codes, vols):
+        """The ``ops.Stitcher`` of this map (``ops.stitch_mode``'s ``w1`` / ``codes``): the whole map on this GPU, into
+        ``vols`` -- for the weighted stitch ``StitchedVolumes.from_block`` volumes of the whole map, zeroed.  Default:
+        new zeroed volumes (the weighted stitch: a block of its own)."""
+        if vols is None and w1 is None:
+            vols = self._new_volumes()
+        return ops.Stitcher(self.cube_shape, self.device, self.grid_size, self.padding, w1, tta=codes, vols=vols)
 
-    def _overlap_stitcher(self, w1, vols, tta=None):
-        """The accumulator of an overlap-weighted map: the whole map in one block on this GPU (``vols``, if given,
-        must be ``StitchedVolumes.from_block`` volumes of the whole map, zeroed)."""
-        return ops.OverlapStitcher(self.cube_shape, self.device, self.grid_size, self.padding, w1, vols=vols, tta=tta)
-
-    def _overlap_done(self, overlap, on_batch, n):
-        vols = overlap.finalize()
-        if on_batch is not None:
+    def _stitch_done(self, st, on_batch, n):
+        """The volumes once every batch has been stitched; ``on_batch`` once if they were not final batch by batch."""
+        vols = st.finalize()
+        if on_batch is not None and not st.per_batch:
             on_batch(vols, n)
         return vols
 

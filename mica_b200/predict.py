@@ -31,8 +31,8 @@ import torch
 
 from . import mrc, ops, pdb, session
 from ._lib import check, lib
-from .pipeline import (MapPipeline, _f32c, _SlabDrain, deal_cubes, run_model_chunks, shared_pipeline,
-                       worker_batches, worker_pipeline)
+from .pipeline import (MapPipeline, _SlabDrain, deal_cubes, run_model_chunks, shared_pipeline, worker_batches,
+                       worker_pipeline)
 
 MAP_TYPES = ('backbone_probability', 'carbon_alpha_probability', 'amino_acid_prediction',
              'amino_acid_probability')
@@ -245,7 +245,7 @@ class CryoEMPredictor:
                                 to the other GPUs, or ``model`` may be a {device: callable} mapping.
         ``overlap_window``      (keyword only) None: the reference's paste of the cube cores.  'uniform',
                                 'triangle' or W = grid_size + 2 * padding weights: overlap-weighted stitching
-                                (``ops.OverlapStitcher``; NOT the reference's arithmetic, DESIGN.md D2), the same bits
+                                (``ops.Stitcher``; NOT the reference's arithmetic, DESIGN.md D2), the same bits
                                 on one device and with ``devices=``.  'core' is the paste.
         ``tta``                 (keyword only) test-time augmentation: 'flips' (8 mirrorings), 'rot90' (the 24
                                 rotations), 'all' (48) or a list of orientation codes (``ops.orientation``).  The
@@ -554,33 +554,15 @@ class CryoEMPredictor:
             torch.cuda.current_stream(vols.device).synchronize()
         return out_host
 
-    def _overlap_weights(self):
-        """The window of an overlap-weighted map (checked before any launch), or None for the paste."""
-        if self.overlap_window is None:
-            return None
-        gs, pad = self._source['grid_size'], self._source['padding']
-        w1 = ops.overlap_window(self.overlap_window, gs, pad)
-        return None if ops.is_core_window(w1, gs, pad) else w1
-
-    def _tta_codes(self):
-        """The orientations of a test-time-augmented map, or None (orientation 0 alone is no augmentation)."""
-        codes = ops.tta_orientations(self.tta)
-        return None if codes in (None, (0,)) else codes
-
     def run_inference_and_reconstruct(self):
         """run_inference + reconstruct_volume (utils/predict.py:307-512) fused.  Returns
         (device volumes, {name: pinned host tensor})."""
-        codes = self._tta_codes()
+        w1, codes = self._stitch_mode
         if codes is not None and self._source['kind'] != 'resident':
             raise ops._lib.MicaError('tta cuts each cube in every orientation from the resident map: the per-cube '
                                      'grid files hold no volume to cut them from')
-        if codes is not None and self._workers:
-            gs, pad = self._source['grid_size'], self._source['padding']
-            return self._run_on_devices(self._workers, ops.overlap_window(
-                'core' if self.overlap_window is None else self.overlap_window, gs, pad), codes)
-        w1 = self._overlap_weights()
         if self._workers:
-            return self._run_on_devices(self._workers, w1)
+            return self._run_on_devices(self._workers, w1, codes)
         dev = torch.device(self.device)
         s = self._source
         gs, pad = s['grid_size'], s['padding']
@@ -594,10 +576,9 @@ class CryoEMPredictor:
                 pipe = self._pipeline(dev)
                 order = self._pipeline_order(pipe)
                 self._pipe = pipe
-                if w1 is not None or codes is not None:     # nothing is final before the last cube: no drain
+                if w1 is not None:                          # nothing is final before the last cube: no drain
                     vols = pipe.predict_and_stitch(model, None, model_batch=self._model_batch(), d8=d8, order=order,
-                                                   overlap_window=self.overlap_window if codes is not None else w1,
-                                                   tta=codes)
+                                                   overlap_window=w1, tta=codes)
                     return vols, self._download(vols)
                 pipe.cube_index()
                 vols = pipe._new_volumes()
@@ -613,34 +594,22 @@ class CryoEMPredictor:
             if dev.type != 'cuda':
                 raise ops._lib.MicaError('mica_b200 has no CPU path')
             ijk_dev = torch.from_numpy(np.ascontiguousarray(s['ijk'], dtype=np.int32)).to(dev)
-            if w1 is not None:
-                overlap = ops.OverlapStitcher(s['cube_shape'], dev, gs, pad, w1)
-                vols = overlap.vols
-            else:
-                overlap, vols = None, ops.StitchedVolumes(s['cube_shape'], dev)
-
-            def stitch(bb, ca, aa, ijk):
-                bb, ca, aa = _f32c(bb, ca, aa)
-                if overlap is not None:
-                    overlap.accumulate(bb, ca, aa, ijk)
-                else:
-                    ops.postproc_stitch(bb, ca, aa, ijk, vols, gs, pad)
+            st = ops.Stitcher(s['cube_shape'], dev, gs, pad, w1)
             step = max(self._model_batch(), 1) * 4
             for b0 in range(0, self.sample_count, step):
                 b1 = min(self.sample_count, b0 + step)
                 x, af, flags = self._fetch_files(b0, b1, dev)
-                run_model_chunks(model, x, af, flags.cpu().numpy(), ijk_dev[b0:b1], stitch, self._model_batch(), d8)
-            if overlap is not None:
-                overlap.finalize()
+                run_model_chunks(model, x, af, flags.cpu().numpy(), ijk_dev[b0:b1], st, self._model_batch(), d8)
+            vols = st.finalize()
             return vols, self._download(vols)
 
     def _run_on_devices(self, workers, w1=None, tta=None):
-        """The map's cubes dealt over ``workers`` (``deal_cubes``), one thread each.  Every worker stores its
-        cores into ONE 23-channel block on workers[0] (``postproc_stitch_peer`` with a one-entry owner table) --
-        or, with the window ``w1``, adds its weighted contributions into it (``ops.OverlapStitcher`` with that
-        table), which workers[0] finalises after the last worker has finished; the host copies run once, after
-        that.  ``tta``: the orientations of a test-time augmentation (with ``w1``; every worker runs its cubes in
-        all of them).  Returns what ``run_inference_and_reconstruct`` returns."""
+        """The map's cubes dealt over ``workers`` (``deal_cubes``), one thread each.  Every worker stitches into ONE
+        23-channel block on workers[0] through an ``ops.Stitcher`` of its device on a one-entry owner table: it stores
+        its cores there (the paste) or, with the window ``w1``, adds its weighted contributions, which workers[0]
+        finalises after the last worker has finished; the host copies run once, after that.  ``tta``: the
+        orientations of a test-time augmentation (with ``w1``; every worker runs its cubes in all of them).  Returns
+        what ``run_inference_and_reconstruct`` returns."""
         s = self._source
         gs, pad = s['grid_size'], s['padding']
         primary, n, mb = workers[0], len(s['ijk']), self._model_batch()
@@ -701,12 +670,9 @@ class CryoEMPredictor:
             zeroed.record()
         vols = ops.StitchedVolumes.from_block(block, cube_shape, (0, 0, 0), (X, Y, Z))
         tables = {d: torch.tensor([block.data_ptr()], dtype=torch.int64, device=d) for d in dict.fromkeys(workers)}
-        overlap = None
-        if w1 is not None:
-            overlap = {d: ops.OverlapStitcher(cube_shape, d, gs, pad, w1, vols=vols if d == primary else None,
-                                              owners=ops.OverlapOwners(tables[d], 0, (0, X), (primary.index,)),
-                                              tta=tta)
-                       for d in dict.fromkeys(workers)}
+        stitchers = {d: ops.Stitcher(cube_shape, d, gs, pad, w1, tta=tta, vols=vols if d == primary else None,
+                                     owners=ops.OverlapOwners(tables[d], 0, (0, X), (primary.index,)))
+                     for d in dict.fromkeys(workers)}
         for dev, st in zip(workers, streams):
             st.wait_stream(torch.cuda.current_stream(dev))     # inputs copied / binned on the current streams
             st.wait_event(zeroed)
@@ -718,23 +684,16 @@ class CryoEMPredictor:
             lo, hi = ranges[w]
             if hi <= lo:
                 return
-            dev, table, model = workers[w], tables[workers[w]], self._model_fn(self._models[workers[w]])
-
-            def stitch(bb, ca, aa, ijk, _vols=None, orient=0):
-                bb, ca, aa = _f32c(bb, ca, aa)
-                if overlap is not None:
-                    overlap[dev].accumulate(bb, ca, aa, ijk, orient=orient)
-                else:
-                    ops.postproc_stitch_peer(bb, ca, aa, ijk, cube_shape, table, (0, X), gs, pad)
+            dev, model = workers[w], self._model_fn(self._models[workers[w]])
             with torch.cuda.device(dev), torch.cuda.stream(streams[w]), torch.no_grad():
                 if resident:
-                    pipes[w].predict_and_stitch(model, vols, model_batch=mb, d8=d8, order=order[lo:hi],
-                                                batches=worker_batches(lo, hi, super_batch), stitch_fn=stitch,
-                                                tta=tta)
+                    pipes[w].predict_and_stitch(model, model_batch=mb, d8=d8, order=order[lo:hi],
+                                                batches=worker_batches(lo, hi, super_batch), stitcher=stitchers[dev])
                     return
                 for b0, b1 in worker_batches(lo, hi, super_batch):
                     x, af, flags = self._fetch_files(lo + b0, lo + b1, dev)
-                    run_model_chunks(model, x, af, flags.cpu().numpy(), ijk_dev[dev][lo + b0:lo + b1], stitch, mb, d8)
+                    run_model_chunks(model, x, af, flags.cpu().numpy(), ijk_dev[dev][lo + b0:lo + b1], stitchers[dev],
+                                     mb, d8)
 
         errors = [None] * len(workers)
 
@@ -760,8 +719,7 @@ class CryoEMPredictor:
         for e in errors:
             if e is not None:
                 raise e
-        if overlap is not None:
-            overlap[primary].finalize()
+        vols = stitchers[primary].finalize()
         return vols, self._download(vols)
 
     # ------------------------------------------------------------------ prediction maps
@@ -823,12 +781,13 @@ class CryoEMPredictor:
     def run_prediction(self):
         t_total = time.time()
         try:
-            self._tta_codes()                                    # a bad tta is refused before any launch
             self._cube_dtype = self._resolve_precision()         # so is a bad precision
             self._workers = self._resolve_workers()
             parse_save_maps(os.environ.get('MICA_SAVE_MAPS') if self.save_maps is None else self.save_maps)
             if not self.select_processing_strategy():
                 return False, {}
+            self._stitch_mode = ops.stitch_mode(self.overlap_window, self.tta, self._source['grid_size'],
+                                                self._source['padding'])      # a bad tta or window: before any launch
             self._maps_target = self._resolve_maps_target()      # refused before any launch
             if not self.load_model():
                 return False, {}

@@ -155,11 +155,11 @@ def exchange_source_halo(own: torch.Tensor, plan: SlabPlan, rank: int, group=Non
 
 class _SplitMap:
     """What the pipelines of one map split over ranks share: meeting the other ranks, the exported volume block
-    (peer.PeerVolumes) the other ranks store into, and the overlap-weighted stitch, whose contributions are added
-    into the block of the rank that owns their plane and finalised by ``finish_map``."""
+    (peer.PeerVolumes) the other ranks store into, and the weighted stitch, whose contributions are added into the
+    block of the rank that owns their plane and finalised by ``finish_map``."""
 
     peer_volumes = None
-    _overlap_pending = None
+    _pending = None
 
     def sync_ranks(self):
         torch.cuda.synchronize(self.device)
@@ -171,13 +171,10 @@ class _SplitMap:
         """All ranks' contributions have landed: after this every rank may read its own volume block (an
         overlap-weighted map is finalised here, each owner its own block)."""
         self.sync_ranks()
-        pending, self._overlap_pending = self._overlap_pending, None
+        pending, self._pending = self._pending, None
         if pending is not None:
-            overlap, on_batch, n = pending
             with torch.cuda.device(self.device):
-                vols = overlap.finalize()
-                if on_batch is not None:
-                    on_batch(vols, n)
+                MapPipeline._stitch_done(self, *pending)
 
     def _exported_volumes(self, n_max):
         """This rank's box as volumes in its exported block (zeroed): the block other ranks store into."""
@@ -201,45 +198,32 @@ class _SplitMap:
         """(cube axis, world + 1 plane bounds) of the output partition."""
         raise NotImplementedError
 
-    def _overlap_stitcher(self, w1, vols, tta=None):
-        if vols is None or getattr(vols, 'block', None) is None:
-            raise MicaError('a split map stitches overlap-weighted into its exported volumes (predict_and_stitch '
-                            'builds them when vols is None)')
+    def _make_stitcher(self, w1, codes, vols):
+        """A stitcher into the owners' exported blocks; ``vols`` (default: this rank's exported volumes, zeroed
+        before the ranks meet, so nobody stores into a block before its owner has cleared it) is this rank's box."""
+        if vols is None:
+            vols = self._exported_volumes(self._n_max())
+            self.sync_ranks()
         axis, bounds = self._owner_bounds()
         pv = self.peer_volumes
-        owners = ops.OverlapOwners(pv.table, axis, tuple(bounds), tuple(pv.devices))
-        return ops.OverlapStitcher(self.cube_shape, self.device, self.grid_size, self.padding, w1, vols=vols,
-                                   owners=owners, tta=tta)
+        return ops.Stitcher(self.cube_shape, self.device, self.grid_size, self.padding, w1, tta=codes, vols=vols,
+                            owners=ops.OverlapOwners(pv.table, axis, tuple(bounds), tuple(pv.devices)))
 
-    def _overlap_done(self, overlap, on_batch, n):
-        self._overlap_pending = (overlap, on_batch, n)        # finalised by finish_map, once every rank has added
-        return overlap.vols
-
-    def _weighted(self, kw):
-        """True when ``kw`` asks for an overlap-weighted stitch other than 'core' (which is the paste), or for a
-        test-time augmentation (other than orientation 0 alone), which always accumulates."""
-        if ops.tta_orientations(kw.get('tta')) not in (None, (0,)):
-            return True
-        kw.pop('tta', None)
-        w = kw.get('overlap_window')
-        if w is None or ops.is_core_window(ops.overlap_window(w, self.grid_size, self.padding), self.grid_size,
-                                           self.padding):
-            kw.pop('overlap_window', None)
-            return False
-        return True
-
-    def _predict_overlap(self, model_fn, vols, on_batch, kw):
-        """predict_and_stitch of an overlap-weighted map: owners zero their blocks, ranks meet, then accumulate."""
-        if vols is None:
-            self.cube_index()
-            vols = self._exported_volumes(self._n_max())
-            self.sync_ranks()                     # nobody adds into a block before its owner has cleared it
-        return MapPipeline.predict_and_stitch(self, model_fn, vols, on_batch, **kw)
+    def _stitch_done(self, st, on_batch, n):
+        if not st.per_batch:
+            self._pending = (st, on_batch, n)         # finalised by finish_map, once every rank has added
+        return st.vols
 
 
 class SlabPipeline(_SplitMap, MapPipeline):
     """One rank's share of a z-slab partitioned map.  ``run`` takes this rank's OWN block
-    of source planes (global planes [own_lo, own_hi) of ``global_src_shape``)."""
+    of source planes (global planes [own_lo, own_hi) of ``global_src_shape``).
+
+    ``predict_and_stitch`` runs this rank's cubes.  The paste stores their cores into this rank's box.  With
+    ``overlap_window`` (or ``tta``) the windows reach ``padding`` planes into the neighbouring slabs: those
+    contributions are added into the neighbours' exported blocks, and the volumes are final after ``finish_map()`` on
+    every rank.  ``min_max``: each rank measures its own cubes on its normalised block (halo included), so the
+    decisions are the one-GPU map's."""
 
     def __init__(self, device, rank, world, grid_size=48, padding=8, order=3, batch_cubes=16,
                  target_voxel_size=1.0, halo_k=16, global_src_shape=None, group=None, af3_mode='sparse',
@@ -496,14 +480,10 @@ class SlabPipeline(_SplitMap, MapPipeline):
         X, Y, _ = self.cube_shape
         return max(r.out_hi - r.out_lo for r in self.plan.ranks) * X * Y
 
-    def predict_and_stitch(self, model_fn, vols=None, on_batch=None, **kw):
-        """As ``MapPipeline.predict_and_stitch`` for this rank's cubes.  With ``overlap_window`` (or ``tta``) the
-        windows reach ``padding`` planes into the neighbouring slabs: those contributions are added into the
-        neighbours' exported blocks, and the volumes are final after ``finish_map()`` on every rank.  ``min_max``: each
-        rank measures its own cubes on its normalised block (halo included), so the decisions are the one-GPU map's."""
-        if self._weighted(kw):
-            return self._predict_overlap(model_fn, vols, on_batch, kw)
-        return super().predict_and_stitch(model_fn, vols, on_batch, **kw)
+    def _make_stitcher(self, w1, codes, vols):
+        if w1 is None:                            # the paste: this rank's cores, into its own box
+            return MapPipeline._make_stitcher(self, w1, codes, vols)
+        return super()._make_stitcher(w1, codes, vols)
 
 
 class BalancedCubePipeline(_SplitMap, MapPipeline):
@@ -516,7 +496,11 @@ class BalancedCubePipeline(_SplitMap, MapPipeline):
     rank that owns that x range: local memory or a peer's over NVLink (``ops.postproc_stitch_peer`` --
     softmax/argmax + stitch fused with its exchange, no NCCL call).  The output is thus partitioned
     along cube axis 0, ``x_bounds[r] .. x_bounds[r+1]`` on rank r; ``finish_map()`` (stream sync +
-    barrier) makes every rank's block final.  No reference counterpart (the reference is single-GPU)."""
+    barrier) makes every rank's block final.  No reference counterpart (the reference is single-GPU).
+
+    With ``overlap_window`` (or ``tta``) every window contribution is added into the block of the rank that owns its x
+    plane; the normaliser comes from the full cube lattice, also under ``cube_subset``.  ``min_max``: every rank
+    measures the whole map and deals the kept cubes as ``cube_subset`` (``cubes_per_rank``)."""
 
     def __init__(self, device, rank, world, grid_size=48, padding=8, order=3, batch_cubes=16,
                  target_voxel_size=1.0, group=None, af3_mode='sparse', cube_subset=None, _peer_volumes=None):
@@ -571,20 +555,3 @@ class BalancedCubePipeline(_SplitMap, MapPipeline):
 
     def _owner_bounds(self):
         return 0, self.x_bounds
-
-    def stitch_fn(self, bb, ca, aa, ijk, vols):
-        ops.postproc_stitch_peer(bb, ca, aa, ijk, self.cube_shape, self.peer_volumes.table, self.x_bounds,
-                                 self.grid_size, self.padding)
-
-    def predict_and_stitch(self, model_fn, vols=None, on_batch=None, **kw):
-        """With ``overlap_window`` (or ``tta``) every window contribution is added into the block of the rank that
-        owns its x plane; the normaliser comes from the full cube lattice, also under ``cube_subset``.  ``min_max``: every
-        rank measures the whole map and deals the kept cubes as ``cube_subset`` (``cubes_per_rank``)."""
-        if self._weighted(kw):
-            return self._predict_overlap(model_fn, vols, on_batch, kw)
-        if vols is None:
-            self.cube_index()
-            vols = self._new_volumes()
-            self.sync_ranks()                     # nobody stores into a block before its owner has cleared it
-        kw.setdefault('stitch_fn', self.stitch_fn)
-        return super().predict_and_stitch(model_fn, vols, on_batch, **kw)

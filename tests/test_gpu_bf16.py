@@ -198,7 +198,7 @@ def _np(vols):
 
 
 @pytest.mark.parametrize('gs,pad', [(32, 16), (48, 8)])
-def test_paste_with_bf16_logits_equals_float32(cuda, gs, pad):
+def test_stitcher_paste_with_bf16_logits_equals_float32(cuda, gs, pad):
     W = gs + 2 * pad
     cube_shape = (70, 50, 90)
     ijk = _dev(ops.cube_origins(cube_shape, gs), cuda)
@@ -210,9 +210,9 @@ def test_paste_with_bf16_logits_equals_float32(cuda, gs, pad):
     a, b = _np(v16), _np(v32)
     for k in MAP_TYPES:
         assert np.array_equal(a[k], b[k]), k
-    # StitchCall, switching dtype between calls
+    # a Stitcher, switching dtype between calls
     v = ops.StitchedVolumes(cube_shape, cuda)
-    call = ops.StitchCall(v, gs, pad)
+    call = ops.Stitcher(cube_shape, cuda, gs, pad, vols=v)
     h = B // 2
     call(bb[:h], ca[:h], aa[:h], ijk[:h])
     call(bb[h:].float(), ca[h:].float(), aa[h:].float(), ijk[h:])
@@ -237,7 +237,7 @@ def test_paste_with_bf16_logits_equals_float32(cuda, gs, pad):
 
 
 @pytest.mark.parametrize('window,tta', [('triangle', None), ('uniform', (0, 5, 30))])
-def test_overlap_accumulate_with_bf16_logits_equals_float32(cuda, window, tta):
+def test_stitcher_accumulate_with_bf16_logits_equals_float32(cuda, window, tta):
     gs, pad = 16, 8
     W = gs + 2 * pad
     cube_shape = (37, 21, 30)
@@ -246,10 +246,10 @@ def test_overlap_accumulate_with_bf16_logits_equals_float32(cuda, window, tta):
     logits = {g: _bf16_logits(len(ijk), W, cuda, seed=g + 1) for g in codes}
     res = {}
     for dt in ('bf16', 'f32'):
-        st = ops.OverlapStitcher(cube_shape, cuda, gs, pad, window, tta=tta)
+        st = ops.Stitcher(cube_shape, cuda, gs, pad, window, tta=tta)
         for g in codes:
             lg = logits[g] if dt == 'bf16' else [t.float() for t in logits[g]]
-            st.accumulate(*lg, ijk, orient=g)
+            st(*lg, ijk, orient=g)
         res[dt] = _np(st.finalize())
     for k in MAP_TYPES:
         assert np.array_equal(res['bf16'][k], res['f32'][k]), k
@@ -263,10 +263,10 @@ def test_overlap_accumulate_with_bf16_logits_equals_float32(cuda, window, tta):
             blocks[dt] = [torch.zeros(23 * m, dtype=torch.float32, device=cuda) for m in n]
             table = torch.tensor([t.data_ptr() for t in blocks[dt]], dtype=torch.int64, device=cuda)
             owners = ops.OverlapOwners(table, axis, bounds, (cuda.index if cuda.index is not None else 0,) * world)
-            st = ops.OverlapStitcher(cube_shape, cuda, gs, pad, window, owners=owners, tta=tta)
+            st = ops.Stitcher(cube_shape, cuda, gs, pad, window, owners=owners, tta=tta)
             for g in codes:
                 lg = logits[g] if dt == 'bf16' else [t.float() for t in logits[g]]
-                st.accumulate(*lg, ijk, orient=g)
+                st(*lg, ijk, orient=g)
         for r in range(world):
             assert torch.equal(blocks['bf16'][r].view(torch.int32), blocks['f32'][r].view(torch.int32)), (axis, r)
 

@@ -1,4 +1,4 @@
-"""Overlap-weighted stitching (``ops.OverlapStitcher``, NOT the reference's arithmetic; DESIGN.md D2) is order free:
+"""Overlap-weighted stitching (``ops.Stitcher``, NOT the reference's arithmetic; DESIGN.md D2) is order free:
 the same bits whatever the batch, the cube order or the partition -- z-slabs, balanced cubes, several workers of
 the drop-in -- and within TOL of the float64 NumPy statement.  The stand-in model gives every position of a window
 its own logits, so a voxel covered by several windows really averages different values."""
@@ -49,17 +49,17 @@ def _lattice_logits(cube_shape, gs, pad, cuda, seed=3):
 
 
 def _stitch(cube_shape, gs, pad, window, cuda, logits, ijk, order, batch):
-    st = ops.OverlapStitcher(cube_shape, cuda, gs, pad, window)
+    st = ops.Stitcher(cube_shape, cuda, gs, pad, window)
     d = [_dev(a[order], cuda) for a in logits]
     ij = _dev(ijk[order].astype(np.int32), cuda)
     for b0 in range(0, len(order), batch):
-        st.accumulate(d[0][b0:b0 + batch], d[1][b0:b0 + batch], d[2][b0:b0 + batch], ij[b0:b0 + batch])
+        st(d[0][b0:b0 + batch], d[1][b0:b0 + batch], d[2][b0:b0 + batch], ij[b0:b0 + batch])
     return st.finalize().as_dict()
 
 
 @pytest.mark.parametrize('cube_shape,gs,pad', [((70, 33, 50), 32, 16), ((21, 13, 9), 8, 2)])
 @pytest.mark.parametrize('window', ['uniform', 'triangle'])
-def test_result_does_not_depend_on_batches_or_cube_order(cuda, cube_shape, gs, pad, window):
+def test_stitcher_result_does_not_depend_on_batches_or_cube_order(cuda, cube_shape, gs, pad, window):
     ijk, logits = _lattice_logits(cube_shape, gs, pad, cuda)
     n = len(ijk)
     ref = _stitch(cube_shape, gs, pad, window, cuda, logits, ijk, np.arange(n), n)
@@ -71,7 +71,7 @@ def test_result_does_not_depend_on_batches_or_cube_order(cuda, cube_shape, gs, p
 
 
 @pytest.mark.parametrize('cube_shape,gs,pad', [((70, 33, 50), 32, 16), ((53, 21, 13), 48, 8), ((21, 13, 9), 8, 2)])
-def test_windows_against_the_float64_statement(cuda, cube_shape, gs, pad):
+def test_stitcher_windows_against_the_float64_statement(cuda, cube_shape, gs, pad):
     ijk, (bb, ca, aa) = _lattice_logits(cube_shape, gs, pad, cuda, seed=11)
     meta = np.concatenate([ijk, np.minimum(gs, np.array(cube_shape)[None] - ijk)], axis=1).astype(np.int64)
     custom = (0.05 + np.random.default_rng(gs).random(gs + 2 * pad)).astype(np.float32)
@@ -245,7 +245,7 @@ def test_dropin_workers_and_sources_equal_one_device(cuda, tmp_path, _clean_sess
     assert np.abs(np.asarray(f1['amino_acid_probability']).sum(0) - 1).max() <= 1e-5
 
 
-def test_refusals(cuda, tmp_path, monkeypatch, _clean_session):
+def test_stitcher_and_split_refusals(cuda, tmp_path, monkeypatch, _clean_session):
     gs, pad = 32, 16
     W = gs + 2 * pad
     bad_windows = [np.full(W, -1.0), np.r_[np.ones(W - 1), np.nan], np.ones(W + 1)]
@@ -256,7 +256,7 @@ def test_refusals(cuda, tmp_path, monkeypatch, _clean_session):
     torch.cuda.synchronize()
     for w in bad_windows:
         with pytest.raises(_lib.MicaError):
-            ops.OverlapStitcher((36, 44, 40), cuda, gs, pad, w)
+            ops.Stitcher((36, 44, 40), cuda, gs, pad, w)
         n0 = ops.launch_count()
         with pytest.raises(_lib.MicaError):
             pipe.predict_and_stitch(WindowModel(W).to(cuda), overlap_window=w)

@@ -530,7 +530,7 @@ def test_postproc_stitch_vs_oracle(cuda, cube_shape, gs, pad):
 
 
 @pytest.mark.parametrize('cube_shape,gs,pad', [((70, 33, 50), 32, 16), ((52, 20, 12), 48, 8)])
-def test_overlap_weighted_stitch_modes(cuda, cube_shape, gs, pad):
+def test_stitcher_window_modes(cuda, cube_shape, gs, pad):
     """The north_star's overlap-weighted stitching (NOT the reference's arithmetic; DESIGN.md D2): with the
     core-indicator window it must reproduce the reference-mode kernel bit for bit, with the uniform and the
     triangle window it must equal the NumPy statement sum(w p) / sum(w) -- float32 atomics in arbitrary
@@ -540,9 +540,9 @@ def test_overlap_weighted_stitch_modes(cuda, cube_shape, gs, pad):
     ijk = dev(np.ascontiguousarray(meta[:, :3], dtype=np.int32), cuda)
     half = len(meta) // 2                                   # two accumulate calls: batches add up
     for window in ('core', 'uniform', 'triangle'):
-        st = ops.OverlapStitcher(cube_shape, cuda, gs, pad, window)
-        st.accumulate(d[0][:half], d[1][:half], d[2][:half], ijk[:half])
-        st.accumulate(d[0][half:], d[1][half:], d[2][half:], ijk[half:])
+        st = ops.Stitcher(cube_shape, cuda, gs, pad, window)
+        st(d[0][:half], d[1][:half], d[2][:half], ijk[:half])
+        st(d[0][half:], d[1][half:], d[2][half:], ijk[half:])
         got = {k: v.cpu().numpy() for k, v in st.finalize().as_dict().items()}
         if window == 'core':
             for k in ('backbone_probability', 'carbon_alpha_probability', 'amino_acid_probability'):
@@ -560,11 +560,11 @@ def test_overlap_weighted_stitch_modes(cuda, cube_shape, gs, pad):
         # every voxel of the map is covered by at least one window: probabilities of the 20 classes sum to 1
         assert np.abs(got['amino_acid_probability'].sum(0) - 1).max() <= 1e-5
     with pytest.raises(_lib.MicaError):
-        ops.OverlapStitcher(cube_shape, cuda, gs, pad, 'hamming')
+        ops.Stitcher(cube_shape, cuda, gs, pad, 'hamming')
 
 
 def test_pipeline_overlap_window_option(cuda):
-    """MapPipeline.predict_and_stitch(overlap_window=...) routes the batches through the OverlapStitcher; 'core'
+    """MapPipeline.predict_and_stitch(overlap_window=...) routes the batches through the weighted ops.Stitcher; 'core'
     equals the default mode."""
     src = synthetic.synthetic_map((40, 44, 36), voxel=1.0, seed=9)
     hdr = MapHeader(voxel_size=(np.float32(1.0),) * 3)

@@ -107,7 +107,7 @@ def test_oriented_af3_fill_and_slot_reuse(cuda):
 
 # ------------------------------------------------------------------------------------------------ accumulate
 @pytest.mark.parametrize('gs,pad,window', [(16, 8, 'triangle'), (8, 2, 'uniform'), (16, 8, 'core')])
-def test_accumulate_against_the_float64_statement(cuda, gs, pad, window):
+def test_stitcher_tta_against_the_float64_statement(cuda, gs, pad, window):
     W = gs + 2 * pad
     cube_shape = (37, 21, 30)
     ijk = ops.cube_origins(cube_shape, gs)
@@ -119,12 +119,12 @@ def test_accumulate_against_the_float64_statement(cuda, gs, pad, window):
         y = (x[0][None] * A + P).astype(np.float32).astype(np.float64)
         return y[:4], y[4:8], y[8:]
     codes = (0, 1, 5, 10, 19, 30, 47)                                    # fastest axis kept, reversed, and moved
-    st = ops.OverlapStitcher(cube_shape, cuda, gs, pad, window, tta=codes)
+    st = ops.Stitcher(cube_shape, cuda, gs, pad, window, tta=codes)
     ij = _dev(ijk.astype(np.int32), cuda)
     for g in codes:
         logits = np.stack([np.concatenate(model(ops.orient_array(w, g).astype(np.float64))) for w in windows])
         t = _dev(logits.astype(np.float32), cuda)
-        st.accumulate(t[:, :4].contiguous(), t[:, 4:8].contiguous(), t[:, 8:].contiguous(), ij, orient=g)
+        st(t[:, :4].contiguous(), t[:, 4:8].contiguous(), t[:, 8:].contiguous(), ij, orient=g)
     got = {k: v.cpu().numpy() for k, v in st.finalize().as_dict().items()}
     want = tto.tta_stitch(windows.astype(np.float64), ijk, cube_shape, gs, pad, ops.overlap_window(window, gs, pad),
                           codes, model)
@@ -294,7 +294,7 @@ def test_dropin_workers_equal_one_device(cuda, tmp_path, _clean_session):
     assert pr.run_prediction() == (False, {})
 
 
-def test_refusals_launch_nothing(cuda, tmp_path, _clean_session):
+def test_tta_refusals_launch_nothing(cuda, tmp_path, _clean_session):
     pipe = _pipe(cuda)
     pipe.cube_index()
     model = WindowModel(32).to(cuda)
@@ -304,7 +304,7 @@ def test_refusals_launch_nothing(cuda, tmp_path, _clean_session):
         with pytest.raises(_lib.MicaError):
             pipe.predict_and_stitch(model, tta=bad)
         with pytest.raises(_lib.MicaError):
-            ops.OverlapStitcher(pipe.cube_shape, cuda, 16, 8, 'core', tta=bad)
+            ops.Stitcher(pipe.cube_shape, cuda, 16, 8, 'core', tta=bad)
         assert ops.launch_count() == n0
     x = torch.zeros((4, 4, 4), device=cuda)
     ijk = torch.zeros((1, 3), dtype=torch.int32, device=cuda)
@@ -312,11 +312,11 @@ def test_refusals_launch_nothing(cuda, tmp_path, _clean_session):
     for g in (48, -1, True):
         with pytest.raises(_lib.MicaError):
             ops.extract_cubes(x, ijk, 2, 1, orient=g)
-    st = ops.OverlapStitcher(pipe.cube_shape, cuda, 16, 8, 'core', tta='flips')
+    st = ops.Stitcher(pipe.cube_shape, cuda, 16, 8, 'core', tta='flips')
     n1 = ops.launch_count()
     t = torch.zeros((1, 4, 32, 32, 32), device=cuda)
     with pytest.raises(_lib.MicaError):
-        st.accumulate(t, t, torch.zeros((1, 21, 32, 32, 32), device=cuda), ijk, orient=9)   # not one of 'flips'
+        st(t, t, torch.zeros((1, 21, 32, 32, 32), device=cuda), ijk, orient=9)              # not one of 'flips'
     assert ops.launch_count() == n1
     grids, _ = _drop_in(tmp_path)
     n0 = ops.launch_count()

@@ -115,6 +115,32 @@ def test_bad_windows_are_refused_on_the_host():
     assert not ops.is_core_window(ops.overlap_window('uniform', 32, 16), 32, 16)
 
 
+def test_stitch_mode_table_and_refusals():
+    """window x tta -> (paste or weighted, orientations): 'core' without augmentation is the paste, tta (0,) is none,
+    and under augmentation the window defaults to 'core' and is weighted.  Bad values raise before any launch."""
+    gs, pad = 32, 16
+    core, uniform = ops.overlap_window('core', gs, pad), ops.overlap_window('uniform', gs, pad)
+    custom = np.linspace(0.5, 1.0, gs + 2 * pad).astype(np.float32)
+    flips = tuple(range(8))
+    table = [((None, None), None, None), (('core', None), None, None), ((core.astype(np.float64), None), None, None),
+             ((None, (0,)), None, None), (('core', [0]), None, None), (('uniform', None), uniform, None),
+             (('uniform', (0,)), uniform, None), ((custom, None), custom, None), ((None, 'flips'), core, flips),
+             (('core', 'flips'), core, flips), (('uniform', (5, 0)), uniform, (5, 0)), ((None, (3,)), core, (3,))]
+    for (window, tta), want_w, want_codes in table:
+        w1, codes = ops.stitch_mode(window, tta, gs, pad)
+        if want_w is None:
+            assert w1 is None, (window, tta)
+        else:
+            assert w1.dtype == np.float32 and np.array_equal(w1, want_w), (window, tta)
+        assert codes == want_codes, (window, tta)
+    n0 = ops.launch_count()
+    for window, tta in (('hamming', None), (np.ones(5), None), (None, 'mirror'), (None, []), (None, [0, 0]),
+                        ('core', [48]), ('hamming', 'flips'), ('uniform', 'ALL')):
+        with pytest.raises(_lib.MicaError):
+            ops.stitch_mode(window, tta, gs, pad)
+    assert ops.launch_count() == n0
+
+
 def test_accumulate_entry_points_reject_bad_arguments_before_touching_the_device():
     import ctypes as C
     lib = _lib.lib

@@ -9,7 +9,7 @@ float32 against bfloat16 model-facing buffers on one GPU (``cube_dtype`` / ``Cry
       extract_map   ops.extract_cubes of the normalised map into [512, 1, 64^3];
       af3_fill      Af3CubeFiller.fill, alternating two batches (every call clears one cube set and sets another);
       paste         ops.postproc_stitch of 512 cubes of logits (the cores);
-      accumulate    OverlapStitcher.accumulate, 'triangle' window (every window voxel).
+      accumulate    the weighted ops.Stitcher, 'triangle' window (every window voxel).
     Algorithmic bytes from the shapes: extract = float32 window read + window written in the dtype; paste = 26 logit
     channels read per core voxel + 23 float32 written; accumulate = 26 logit channels read + 22 uint32 sums added per
     window voxel; the fill moves a few bytes per atom voxel and is reported as time only.  Every working set is larger
@@ -92,7 +92,7 @@ def kernels(dev, reps, warmup):
     logits32 = [torch.randn((B, c, W, W, W), device=dev, generator=g) for c in (4, 4, 21)]
     logits = {'fp32': logits32, 'bf16': [t.to(torch.bfloat16) for t in logits32]}
     vols = ops.StitchedVolumes(pipe.cube_shape, dev)
-    acc = ops.OverlapStitcher(pipe.cube_shape, dev, GS, PAD, 'triangle')
+    acc = ops.Stitcher(pipe.cube_shape, dev, GS, PAD, 'triangle')
     turn = {k: 0 for k in DTYPES}
 
     def fill(k):
@@ -103,7 +103,7 @@ def kernels(dev, reps, warmup):
         fns['extract_map', k] = (lambda k=k: ops.extract_cubes(pipe.normalized, ijk, GS, PAD, pipe.perm, out=xs[k]))
         fns['af3_fill', k] = (lambda k=k: fill(k))
         fns['paste', k] = (lambda k=k: ops.postproc_stitch(*logits[k], ijk, vols, GS, PAD))
-        fns['accumulate', k] = (lambda k=k: acc.accumulate(*logits[k], ijk))
+        fns['accumulate', k] = (lambda k=k: acc(*logits[k], ijk))
     ms = _alternate(fns, reps, warmup)
     for (name, k), t in ms.items():
         e = 4 if k == 'fp32' else 2

@@ -7,7 +7,7 @@ launch, median over R repetitions after W warm-ups, for orientation 0, 4 (the fa
 (2, 1, 0): the fastest axis moved):
   extract_map   ops.extract_cubes of the normalised map into [512, 1, 64^3];
   af3_fill      Af3CubeFiller.fill, alternating two batches so that every call clears one cube set and sets another;
-  accumulate    OverlapStitcher.accumulate ('triangle' window, every window voxel contributes), 512 cubes of logits.
+  accumulate    ops.Stitcher ('triangle' window, every window voxel contributes), 512 cubes of logits.
 Algorithmic bytes: extract = window bytes read + written; accumulate = 26 logit channels read + 22 uint32 sums
 added per window voxel; the fill moves a few bytes per atom voxel and is reported as time only.  ``copy_peak``: a
 2 GiB device-to-device copy in the same run (read + write bytes / time), the reference for ``frac_copy``.
@@ -99,7 +99,7 @@ def main():
     bb = torch.randn((B, 4, W, W, W), device=dev)
     ca = torch.randn((B, 4, W, W, W), device=dev)
     aa = torch.randn((B, 21, W, W, W), device=dev)
-    acc = ops.OverlapStitcher(pipe.cube_shape, dev, GS, PAD, 'triangle', tta='all')
+    acc = ops.Stitcher(pipe.cube_shape, dev, GS, PAD, 'triangle', tta='all')
     acc_bytes = B * W ** 3 * (26 + 22) * 4
     for g in CODES:
         ms = _time(lambda: ops.extract_cubes(pipe.normalized, ijk, GS, PAD, pipe.perm, out=x, orient=g),
@@ -112,7 +112,7 @@ def main():
             turn[0] ^= 1
             filler.fill(ijk if turn[0] else ijk2, orient=g)
         c['af3_fill_ms'] = round(_time(fill, args.reps, args.warmup), 4)
-        ms = _time(lambda: acc.accumulate(bb, ca, aa, ijk, orient=g), args.reps, args.warmup)
+        ms = _time(lambda: acc(bb, ca, aa, ijk, orient=g), args.reps, args.warmup)
         c.update({'accumulate_ms': round(ms, 4), 'accumulate_GBps': round(acc_bytes / (ms * 1e-3) / 1e9, 1),
                   'accumulate_frac_copy': round(acc_bytes / (ms * 1e-3) / peak, 3)})
         cases[str(g)] = c
